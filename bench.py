@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the PlanGen CFG image-token decode path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one batch through the hot path: prompt embed + prefill + 576 x (gen_head, CFG, Philox
@@ -18,7 +18,7 @@ cond/uncond pair, synthetic LayoutSAM-shaped prompts with 4-8 boxes).  Prints ON
 
 `--impl reference` times the reference's own CPU implementation of the path: the oracle restatement
 of System.t2i / sample_image (oracle/janus_oracle.py; the reference itself cannot be imported here,
-see DESIGN.md) on all host threads: ONE full 576-token image, wall clock, nothing extrapolated.
+see DESIGN.md) on all host threads: one full 576-token image per step, wall clock, nothing extrapolated.
 """
 from __future__ import annotations
 
@@ -49,7 +49,16 @@ def parse():
     ap.add_argument("--no-roofline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the bounded configs[2]/[3]/[4] measurements after the timed region")
     ap.add_argument("--option", action="append", default=[], help="engine option key=value")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (uint8 images, image tokens) and "
+                         "which batch rows they are as DIR/<name>.npy in float32, at most 64 MB in all, so that two builds "
+                         "can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
 
 
 # ----------------------------------------------------------------------------- clocks sampler
@@ -144,10 +153,13 @@ def cpu_reference_sample(model_name: str, threads: int, prompt_len: int = 256, r
             "sample_wall_s": loop_s + vq_s}
 
 
-def cpu_reference_full_image(model_name: str, threads: int, prompt_len: int = 256, sd=None):
-    """ONE full image through the oracle port of System.t2i on host cores, nothing extrapolated: embed + prefill +
-    575 decode steps (each LlamaModel.forward timed) + gen_head / CFG / sampling / embed per token + VQ decode_code.
-    BASELINE configs[0]: B=1 (R=2 rows with the CFG pair), P=256, fp32."""
+def cpu_reference_full_image(model_name: str, threads: int, prompt_len: int = 256, sd=None, images: int = 1,
+                             warmup: int = 1):
+    """`images` full images, one after the other, through the oracle port of System.t2i on host cores, nothing
+    extrapolated: each is embed + prefill + 575 decode steps (each LlamaModel.forward timed) + gen_head / CFG /
+    sampling / embed per token + VQ decode_code.  `warmup` untimed short passes (prefill + 2 tokens) page the weights
+    in first.  BASELINE configs[0]: B=1 (R=2 rows with the CFG pair), P=256, fp32.  wall_s and loop_s cover all the
+    images; prefill_s and vq_s are per image (median, mean)."""
     import torch
     from oracle import janus_oracle as O
     torch.set_num_threads(threads)
@@ -164,21 +176,31 @@ def cpu_reference_full_image(model_name: str, threads: int, prompt_len: int = 25
         times.append(time.perf_counter() - t0)
         return out
 
-    g = torch.Generator().manual_seed(0)
-    with torch.inference_mode():                                        # warm: page the weights in, untimed
-        O.sample_image(sd, d, O.embed_tokens(sd, ids), 1, 3, mask, 5.0, 1.0, O.make_torch_sampler(g), mode="fp32")
-    times.clear()
-    g = torch.Generator().manual_seed(0)
+    for _ in range(warmup):
+        g = torch.Generator().manual_seed(0)
+        with torch.inference_mode():
+            O.sample_image(sd, d, O.embed_tokens(sd, ids), 1, 3, mask, 5.0, 1.0, O.make_torch_sampler(g), mode="fp32")
+    prefill, dec, loop_s, vq_s = [], [], 0.0, 0.0
     t0 = time.perf_counter()
-    with torch.inference_mode():
-        emb = O.embed_tokens(sd, ids)
-        toks = O.sample_image(sd, d, emb, 1, d.n_img_tokens, mask, 5.0, 1.0, O.make_torch_sampler(g), mode="fp32",
-                              lm_forward=timed_forward)
-        t1 = time.perf_counter()
-        O.decode_code(sd, d, toks.to(torch.int32), [1, d.code_dim, d.grid, d.grid])
-    t2 = time.perf_counter()
-    dec = sorted(times[1:])
-    return {"wall_s": t2 - t0, "loop_s": t1 - t0, "vq_s": t2 - t1, "prefill_s": times[0],
+    for _ in range(images):
+        times.clear()
+        g = torch.Generator().manual_seed(0)
+        ta = time.perf_counter()
+        with torch.inference_mode():
+            emb = O.embed_tokens(sd, ids)
+            toks = O.sample_image(sd, d, emb, 1, d.n_img_tokens, mask, 5.0, 1.0, O.make_torch_sampler(g), mode="fp32",
+                                  lm_forward=timed_forward)
+            tb = time.perf_counter()
+            O.decode_code(sd, d, toks.to(torch.int32), [1, d.code_dim, d.grid, d.grid])
+        tc = time.perf_counter()
+        loop_s, vq_s = loop_s + tb - ta, vq_s + tc - tb
+        prefill.append(times[0])
+        dec += times[1:]
+    wall_s = time.perf_counter() - t0
+    prefill.sort()
+    dec.sort()
+    return {"wall_s": wall_s, "images": images, "loop_s": loop_s, "vq_s": vq_s / images,
+            "prefill_s": prefill[len(prefill) // 2],
             "ms_per_decode_step_median": 1e3 * dec[len(dec) // 2], "ms_per_decode_step_p90": 1e3 * dec[int(0.9 * len(dec))],
             "decode_steps_timed": len(dec), "rows": 2, "prompt_len": prompt_len}
 
@@ -218,10 +240,9 @@ def cpu_b16_estimate(model_name: str, threads: int, sd, vq_s_per_image: float):
 
 def run_reference_arm(args):
     """Reference arm: the reference's CPU PyTorch path (oracle port; the reference itself cannot be imported, DESIGN.md)
-    on all host threads.  The timed region is exactly ONE full 576-token image of BASELINE configs[0] (B=1, R=2, P=256,
-    fp32): embed + prefill + 575 decode steps + VQ decode, wall clock, nothing extrapolated.  That costs ~25-30 s, so
-    whatever --steps K asks for, K 'steps' are K equal slices of that one image: ms_per_step x K = the wall time that was
-    actually measured.  --warmup: one short untimed pass (prefill + 2 tokens) pages the weights in."""
+    on all host threads.  One step is one full 576-token image of BASELINE configs[0] (B=1, R=2, P=256, fp32): embed +
+    prefill + 575 decode steps + VQ decode, wall clock, nothing extrapolated; the timed region is --steps K such images
+    (~25-30 s each).  --warmup W: W short untimed passes (prefill + 2 tokens) page the weights in."""
     import torch
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -230,25 +251,24 @@ def run_reference_arm(args):
     from oracle import janus_oracle as O
     d = O.PRESETS[args.model]
     sd = O.init_state_dict(d, seed=0, with_vq=True)
-    r = cpu_reference_full_image(args.model, threads, prompt_len=256, sd=sd)
-    ips = 1.0 / r["wall_s"]
+    r = cpu_reference_full_image(args.model, threads, prompt_len=256, sd=sd, images=args.steps, warmup=args.warmup)
+    ips = args.steps / r["wall_s"]
     b16 = cpu_b16_estimate(args.model, threads, sd, r["vq_s"])
     line = {
         "metric": METRIC, "value": ips, "unit": UNIT, "impl": "reference", "n_gpus": args.gpus, "steps": args.steps,
-        "warmup": args.warmup, "ms_per_step": 1e3 * r["wall_s"] / max(args.steps, 1), "higher_is_better": True, "scaling": "weak",
+        "warmup": args.warmup, "ms_per_step": 1e3 * r["wall_s"] / args.steps, "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": "configs[0] layout2image (task_type=uni), Janus-1.3B-arch random init, B=1 (R=2 rows with the CFG "
                                "pair), P=256, 576 VQ tokens, CFG 5, fp32 on CPU; reference arm = oracle port of System.t2i / "
-                               "sample_image (the reference cannot be imported here); timed region = ONE full image (embed + "
-                               "prefill + 575 decode steps + VQ decode), wall clock, no extrapolation; the K 'steps' are K equal "
-                               "slices of that one image",
+                               "sample_image (the reference cannot be imported here); timed region = --steps full images, one "
+                               "per step (embed + prefill + 575 decode steps + VQ decode), wall clock, no extrapolation",
                    "same_config_as_b200_arm": False,
                    "note": "the B200 arm runs configs[1] (B=16 per GPU, bf16); cpu_baseline_b16 below estimates this CPU path at B=16"},
-        "timed": {"images": 1, "wall_s": r["wall_s"], "prefill_s": r["prefill_s"], "decode_steps": r["decode_steps_timed"],
+        "timed": {"images": r["images"], "wall_s": r["wall_s"], "prefill_s": r["prefill_s"], "decode_steps": r["decode_steps_timed"],
                   "ms_per_decode_step_median": r["ms_per_decode_step_median"], "ms_per_decode_step_p90": r["ms_per_decode_step_p90"],
-                  "vq_decode_s": r["vq_s"]},
+                  "vq_decode_s_per_image": r["vq_s"]},
         "cpu_baseline": {"value": ips, "unit": UNIT, "cores": threads, "kind": "port",
-                         "sample": "one full image: R=2 rows, P=256: prefill + 575 decode steps + VQ decode (nothing extrapolated)",
+                         "sample": "--steps full images: R=2 rows, P=256: prefill + 575 decode steps + VQ decode (nothing extrapolated)",
                          "ms_per_decode_step": r["ms_per_decode_step_median"], "ms_per_decode_step_p90": r["ms_per_decode_step_p90"],
                          "prefill_s": r["prefill_s"], "vq_decode_s_per_image": r["vq_s"], "torch": torch.__version__},
         "cpu_baseline_b16": b16,
@@ -322,6 +342,26 @@ def _ncu_traffic_bytes():
     except OSError:
         return None
     return int(total) if seen == 2 else None
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path: str, images, tokens):
+    """Write one step's (B, 3, H, W) uint8 images and (B, n) image tokens, and the batch rows they are, as float32 .npy
+    files.  When the batch does not fit DUMP_BYTES, the rows are a fixed seeded sample of whole images."""
+    import numpy as np
+    import torch
+    n = images.shape[0]
+    per_row = 4 * (images[0].numel() + tokens[0].numel() + 1)
+    keep = min(n, DUMP_BYTES // per_row)
+    rows = torch.arange(n)
+    if keep < n:
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    out = {"images": images[rows.to(images.device)], "tokens": tokens[rows.to(tokens.device)], "rows": rows}
+    os.makedirs(path, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy().astype(np.float32))
 
 
 def _timed(st, fn):
@@ -527,12 +567,16 @@ def run_b200_arm(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     e0.record(st)
-    run_resident(range(args.warmup, total))
+    images_out = run_resident(range(args.warmup, total))
     e1.record(st)
     barrier()
     elapsed = dp.max_over_ranks(e0.elapsed_time(e1) / 1e3, dev)
     launches = eng.counter("launches")
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # the gathered images are rank-major: rank 0's last batch sits at the end of its own steps
+        dump_outputs(args.dump_outputs, images_out[(args.steps - 1) * B:args.steps * B], eng.last_tokens)
+    del images_out
 
     # decode-step time alone (graph replays), for the roofline of the step
     P = dev_batches[args.warmup][0].shape[1]

@@ -57,7 +57,15 @@ def versions():
     return np.array([torch.__version__, transformers.__version__])
 
 
-def golden_lm(name: str, d: O.JanusDims, batch: int, steps: int, lo: int, hi: int, neg_len: int):
+def logit_columns(vocab: int, keep: int) -> np.ndarray:
+    """The image-vocab columns whose CFG logits a golden stores: all of them, or a fixed seeded sorted sample of `keep`
+    (a golden file stays under 1 MB; random fp32 logits do not compress)."""
+    if keep >= vocab:
+        return np.arange(vocab, dtype=np.int64)
+    return np.sort(np.random.default_rng(0).choice(vocab, keep, replace=False)).astype(np.int64)
+
+
+def golden_lm(name: str, d: O.JanusDims, batch: int, steps: int, lo: int, hi: int, neg_len: int, logit_cols: int):
     sd = O.init_state_dict(d, seed=0, with_vq=False)
     hf = hf_llama(d, sd)
     cond, neg = O.synthetic_prompts(d, batch, seed=1234, lo=lo, hi=hi, neg_len=neg_len)
@@ -68,10 +76,11 @@ def golden_lm(name: str, d: O.JanusDims, batch: int, steps: int, lo: int, hi: in
         toks = O.sample_image(sd, d, emb, batch, steps, mask, 5.0, 1.0, PhiloxSampler(0, 148),
                               mode="fp32", trace=trace,
                               lm_forward=lambda **kw: hf(**kw))
+    cols = logit_columns(d.img_vocab, logit_cols)
     np.savez_compressed(
         os.path.join(OUT, name), dims=np.array(d.name), ids=ids.numpy(), mask=mask.numpy(),
-        hidden=torch.stack(trace["hidden"]).numpy(), logits=torch.stack(trace["logits"]).numpy(),
-        tokens=toks.numpy(), cfg_weight=5.0, temperature=1.0, seed=0, num_sms=148,
+        hidden=torch.stack(trace["hidden"]).numpy(), logits=torch.stack(trace["logits"]).numpy()[..., cols],
+        logit_cols=cols, tokens=toks.numpy(), cfg_weight=5.0, temperature=1.0, seed=0, num_sms=148,
         versions=versions())
     print(name, "tokens", toks.tolist())
 
@@ -232,8 +241,8 @@ def main():
         golden_x2t("x2t_small_fp32.npz", O.SMALL, batch=4, max_new=20, lo=9, hi=40, eos_from=(1, 5))
         golden_x2t("x2t_tiny_stop_fp32.npz", O.TINY, batch=1, max_new=24, lo=11, hi=11, eos_from=(0, 6))   # all rows finish early
         return
-    golden_lm("lm_tiny_fp32.npz", O.TINY, batch=2, steps=8, lo=5, hi=12, neg_len=7)
-    golden_lm("lm_small_fp32.npz", O.SMALL, batch=3, steps=6, lo=9, hi=40, neg_len=13)
+    golden_lm("lm_tiny_fp32.npz", O.TINY, batch=2, steps=8, lo=5, hi=12, neg_len=7, logit_cols=O.TINY.img_vocab)
+    golden_lm("lm_small_fp32.npz", O.SMALL, batch=3, steps=6, lo=9, hi=40, neg_len=13, logit_cols=8192)
     golden_vq_tiny("vq_tiny.npz", O.TINY, batch=2)
     golden_vq_tiny("vq_small.npz", O.SMALL, batch=1)
     golden_vq_ref_class("vq16_grid4.npz")

@@ -162,6 +162,8 @@ class _CharTok:
 
 
 def test_sft_prompt_matches_reference_conversation_template():
+    """`want` holds the prompts the reference's own `get_conv_template("deepseek")` (Janus conversation.py) builds for
+    these conversations with an empty system message (its stripped `get_prompt()`)."""
     from plangen_b200 import prompts as PR
     convs = [
         [{"role": PR.USER, "content": "a yellow car in front of the tree"}, {"role": PR.ASSISTANT, "content": ""}],
@@ -175,18 +177,6 @@ def test_sft_prompt_matches_reference_conversation_template():
     ]
     assert [PR.sft_prompt(c) for c in convs] == want
     assert PR.sft_prompt(convs[0], system_prompt="be brief") == "be brief\n\n" + want[0]
-    ref_path = "/root/reference/three_party/Janus/janus/utils/conversation.py"
-    if os.path.exists(ref_path):          # the reference's own template code, when the tree is mounted (authoring container)
-        import importlib.util
-        spec = importlib.util.spec_from_file_location("ref_conversation", ref_path)
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        for c, w in zip(convs, want):
-            conv = mod.get_conv_template("deepseek")
-            conv.set_system_message("")
-            for m in c:
-                conv.append_message(m["role"], m["content"].strip())
-            assert conv.get_prompt().strip() == w
 
 
 def test_prompt_pipeline_wraps_pads_and_collates_like_the_reference():
@@ -227,7 +217,7 @@ def test_bench_reference_arm_prints_the_contract_line(capsys):
     import argparse
     import json
     import bench
-    args = argparse.Namespace(model="tiny", gpus=1, steps=1, warmup=1, impl="reference")
+    args = argparse.Namespace(model="tiny", gpus=1, steps=2, warmup=1, impl="reference")
     os.environ.pop("RANK", None)
     bench.run_reference_arm(args)
     lines = [l for l in capsys.readouterr().out.splitlines() if l.startswith("{")]
@@ -239,9 +229,10 @@ def test_bench_reference_arm_prints_the_contract_line(capsys):
     assert d["impl"] == "reference" and d["metric"] == bench.METRIC and d["unit"] == bench.UNIT and d["value"] > 0
     assert d["e2e"] == {"value": d["value"], "unit": bench.UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1 and d["vs_baseline"] is None
-    # nothing is extrapolated: the line's time is the wall time of the one image that was run, value = 1 / that time
+    # nothing is extrapolated: one full image per step, the line's time is the wall time of the images that were run
+    assert d["steps"] == 2 and d["timed"]["images"] == 2 and d["timed"]["decode_steps"] == 2 * (O.TINY.n_img_tokens - 1)
     assert abs(d["ms_per_step"] * d["steps"] - 1e3 * d["timed"]["wall_s"]) < 1e-6 * d["timed"]["wall_s"] * 1e3 + 1e-9
-    assert abs(d["value"] * d["timed"]["wall_s"] - 1.0) < 1e-9 and d["timed"]["decode_steps"] == O.TINY.n_img_tokens - 1
+    assert abs(d["value"] * d["timed"]["wall_s"] - d["steps"]) < 1e-9
     assert d["cpu_baseline_b16"]["images_per_s_estimate"] > 0
     # ranks other than 0 do no work and print nothing
     os.environ["RANK"] = "1"
@@ -250,6 +241,38 @@ def test_bench_reference_arm_prints_the_contract_line(capsys):
         assert capsys.readouterr().out.strip() == ""
     finally:
         os.environ.pop("RANK", None)
+
+
+def test_bench_dump_outputs_float32_within_budget(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: the step's images and tokens and their batch rows as float32 .npy; a batch over the
+    byte budget is cut to the same seeded sample of whole images on every call; a later dump into the same directory
+    leaves no file of the earlier one behind."""
+    import numpy as np
+    import bench
+    g = torch.Generator().manual_seed(0)
+    images = torch.randint(0, 256, (6, 3, 8, 8), generator=g, dtype=torch.uint8)
+    tokens = torch.randint(0, 16384, (6, 10), generator=g, dtype=torch.int32)
+
+    def load(d):
+        assert sorted(os.listdir(d)) == ["images.npy", "rows.npy", "tokens.npy"]
+        got = {n: np.load(d / (n + ".npy")) for n in ("images", "tokens", "rows")}
+        assert all(a.dtype == np.float32 for a in got.values())
+        return got
+
+    budget = bench.DUMP_BYTES
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4 * 4 * (3 * 8 * 8 + 10 + 1))         # room for 4 of the 6 images
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), images, tokens)
+    a, b = load(tmp_path / "a"), load(tmp_path / "b")
+    r = a["rows"].astype(np.int64)
+    assert len(r) == 4 and np.all(np.diff(r) > 0) and np.array_equal(a["rows"], b["rows"])
+    assert np.array_equal(a["images"], images.numpy()[r]) and np.array_equal(a["tokens"], tokens.numpy()[r])
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= bench.DUMP_BYTES + 3 * 128   # + .npy headers
+    monkeypatch.setattr(bench, "DUMP_BYTES", budget)
+    bench.dump_outputs(str(tmp_path / "a"), images, tokens)                          # the whole batch fits
+    a = load(tmp_path / "a")
+    assert np.array_equal(a["rows"], np.arange(6)) and np.array_equal(a["images"], images.numpy())
+    assert np.array_equal(a["tokens"], tokens.numpy())
 
 
 # ------------------------------------------------------------------ teacher-forcing gate (ADVICE r1, plangen_base.py:528,593)
