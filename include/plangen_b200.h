@@ -20,7 +20,7 @@
 extern "C" {
 #endif
 
-#define PG_ABI_VERSION 2
+#define PG_ABI_VERSION 3
 
 /* arithmetic regimes */
 #define PG_MODE_BF16 0 /* the reference's regime: fp32 master weights under autocast(bf16), plangen_base.py:360 */
@@ -92,10 +92,13 @@ int pg_gen_head(pg_engine* e, const float* hidden, int R, float* logits_out, voi
  * args.use_teacher_forcing as the reference does, :593).  greedy != 0 -> argmax.
  * top_k > 0: only CFG logits >= the k-th largest survive (`logits[logits < topk(logits,k)[..., -1:]] = -inf`) before
  * the softmax; 0 = off = the reference (it has no top-k; north_star names the option).
+ * top_p in [0, 1) (after top-k): HF TopPLogitsWarper with min_tokens_to_keep = 1 - in ascending (logit, index) order
+ * the longest prefix whose cumulative probability is <= fp32(1 - top_p) is removed, the largest logit always stays;
+ * 1 = off (the default, the unfiltered path).  Outside [0, 1] or NaN: failure.  Ignored when greedy != 0.
  * tokens_out int32 [B, n_steps] (column `step` written); x_next fp32 [2B, D]. */
 int pg_cfg_sample_embed(pg_engine* e, const float* logits, int B, float cfg_weight,
                         float temperature, uint64_t seed, uint64_t philox_offset, int greedy, int top_k,
-                        const int32_t* edit_region, const int32_t* gt_labels, int step,
+                        double top_p, const int32_t* edit_region, const int32_t* gt_labels, int step,
                         int n_steps, int32_t* tokens_out, float* x_next, void* stream);
 
 /* replaces: vl_gpt.prepare_gen_img_embeds(ids)     modeling_vlm.py:270-271
@@ -105,10 +108,11 @@ int pg_prepare_gen_img_embeds(pg_engine* e, const int32_t* ids, int n, float* ou
 /* replaces: System.sample_image (plangen_base.py:567-607), whole loop on the device:
  * prefill + n_steps x (gen_head, CFG, sample, embed, decode step) with no host sync.
  * x_prompt fp32 [R,P,D] (consumed).  tokens_out int32 [R/2, n_steps].  kv_start / edit_region / gt_labels are copied
- * into engine-owned buffers at entry (captured graphs are keyed on shapes and scalars, not on caller addresses). */
+ * into engine-owned buffers at entry (captured graphs are keyed on shapes and scalars, not on caller addresses).
+ * top_k / top_p as for pg_cfg_sample_embed. */
 int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P,
                     int n_steps, float cfg_weight, float temperature, uint64_t seed, int greedy, int top_k,
-                    const int32_t* edit_region, const int32_t* gt_labels,
+                    double top_p, const int32_t* edit_region, const int32_t* gt_labels,
                     int32_t* tokens_out, void* stream);
 
 /* replaces: System.x2t (plangen_base.py:513-523) = vl_gpt.language_model.generate(inputs_embeds=,

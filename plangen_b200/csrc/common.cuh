@@ -146,6 +146,13 @@ PG_DEVINL uint32_t dsmem_ld_u32(const void* my_smem_ptr, uint32_t rank) {
   asm volatile("ld.shared::cluster.u32 %0, [%1];" : "=r"(v) : "r"(remote) : "memory");
   return v;
 }
+PG_DEVINL uint64_t dsmem_ld_u64(const void* my_smem_ptr, uint32_t rank) {
+  uint32_t remote;
+  uint64_t v;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(smem_u32(my_smem_ptr)), "r"(rank));
+  asm volatile("ld.shared::cluster.u64 %0, [%1];" : "=l"(v) : "r"(remote) : "memory");
+  return v;
+}
 
 
 // generic-proxy writes (st.shared) made visible to the async proxy (TMA / tcgen05)

@@ -1179,36 +1179,45 @@ static void philox_policy(pg_engine* e, size_t numel, uint64_t* counter_offset, 
 }
 
 static int k_sample(pg_engine* e, const float* part, int S, size_t sstride, const float* bias, int B, float cfg_weight,
-                    float temperature, uint64_t seed, uint64_t offset_base, int greedy, int top_k, const int32_t* edit_region,
-                    const int32_t* gt_labels, int step_base, const int* step_ptr, int n_steps, int32_t* tokens_out,
-                    float* x_next, const float* next_norm_w, void* xn_next, cudaStream_t st) {
+                    float temperature, uint64_t seed, uint64_t offset_base, int greedy, int top_k, double top_p,
+                    const int32_t* edit_region, const int32_t* gt_labels, int step_base, const int* step_ptr, int n_steps,
+                    int32_t* tokens_out, float* x_next, const float* next_norm_w, void* xn_next, cudaStream_t st) {
   const pg_dims& d = e->d;
   uint64_t per_step, stride;
   philox_policy(e, (size_t)B * d.img_vocab, &per_step, &stride);
-  const size_t csm = (size_t)((d.img_vocab + SAMPLE_CLUSTER - 1) / SAMPLE_CLUSTER) * 4;
+  const size_t chunk = (size_t)((d.img_vocab + SAMPLE_CLUSTER - 1) / SAMPLE_CLUSTER);
+  size_t csm = chunk * 4;
+  // top-p: the threshold torch compares the fp32 cumulative sum with, fp32(1 - top_p) with 1 - top_p in double;
+  // the kernel then keeps the logits and the select's 5 x 256 fixed-point mass histograms in dynamic shared memory
+  const float top_p_thr = top_p < 1.0 ? (float)(1.0 - top_p) : -1.f;
+  if (top_p < 1.0) {
+    csm = ((chunk + 1) & ~(size_t)1) * 8 + 5 * 256 * 8;
+    if (csm > 48 * 1024) return fail("top_p needs %zu B of shared memory per CTA at img_vocab %d (48 KB available)", csm, d.img_vocab);
+  }
   DISPATCH_T(e,
              launch(e, cfg_sample_embed_cluster_kernel<bf16>, dim3(B * SAMPLE_CLUSTER), dim3(SAMPLE_CL_THREADS), csm, st, part, S, sstride, bias, B, d.img_vocab,
-                    cfg_weight, temperature, seed, offset_base, per_step, stride, greedy, top_k, edit_region, gt_labels, step_base,
-                    step_ptr, n_steps, tokens_out, (const bf16*)e->embed_table, d.D, x_next, next_norm_w, (bf16*)xn_next,
+                    cfg_weight, temperature, seed, offset_base, per_step, stride, greedy, top_k, top_p_thr, edit_region, gt_labels,
+                    step_base, step_ptr, n_steps, tokens_out, (const bf16*)e->embed_table, d.D, x_next, next_norm_w, (bf16*)xn_next,
                     d.rms_eps, 1, e->dbg_logits),
              launch(e, cfg_sample_embed_cluster_kernel<float>, dim3(B * SAMPLE_CLUSTER), dim3(SAMPLE_CL_THREADS), csm, st, part, S, sstride, bias, B, d.img_vocab,
-                    cfg_weight, temperature, seed, offset_base, per_step, stride, greedy, top_k, edit_region, gt_labels, step_base,
-                    step_ptr, n_steps, tokens_out, (const float*)e->embed_table, d.D, x_next, next_norm_w, (float*)xn_next,
+                    cfg_weight, temperature, seed, offset_base, per_step, stride, greedy, top_k, top_p_thr, edit_region, gt_labels,
+                    step_base, step_ptr, n_steps, tokens_out, (const float*)e->embed_table, d.D, x_next, next_norm_w, (float*)xn_next,
                     d.rms_eps, 0, e->dbg_logits));
   return 0;
 }
 
 // a6-a8
 extern "C" int pg_cfg_sample_embed(pg_engine* e, const float* logits, int B, float cfg_weight, float temperature,
-                                   uint64_t seed, uint64_t philox_offset, int greedy, int top_k,
+                                   uint64_t seed, uint64_t philox_offset, int greedy, int top_k, double top_p,
                                    const int32_t* edit_region, const int32_t* gt_labels, int step, int n_steps,
                                    int32_t* tokens_out, float* x_next, void* stream) {
   TRY(check_ready(e));
   if (B < 1 || 2 * B > e->d.max_rows) return fail("sample B=%d exceeds engine limits", B);
   if (step < 0 || step >= n_steps) return fail("step %d out of range", step);
   if (top_k < 0) return fail("top_k must be >= 0");
+  if (!(top_p >= 0.0 && top_p <= 1.0)) return fail("top_p must be in [0, 1], got %g", top_p);
   if ((edit_region == nullptr) != (gt_labels == nullptr)) return fail("edit_region and gt_labels go together");
-  return k_sample(e, logits, 1, 0, nullptr, B, cfg_weight, temperature, seed, philox_offset, greedy, top_k, edit_region,
+  return k_sample(e, logits, 1, 0, nullptr, B, cfg_weight, temperature, seed, philox_offset, greedy, top_k, top_p, edit_region,
                   gt_labels, step, nullptr, n_steps, tokens_out, x_next, nullptr, nullptr, (cudaStream_t)stream);
 }
 
@@ -1226,8 +1235,8 @@ extern "C" int pg_prepare_gen_img_embeds(pg_engine* e, const int32_t* ids, int n
 // (graph replays; consecutive graph launches are fully ordered, so kernels may read it before their
 // PDL wait).
 static int one_step(pg_engine* e, const int32_t* kv_start, int R, int P, int n_steps, float cfg_weight, float temperature,
-                    uint64_t seed, int greedy, int top_k, const int32_t* edit_region, const int32_t* gt_labels,
-                    int32_t* tokens_out, bool with_lm, int step_host, cudaStream_t st) {
+                    uint64_t seed, int greedy, int top_k, double top_p, const int32_t* edit_region,
+                    const int32_t* gt_labels, int32_t* tokens_out, bool with_lm, int step_host, cudaStream_t st) {
   NEED(b1, float, "head.b1");
   LayerW w0;
   TRY(layer_weights(e, 0, &w0));
@@ -1237,7 +1246,7 @@ static int one_step(pg_engine* e, const int32_t* kv_start, int R, int P, int n_s
   uint64_t per_step, stride;
   philox_policy(e, (size_t)(R / 2) * e->d.img_vocab, &per_step, &stride);
   TRY(k_sample(e, e->part, S, (size_t)R * e->d.img_vocab, b1, R / 2, cfg_weight, temperature, seed,
-               host ? per_step * (uint64_t)step_host : 0, greedy, top_k, edit_region, gt_labels, host ? step_host : 0,
+               host ? per_step * (uint64_t)step_host : 0, greedy, top_k, top_p, edit_region, gt_labels, host ? step_host : 0,
                host ? nullptr : e->step_ctr, n_steps, tokens_out, with_lm ? e->x_dec : nullptr, w0.ln1,
                with_lm ? e->xn : nullptr, st));
   if (with_lm)
@@ -1274,13 +1283,14 @@ static int graph_for(pg_engine* e, const std::string& key, cudaStream_t st, F&& 
 }
 
 extern "C" int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
-                               float cfg_weight, float temperature, uint64_t seed, int greedy, int top_k,
+                               float cfg_weight, float temperature, uint64_t seed, int greedy, int top_k, double top_p,
                                const int32_t* edit_region, const int32_t* gt_labels, int32_t* tokens_out, void* stream) {
   TRY(check_ready(e));
   if (R % 2) return fail("R must be even (interleaved cond/uncond rows)");
   if (R < 2 || R > e->d.max_rows) return fail("sample_image R=%d exceeds engine limits", R);
   if (n_steps < 1 || n_steps > e->d.max_steps) return fail("n_steps %d exceeds engine limit %d", n_steps, e->d.max_steps);
   if (top_k < 0) return fail("top_k must be >= 0");
+  if (!(top_p >= 0.0 && top_p <= 1.0)) return fail("top_p must be in [0, 1], got %g", top_p);
   if ((edit_region == nullptr) != (gt_labels == nullptr)) return fail("edit_region and gt_labels go together ([R/2][n_steps] each)");
   if (!kv_start || !tokens_out) return fail("null argument");
   cudaStream_t user = (cudaStream_t)stream;
@@ -1303,13 +1313,13 @@ extern "C" int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_
   if (n_steps > 1) {
     if (e->use_graph) {
       char key[256];
-      snprintf(key, sizeof(key), "img/%d/%d/%d/%a/%a/%llu/%d/%d/%d/%d", R, P, n_steps, cfg_weight, temperature,
-               (unsigned long long)seed, greedy, top_k, edit_region ? 1 : 0, (e->prof_buf && e->prof_step >= 0) ? 1 : 0);
+      snprintf(key, sizeof(key), "img/%d/%d/%d/%a/%a/%llu/%d/%d/%a/%d/%d", R, P, n_steps, cfg_weight, temperature,
+               (unsigned long long)seed, greedy, top_k, top_p, edit_region ? 1 : 0, (e->prof_buf && e->prof_step >= 0) ? 1 : 0);
       pg_engine::GraphEntry* ge = nullptr;
       TRY(graph_for(e, key, st, [&]() {
         e->prof_active = (e->prof_buf != nullptr && e->prof_step >= 0);
         e->prof_slot = 0;
-        int rc = one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, er, gl, toks, true, -1, st);
+        int rc = one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, true, -1, st);
         e->prof_active = false;
         return rc;
       }, &ge));
@@ -1332,7 +1342,7 @@ extern "C" int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_
           CK(cudaMemsetAsync(e->prof_buf, 0xFF, PROF_SLOTS * 8, st));
           CK(cudaMemsetAsync(e->prof_buf + PROF_SLOTS, 0, PROF_SLOTS * 8, st));
         }
-        int rc = one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, er, gl, toks, true, i, st);
+        int rc = one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, true, i, st);
         if (e->prof_active)
           CK(cudaMemcpyAsync(e->prof_buf + 2 * PROF_SLOTS, e->prof_buf, 2 * PROF_SLOTS * 8, cudaMemcpyDeviceToDevice, st));
         e->prof_active = false;
@@ -1341,7 +1351,7 @@ extern "C" int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_
     }
   }
   // last token: head + sample only (the reference computes and drops one more embed, SURVEY appendix A.12)
-  TRY(one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, er, gl, toks, false, n_steps - 1, st));
+  TRY(one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, false, n_steps - 1, st));
   CK(cudaMemcpyAsync(tokens_out, toks, tok_bytes, cudaMemcpyDeviceToDevice, st));
   CK(cudaEventRecord(e->ev_out, st));
   CK(cudaStreamWaitEvent(user, e->ev_out, 0));

@@ -62,36 +62,125 @@ __device__ unsigned long long* g_sample_dbg = nullptr;   // debug timeline (tool
 // result equals torch.multinomial on the masked distribution with the same generator.  The threshold is found by
 // a 4-pass radix select (8 bits per pass) over an order-preserving integer key, histograms summed across the
 // cluster through distributed shared memory.
+//
+// top_p < 1 (HF TopPLogitsWarper after TopKLogitsWarper, min_tokens_to_keep = 1; 1 = off is the default): in the
+// ascending order of (t, index), the longest prefix whose cumulative probability is <= thr = fp32(1 - top_p) leaves
+// the distribution, except the largest element.  The boundary key is the same radix select weighted by probability
+// mass p_v = e_v / sum (the softmax's own numbers) in 2^62 fixed point, so the result does not depend on the order of
+// the shared-memory atomics.  The tie group at the boundary key all has the same p; its members leave in index order
+// while mass_below + j * p <= thr.  The removed e_v are zeroed and the sum recomputed over the kept set.  Greedy
+// sampling skips it (the arg-max is always kept).
 constexpr int SAMPLE_CLUSTER = 8;
 // order-preserving map float -> uint32 (larger value, larger key; -0 < +0 is harmless here)
 PG_DEVINL uint32_t sample_order_key(float t) {
   const uint32_t u = __float_as_uint(t);
   return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
+PG_DEVINL float sample_key_value(uint32_t k) { return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k); }
 #ifndef PG_SAMPLE_CL_THREADS
 #define PG_SAMPLE_CL_THREADS 256
 #endif
 constexpr int SAMPLE_CL_THREADS = PG_SAMPLE_CL_THREADS;   // light CTAs: a cluster needs 8 co-scheduled SMs of one GPC
+constexpr float SAMPLE_MASS_ONE = 4611686018427387904.f;  // 2^62: fixed-point scale of the top-p probability masses
 
 struct SampleXchg {
   float mx, sum, bv, ss;
-  int bi;
+  int bi, ties;
 };
+
+PG_DEVINL void sample_hist_add(uint32_t* h, uint32_t w) { atomicAdd(h, w); }
+// a 64-bit shared-memory atomicAdd is a compare-and-swap loop, slow under the contention of the first passes: add the
+// two halves with native 32-bit atomics and carry into the high word (the histograms are read only after a barrier)
+PG_DEVINL void sample_hist_add(unsigned long long* h, unsigned long long w) {
+  uint32_t* h32 = reinterpret_cast<uint32_t*>(h);
+  const uint32_t lo = (uint32_t)w, old = atomicAdd(h32, lo);
+  atomicAdd(h32 + 1, (uint32_t)(w >> 32) + (old + lo < old ? 1u : 0u));
+}
+
+// Cluster-wide radix select: the largest 32-bit key K with W(key < K) <= thr, where W sums weight(i) over the image's
+// elements (each CTA contributes i in [0, n) of its slice).  Count weights with thr = V - k give the k-th largest key;
+// probability-mass weights give the top-p boundary.  thr is first clamped to W(all) - 1, so K is always a present key.
+// Returns K, *below = W(key < K) and, if total != nullptr, *total = W(all).  hist: [4][256], one histogram per pass, read by the other CTAs through DSMEM (so
+// no pass overwrites what a peer may still be reading).  Called by the whole CTA of every CTA of the cluster.
+template <typename W, typename KeyF, typename WeightF>
+PG_DEVINL uint32_t cluster_radix_select(W (*hist)[256], W* hsum, W* sel_w, uint32_t* sel_d, int n, KeyF key,
+                                        WeightF weight, W thr, W* below_out, W* total = nullptr) {
+  const int tid = threadIdx.x;
+  for (int i = tid; i < 4 * 256; i += SAMPLE_CL_THREADS) (&hist[0][0])[i] = 0;
+  __syncthreads();
+  uint32_t prefix = 0;
+  W below = 0;
+  for (int pass = 0; pass < 4; ++pass) {
+    const int shift = 24 - 8 * pass;
+    const uint32_t himask = pass == 0 ? 0u : (0xffffffffu << (shift + 8));
+    for (int i = tid; i < n; i += SAMPLE_CL_THREADS) {
+      const uint32_t k = key(i);
+      if ((k & himask) == prefix) sample_hist_add(&hist[pass][(k >> shift) & 255u], weight(i));
+    }
+    cluster_sync_all();                                  // every CTA's histogram of this pass is complete
+    for (int d = tid; d < 256; d += SAMPLE_CL_THREADS) {
+      W c = 0;
+#pragma unroll
+      for (uint32_t r = 0; r < SAMPLE_CLUSTER; ++r) {
+        if constexpr (sizeof(W) == 8) c += dsmem_ld_u64(&hist[pass][d], r);
+        else c += dsmem_ld_u32(&hist[pass][d], r);
+      }
+      hsum[d] = c;
+    }
+    __syncthreads();
+    if (tid < 32) {
+      // lane l owns digits 8l .. 8l+7; prefix weights from the lowest digit up
+      W mine = 0;
+#pragma unroll
+      for (int j = 0; j < 8; ++j) mine += hsum[tid * 8 + j];
+      W run = mine;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const W t = __shfl_up_sync(0xffffffffu, run, o);
+        if (tid >= o) run += t;
+      }
+      if (pass == 0) {
+        const W all = __shfl_sync(0xffffffffu, run, 31);
+        thr = min(thr, (W)(all - 1));
+        if (total && tid == 0) *total = all;
+      }
+      W lo = below + (run - mine);                       // weight of the keys below this lane's first digit
+      const uint32_t ok = __ballot_sync(0xffffffffu, lo <= thr);   // lane 0 always: below <= thr
+      if (tid == 31 - __clz(ok)) {
+        uint32_t d = (uint32_t)tid * 8;
+        for (int j = 1; j < 8; ++j) {
+          const W nx = lo + hsum[tid * 8 + j - 1];
+          if (nx > thr) break;
+          lo = nx; d = (uint32_t)(tid * 8 + j);
+        }
+        *sel_d = d; *sel_w = lo;
+      }
+    }
+    __syncthreads();
+    prefix |= *sel_d << shift;
+    below = *sel_w;
+    __syncthreads();
+  }
+  *below_out = below;
+  return prefix;
+}
 
 template <typename T>
 __global__ void __cluster_dims__(SAMPLE_CLUSTER, 1, 1) __launch_bounds__(SAMPLE_CL_THREADS)
 cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t split_stride, const float* __restrict__ bias,
                                 int B, int V, float cfg_weight, float temperature, uint64_t seed, uint64_t offset_base,
                                 uint64_t offset_per_step, uint64_t philox_stride, int greedy, int top_k,
-                                const int32_t* __restrict__ edit_region, const int32_t* __restrict__ gt_labels,
+                                float top_p_thr, const int32_t* __restrict__ edit_region, const int32_t* __restrict__ gt_labels,
                                 int step_base, const int* __restrict__ step_ptr, int n_steps,
                                 int32_t* __restrict__ tokens_out, const T* __restrict__ embed_table, int D,
                                 float* __restrict__ x_next, const float* __restrict__ next_norm_w, T* __restrict__ xn_next,
                                 float eps, int round_resid, float* __restrict__ dbg_logits) {
-  extern __shared__ float sh[];      // this CTA's slice of the CFG logits -> unnormalised probabilities
-  __shared__ int hist[4][256];       // top-k radix select: one histogram per pass (read by the other CTAs)
-  __shared__ int hsum[256];
-  __shared__ uint32_t sel_s[2];      // {digit, remaining k} of the current pass
+  extern __shared__ __align__(16) float sh[];   // this CTA's slice of the CFG logits -> unnormalised probabilities
+  // top_p_thr >= 0 (top-p on): sh is followed by the slice's logits t and the mass histograms of its radix select
+  __shared__ uint32_t hist[4][256];  // top-k radix select: one histogram per pass (read by the other CTAs)
+  __shared__ uint32_t hsum[256];
+  __shared__ uint32_t sel_d, sel_c;  // digit and count below of the current pass
+  __shared__ unsigned long long sel_m, mass_all;
   __shared__ float red[32];
   __shared__ float bestv[32];
   __shared__ int besti[32];
@@ -162,58 +251,16 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
   }
   SAMPLE_STAMP(2);
   if (top_k > 0 && top_k < V) {
-    // k-th largest CFG logit of the image: radix select on key(t) (monotone in t), most significant byte first
-    for (int i = tid; i < 4 * 256; i += SAMPLE_CL_THREADS) (&hist[0][0])[i] = 0;
-    __syncthreads();
-    uint32_t prefix = 0, krem = (uint32_t)top_k;
-    for (int pass = 0; pass < 4; ++pass) {
-      const int shift = 24 - 8 * pass;
-      const uint32_t himask = pass == 0 ? 0u : (0xffffffffu << (shift + 8));
-      for (int v = v_lo + tid; v < v_hi; v += SAMPLE_CL_THREADS) {
-        const uint32_t key = sample_order_key(sh[v - v_lo]);
-        if ((key & himask) == prefix) atomicAdd(&hist[pass][(key >> shift) & 255u], 1);
-      }
-      cluster_sync_all();                                  // every CTA's histogram of this pass is complete
-      for (int d = tid; d < 256; d += SAMPLE_CL_THREADS) {
-        int c = 0;
-#pragma unroll
-        for (uint32_t r = 0; r < SAMPLE_CLUSTER; ++r) c += (int)dsmem_ld_u32(&hist[pass][d], r);
-        hsum[d] = c;
-      }
-      __syncthreads();
-      if (tid < 32) {
-        // lane l owns digits 8l .. 8l+7; suffix counts from the top digit down
-        int mine = 0;
-#pragma unroll
-        for (int j = 0; j < 8; ++j) mine += hsum[tid * 8 + j];
-        // suffix scan over the 32 lanes: above = elements in digits owned by higher lanes
-        int run = mine;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-          const int t = __shfl_down_sync(0xffffffffu, run, o);
-          if (tid + o < 32) run += t;
-        }
-        const int above = run - mine;
-        const bool here = (uint32_t)above < krem && (uint32_t)(above + mine) >= krem;   // exactly one lane
-        if (here) {
-          int cum = above;
-          for (int j = 7; j >= 0; --j) {
-            const int c = hsum[tid * 8 + j];
-            if ((uint32_t)(cum + c) >= krem) { sel_s[0] = (uint32_t)(tid * 8 + j); sel_s[1] = krem - (uint32_t)cum; break; }
-            cum += c;
-          }
-        }
-      }
-      __syncthreads();
-      prefix |= sel_s[0] << shift;
-      krem = sel_s[1];
-      __syncthreads();
-    }
-    // prefix = key of the k-th largest logit: everything below it leaves the distribution
+    // k-th largest CFG logit of the image = the largest key with at most V - k keys below it
+    uint32_t below;
+    const uint32_t kth = cluster_radix_select<uint32_t>(
+        hist, hsum, &sel_c, &sel_d, v_hi - v_lo, [&](int i) { return sample_order_key(sh[i]); }, [](int) { return 1u; },
+        (uint32_t)(V - top_k), &below);
+    // everything below the k-th largest leaves the distribution
     mx = -INFINITY;
     for (int v = v_lo + tid; v < v_hi; v += SAMPLE_CL_THREADS) {
       float t = sh[v - v_lo];
-      if (sample_order_key(t) < prefix) { t = -INFINITY; sh[v - v_lo] = t; }
+      if (sample_order_key(t) < kth) { t = -INFINITY; sh[v - v_lo] = t; }
       mx = fmaxf(mx, t);
     }
   }
@@ -222,9 +269,13 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
   cluster_sync_all();
 #pragma unroll
   for (uint32_t r = 0; r < SAMPLE_CLUSTER; ++r) mx = fmaxf(mx, __uint_as_float(dsmem_ld_u32(&xc.mx, r)));
+  const bool top_p = top_p_thr >= 0.f && !greedy;
+  float* const tsh = sh + chunk;                            // top-p: the logits t, ordering key of the select
   float sum = 0.f;
   for (int v = v_lo + tid; v < v_hi; v += SAMPLE_CL_THREADS) {
-    const float e = expf(sh[v - v_lo] - mx);
+    const float t = sh[v - v_lo];
+    if (top_p) tsh[v - v_lo] = t;
+    const float e = expf(t - mx);
     sh[v - v_lo] = e;
     sum += e;
   }
@@ -235,6 +286,68 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
   sum = 0.f;
 #pragma unroll
   for (uint32_t r = 0; r < SAMPLE_CLUSTER; ++r) sum += __uint_as_float(dsmem_ld_u32(&xc.sum, r));   // rank order
+  if (top_p) {
+    typedef unsigned long long u64;
+    u64(*mhist)[256] = reinterpret_cast<u64(*)[256]>(sh + 2 * ((chunk + 1) & ~1));
+    u64* mhsum = &mhist[4][0];
+    const u64 thr = __float2ull_rn(top_p_thr * SAMPLE_MASS_ONE);
+    u64 below;
+    const uint32_t kb = cluster_radix_select<u64>(
+        mhist, mhsum, &sel_m, &sel_d, v_hi - v_lo, [&](int i) { return sample_order_key(tsh[i]); },
+        [&](int i) { return __float2ull_rn(__fdiv_rn(sh[i], sum) * SAMPLE_MASS_ONE); }, thr, &below, &mass_all);
+    // the tie group at kb: members per CTA (ranks own ascending index ranges), then how many of them leave
+    const u64 pk = __float2ull_rn(__fdiv_rn(expf(sample_key_value(kb) - mx), sum) * SAMPLE_MASS_ONE);
+    int mine = 0;
+    for (int v0 = v_lo; v0 < v_hi; v0 += SAMPLE_CL_THREADS) {
+      const int v = v0 + tid;
+      mine += __syncthreads_count(v < v_hi && sample_order_key(tsh[v - v_lo]) == kb);
+    }
+    if (tid == 0) xc.ties = mine;
+    cluster_sync_all();
+    int first = 0, ties = 0;                                 // group members in lower ranks, in the whole image
+#pragma unroll
+    for (uint32_t r = 0; r < SAMPLE_CLUSTER; ++r) {
+      const int c = (int)dsmem_ld_u32(&xc.ties, r);
+      if (r < rank) first += c;
+      ties += c;
+    }
+    // member j = 1, 2, ... (index order) leaves while below + j * pk <= thr; the group of the largest key keeps one
+    u64 drop = pk ? (thr - below) / pk : (u64)ties;
+    if (below + (u64)ties * pk == mass_all) drop = min(drop, (u64)(ties - 1));
+    drop = min(drop, (u64)ties);
+    // zero the removed e_v and sum the kept set as the softmax of the masked logits does (same per-thread order)
+    __shared__ int wcnt[SAMPLE_CL_THREADS / 32];
+    const int lane = tid & 31, warp = tid >> 5;
+    int seen = first;                                        // group members before this iteration's elements
+    float kept = 0.f;
+    for (int v0 = v_lo; v0 < v_hi; v0 += SAMPLE_CL_THREADS) {
+      const int v = v0 + tid;
+      const uint32_t k = v < v_hi ? sample_order_key(tsh[v - v_lo]) : 0u;
+      const bool tie = v < v_hi && k == kb;
+      const uint32_t bal = __ballot_sync(0xffffffffu, tie);
+      if (lane == 0) wcnt[warp] = __popc(bal);
+      __syncthreads();
+      int before = seen + __popc(bal & ((1u << lane) - 1u)), all = 0;
+#pragma unroll
+      for (int w = 0; w < SAMPLE_CL_THREADS / 32; ++w) {
+        if (w < warp) before += wcnt[w];
+        all += wcnt[w];
+      }
+      __syncthreads();
+      seen += all;
+      if (v < v_hi) {
+        float e = sh[v - v_lo];
+        if (k < kb || (tie && (u64)before < drop)) { e = 0.f; sh[v - v_lo] = e; }
+        kept += e;
+      }
+    }
+    kept = block_sum(kept, red);
+    if (tid == 0) xc.sum = kept;
+    cluster_sync_all();
+    sum = 0.f;
+#pragma unroll
+    for (uint32_t r = 0; r < SAMPLE_CLUSTER; ++r) sum += __uint_as_float(dsmem_ld_u32(&xc.sum, r));
+  }
   // argmax over p/q (first index wins ties, like torch.argmax)
   float bv = -INFINITY;
   int bi = 0x7fffffff;

@@ -211,7 +211,7 @@ class FastJanus:
     def __init__(self, state_dict: Dict[str, torch.Tensor], dims: Dims, mode: str = "bf16",
                  max_batch: int = 16, max_prompt: int = 512, max_steps: Optional[int] = None,
                  device: str = "cuda:0", seed: int = 0, with_vq: bool = True, options: Optional[dict] = None,
-                 use_teacher_forcing: bool = False, top_k: int = 0, max_images: int = 0):
+                 use_teacher_forcing: bool = False, top_k: int = 0, max_images: int = 0, top_p: float = 1.0):
         if not torch.cuda.is_available():
             raise RuntimeError("plangen_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         if mode not in MODE_IDS:
@@ -219,6 +219,8 @@ class FastJanus:
         self.dims, self.mode, self.seed = dims, mode, seed
         self.use_teacher_forcing = bool(use_teacher_forcing)      # args.use_teacher_forcing (plangen_base.py:528,556,593)
         self.top_k = int(top_k)                                   # 0 = off (the reference has no top-k)
+        self.top_p = float(top_p)                                 # 1 = off (nor top-p)
+        _ops._top_p(self.top_p)
         self.device = torch.device(device)
         self.out_dtype = torch.bfloat16 if mode == "bf16" else torch.float32
         self.max_rows = 2 * max_batch
@@ -362,13 +364,14 @@ class FastJanus:
     def cfg_sample_embed(self, logits: torch.Tensor, cfg_weight: float, temperature: float, seed: int, offset: int,
                          step: int, n_steps: int, tokens_out: torch.Tensor, greedy: bool = False,
                          edit_region: Optional[torch.Tensor] = None, gt_labels: Optional[torch.Tensor] = None,
-                         top_k: int = 0):
-        """plangen_base.py:580-604 in one launch; returns the next inputs_embeds (2B, D) fp32."""
+                         top_k: int = 0, top_p: float = 1.0):
+        """plangen_base.py:580-604 in one launch; returns the next inputs_embeds (2B, D) fp32.  `top_k` / `top_p` filter the
+        CFG logits as HF's TopKLogitsWarper then TopPLogitsWarper do (0 / 1 = off)."""
         B = logits.shape[0] // 2
         lg = logits.to(device=self.device, dtype=torch.float32).contiguous()
         x_next = torch.empty(2 * B, self.dims.D, device=self.device, dtype=torch.float32)
         OPS.cfg_sample_embed(self.handle, lg, float(cfg_weight), float(temperature), _i64(seed), int(offset), bool(greedy), int(top_k),
-                             edit_region, gt_labels, int(step), int(n_steps), tokens_out, x_next)
+                             edit_region, gt_labels, int(step), int(n_steps), tokens_out, x_next, float(top_p))
         return x_next
 
     def philox_offset_per_step(self, B: int) -> int:
@@ -404,12 +407,15 @@ class FastJanus:
     @torch.inference_mode()
     def sample_image(self, inputs_embeds, num_gen, image_token_num_per_image, mask, cfg_weight, temperature,
                      generator=None, batch=None, gt_labels=None, greedy: bool = False,
-                     use_teacher_forcing: Optional[bool] = None, top_k: Optional[int] = None):
+                     use_teacher_forcing: Optional[bool] = None, top_k: Optional[int] = None,
+                     top_p: Optional[float] = None):
         """System.sample_image (plangen_base.py:567-607).  `generator`: torch CUDA generator (its seed and
         philox offset are honoured and advanced) or an int seed.  Teacher forcing (:593-598) is gated on
         `use_teacher_forcing` (default: the engine's flag = `args.use_teacher_forcing`), never on the mere presence
         of batch['edit_region'] - the reference's datasets emit an all-zero edit_region for non-edit samples.
-        `top_k` > 0 keeps the k largest CFG logits before the softmax (north_star (4); 0 = off = the reference)."""
+        `top_k` > 0 keeps the k largest CFG logits before the softmax (north_star (4); 0 = off = the reference).
+        `top_p` < 1 then keeps the nucleus, as HF's TopPLogitsWarper after TopKLogitsWarper (1 = off = the reference).
+        None: the engine's defaults."""
         R, P, D = inputs_embeds.shape
         if R != 2 * num_gen:
             raise ValueError("inputs_embeds rows must be 2 * num_gen (interleaved cond/uncond)")
@@ -429,8 +435,9 @@ class FastJanus:
         if teacher:
             er, gl = self._teacher_inputs(batch, gt_labels, num_gen, n)
         k = int(self.top_k if top_k is None else top_k)
+        p = float(self.top_p if top_p is None else top_p)
         self._keep = (kv_start, x, er, gl)        # keep alive until the stream has consumed them
-        OPS.sample_image(self.handle, x, kv_start, n, float(cfg_weight), float(temperature), _i64(seed), bool(greedy), k, er, gl, tokens)
+        OPS.sample_image(self.handle, x, kv_start, n, float(cfg_weight), float(temperature), _i64(seed), bool(greedy), k, er, gl, tokens, p)
         self._serial += 1
         if isinstance(generator, torch.Generator):
             generator.set_offset(off + n * self.philox_offset_per_step(num_gen))
@@ -439,7 +446,8 @@ class FastJanus:
     @torch.inference_mode()
     def t2i(self, inputs_ids=None, parallel_size=1, image_token_num_per_image=None, cfg_weight=5.0, temperature=1.0,
             img_size=None, patch_size=None, gt_image=None, batch=None, mask=None, tokens=None, emb=None,
-            gt_labels=None, greedy: bool = False, use_teacher_forcing: Optional[bool] = None, top_k: Optional[int] = None):
+            gt_labels=None, greedy: bool = False, use_teacher_forcing: Optional[bool] = None, top_k: Optional[int] = None,
+            top_p: Optional[float] = None):
         """System.t2i (plangen_base.py:525-565), `tokens`/`emb` branches.  Returns (dec, mask_image).
         Teacher forcing (layout-guided editing, :528-532, :593-598, :557-562) follows `use_teacher_forcing` (default: the
         engine's flag, the counterpart of `args.use_teacher_forcing`): `gt_image` is encoded with the VQ encoder as the
@@ -462,7 +470,7 @@ class FastJanus:
         mask = torch.cat([mask.to(self.device)] * parallel_size)
         num_gen = inputs_embeds.shape[0] // 2
         gen = self.sample_image(inputs_embeds, num_gen, n, mask, cfg_weight, temperature, None, batch, gt_labels, greedy,
-                                use_teacher_forcing=teacher, top_k=top_k)
+                                use_teacher_forcing=teacher, top_k=top_k, top_p=top_p)
         g = img_size // patch_size
         dec = self.gen_vision_model.decode_code(gen.to(dtype=torch.int), shape=[num_gen, self.dims.code_dim, g, g])
         self.last_tokens = gen

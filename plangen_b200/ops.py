@@ -61,6 +61,11 @@ def _cuda(*ts):
             raise RuntimeError("plangen_b200 ops take CUDA tensors only (there is no CPU path)")
 
 
+def _top_p(top_p: float):
+    if not 0.0 <= float(top_p) <= 1.0:          # NaN fails too
+        raise ValueError(f"`top_p` has to be a float in [0, 1], but is {top_p}")
+
+
 @torch.library.custom_op(f"{NS}::embed_tokens", mutates_args=("out",), device_types="cuda")
 def embed_tokens(handle: int, ids: torch.Tensor, out: torch.Tensor) -> None:
     e = _eng(handle); _cuda(ids, out)
@@ -95,21 +100,21 @@ def prepare_gen_img_embeds(handle: int, ids: torch.Tensor, out: torch.Tensor) ->
 @torch.library.custom_op(f"{NS}::cfg_sample_embed", mutates_args=("tokens_out", "x_next"), device_types="cuda")
 def cfg_sample_embed(handle: int, logits: torch.Tensor, cfg_weight: float, temperature: float, seed: int, philox_offset: int,
                      greedy: bool, top_k: int, edit_region: Optional[torch.Tensor], gt_labels: Optional[torch.Tensor], step: int,
-                     n_steps: int, tokens_out: torch.Tensor, x_next: torch.Tensor) -> None:
-    e = _eng(handle); _cuda(logits, edit_region, gt_labels, tokens_out, x_next)
+                     n_steps: int, tokens_out: torch.Tensor, x_next: torch.Tensor, top_p: float = 1.0) -> None:
+    e = _eng(handle); _cuda(logits, edit_region, gt_labels, tokens_out, x_next); _top_p(top_p)
     _lib.check(e._lib.pg_cfg_sample_embed(e._h, _p(logits), logits.shape[0] // 2, float(cfg_weight), float(temperature), int(seed) & 0xFFFFFFFFFFFFFFFF,
-                                          int(philox_offset), int(greedy), int(top_k), _p(edit_region), _p(gt_labels), int(step),
+                                          int(philox_offset), int(greedy), int(top_k), float(top_p), _p(edit_region), _p(gt_labels), int(step),
                                           int(n_steps), _p(tokens_out), _p(x_next), _st(logits)))
 
 
 @torch.library.custom_op(f"{NS}::sample_image", mutates_args=("x_prompt", "tokens_out"), device_types="cuda")
 def sample_image(handle: int, x_prompt: torch.Tensor, kv_start: torch.Tensor, n_steps: int, cfg_weight: float, temperature: float,
                  seed: int, greedy: bool, top_k: int, edit_region: Optional[torch.Tensor], gt_labels: Optional[torch.Tensor],
-                 tokens_out: torch.Tensor) -> None:
-    e = _eng(handle); _cuda(x_prompt, kv_start, edit_region, gt_labels, tokens_out)
+                 tokens_out: torch.Tensor, top_p: float = 1.0) -> None:
+    e = _eng(handle); _cuda(x_prompt, kv_start, edit_region, gt_labels, tokens_out); _top_p(top_p)
     R, P = x_prompt.shape[0], x_prompt.shape[1]
     _lib.check(e._lib.pg_sample_image(e._h, _p(x_prompt), _p(kv_start), R, P, int(n_steps), float(cfg_weight), float(temperature),
-                                      int(seed) & 0xFFFFFFFFFFFFFFFF, int(greedy), int(top_k), _p(edit_region), _p(gt_labels), _p(tokens_out), _st(x_prompt)))
+                                      int(seed) & 0xFFFFFFFFFFFFFFFF, int(greedy), int(top_k), float(top_p), _p(edit_region), _p(gt_labels), _p(tokens_out), _st(x_prompt)))
 
 
 @torch.library.custom_op(f"{NS}::vq_decode_code", mutates_args=("image_out",), device_types="cuda")

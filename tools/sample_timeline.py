@@ -1,4 +1,5 @@
-"""In-kernel timeline of the fused CFG + softmax + multinomial + embed kernel inside the decode graph."""
+"""In-kernel timeline of the fused CFG + softmax + multinomial + embed kernel inside the decode graph.
+PG_TOP_P (default 1.0 = off) sets the sampler's top-p."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -13,7 +14,7 @@ ids, mask = synthetic.collate_cfg_batch(cond, neg, dims.pad_id, dims.n_img_token
 emb = eng.language_model.get_input_embeddings()(ids.to(dev))
 dbg = torch.zeros(256 * 16, dtype=torch.int64, device=dev)
 eng.set_option("sample_dbg_ptr", dbg.data_ptr())
-eng.sample_image(emb, B, 40, mask.to(dev), 5.0, 1.0, generator=0)
+eng.sample_image(emb, B, 40, mask.to(dev), 5.0, 1.0, generator=0, top_p=float(os.environ.get("PG_TOP_P", "1.0")))
 torch.cuda.synchronize()
 eng.set_option("sample_dbg_ptr", 0)
 t = dbg.cpu().numpy().reshape(-1, 16).astype(np.float64)

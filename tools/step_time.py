@@ -1,4 +1,6 @@
-"""Decode-loop timing sweeps over engine options (one engine, graph re-captured per setting)."""
+"""Decode-loop timing sweeps over engine options (one engine, graph re-captured per setting).
+
+PG_TOP_P=1.0,0.9 times the sampler's top-p settings instead, alternated three times in this one process."""
 import os
 import sys
 
@@ -21,21 +23,27 @@ st = torch.cuda.current_stream(dev)
 DEFAULTS = {"use_pdl": 1, "use_graph": 1, "use_tc": 1, "attn_impl": 3, "attn_trigger": 1, "attn_attr": 1}
 
 
-def loop_ms(n=576):
+def loop_ms(n=576, top_p=1.0):
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
-    eng.sample_image(emb, B, n, mask, 5.0, 1.0, generator=0)       # warm (captures the graph)
-    eng.sample_image(emb, B, 1, mask, 5.0, 1.0, generator=0)       # warm the 1-token path too (its first run is ~90 ms slower,
-    torch.cuda.synchronize()                                        # which used to deflate the first ms/step figure by 0.16 ms)
+    eng.sample_image(emb, B, n, mask, 5.0, 1.0, generator=0, top_p=top_p)   # warm (captures the graph)
+    eng.sample_image(emb, B, 1, mask, 5.0, 1.0, generator=0, top_p=top_p)   # warm the 1-token path too (its first run is
+    torch.cuda.synchronize()                                        # ~90 ms slower, which used to deflate the first ms/step by 0.16 ms)
     ev[0].record(st)
-    eng.sample_image(emb, B, 1, mask, 5.0, 1.0, generator=0)
+    eng.sample_image(emb, B, 1, mask, 5.0, 1.0, generator=0, top_p=top_p)
     ev[1].record(st)
-    eng.sample_image(emb, B, n, mask, 5.0, 1.0, generator=0)
+    eng.sample_image(emb, B, n, mask, 5.0, 1.0, generator=0, top_p=top_p)
     ev[2].record(st)
     torch.cuda.synchronize()
     pre = ev[0].elapsed_time(ev[1])
     return round(pre, 2), round((ev[1].elapsed_time(ev[2]) - pre) / (n - 1), 4)
 
 
+top_ps = [float(x) for x in os.environ.get("PG_TOP_P", "").split(",") if x]
+if top_ps:
+    for rep in range(3):
+        for p in top_ps:
+            print(f"top_p={p} (prefill ms, ms/decode step)", loop_ms(top_p=p), flush=True)
+    sys.exit(0)
 sweeps = [s for s in os.environ.get("PG_SWEEP", "").split(";") if s]
 print("baseline (prefill ms, ms/decode step)", loop_ms(), flush=True)
 for s in sweeps:
