@@ -7,8 +7,8 @@
 //   P   = online softmax of S, one thread per query row (= TMEM lane): two passes over the row with tcgen05.ld
 //         (masked max, then exp2 + running sum), written as bf16 into shared memory in the K-major swizzled
 //         image the second MMA reads as its A operand
-//   O_b = P V_blk        tcgen05.mma 128x128x128 into TMEM columns 128..255; V comes from a key-contiguous
-//         (transposed) copy the prefill writes next to the cache, so both operands are K-major
+//   O_b = P V_blk        tcgen05.mma 128x128x128 into TMEM columns 128..255; V is read straight from the cache rows
+//         ([key][dim], dims contiguous) as an MN-major B operand
 //   O   = O * exp(m_old - m_new) + O_b   in registers (128 fp32 per thread)
 // Rounding points of the reference under autocast: scores are a bf16 matmul output, scaled in bf16; softmax in
 // fp32; probabilities enter the second matmul as bf16.  (The probabilities here are rounded before the final
@@ -23,41 +23,15 @@ constexpr int PA_BK = 128;                     // keys per block (MMA N of the f
 constexpr int PA_TILE = 128 * 64 * 2;          // one [128 rows][64 bf16] swizzled tile = 16 KB
 constexpr int PA_SMEM = 6 * PA_TILE + 1024 + 64;   // Q, K (later P), V: two tiles each; 97 KB -> two CTAs per SM
 
-// V [r][h][key][128] (cache layout) -> vT [r][h][128][Ppad] (keys contiguous) for keys < P
-__global__ void __launch_bounds__(256)
-v_transpose_kernel(const bf16* __restrict__ vcache, bf16* __restrict__ vT, int P, int Ppad, int H, int Tmax) {
-  __shared__ bf16 tile[64][HEAD_DIM + 2];
-  pdl_launch_dependents();
-  pdl_wait();
-  const int k0 = blockIdx.x * 64, h = blockIdx.y, r = blockIdx.z;
-  const bf16* src = vcache + (((size_t)r * H + h) * Tmax + k0) * HEAD_DIM;
-  for (int i = threadIdx.x; i < 64 * HEAD_DIM / 2; i += 256) {
-    const int kk = i / (HEAD_DIM / 2), d2 = i % (HEAD_DIM / 2);
-    __nv_bfloat162 v = __floats2bfloat162_rn(0.f, 0.f);
-    if (k0 + kk < P) v = *reinterpret_cast<const __nv_bfloat162*>(src + (size_t)kk * HEAD_DIM + 2 * d2);
-    tile[kk][2 * d2] = v.x; tile[kk][2 * d2 + 1] = v.y;
-  }
-  __syncthreads();
-  bf16* dst = vT + ((size_t)r * H + h) * HEAD_DIM * Ppad + k0;
-  for (int i = threadIdx.x; i < HEAD_DIM * 32; i += 256) {
-    const int d = i >> 5, k2 = i & 31;
-    if (k0 + 2 * k2 < Ppad) {
-      __nv_bfloat162 v; v.x = tile[2 * k2][d]; v.y = tile[2 * k2 + 1][d];
-      *reinterpret_cast<__nv_bfloat162*>(dst + (size_t)d * Ppad + 2 * k2) = v;
-    }
-  }
-}
-
 __global__ void __launch_bounds__(128, 2)
 attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
-                       const __grid_constant__ CUtensorMap map_vt, const int32_t* __restrict__ kv_start,
-                       bf16* __restrict__ out, int P, int H, int Tmax, float scale, const int32_t* __restrict__ row_off,
-                       int v_direct) {
+                       const __grid_constant__ CUtensorMap map_v, const int32_t* __restrict__ kv_start,
+                       bf16* __restrict__ out, int P, int H, int Tmax, float scale, const int32_t* __restrict__ row_off) {
   extern __shared__ uint8_t pa_smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)pa_smem_raw + 1023) & ~(uintptr_t)1023);
   uint8_t* sQ = smem;                      // 2 tiles: dims 0-63 | 64-127 of the 128 queries
   uint8_t* sK = smem + 2 * PA_TILE;        // 2 tiles: dims 0-63 | 64-127 of the 128 keys
-  uint8_t* sV = smem + 4 * PA_TILE;        // 2 tiles: keys 0-63 | 64-127 of the 128 dims (V^T)
+  uint8_t* sV = smem + 4 * PA_TILE;        // 2 tiles: dims 0-63 | 64-127 of the 128 keys
   uint8_t* sP = sK;                        // probabilities (2 tiles: keys 0-63 | 64-127 of the 128 queries) overwrite the K tiles:
                                            // every thread has waited for S = Q K^T before it writes P, and the next K load is
                                            // issued only after O_b = P V has completed
@@ -74,7 +48,7 @@ attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_c
   // written before the first prefill kernel is launched, so reading it ahead of the dependency wait is safe.
   if (row_off != nullptr && row_off[r + 1] == row_off[r]) return;
   if (tid == 0) {
-    tma_prefetch_desc(&map_q); tma_prefetch_desc(&map_k); tma_prefetch_desc(&map_vt);
+    tma_prefetch_desc(&map_q); tma_prefetch_desc(&map_k); tma_prefetch_desc(&map_v);
     mbar_init(bar_load, 1); mbar_init(bar_mma, 1);
     mbar_fence_init();
   }
@@ -117,14 +91,9 @@ attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_c
         const int krow = (r * H + h) * Tmax + key0;
         tma_load_2d(sK, &map_k, bar_load, 0, krow, pol);
         tma_load_2d(sK + PA_TILE, &map_k, bar_load, 64, krow, pol);
-        if (v_direct) {          // V rows of the cache, [128 keys][64 dims] per tile: dims 0-63 | 64-127 (MN-major B operand)
-          tma_load_2d(sV, &map_vt, bar_load, 0, krow, pol);
-          tma_load_2d(sV + PA_TILE, &map_vt, bar_load, 64, krow, pol);
-        } else {                 // key-contiguous copy, [128 dims][64 keys] per tile: keys 0-63 | 64-127
-          const int vrow = (r * H + h) * HEAD_DIM;
-          tma_load_2d(sV, &map_vt, bar_load, key0, vrow, pol);
-          tma_load_2d(sV + PA_TILE, &map_vt, bar_load, key0 + 64, vrow, pol);
-        }
+        // V rows of the cache, [128 keys][64 dims] per tile: dims 0-63 | 64-127 (MN-major B operand)
+        tma_load_2d(sV, &map_v, bar_load, 0, krow, pol);
+        tma_load_2d(sV + PA_TILE, &map_v, bar_load, 64, krow, pol);
         mbar_wait(bar_load, (uint32_t)(it & 1), 50);
         tc_fence_after();
         // S = Q K^T : 8 K-steps of 16 dims over the two dim tiles
@@ -197,9 +166,8 @@ attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_c
         for (int kk = 0; kk < 8; ++kk) {
           const uint64_t da = umma_desc_k_sw128(smem_u32(sP + (kk >> 2) * PA_TILE)) + (uint64_t)(2 * (kk & 3));
           // MN-major V: 16 keys = 2048 bytes down each [keys][64 dims] tile, the second 64 dims one tile further
-          const uint64_t db = v_direct ? umma_desc_mn_sw128(smem_u32(sV) + (uint32_t)kk * 2048u, (uint32_t)PA_TILE)
-                                       : umma_desc_k_sw128(smem_u32(sV + (kk >> 2) * PA_TILE)) + (uint64_t)(2 * (kk & 3));
-          umma_bf16(tmem_base + 128u, da, db, v_direct ? umma_idesc_bf16_bmn(PA_BQ, HEAD_DIM) : idesc, kk != 0);
+          const uint64_t db = umma_desc_mn_sw128(smem_u32(sV) + (uint32_t)kk * 2048u, (uint32_t)PA_TILE);
+          umma_bf16(tmem_base + 128u, da, db, umma_idesc_bf16_bmn(PA_BQ, HEAD_DIM), kk != 0);
         }
         umma_commit(bar_mma);
       }
@@ -214,7 +182,7 @@ attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_c
         for (int j = 0; j < 64; ++j) o[c0 + j] = o[c0 + j] * alpha + __uint_as_float(v[j]);
       }
       tc_fence_before();
-      __syncthreads();          // next block: TMA overwrites K / V^T, the first MMA overwrites S
+      __syncthreads();          // next block: TMA overwrites K / V, the first MMA overwrites S
     }
   }
   if (q < P && (row_off == nullptr || q >= start)) {

@@ -78,14 +78,12 @@ struct pg_engine {
   std::unordered_map<const void*, Tiled> tiled;      // row-major weight -> engine-owned tile-major copy (bf16 mode)
   uint8_t* tiled_buf = nullptr;
   int prefill_attn_tc = 1;                   // prompt-prefill attention on tcgen05 (attn_prefill_tc.cuh); 0 = CUDA-core kernel
-  void* vT = nullptr;                        // [R][H][128][Ppad] key-contiguous copy of V for the prefill attention
-  int norm_tma = 3;      // bit 0: decode-step norms through the TMA-staged kernel, bit 1: prefill norms too
-  int use_tiled = 1, use_implicit_conv = 1, tc_wide_stages = 2, fuse_conv_epilogue = 1;   // conv bias / residual / bf16 store in the contraction epilogue
+  int tc_wide_stages = 2, fuse_conv_epilogue = 1;   // conv bias / residual / bf16 store in the contraction epilogue
   EncodeTiledFn encode = nullptr;
   // options
   uint64_t attn_dbg_ptr = 0;
   int64_t attn_test_flags = 0;
-  int use_tc = 1, use_pdl = 1, use_graph = 1, attn_impl = 3, attn_ctas = 0, attn_trigger = 1, attn_attr = 1, fuse_swiglu = 1, tc_stages = 0, tc_stages_gu = 0, vq_chunk = 0, attn_splits = 0, gemm_splits = 0;
+  int use_tc = 1, use_pdl = 1, use_graph = 1, attn_impl = 3, attn_ctas = 0, tc_stages = 0, tc_stages_gu = 0, vq_chunk = 0, attn_splits = 0, gemm_splits = 0;
   float* dbg_logits = nullptr;
   float* dbg_text_logits = nullptr;
   unsigned long long* prof_buf = nullptr;   // per-kernel timeline of ONE decode step (plain-launch mode)
@@ -105,10 +103,10 @@ struct pg_engine {
   // mmu front-end (SigLIP tower + aligner + scatter, vit_kernels.cuh); carved only when dims.sig_layers > 0
   int sig_chunk = 0, sig_np = 0;                      // images per pass, patches per image
   float *sig_x = nullptr, *sig_part = nullptr;
-  void *sig_xn = nullptr, *sig_qkv = nullptr, *sig_vT = nullptr, *sig_attn = nullptr, *sig_h = nullptr, *sig_feat = nullptr;
+  void *sig_xn = nullptr, *sig_qkv = nullptr, *sig_attn = nullptr, *sig_h = nullptr, *sig_feat = nullptr;
   size_t sig_part_bytes = 0;
   int32_t *sig_rank_dst = nullptr, *sig_inv_src = nullptr, *sig_counts = nullptr;
-  int use_tc2 = 1, tc2_stages = 4;                    // wide-tile contractions on CTA pairs (gemm_tc2.cuh, tcgen05 cta_group::2)
+  int tc2_stages = 4;                                 // wide-tile contractions on CTA pairs (gemm_tc2.cuh, tcgen05 cta_group::2)
   int stage_cap_once = 0, down_stages = 4;            // ring cap of the next launch_tc; decode down projection (see decode_layers)
   int tc_stages_k = 0;
   int tc_stages_n = 0;                                // tc_stages applies to contractions with this N only (0 = all)
@@ -119,17 +117,11 @@ struct pg_engine {
   unsigned long long* row_hash = nullptr; unsigned long long* row_hash_host = nullptr;   // content hash per prompt row (device / pinned)
   int prefill_pack = 1;                               // fused loops prefill the real tokens only (lm_kernels.cuh packed_row_of)
   float* xpack = nullptr; float* x_last = nullptr; int32_t* row_off = nullptr; int32_t* row_off_host = nullptr;
-  int prefill_fuse = 1;                               // prefill contractions with bf16 / residual epilogues (gemm.cuh EpiFuse) instead of fp32 partials
   int gu_streamk = 1;                                 // decode gate|up + SwiGLU as a stream-K launch over all SMs (gemm_sk.cuh)
   int* sk_counters = nullptr;
   int prefill_qkv_fuse = 1;                           // prefill QKV: RoPE + q / cache stores in the CTA-pair contraction's epilogue
   QkvEpi qkv_epi_next = {};                           // consumed (and cleared) by the next CTA-pair launch
-  int prefill_swiglu_fuse = 1;                        // prefill gate|up: SwiGLU in the CTA-pair contraction's epilogue
-  int norm_warp = 1;                                  // prefill RMSNorm: one warp per row (lm_kernels.cuh rmsnorm_rows_warp_kernel)
-  int prefill_v_direct = 1;                           // prefill attention reads V from the cache rows (MN-major operand), no transposed copy
-  int sig_v_direct = 1;                               // ViT attention reads V in place (MN-major operand) instead of a transposed copy
   int sig_attn_tc = 1;                                // tcgen05 attention (bf16, head_dim 64); 0 = CUDA-core kernel
-  int sig_fuse = 1;                                   // bias / GELU / residual in the contraction epilogues (gemm.cuh EpiFuse)
   size_t part_bytes = 0;
   int *attn_cnt = nullptr, *attn_flag = nullptr, *step_ctr = nullptr, *greedy_state = nullptr;
   int* poll_host = nullptr;                          // pinned: early-exit poll of the greedy loop
@@ -238,7 +230,7 @@ constexpr int CONV_NT = 192;
 static int run_conv_gemm(pg_engine* e, const void* act, const void* Wc, int B, int H, int W, int Cin, int Cout, float* C,
                          size_t c_bytes, cudaStream_t st, int* taken, const EpiFuse* epi = nullptr) {
   *taken = 0;
-  if (!e->bf16 || !e->use_tc || !e->use_implicit_conv || Cin % TC_BK != 0) return 0;
+  if (!e->bf16 || !e->use_tc || Cin % TC_BK != 0) return 0;
   if ((((uintptr_t)act) & 15) || (((uintptr_t)Wc) & 15)) return 0;
   int bw = 0;
   if (W <= CONV_NT && CONV_NT % W == 0) bw = W;
@@ -301,13 +293,13 @@ static int run_gemm(pg_engine* e, const void* X, const void* W, int M, int N, in
     const int kb_per_split = (num_kb + want - 1) / want;
     splits = (num_kb + kb_per_split - 1) / kb_per_split;
     if ((size_t)splits * M * N * 4 > c_bytes) return fail("GEMM partial buffer too small (%d x %d x %d)", splits, M, N);
-    if (!w_tiled && w_const && e->use_tiled) {             // stream the tile-major copy when the weight has one
+    if (!w_tiled && w_const) {                             // stream the tile-major copy when the weight has one
       auto it = e->tiled.find(W);
       if (it != e->tiled.end() && it->second.N == N && it->second.K == K) w_tiled = it->second.ptr;
     }
     CUtensorMap mw, mx;
     TRY(make_map_2d(e, &mw, W, (uint64_t)N, (uint64_t)K, TC_BM));
-    if (e->use_tc2 && NT == 256 && splits == 1 && !swiglu_out && N > TC_BM) {
+    if (NT == 256 && splits == 1 && !swiglu_out && N > TC_BM) {
       // tensor-bound shape: CTA pairs, one 256 x 256 x 16 MMA per pair and k-step (gemm_tc2.cuh)
       TRY(make_map_2d(e, &mx, X, (uint64_t)M, (uint64_t)K, (uint32_t)(TC2_NT / 2)));
       EpiFuse ep2 = {};
@@ -391,7 +383,6 @@ static void layout_workspace(pg_engine* e, Carve& c) {
   e->step_ctr = (int*)c.take(256);
   e->sk_counters = (int*)c.take((size_t)((2 * d.F + TC_BM - 1) / TC_BM) * 4);
   e->greedy_state = (int*)c.take(256 + R * 4);      // [0] rows unfinished, [1] steps generated, [64..] per-row flags
-  e->vT = c.take(R * d.H * HEAD_DIM * align_up((size_t)std::max(d.max_prompt, 1), 64) * 2);
   e->embed_table = c.take((size_t)d.img_vocab * d.D * es);
   e->align_tmp = c.take((size_t)d.img_vocab * d.D * es);
   {
@@ -410,7 +401,6 @@ static void layout_workspace(pg_engine* e, Carve& c) {
     e->sig_x = (float*)c.take(Mc * W * 4);
     e->sig_xn = c.take(Mc * std::max(W, Kp) * es);
     e->sig_qkv = c.take(Mc * 3 * W * es);
-    e->sig_vT = c.take((size_t)e->sig_chunk * W * align_up((size_t)e->sig_np, 8) * 2);
     e->sig_attn = c.take(Mc * W * es);
     e->sig_h = c.take(Mc * std::max<size_t>(d.sig_mlp, d.D) * es);
     e->sig_part_bytes = Mc * widest * 4;
@@ -589,27 +579,17 @@ extern "C" int pg_engine_set_option(pg_engine* e, const char* key, int64_t value
   else if (k == "vq_chunk") e->vq_chunk = (int)value;
   else if (k == "attn_splits") e->attn_splits = (int)value;
   else if (k == "attn_impl") e->attn_impl = (int)value;
-  else if (k == "use_tiled") e->use_tiled = (int)value;
-  else if (k == "norm_tma") e->norm_tma = (int)value;
   else if (k == "prefill_attn_tc") e->prefill_attn_tc = (int)value;
   else if (k == "sig_attn_tc") e->sig_attn_tc = (int)value;
-  else if (k == "sig_v_direct") e->sig_v_direct = (int)value;
-  else if (k == "prefill_v_direct") e->prefill_v_direct = (int)value;
-  else if (k == "norm_warp") e->norm_warp = (int)value;
-  else if (k == "prefill_swiglu_fuse") e->prefill_swiglu_fuse = (int)value;
   else if (k == "prefill_qkv_fuse") e->prefill_qkv_fuse = (int)value;
   else if (k == "gu_streamk") e->gu_streamk = (int)value;
-  else if (k == "prefill_fuse") e->prefill_fuse = (int)value;
   else if (k == "prefill_pack") e->prefill_pack = (int)value;
   else if (k == "prefill_dedup") e->prefill_dedup = (int)value;
   else if (k == "attn_alias") e->attn_alias = (int)value;
   else if (k == "attn_test_alias_p") e->attn_test_alias_p = (int)value;
-  else if (k == "use_tc2") e->use_tc2 = (int)value;
   else if (k == "tc2_stages") e->tc2_stages = std::max(2, std::min(4, (int)value));
-  else if (k == "sig_fuse") e->sig_fuse = (int)value;
   else if (k == "fuse_conv_epilogue") e->fuse_conv_epilogue = (int)value;
   else if (k == "tc_wide_stages") e->tc_wide_stages = std::max(2, (int)value);
-  else if (k == "use_implicit_conv") e->use_implicit_conv = (int)value;
   else if (k == "attn_dbg_ptr") e->attn_dbg_ptr = (uint64_t)value;
   else if (k == "gemm_dbg_ptr") { unsigned long long* p = (unsigned long long*)value; CK(cudaMemcpyToSymbol(g_gemm_dbg, &p, sizeof(p))); }
   else if (k == "sample_dbg_ptr") { unsigned long long* p = (unsigned long long*)value; CK(cudaMemcpyToSymbol(g_sample_dbg, &p, sizeof(p))); }
@@ -618,9 +598,6 @@ extern "C" int pg_engine_set_option(pg_engine* e, const char* key, int64_t value
   else if (k == "gemm_dbg_n") { int n = (int)value; CK(cudaMemcpyToSymbol(g_gemm_dbg_n, &n, sizeof(n))); }
   else if (k == "attn_test_flags") e->attn_test_flags = value;
   else if (k == "attn_ctas") e->attn_ctas = (int)value;
-  else if (k == "attn_trigger") e->attn_trigger = (int)value;
-  else if (k == "fuse_swiglu") e->fuse_swiglu = (int)value;
-  else if (k == "attn_attr") e->attn_attr = (int)value;
   else if (k == "gemm_splits") e->gemm_splits = (int)value;
   else if (k == "dbg_logits_ptr") e->dbg_logits = (float*)(uintptr_t)value;
   else if (k == "dbg_text_logits_ptr") e->dbg_text_logits = (float*)(uintptr_t)value;   // [max_new][R][vocab] fp32
@@ -654,10 +631,10 @@ extern "C" int pg_engine_get_counter(const pg_engine* e, const char* key, int64_
 static int k_resid_norm(pg_engine* e, float* x, const float* part, int S, size_t sstride, const float* w, void* xn,
                         float* y, int rows, int in_stride, int in_off, int flags, cudaStream_t st) {
   const int D = e->d.D;
-  // decode steps: slabs + residual row through TMA bulk copies into shared memory (bit-identical, see lm_kernels.cuh)
+  // split-K slabs + residual row through TMA bulk copies into shared memory (bit-identical, see lm_kernels.cuh)
   const size_t tma_smem = (size_t)(S + 1) * D * 4 + 128;
   const int tma_threads = std::min(RN_THREADS, std::max(128, (D / 4 + 31) / 32 * 32));   // one element quad per thread
-  if (e->norm_tma && part != nullptr && in_stride == 1 && in_off == 0 && (rows <= 256 || (e->norm_tma & 2)) && D % 4 == 0 &&
+  if (part != nullptr && in_stride == 1 && in_off == 0 && D % 4 == 0 &&
       D <= RN_MAX_PER_THREAD * tma_threads && tma_smem <= 200 * 1024 && (sstride * 4) % 16 == 0 &&
       (((uintptr_t)part | (uintptr_t)x) & 15) == 0) {
     DISPATCH_T(e,
@@ -668,7 +645,7 @@ static int k_resid_norm(pg_engine* e, float* x, const float* part, int S, size_t
     return 0;
   }
   // prefill with fused epilogues: plain RMSNorm of thousands of rows to bf16 - one warp per row (lm_kernels.cuh)
-  if (e->bf16 && e->norm_warp && part == nullptr && y == nullptr && xn != nullptr && in_stride == 1 && in_off == 0 && flags == 0 &&
+  if (e->bf16 && part == nullptr && y == nullptr && xn != nullptr && in_stride == 1 && in_off == 0 && flags == 0 &&
       rows > 256 && D % 128 == 0 && (((uintptr_t)x | (uintptr_t)xn | (uintptr_t)w) & 15) == 0) {
     const dim3 grid((rows + 7) / 8);
     if (D == 2048) return launch(e, rmsnorm_rows_warp_kernel<16>, grid, dim3(256), 0, st, (const float*)x, w, (bf16*)xn, rows, D, e->d.rms_eps);
@@ -744,7 +721,6 @@ extern "C" int pg_engine_finalize(pg_engine* e, void* stream) {
   CK(cudaMemsetAsync(e->attn_ll, 0, (size_t)d.max_rows * d.H * 64 * (HEAD_DIM + 2) * 8, st));
   CK(cudaMemsetAsync(e->step_ctr, 0, 256, st));
   CK(cudaMemsetAsync(e->sk_counters, 0, (size_t)((2 * d.F + TC_BM - 1) / TC_BM) * 4, st));
-  CK(cudaMemsetAsync(e->vT, 0, (size_t)d.max_rows * d.H * HEAD_DIM * align_up((size_t)std::max(d.max_prompt, 1), 64) * 2, st));   // must stay finite
   if (e->bf16 && !e->tiled_buf) {
     // tile-major copies of the weights that are streamed once per step (see tile_weight_kernel)
     struct Item { const void* w; int N, K; };
@@ -796,7 +772,7 @@ static int elementwise_blocks(pg_engine* e, size_t total) {
 // gate|up projection + SwiGLU -> hbuf.  bf16 + tcgen05: one kernel (fused epilogue, interleaved weight rows);
 // otherwise the contraction followed by swiglu_kernel.
 // (decode-sized token counts only: with 256-token tiles the two gate warps' expf work would outlast the MMAs)
-static bool fused_swiglu_ok(const pg_engine* e, int tok) { return e->bf16 && e->use_tc && e->fuse_swiglu && e->d.F % 64 == 0 && tok <= 128; }
+static bool fused_swiglu_ok(const pg_engine* e, int tok) { return e->bf16 && e->use_tc && e->d.F % 64 == 0 && tok <= 128; }
 static int k_gate_up(pg_engine* e, const LayerW& w, int tok, cudaStream_t st) {
   const pg_dims& d = e->d;
   const int F = d.F, D = d.D;
@@ -805,7 +781,7 @@ static int k_gate_up(pg_engine* e, const LayerW& w, int tok, cudaStream_t st) {
   // 172 tiles on 148 SMs; measured 4.17 -> 3.98 ms per step at B=16).  With fewer tiles than SMs (Janus-1.3B: 88) the
   // plain launch is faster (1.49 vs 1.58 ms per step): the SMs it leaves free are not idle, they host the early-launched
   // CTAs of the down projection prefetching their weights.  gu_streamk = 2 forces it.
-  if (fused_swiglu_ok(e, tok) && tok <= 64 && D % TC_BK == 0 && e->use_tiled &&
+  if (fused_swiglu_ok(e, tok) && tok <= 64 && D % TC_BK == 0 &&
       (e->gu_streamk == 2 || (e->gu_streamk == 1 && 2 * F / TC_BM > e->num_sms))) {
     auto it = e->tiled.find(w.wgu);
     if (it != e->tiled.end() && it->second.N == 2 * F && it->second.K == D) {
@@ -878,7 +854,7 @@ static int prefill_impl(pg_engine* e, float* x, const int32_t* kv_start, int R, 
   // ---- packed prefill (fused loops only: the drop-in call returns every position, pads included)
   const int32_t* row_off = nullptr;
   int packed_dups = 0;
-  if (!all_positions && e->bf16 && e->use_tc && e->prefill_attn_tc && e->prefill_fuse && e->prefill_pack && D % 8 == 0 && HD % 8 == 0 &&
+  if (!all_positions && e->bf16 && e->use_tc && e->prefill_attn_tc && e->prefill_pack && D % 8 == 0 && HD % 8 == 0 &&
       F % 64 == 0) {
     if (!e->row_off_host) CK(cudaMallocHost(&e->row_off_host, (size_t)(3 * d.max_rows + 2) * 4));
     if (!e->row_hash_host) CK(cudaMallocHost(&e->row_hash_host, (size_t)d.max_rows * 8));
@@ -938,14 +914,14 @@ static int prefill_impl(pg_engine* e, float* x, const int32_t* kv_start, int R, 
   }
   // fused epilogues (bf16 regime on tcgen05): QKV and gate|up leave the contraction as bf16 rows, O and down add straight
   // into the fp32 residual stream - no fp32 partial round trip (same values: the row kernels rounded the partials first)
-  const bool fuse = e->bf16 && e->use_tc && e->prefill_fuse && D % 8 == 0 && HD % 8 == 0 && F % 64 == 0 &&
+  const bool fuse = e->bf16 && e->use_tc && D % 8 == 0 && HD % 8 == 0 && F % 64 == 0 &&
                     (size_t)tok * std::max(3 * HD, 2 * F) * 2 <= e->part_bytes;
   bf16* stage16 = (bf16*)e->part;
   for (int l = 0; l < d.L; ++l) {
     LayerW w;
     TRY(layer_weights(e, l, &w));
     if (l == 0) TRY(k_resid_norm(e, x, nullptr, 0, 0, w.ln1, e->xn, nullptr, tok, 1, 0, 0, st));
-    if (fuse && e->prefill_qkv_fuse && e->use_tc2 && tok > 128) {
+    if (fuse && e->prefill_qkv_fuse && tok > 128) {
       // RoPE + q / K / V stores in the contraction's epilogue (gemm.cuh QkvEpi)
       EpiFuse ep = {nullptr, (bf16*)e->qbuf, nullptr, 3};
       e->qkv_epi_next = QkvEpi{cosT, sinT, (bf16*)e->qbuf, (bf16*)kv_ptr(e, l, 0, R), (bf16*)kv_ptr(e, l, 1, R), row_off, kv_start,
@@ -970,20 +946,12 @@ static int prefill_impl(pg_engine* e, float* x, const int32_t* kv_start, int R, 
     }
     if (e->bf16 && e->use_tc && e->prefill_attn_tc) {
       // tensor-core path: one CTA per (row, head, 128-query tile); V is read from the cache rows as an MN-major operand
-      // (prefill_v_direct = 0: from a key-contiguous copy made first)
-      const int Ppad = (int)align_up((size_t)P, 64);
       CUtensorMap mq, mk, mv;
       TRY(make_map_2d(e, &mq, e->qbuf, (uint64_t)tok, (uint64_t)HD, PA_BQ));
       TRY(make_map_2d(e, &mk, kv_ptr(e, l, 0, R), (uint64_t)R * d.H * e->Tmax, (uint64_t)HEAD_DIM, PA_BK));
-      if (e->prefill_v_direct) {
-        TRY(make_map_2d(e, &mv, kv_ptr(e, l, 1, R), (uint64_t)R * d.H * e->Tmax, (uint64_t)HEAD_DIM, PA_BK));
-      } else {
-        TRY(launch(e, v_transpose_kernel, dim3(Ppad / 64, d.H, R), dim3(256), 0, st, (const bf16*)kv_ptr(e, l, 1, R), (bf16*)e->vT, P, Ppad,
-                   d.H, e->Tmax));
-        TRY(make_map_2d(e, &mv, e->vT, (uint64_t)R * d.H * HEAD_DIM, (uint64_t)Ppad, HEAD_DIM));
-      }
+      TRY(make_map_2d(e, &mv, kv_ptr(e, l, 1, R), (uint64_t)R * d.H * e->Tmax, (uint64_t)HEAD_DIM, PA_BK));
       TRY(launch(e, attn_prefill_tc_kernel, dim3((P + PA_BQ - 1) / PA_BQ, d.H, R), dim3(128), PA_SMEM, st, mq, mk, mv, kv_start,
-                 (bf16*)e->attn_out, P, d.H, e->Tmax, scale, row_off, e->prefill_v_direct));
+                 (bf16*)e->attn_out, P, d.H, e->Tmax, scale, row_off));
     } else
     DISPATCH_T(e,
                launch(e, attn_prefill_kernel<bf16>, dim3((P + 63) / 64, d.H, R), dim3(256), ATTN_PREFILL_SMEM, st,
@@ -999,16 +967,9 @@ static int prefill_impl(pg_engine* e, float* x, const int32_t* kv_start, int R, 
       if (fused_swiglu_ok(e, tok)) {
         TRY(k_gate_up(e, w, tok, st));
       } else {
-        if (e->prefill_swiglu_fuse && e->use_tc2 && tok > 128 && (2 * F) % TC_BM == 0) {
-          // SwiGLU in the CTA-pair contraction's epilogue (gemm_tc2.cuh, EpiFuse::gelu == 2): h leaves the kernel directly
-          EpiFuse eg = {nullptr, (bf16*)e->hbuf, nullptr, 2};
-          TRY(run_gemm(e, e->xn, w.wgu, tok, 2 * F, D, e->part, e->part_bytes, &S, st, -1, 0, true, nullptr, nullptr, &eg));
-        } else {
-        EpiFuse eg = {nullptr, stage16, nullptr, 0};
+        // SwiGLU in the CTA-pair contraction's epilogue (gemm_tc2.cuh, EpiFuse::gelu == 2): h leaves the kernel directly
+        EpiFuse eg = {nullptr, (bf16*)e->hbuf, nullptr, 2};
         TRY(run_gemm(e, e->xn, w.wgu, tok, 2 * F, D, e->part, e->part_bytes, &S, st, -1, 0, true, nullptr, nullptr, &eg));
-        const size_t total8 = (size_t)tok * F / 8;
-        TRY(launch(e, swiglu_bf16_kernel, dim3(elementwise_blocks(e, total8)), dim3(256), 0, st, (const bf16*)stage16, (bf16*)e->hbuf, F, total8));
-        }
       }
       TRY(run_gemm(e, e->hbuf, w.wd, tok, D, F, e->part, e->part_bytes, &S, st, -1, 0, true, nullptr, nullptr, &er));
       if (l + 1 < d.L) {
@@ -1079,14 +1040,10 @@ static int decode_layers(pg_engine* e, const int32_t* kv_start, int R, int pos_b
     TRY(run_gemm(e, e->xn, w.wqkv, R, 3 * HD, D, e->part, e->part_bytes, &S, st));
     if (e->bf16 && e->attn_impl >= 1 && R <= AT_MAX_ROWS) {
       const int ctas = e->attn_ctas > 0 ? e->attn_ctas : e->num_sms;
-      const int saved = e->use_pdl;
-      if (!e->attn_attr) e->use_pdl = 0;
-      int rc = launch(e, attn_decode_v5_kernel, dim3(ctas), dim3(AT_THREADS), A5_SMEM, st, e->part, S, (size_t)R * 3 * HD, cosT, sinT,
-                      (bf16*)kv_ptr(e, l, 0, R), (bf16*)kv_ptr(e, l, 1, R), kv_start, (bf16*)e->attn_out, e->attn_ll,
-                      R, d.H, e->Tmax, pos_base, step_ptr, scale, trig, e->attn_trigger, next_prof(e), (unsigned long long*)nullptr,
-                      (const int32_t*)((alias_P > 0 && e->attn_alias) ? e->dup_of : nullptr), alias_P);
-      e->use_pdl = saved;
-      TRY(rc);
+      TRY(launch(e, attn_decode_v5_kernel, dim3(ctas), dim3(AT_THREADS), A5_SMEM, st, e->part, S, (size_t)R * 3 * HD, cosT, sinT,
+                 (bf16*)kv_ptr(e, l, 0, R), (bf16*)kv_ptr(e, l, 1, R), kv_start, (bf16*)e->attn_out, e->attn_ll,
+                 R, d.H, e->Tmax, pos_base, step_ptr, scale, trig, 1, next_prof(e), (unsigned long long*)nullptr,
+                 (const int32_t*)((alias_P > 0 && e->attn_alias) ? e->dup_of : nullptr), alias_P));
     } else {
     DISPATCH_T(e,
                  launch(e, attn_decode_kernel<bf16>, dim3(d.H, R, nsp), dim3(128), 0, st, e->part, S, (size_t)R * 3 * HD, cosT, sinT,
@@ -1486,7 +1443,7 @@ static int sig_tower(pg_engine* e, const float* pixel, int n, void* feat, cudaSt
     return 0;
   };
   const bool tc_attn = e->bf16 && e->use_tc && e->sig_attn_tc && hd == VT_HD;
-  const bool fuse = e->bf16 && e->use_tc && e->sig_fuse;
+  const bool fuse = e->bf16 && e->use_tc;
   // contraction + bias (+ GELU) -> T, or contraction + bias + residual add; fused into the tcgen05 epilogue when possible
   auto linear_out = [&](const void* X, const void* Wt, const float* bias, void* out, int N, int K, int gelu) {
     if (fuse) {
@@ -1513,18 +1470,11 @@ static int sig_tower(pg_engine* e, const float* pixel, int n, void* feat, cudaSt
     if (l == 0) TRY(resid_ln(nullptr, nullptr, ln1w, ln1b));
     TRY(linear_out(e->sig_xn, wqkv, bqkv, e->sig_qkv, 3 * W, W, 0));
     if (tc_attn) {
-      const int NPpad = (int)align_up((size_t)NP, 8);
-      CUtensorMap mq, mk, mv;
+      CUtensorMap mq, mk;      // K and V rows both through mk (V read in place as an MN-major operand)
       TRY(make_map_2d(e, &mq, e->sig_qkv, (uint64_t)M, (uint64_t)3 * W, VT_BQ));
       TRY(make_map_2d(e, &mk, e->sig_qkv, (uint64_t)M, (uint64_t)3 * W, VT_BK));
-      if (e->sig_v_direct) {
-        mv = mk;            // V rows are read in place as an MN-major operand: no key-contiguous copy
-      } else {
-        TRY(launch(e, vit_v_transpose_kernel, dim3((NPpad + 63) / 64, heads, n), dim3(256), 0, st, (const bf16*)e->sig_qkv, (bf16*)e->sig_vT, NP, NPpad, W, heads, hd));
-        TRY(make_map_2d(e, &mv, e->sig_vT, (uint64_t)n * heads * hd, (uint64_t)NPpad, 64));
-      }
-      TRY(launch(e, vit_attn_tc_kernel, dim3((NP + VT_BQ - 1) / VT_BQ, heads, n), dim3(128), VT_SMEM, st, mq, mk, mv, (bf16*)e->sig_attn, NP, W,
-                 heads, 1.0f / sqrtf((float)hd), e->sig_v_direct));
+      TRY(launch(e, vit_attn_tc_kernel, dim3((NP + VT_BQ - 1) / VT_BQ, heads, n), dim3(128), VT_SMEM, st, mq, mk, (bf16*)e->sig_attn, NP, W,
+                 1.0f / sqrtf((float)hd)));
     } else {
       DISPATCH_T(e,
                  launch(e, vit_attn_kernel<bf16>, dim3((NP + 3) / 4, heads, n), dim3(128), 0, st, (const bf16*)e->sig_qkv, (bf16*)e->sig_attn, NP, W, heads, hd, 1.0f / sqrtf((float)hd)),
@@ -1714,7 +1664,7 @@ static int vq_conv(VqCtx& c, const void* in, int Hi, int Wi, int Cin, const std:
   if (ks == 3) {
     // implicit GEMM: only the (normalised, activated, upsampled) activation is materialised, not its 9 taps
     const void* act = in;
-    const bool qualifies = e->bf16 && e->use_tc && e->use_implicit_conv && Cin % TC_BK == 0 &&
+    const bool qualifies = e->bf16 && e->use_tc && Cin % TC_BK == 0 &&
                            ((Wo <= CONV_NT && CONV_NT % Wo == 0) || Wo % CONV_NT == 0);
     if (qualifies) {
       if (gn_name || up != 1) {

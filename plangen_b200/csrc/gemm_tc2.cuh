@@ -243,7 +243,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant
         if (ep.gelu == 2) {
           // SwiGLU (prefill gate|up): the tile's 128 weight rows are gate(f0 .. f0+63) | up(f0 .. f0+63) (rows interleaved in
           // blocks of 64, weights.py), so a staged token row holds g in bytes 0-127 and u in bytes 128-255:
-          // h = rnd(rnd(silu(g)) * u), 64 values = 128 bytes per token into out [M][N / 2]  (swiglu_bf16_kernel's arithmetic)
+          // h = rnd(rnd(silu(g)) * u), 64 values = 128 bytes per token into out [M][N / 2]  (values identical to swiglu_kernel<bf16>)
           const int c8 = tE & 7, rr0 = tE >> 3, F = N >> 1, f0 = (n0 / TC_BM) * 64;
           if (n0 < N) {
 #pragma unroll 2

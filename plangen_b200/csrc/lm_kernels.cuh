@@ -570,31 +570,6 @@ qkv_rope_store_bf16_kernel(const bf16* __restrict__ qkv, const float* __restrict
   }
 }
 
-// h = rnd(silu(g)) * u on bf16 gate | up projections ([tok][2F], interleaved in blocks of 64 as the weight rows are
-// packed): the prefill's SwiGLU behind the fused bf16 epilogue; values identical to swiglu_kernel<bf16>.
-__global__ void __launch_bounds__(256)
-swiglu_bf16_kernel(const bf16* __restrict__ gu, bf16* __restrict__ h, int F, size_t total8) {
-  pdl_launch_dependents();
-  pdl_wait();
-  const int F8 = F / 8;
-  for (size_t i8 = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i8 < total8; i8 += (size_t)gridDim.x * blockDim.x) {
-    const size_t tok = i8 / F8;
-    const int f = (int)(i8 - tok * F8) * 8;
-    const bf16* row = gu + tok * 2 * F + (size_t)(f >> 6) * 128 + (f & 63);
-    const uint4 g4 = *reinterpret_cast<const uint4*>(row), u4 = *reinterpret_cast<const uint4*>(row + 64);
-    const uint32_t gw[4] = {g4.x, g4.y, g4.z, g4.w}, uw[4] = {u4.x, u4.y, u4.z, u4.w};
-    uint32_t ow[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const float g0 = bf16lo(gw[j]), g1 = bf16hi(gw[j]), u0 = bf16lo(uw[j]), u1 = bf16hi(uw[j]);
-      const float h0 = bf16_round(g0 / (1.0f + expf(-g0))) * u0, h1 = bf16_round(g1 / (1.0f + expf(-g1))) * u1;
-      const __nv_bfloat162 o = __floats2bfloat162_rn(h0, h1);
-      ow[j] = *reinterpret_cast<const uint32_t*>(&o);
-    }
-    *reinterpret_cast<uint4*>(h + tok * F + f) = make_uint4(ow[0], ow[1], ow[2], ow[3]);
-  }
-}
-
 // ---------------------------------------------------------------- a4.3: SwiGLU
 // h = silu(gate) * up   (HF LlamaMLP :182-184); partial layout [S][tok][2F]: [gate | up], or - when the
 // weight rows were packed for the fused tcgen05 epilogue - interleaved in blocks of 64 (g0-63, u0-63, g64-127, ...)

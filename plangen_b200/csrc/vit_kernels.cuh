@@ -182,35 +182,6 @@ vit_resid_ln_warp_kernel(float* __restrict__ x, const float* __restrict__ part, 
   }
 }
 
-// ---------------------------------------------------------------- V^T for the tensor-core attention
-// qkv bf16 [M][3*W] (q | k | v, head-major inside each) -> vT [(img*heads + h)*hd + d][NPpad] (keys contiguous; NPpad =
-// NP rounded up to 8 so rows are 16-byte multiples for TMA; the pad keys are written as zeros - they meet P = 0)
-__global__ void __launch_bounds__(256)
-vit_v_transpose_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ vT, int NP, int NPpad, int W, int heads, int hd) {
-  __shared__ bf16 tile[64][64 + 2];
-  pdl_launch_dependents();
-  pdl_wait();
-  const int k0 = blockIdx.x * 64, h = blockIdx.y, img = blockIdx.z;
-  for (int d0 = 0; d0 < hd; d0 += 64) {
-    for (int i = threadIdx.x; i < 64 * 32; i += 256) {
-      const int kk = i >> 5, d2 = (i & 31) * 2;
-      __nv_bfloat162 v = __floats2bfloat162_rn(0.f, 0.f);
-      if (k0 + kk < NP && d0 + d2 < hd)
-        v = *reinterpret_cast<const __nv_bfloat162*>(qkv + ((size_t)img * NP + k0 + kk) * 3 * W + 2 * W + h * hd + d0 + d2);
-      tile[kk][d2] = v.x; tile[kk][d2 + 1] = v.y;
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < 64 * 32; i += 256) {
-      const int d = i >> 5, k2 = (i & 31) * 2;
-      if (d0 + d < hd && k0 + k2 < NPpad) {                    // NPpad is even
-        __nv_bfloat162 v; v.x = tile[k2][d]; v.y = tile[k2 + 1][d];
-        *reinterpret_cast<__nv_bfloat162*>(vT + ((size_t)(img * heads + h) * hd + d0 + d) * NPpad + k0 + k2) = v;
-      }
-    }
-    __syncthreads();
-  }
-}
-
 // ---------------------------------------------------------------- attention, CUDA cores (fp32 check mode / fallback)
 // F.scaled_dot_product_attention(q, k, v) without mask (siglip_vit.py:176): one warp per query, the whole score row
 // in registers (NP <= 32 * VA_MAXI keys), exact two-pass softmax in fp32.
@@ -279,8 +250,8 @@ vit_attn_kernel(const T* __restrict__ qkv, T* __restrict__ out, int NP, int W, i
 //   P   = online softmax of S, one thread per query row (= TMEM lane), two tcgen05.ld passes (row maximum, then
 //         exp2 + running sum), written as bf16 into shared memory in the K-major swizzled image the second MMA
 //         reads as its A operand - over the K tile, which is dead once S is complete
-//   O_b = P V_blk        tcgen05.mma 128 x 64 x VT_BK into TMEM columns VT_BK .. VT_BK+63; V comes from the
-//         key-contiguous copy (vit_v_transpose_kernel), so both operands are K-major
+//   O_b = P V_blk        tcgen05.mma 128 x 64 x VT_BK into TMEM columns VT_BK .. VT_BK+63; V is taken straight from
+//         the qkv rows ([key][64 dims], one TMA box) as an MN-major B operand
 //   O   = O * exp(m_old - m_new) + O_b   in registers (64 fp32 per thread)
 // Scores stay fp32 (fused SDPA kernels do not round them), probabilities enter the second product as bf16.
 // 88 KB of shared memory and 256 TMEM columns per CTA: two CTAs per SM overlap each other's load / MMA / softmax phases.
@@ -290,21 +261,20 @@ constexpr int VT_HD = 64;
 constexpr int VT_QTILE = VT_BQ * 64 * 2;        // 16 KB
 constexpr int VT_KTILE = VT_BK * 64 * 2;        // 24 KB
 constexpr int VT_PTILE = VT_BQ * 64 * 2;        // one [128][64] tile of P, VT_BK / 64 of them
-constexpr int VT_VTILE = 64 * 64 * 2;           // one [64 dims][64 keys] tile of V^T, VT_BK / 64 of them
+constexpr int VT_VTILE = VT_BK * 64 * 2;        // V tile [VT_BK keys][64 dims] (24 KB)
 constexpr int VT_KP_BYTES = (VT_BK / 64) * VT_PTILE;          // K tile, later the P tiles (48 KB)
-constexpr int VT_SMEM = VT_QTILE + VT_KP_BYTES + (VT_BK / 64) * VT_VTILE + 1024 + 64;
+constexpr int VT_SMEM = VT_QTILE + VT_KP_BYTES + VT_VTILE + 1024 + 64;
 
 __global__ void __launch_bounds__(128, 2)
 vit_attn_tc_kernel(const __grid_constant__ CUtensorMap map_qk, const __grid_constant__ CUtensorMap map_k,
-                   const __grid_constant__ CUtensorMap map_vt, bf16* __restrict__ out, int NP, int W, int heads, float scale,
-                   int v_direct) {
+                   bf16* __restrict__ out, int NP, int W, float scale) {
   extern __shared__ uint8_t vt_smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)vt_smem_raw + 1023) & ~(uintptr_t)1023);
   uint8_t* sQ = smem;
   uint8_t* sK = smem + VT_QTILE;                 // K tile [VT_BK][64]; overwritten by P [128][VT_BK] (3 tiles)
   uint8_t* sP = sK;
-  uint8_t* sV = sK + VT_KP_BYTES;                // V^T: VT_BK/64 tiles of [64 dims][64 keys]
-  uint64_t* bars = (uint64_t*)(sV + (VT_BK / 64) * VT_VTILE);
+  uint8_t* sV = sK + VT_KP_BYTES;                // V tile [VT_BK keys][64 dims]
+  uint64_t* bars = (uint64_t*)(sV + VT_VTILE);
   uint64_t* bar_load = bars;
   uint64_t* bar_mma = bars + 1;
   uint32_t* tmem_slot = (uint32_t*)(bars + 2);
@@ -313,7 +283,7 @@ vit_attn_tc_kernel(const __grid_constant__ CUtensorMap map_qk, const __grid_cons
   const int q0 = blockIdx.x * VT_BQ, h = blockIdx.y, img = blockIdx.z;
   pdl_launch_dependents();
   if (tid == 0) {
-    tma_prefetch_desc(&map_qk); tma_prefetch_desc(&map_k); tma_prefetch_desc(&map_vt);
+    tma_prefetch_desc(&map_qk); tma_prefetch_desc(&map_k);
     mbar_init(bar_load, 1); mbar_init(bar_mma, 1);
     mbar_fence_init();
   }
@@ -333,24 +303,16 @@ vit_attn_tc_kernel(const __grid_constant__ CUtensorMap map_qk, const __grid_cons
   const float sl2 = scale * 1.4426950408889634f;     // scores in log2 units
   const uint32_t t_lane = tmem_base + ((uint32_t)(warp * 32) << 16);
   const uint32_t idesc_s = umma_idesc_bf16(VT_BQ, VT_BK);
-  // v_direct: V is taken straight from the qkv rows ([key][64 dims], one TMA box) as an MN-major B operand; otherwise
-  // from the key-contiguous copy vit_v_transpose_kernel made (K-major)
-  const uint32_t idesc_o = v_direct ? umma_idesc_bf16_bmn(VT_BQ, VT_HD) : umma_idesc_bf16(VT_BQ, VT_HD);
+  const uint32_t idesc_o = umma_idesc_bf16_bmn(VT_BQ, VT_HD);
   const int nkb = (NP + VT_BK - 1) / VT_BK;
   for (int kb = 0; kb < nkb; ++kb) {
     const int key0 = kb * VT_BK;
     if (tid == 0) {
       const uint64_t pol = policy_evict_first();
-      mbar_expect_tx(bar_load, (kb == 0 ? VT_QTILE : 0) + VT_KTILE + (VT_BK / 64) * VT_VTILE);
+      mbar_expect_tx(bar_load, (kb == 0 ? VT_QTILE : 0) + VT_KTILE + VT_VTILE);
       if (kb == 0) tma_load_2d(sQ, &map_qk, bar_load, h * VT_HD, img * NP + q0, pol);
       tma_load_2d(sK, &map_k, bar_load, W + h * VT_HD, img * NP + key0, pol);
-      if (v_direct) {
-        tma_load_2d(sV, &map_k, bar_load, 2 * W + h * VT_HD, img * NP + key0, pol);
-      } else {
-#pragma unroll
-        for (int t = 0; t < VT_BK / 64; ++t)
-          tma_load_2d(sV + t * VT_VTILE, &map_vt, bar_load, key0 + 64 * t, (img * heads + h) * VT_HD, pol);
-      }
+      tma_load_2d(sV, &map_k, bar_load, 2 * W + h * VT_HD, img * NP + key0, pol);
       mbar_wait(bar_load, (uint32_t)(kb & 1), 60);
       tc_fence_after();
 #pragma unroll
@@ -410,8 +372,7 @@ vit_attn_tc_kernel(const __grid_constant__ CUtensorMap map_qk, const __grid_cons
 #pragma unroll
       for (int kk = 0; kk < VT_BK / 16; ++kk)
         umma_bf16(tmem_base + (uint32_t)VT_BK, umma_desc_k_sw128(smem_u32(sP + (kk >> 2) * VT_PTILE)) + (uint64_t)(2 * (kk & 3)),
-                  v_direct ? umma_desc_mn_sw128(smem_u32(sV) + (uint32_t)kk * 2048u, 1024u)
-                           : umma_desc_k_sw128(smem_u32(sV + (kk >> 2) * VT_VTILE)) + (uint64_t)(2 * (kk & 3)),
+                  umma_desc_mn_sw128(smem_u32(sV) + (uint32_t)kk * 2048u, 1024u),
                   idesc_o, kk != 0);
       umma_commit(bar_mma);
     }
@@ -425,7 +386,7 @@ vit_attn_tc_kernel(const __grid_constant__ CUtensorMap map_qk, const __grid_cons
       for (int j = 0; j < VT_HD; ++j) o[j] = o[j] * alpha + __uint_as_float(v[j]);
     }
     tc_fence_before();
-    __syncthreads();          // next block: TMA overwrites K (= P) / V^T, the first MMA overwrites S
+    __syncthreads();          // next block: TMA overwrites K (= P) / V, the first MMA overwrites S
   }
   if (q < NP) {
     const float inv = 1.f / l_run;

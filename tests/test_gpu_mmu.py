@@ -118,15 +118,6 @@ def test_bf16_small_tower_vs_autocast_reference(tc):
     finally:
         eng.set_option("sig_attn_tc", 1)
     assert_close(got.numpy(), want.numpy(), 2e-2, 2e-2, f"bf16 SigLIP features (tc attention = {tc})")
-    if tc:
-        # V read in place as an MN-major operand (default) vs from the key-contiguous copy: the same products summed in the
-        # same order - identical features
-        eng.set_option("sig_v_direct", 0)
-        try:
-            got2 = eng.vision_features(img).float().cpu()
-        finally:
-            eng.set_option("sig_v_direct", 1)
-        assert torch.equal(got, got2)
 
 
 def test_fullsize_siglip_l_bf16_vs_autocast_reference():

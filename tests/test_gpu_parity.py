@@ -255,13 +255,10 @@ def test_packed_prefill_is_bit_identical_to_padded_prefill():
     ids, mask = O.t2i_infer_collate_batch(cond, neg, dims.pad_id, dims.n_img_tokens)
     eng = get_engine(dims, "bf16", with_vq=False, max_batch=8, max_prompt=256)
     outs, toks = [], []
-    # third pass: V from the key-contiguous copy instead of the cache rows read in place (MN-major operand, the default);
-    # fourth: SwiGLU as its own kernel instead of in the gate|up contraction's epilogue
-    # fifth: RoPE + q / cache stores as their own kernel instead of in the QKV contraction's epilogue (also with the padded block)
-    for pack, v_direct, swiglu_fuse, qkv_fuse in ((1, 1, 1, 1), (0, 1, 1, 1), (1, 0, 1, 1), (1, 1, 0, 1), (1, 1, 1, 0), (0, 1, 1, 0)):
+    # third pass: RoPE + q / cache stores as their own kernel instead of in the QKV contraction's epilogue (also with the
+    # padded block)
+    for pack, qkv_fuse in ((1, 1), (0, 1), (1, 0), (0, 0)):
         eng.set_option("prefill_pack", pack)
-        eng.set_option("prefill_v_direct", v_direct)
-        eng.set_option("prefill_swiglu_fuse", swiglu_fuse)
         eng.set_option("prefill_qkv_fuse", qkv_fuse)
         dbg = torch.zeros(steps, len(lens), dims.img_vocab, device="cuda")
         eng.set_option("dbg_logits_ptr", dbg.data_ptr())
@@ -272,11 +269,9 @@ def test_packed_prefill_is_bit_identical_to_padded_prefill():
         finally:
             eng.set_option("dbg_logits_ptr", 0)
             eng.set_option("prefill_pack", 1)
-            eng.set_option("prefill_v_direct", 1)
-            eng.set_option("prefill_swiglu_fuse", 1)
             eng.set_option("prefill_qkv_fuse", 1)
         outs.append(dbg.cpu())
-    for k in (1, 2, 3, 4, 5):
+    for k in (1, 2, 3):
         assert torch.equal(outs[0], outs[k]) and torch.equal(toks[0], toks[k]), k
     # and for the text prefill of language_model.generate (mask-aware RoPE positions)
     sd = O.init_state_dict(dims, seed=0, with_vq=False, with_lm_head=True)

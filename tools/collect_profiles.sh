@@ -18,7 +18,7 @@ PG_STEPS=300 PG_GRAPH=0 timeout 400 ncu --set full --clock-control none --import
 PG_STEPS=300 PG_GRAPH=0 timeout 400 ncu --set full --clock-control none --import-source on -k regex:"gemm_tc_kernel" -s 28900 -c 4 \
   -o gpurun_out/${R}_gemm_tc python tools/profile_step.py > gpurun_out/p_c.log 2>&1
 PG_STEPS=2 PG_GRAPH=0 PG_VQ=1 timeout 400 ncu --metrics gpu__time_duration.sum --clock-control none \
-  -k regex:"^(gemm_tc|gemm_simt|im2col|v_transpose|gn_|conv_epilogue|softmax_rows|vq_codebook|attn_prefill|qkv_rope|resid_rmsnorm|swiglu|prefill_|gather_last|kv_broadcast)" -c 2000 \
+  -k regex:"^(gemm_tc|gemm_simt|im2col|gn_|conv_epilogue|softmax_rows|vq_codebook|attn_prefill|qkv_rope|resid_rmsnorm|swiglu|prefill_|gather_last|kv_broadcast)" -c 2000 \
   --csv --log-file gpurun_out/${R}_launches_prefill_vq.csv python tools/profile_step.py > gpurun_out/p_d.log 2>&1
 PG_STEPS=2 PG_GRAPH=0 timeout 400 ncu --set full --clock-control none --import-source on -k regex:"gemm_tc2_kernel" -s 1 -c 4 \
   -o gpurun_out/${R}_gemm_prefill python tools/profile_step.py > gpurun_out/p_e.log 2>&1

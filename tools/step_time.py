@@ -20,7 +20,7 @@ ids, mask = synthetic.collate_cfg_batch(cond, neg, dims.pad_id, dims.n_img_token
 ids, mask = ids.to(dev), mask.to(dev)
 emb = eng.language_model.get_input_embeddings()(ids)
 st = torch.cuda.current_stream(dev)
-DEFAULTS = {"use_pdl": 1, "use_graph": 1, "use_tc": 1, "attn_impl": 3, "attn_trigger": 1, "attn_attr": 1}
+DEFAULTS = {"use_pdl": 1, "use_graph": 1, "use_tc": 1, "attn_impl": 3}
 
 
 def loop_ms(n=576, top_p=1.0):

@@ -6,7 +6,7 @@ from plangen_b200 import JANUS_1P3B, synthetic
 from plangen_b200.engine import FastJanus
 B = int(os.environ.get("PG_B", "16")); dims = JANUS_1P3B; dev = torch.device("cuda", 0)
 sd = synthetic.random_state_dict(dims, dev, seed=0, with_vq=False)
-eng = FastJanus(sd, dims, mode="bf16", max_batch=B, max_prompt=512, with_vq=False, options={"use_graph": int(os.environ.get("PG_GRAPH", "1")), "fuse_swiglu": int(os.environ.get("PG_FUSE", "1"))})
+eng = FastJanus(sd, dims, mode="bf16", max_batch=B, max_prompt=512, with_vq=False, options={"use_graph": int(os.environ.get("PG_GRAPH", "1"))})
 del sd
 cond, neg = synthetic.layoutsam_prompts(dims, B, seed=1234)
 ids, mask = synthetic.collate_cfg_batch(cond, neg, dims.pad_id, dims.n_img_tokens)
@@ -22,10 +22,8 @@ t = torch.stack([snap[:NS], snap[NS:]], 1)
 used = (t[:, 1] > 0).nonzero().flatten().tolist()
 t0 = int(t[used, 0].min())
 names = []
-# launch order of instrumented kernels in a step: head gemm, head gemm, then per layer: qkv, attn, o, norm, gu, swiglu, down, norm
-per_layer = ["qkv", "attn", "o", "norm1", "gu", "swiglu", "down", "norm2"] if int(os.environ.get("PG_FUSE", "1")) == 0 else ["qkv", "attn", "o", "norm1", "gu", "down", "norm2"]
-if int(os.environ.get("PG_FUSE_NORM", "0")) == 1 and B <= 16:
-    per_layer = ["qkv", "attn", "o", "gu", "down"]
+# launch order of instrumented kernels in a step: head gemm, head gemm, then per layer: qkv, attn, o, norm, gu, down, norm
+per_layer = ["qkv", "attn", "o", "norm1", "gu", "down", "norm2"]
 labels = ["head0", "head1"] + [f"L{l}.{n}" for l in range(dims.L) for n in per_layer]
 rows = [(labels[i] if i < len(labels) else str(i), (int(t[i, 0]) - t0) / 1e3, (int(t[i, 1]) - t0) / 1e3) for i in used]
 print("slots used", len(used), "step span us", rows[-1][2] - rows[0][1])
