@@ -20,7 +20,7 @@
 extern "C" {
 #endif
 
-#define PG_ABI_VERSION 3
+#define PG_ABI_VERSION 4
 
 /* arithmetic regimes */
 #define PG_MODE_BF16 0 /* the reference's regime: fp32 master weights under autocast(bf16), plangen_base.py:360 */
@@ -101,6 +101,30 @@ int pg_cfg_sample_embed(pg_engine* e, const float* logits, int B, float cfg_weig
                         double top_p, const int32_t* edit_region, const int32_t* gt_labels, int step,
                         int n_steps, int32_t* tokens_out, float* x_next, void* stream);
 
+/* Sampling settings of one image for the *_per_image entry points, passed as a HOST array of B entries (copied at entry;
+ * the array may be reused when the call returns).  Image b is sampled exactly as the scalar entry points sample a whole
+ * batch run with (cfg_weight, temperature, top_k, top_p): CFG per op in the engine dtype, a correctly rounded
+ * /temperature, top-k, top-p, softmax.  top_k >= 0 and top_p in [0, 1] (NaN fails) are checked per image and a failure
+ * names the image.  top_p is a double, like the scalar entries' argument: the kernel compares against fp32(1 - top_p)
+ * with 1 - top_p in double, as torch does.
+ * seed / offset: rng_per_image != 0 - image b draws as torch.multinomial(probs[b:b+1], 1, generator=g_b) with g_b at
+ * (seed, offset): element v of a (1, V) tensor, so its tokens depend neither on b nor on B; each step advances its
+ * offset by torch's per-draw increment for numel = V (4 at V = 16384).  rng_per_image == 0 - entry 0's seed and offset
+ * serve the whole call with the scalar path's mapping (element b * V + v of one (B, V) draw); the other entries' seed
+ * and offset are ignored. */
+typedef struct pg_image_sampling {
+  uint64_t seed, offset;
+  float cfg_weight, temperature;
+  int32_t top_k;
+  double top_p;
+} pg_image_sampling;
+
+/* pg_cfg_sample_embed with per-image settings: per_image = HOST array [B] (see pg_image_sampling; its offsets are the
+ * offsets of this draw).  greedy, teacher forcing, step, n_steps and the outputs as for pg_cfg_sample_embed. */
+int pg_cfg_sample_embed_per_image(pg_engine* e, const float* logits, int B, const pg_image_sampling* per_image,
+                                  int rng_per_image, int greedy, const int32_t* edit_region, const int32_t* gt_labels,
+                                  int step, int n_steps, int32_t* tokens_out, float* x_next, void* stream);
+
 /* replaces: vl_gpt.prepare_gen_img_embeds(ids)     modeling_vlm.py:270-271
  * ids int32 [n] -> fp32 [n, D] */
 int pg_prepare_gen_img_embeds(pg_engine* e, const int32_t* ids, int n, float* out, void* stream);
@@ -109,11 +133,19 @@ int pg_prepare_gen_img_embeds(pg_engine* e, const int32_t* ids, int n, float* ou
  * prefill + n_steps x (gen_head, CFG, sample, embed, decode step) with no host sync.
  * x_prompt fp32 [R,P,D] (consumed).  tokens_out int32 [R/2, n_steps].  kv_start / edit_region / gt_labels are copied
  * into engine-owned buffers at entry (captured graphs are keyed on shapes and scalars, not on caller addresses).
- * top_k / top_p as for pg_cfg_sample_embed. */
+ * top_k / top_p as for pg_cfg_sample_embed.  pg_sample_image_per_image below takes these settings per image. */
 int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P,
                     int n_steps, float cfg_weight, float temperature, uint64_t seed, int greedy, int top_k,
                     double top_p, const int32_t* edit_region, const int32_t* gt_labels,
                     int32_t* tokens_out, void* stream);
+
+/* pg_sample_image with per-image settings: per_image = HOST array [R/2] (see pg_image_sampling), so one batch can serve
+ * requests with different seeds, guidance scales, temperatures, top-k and top-p.  The settings are staged in the engine
+ * and read on the device, so the captured decode-step graph depends on the shape, greedy, teacher forcing,
+ * rng_per_image and whether any image uses top-p - not on the values: new seeds and settings replay the same graph. */
+int pg_sample_image_per_image(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
+                              const pg_image_sampling* per_image, int rng_per_image, int greedy,
+                              const int32_t* edit_region, const int32_t* gt_labels, int32_t* tokens_out, void* stream);
 
 /* replaces: System.x2t (plangen_base.py:513-523) = vl_gpt.language_model.generate(inputs_embeds=,
  *           attention_mask=, pad_token_id=, eos_token_id=, max_new_tokens=, do_sample=False, use_cache=True),

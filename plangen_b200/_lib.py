@@ -25,6 +25,12 @@ class PgDims(C.Structure):
     ]
 
 
+class PgImageSampling(C.Structure):
+    """pg_image_sampling: one image's settings for the *_per_image entry points."""
+    _fields_ = [("seed", C.c_uint64), ("offset", C.c_uint64), ("cfg_weight", C.c_float), ("temperature", C.c_float),
+                ("top_k", C.c_int32), ("top_p", C.c_double)]
+
+
 class PgError(RuntimeError):
     pass
 
@@ -45,9 +51,14 @@ EXPORTS = {
     "pg_cfg_sample_embed": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_float, C.c_float, C.c_uint64, C.c_uint64,
                                       C.c_int, C.c_int, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                       C.c_void_p]),
+    "pg_cfg_sample_embed_per_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(PgImageSampling), C.c_int, C.c_int,
+                                                C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pg_prepare_gen_img_embeds": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "pg_sample_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float,
                                   C.c_uint64, C.c_int, C.c_int, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "pg_sample_image_per_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                            C.POINTER(PgImageSampling), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_void_p]),
     "pg_generate_greedy": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_void_p, C.POINTER(C.c_int), C.c_void_p]),
     "pg_vq_decode_code": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
@@ -88,7 +99,7 @@ def load(build_if_missing: bool = True):
         fn = getattr(lib, name)      # AttributeError if the symbol is not exported
         fn.restype = res
         fn.argtypes = args
-    if lib.pg_abi_version() != 3:
+    if lib.pg_abi_version() != 4:
         raise PgError("ABI version mismatch")
     _LIB = lib
     return lib

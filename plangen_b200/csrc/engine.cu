@@ -90,6 +90,7 @@ struct pg_engine {
   int prof_step = -1, prof_slot = 0;
   bool prof_active = false;
   int64_t launches = 0;
+  int64_t graph_captures = 0;                // decode-step graphs captured (graph_for misses)
   bool finalized = false;
   // bound buffers
   void* kv = nullptr; size_t kv_bytes = 0;
@@ -100,6 +101,7 @@ struct pg_engine {
   // engine-owned staging of the per-call inputs / outputs of the fused loops, so captured graphs depend on shapes
   // and scalars only (the caller's tensors are fresh allocations on every call)
   int32_t *st_kv_start = nullptr, *st_edit = nullptr, *st_gt = nullptr, *st_tokens = nullptr;
+  ImageSampling* st_sampling = nullptr;               // per-image entry points: [B] settings (sample.cuh)
   // mmu front-end (SigLIP tower + aligner + scatter, vit_kernels.cuh); carved only when dims.sig_layers > 0
   int sig_chunk = 0, sig_np = 0;                      // images per pass, patches per image
   float *sig_x = nullptr, *sig_part = nullptr;
@@ -391,6 +393,7 @@ static void layout_workspace(pg_engine* e, Carve& c) {
     e->st_edit = (int32_t*)c.take(B * std::max(d.max_steps, 1) * 4);
     e->st_gt = (int32_t*)c.take(B * std::max(d.max_steps, 1) * 4);
     e->st_tokens = (int32_t*)c.take(R * (size_t)e->Tmax * 4);      // image loop: [B][n_steps]; text loop: [R][max_new]
+    e->st_sampling = (ImageSampling*)c.take(B * sizeof(ImageSampling));
   }
   if (d.sig_layers > 0 && d.max_images > 0) {
     // SigLIP tower scratch for one pass of sig_chunk images; features of ALL images stay (the scatter needs them)
@@ -616,6 +619,7 @@ extern "C" int pg_engine_get_counter(const pg_engine* e, const char* key, int64_
   else if (k == "num_sms") *value = e->num_sms;
   else if (k == "max_threads_per_sm") *value = e->max_threads_per_sm;
   else if (k == "tmax") *value = e->Tmax;
+  else if (k == "graph_captures") *value = e->graph_captures;
   else if (k == "philox_offset_per_step") *value = 0;
   else return fail("unknown counter '%s'", key);
   return 0;
@@ -1135,19 +1139,36 @@ static void philox_policy(pg_engine* e, size_t numel, uint64_t* counter_offset, 
   *stride = grid * block;
 }
 
+// Per-image settings of one sampler launch or decode loop (the per-image entry points; nullptr everywhere else):
+// `dev` holds B staged entries; the scalar settings arguments are then ignored.  any_top_p: some image has top_p < 1.
+struct PerImage {
+  const ImageSampling* dev;
+  int rng_per_image;
+  bool any_top_p;
+};
+
+// Philox element count of one draw: the whole (B, V) tensor, or one image's (1, V) row with per-image generators
+static size_t philox_numel(const pg_engine* e, int B, const PerImage* pi) {
+  return (pi && pi->rng_per_image ? 1 : (size_t)B) * e->d.img_vocab;
+}
+
+// top-p threshold: what torch compares the fp32 cumulative sum with, fp32(1 - top_p) with 1 - top_p in double; -1 = off
+static float top_p_threshold(double top_p) { return top_p < 1.0 ? (float)(1.0 - top_p) : -1.f; }
+
 static int k_sample(pg_engine* e, const float* part, int S, size_t sstride, const float* bias, int B, float cfg_weight,
                     float temperature, uint64_t seed, uint64_t offset_base, int greedy, int top_k, double top_p,
                     const int32_t* edit_region, const int32_t* gt_labels, int step_base, const int* step_ptr, int n_steps,
-                    int32_t* tokens_out, float* x_next, const float* next_norm_w, void* xn_next, cudaStream_t st) {
+                    int32_t* tokens_out, float* x_next, const float* next_norm_w, void* xn_next, cudaStream_t st,
+                    const PerImage* pi = nullptr) {
   const pg_dims& d = e->d;
   uint64_t per_step, stride;
-  philox_policy(e, (size_t)B * d.img_vocab, &per_step, &stride);
+  philox_policy(e, philox_numel(e, B, pi), &per_step, &stride);
   const size_t chunk = (size_t)((d.img_vocab + SAMPLE_CLUSTER - 1) / SAMPLE_CLUSTER);
   size_t csm = chunk * 4;
-  // top-p: the threshold torch compares the fp32 cumulative sum with, fp32(1 - top_p) with 1 - top_p in double;
-  // the kernel then keeps the logits and the select's 5 x 256 fixed-point mass histograms in dynamic shared memory
-  const float top_p_thr = top_p < 1.0 ? (float)(1.0 - top_p) : -1.f;
-  if (top_p < 1.0) {
+  // top-p: the kernel keeps the logits and the select's 5 x 256 fixed-point mass histograms in dynamic shared memory
+  // (per image: sized when any image uses it; the others skip the select)
+  const float top_p_thr = top_p_threshold(top_p);
+  if (pi ? pi->any_top_p : top_p < 1.0) {
     csm = ((chunk + 1) & ~(size_t)1) * 8 + 5 * 256 * 8;
     if (csm > 48 * 1024) return fail("top_p needs %zu B of shared memory per CTA at img_vocab %d (48 KB available)", csm, d.img_vocab);
   }
@@ -1155,11 +1176,11 @@ static int k_sample(pg_engine* e, const float* part, int S, size_t sstride, cons
              launch(e, cfg_sample_embed_cluster_kernel<bf16>, dim3(B * SAMPLE_CLUSTER), dim3(SAMPLE_CL_THREADS), csm, st, part, S, sstride, bias, B, d.img_vocab,
                     cfg_weight, temperature, seed, offset_base, per_step, stride, greedy, top_k, top_p_thr, edit_region, gt_labels,
                     step_base, step_ptr, n_steps, tokens_out, (const bf16*)e->embed_table, d.D, x_next, next_norm_w, (bf16*)xn_next,
-                    d.rms_eps, 1, e->dbg_logits),
+                    d.rms_eps, 1, e->dbg_logits, pi ? pi->dev : nullptr, pi ? pi->rng_per_image : 0),
              launch(e, cfg_sample_embed_cluster_kernel<float>, dim3(B * SAMPLE_CLUSTER), dim3(SAMPLE_CL_THREADS), csm, st, part, S, sstride, bias, B, d.img_vocab,
                     cfg_weight, temperature, seed, offset_base, per_step, stride, greedy, top_k, top_p_thr, edit_region, gt_labels,
                     step_base, step_ptr, n_steps, tokens_out, (const float*)e->embed_table, d.D, x_next, next_norm_w, (float*)xn_next,
-                    d.rms_eps, 0, e->dbg_logits));
+                    d.rms_eps, 0, e->dbg_logits, pi ? pi->dev : nullptr, pi ? pi->rng_per_image : 0));
   return 0;
 }
 
@@ -1178,6 +1199,53 @@ extern "C" int pg_cfg_sample_embed(pg_engine* e, const float* logits, int B, flo
                   gt_labels, step, nullptr, n_steps, tokens_out, x_next, nullptr, nullptr, (cudaStream_t)stream);
 }
 
+// The caller's per-image settings, validated (naming the image) and converted to the kernel's entries.  Batch-wide RNG:
+// every entry takes image 0's seed and offset.
+struct StagedSampling {
+  std::vector<ImageSampling> dev;
+  int rng_per_image = 0;
+  bool any_top_p = false;
+};
+
+static int convert_per_image(const pg_image_sampling* h, int B, int rng_per_image, StagedSampling* out) {
+  if (!h) return fail("null argument");
+  out->dev.resize((size_t)B);
+  out->rng_per_image = rng_per_image ? 1 : 0;
+  out->any_top_p = false;
+  for (int b = 0; b < B; ++b) {
+    if (h[b].top_k < 0) return fail("image %d: top_k must be >= 0, got %d", b, h[b].top_k);
+    if (!(h[b].top_p >= 0.0 && h[b].top_p <= 1.0)) return fail("image %d: top_p must be in [0, 1], got %g", b, h[b].top_p);
+    const pg_image_sampling& rng = h[rng_per_image ? b : 0];
+    out->dev[b] = {rng.seed, rng.offset, h[b].cfg_weight, h[b].temperature, h[b].top_k, top_p_threshold(h[b].top_p)};
+    out->any_top_p |= h[b].top_p < 1.0;
+  }
+  return 0;
+}
+
+// copy into st_sampling on `st` (a plain copy from pageable memory: `ss` may go when it returns)
+static int stage_per_image(pg_engine* e, const StagedSampling& ss, cudaStream_t st, PerImage* out) {
+  CK(cudaMemcpyAsync(e->st_sampling, ss.dev.data(), ss.dev.size() * sizeof(ImageSampling), cudaMemcpyHostToDevice, st));
+  *out = {e->st_sampling, ss.rng_per_image, ss.any_top_p};
+  return 0;
+}
+
+extern "C" int pg_cfg_sample_embed_per_image(pg_engine* e, const float* logits, int B, const pg_image_sampling* per_image,
+                                             int rng_per_image, int greedy, const int32_t* edit_region,
+                                             const int32_t* gt_labels, int step, int n_steps, int32_t* tokens_out,
+                                             float* x_next, void* stream) {
+  TRY(check_ready(e));
+  if (B < 1 || 2 * B > e->d.max_rows) return fail("sample B=%d exceeds engine limits", B);
+  if (step < 0 || step >= n_steps) return fail("step %d out of range", step);
+  if ((edit_region == nullptr) != (gt_labels == nullptr)) return fail("edit_region and gt_labels go together");
+  StagedSampling ss;
+  TRY(convert_per_image(per_image, B, rng_per_image, &ss));
+  cudaStream_t st = (cudaStream_t)stream;
+  PerImage pi;
+  TRY(stage_per_image(e, ss, st, &pi));
+  return k_sample(e, logits, 1, 0, nullptr, B, 0.f, 1.f, 0, 0, greedy, 0, 1.0, edit_region, gt_labels, step, nullptr,
+                  n_steps, tokens_out, x_next, nullptr, nullptr, st, &pi);
+}
+
 extern "C" int pg_prepare_gen_img_embeds(pg_engine* e, const int32_t* ids, int n, float* out, void* stream) {
   TRY(check_ready(e));
   cudaStream_t st = (cudaStream_t)stream;
@@ -1193,7 +1261,8 @@ extern "C" int pg_prepare_gen_img_embeds(pg_engine* e, const int32_t* ids, int n
 // PDL wait).
 static int one_step(pg_engine* e, const int32_t* kv_start, int R, int P, int n_steps, float cfg_weight, float temperature,
                     uint64_t seed, int greedy, int top_k, double top_p, const int32_t* edit_region,
-                    const int32_t* gt_labels, int32_t* tokens_out, bool with_lm, int step_host, cudaStream_t st) {
+                    const int32_t* gt_labels, int32_t* tokens_out, bool with_lm, int step_host, cudaStream_t st,
+                    const PerImage* pi) {
   NEED(b1, float, "head.b1");
   LayerW w0;
   TRY(layer_weights(e, 0, &w0));
@@ -1201,11 +1270,11 @@ static int one_step(pg_engine* e, const int32_t* kv_start, int R, int P, int n_s
   TRY(head_gemms(e, R, &S, st));
   const bool host = step_host >= 0;
   uint64_t per_step, stride;
-  philox_policy(e, (size_t)(R / 2) * e->d.img_vocab, &per_step, &stride);
+  philox_policy(e, philox_numel(e, R / 2, pi), &per_step, &stride);
   TRY(k_sample(e, e->part, S, (size_t)R * e->d.img_vocab, b1, R / 2, cfg_weight, temperature, seed,
                host ? per_step * (uint64_t)step_host : 0, greedy, top_k, top_p, edit_region, gt_labels, host ? step_host : 0,
                host ? nullptr : e->step_ctr, n_steps, tokens_out, with_lm ? e->x_dec : nullptr, w0.ln1,
-               with_lm ? e->xn : nullptr, st));
+               with_lm ? e->xn : nullptr, st, pi));
   if (with_lm)
     TRY(decode_layers(e, kv_start, R, host ? P + step_host : P, host ? nullptr : e->step_ctr, true, !host,
                       P + n_steps / 2, st, 0, P));
@@ -1235,21 +1304,28 @@ static int graph_for(pg_engine* e, const std::string& key, cudaStream_t st, F&& 
   if (ce != cudaSuccess) return fail("graph instantiate failed: %s", cudaGetErrorString(ce));
   pg_engine::GraphEntry& ge = e->graphs[key];
   ge.exec = exec; ge.launches = per_replay;
+  ++e->graph_captures;
   *out = &ge;
   return 0;
 }
 
-extern "C" int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
-                               float cfg_weight, float temperature, uint64_t seed, int greedy, int top_k, double top_p,
-                               const int32_t* edit_region, const int32_t* gt_labels, int32_t* tokens_out, void* stream) {
+static int check_image_loop(pg_engine* e, const int32_t* kv_start, int R, int n_steps, const int32_t* edit_region,
+                            const int32_t* gt_labels, int32_t* tokens_out) {
   TRY(check_ready(e));
   if (R % 2) return fail("R must be even (interleaved cond/uncond rows)");
   if (R < 2 || R > e->d.max_rows) return fail("sample_image R=%d exceeds engine limits", R);
   if (n_steps < 1 || n_steps > e->d.max_steps) return fail("n_steps %d exceeds engine limit %d", n_steps, e->d.max_steps);
-  if (top_k < 0) return fail("top_k must be >= 0");
-  if (!(top_p >= 0.0 && top_p <= 1.0)) return fail("top_p must be in [0, 1], got %g", top_p);
   if ((edit_region == nullptr) != (gt_labels == nullptr)) return fail("edit_region and gt_labels go together ([R/2][n_steps] each)");
   if (!kv_start || !tokens_out) return fail("null argument");
+  return 0;
+}
+
+// The image loop of pg_sample_image (pi == nullptr: the scalar settings) and pg_sample_image_per_image (per_image:
+// the caller's settings, staged here).  Arguments are checked by the callers.
+static int image_loop(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
+                      float cfg_weight, float temperature, uint64_t seed, int greedy, int top_k, double top_p,
+                      const int32_t* edit_region, const int32_t* gt_labels, int32_t* tokens_out, void* stream,
+                      const StagedSampling* per_image) {
   cudaStream_t user = (cudaStream_t)stream;
   cudaStream_t st = e->own_stream;
   const int B = R / 2;
@@ -1261,6 +1337,12 @@ extern "C" int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_
     CK(cudaMemcpyAsync(e->st_edit, edit_region, tok_bytes, cudaMemcpyDeviceToDevice, st));
     CK(cudaMemcpyAsync(e->st_gt, gt_labels, tok_bytes, cudaMemcpyDeviceToDevice, st));
   }
+  PerImage pi_v = {};
+  const PerImage* pi = nullptr;
+  if (per_image) {
+    TRY(stage_per_image(e, *per_image, st, &pi_v));
+    pi = &pi_v;
+  }
   const int32_t* kvs = e->st_kv_start;
   const int32_t* er = edit_region ? e->st_edit : nullptr;
   const int32_t* gl = edit_region ? e->st_gt : nullptr;
@@ -1270,13 +1352,18 @@ extern "C" int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_
   if (n_steps > 1) {
     if (e->use_graph) {
       char key[256];
-      snprintf(key, sizeof(key), "img/%d/%d/%d/%a/%a/%llu/%d/%d/%a/%d/%d", R, P, n_steps, cfg_weight, temperature,
-               (unsigned long long)seed, greedy, top_k, top_p, edit_region ? 1 : 0, (e->prof_buf && e->prof_step >= 0) ? 1 : 0);
+      const int prof = (e->prof_buf && e->prof_step >= 0) ? 1 : 0;
+      if (pi)   // the settings are read from st_sampling: one graph serves every seed and setting of this shape
+        snprintf(key, sizeof(key), "imgpi/%d/%d/%d/%d/%d/%d/%d/%d", R, P, n_steps, greedy, edit_region ? 1 : 0,
+                 pi->rng_per_image, pi->any_top_p ? 1 : 0, prof);
+      else
+        snprintf(key, sizeof(key), "img/%d/%d/%d/%a/%a/%llu/%d/%d/%a/%d/%d", R, P, n_steps, cfg_weight, temperature,
+                 (unsigned long long)seed, greedy, top_k, top_p, edit_region ? 1 : 0, prof);
       pg_engine::GraphEntry* ge = nullptr;
       TRY(graph_for(e, key, st, [&]() {
         e->prof_active = (e->prof_buf != nullptr && e->prof_step >= 0);
         e->prof_slot = 0;
-        int rc = one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, true, -1, st);
+        int rc = one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, true, -1, st, pi);
         e->prof_active = false;
         return rc;
       }, &ge));
@@ -1299,7 +1386,7 @@ extern "C" int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_
           CK(cudaMemsetAsync(e->prof_buf, 0xFF, PROF_SLOTS * 8, st));
           CK(cudaMemsetAsync(e->prof_buf + PROF_SLOTS, 0, PROF_SLOTS * 8, st));
         }
-        int rc = one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, true, i, st);
+        int rc = one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, true, i, st, pi);
         if (e->prof_active)
           CK(cudaMemcpyAsync(e->prof_buf + 2 * PROF_SLOTS, e->prof_buf, 2 * PROF_SLOTS * 8, cudaMemcpyDeviceToDevice, st));
         e->prof_active = false;
@@ -1308,11 +1395,32 @@ extern "C" int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_
     }
   }
   // last token: head + sample only (the reference computes and drops one more embed, SURVEY appendix A.12)
-  TRY(one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, false, n_steps - 1, st));
+  TRY(one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, false, n_steps - 1, st, pi));
   CK(cudaMemcpyAsync(tokens_out, toks, tok_bytes, cudaMemcpyDeviceToDevice, st));
   CK(cudaEventRecord(e->ev_out, st));
   CK(cudaStreamWaitEvent(user, e->ev_out, 0));
   return 0;
+}
+
+extern "C" int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
+                               float cfg_weight, float temperature, uint64_t seed, int greedy, int top_k, double top_p,
+                               const int32_t* edit_region, const int32_t* gt_labels, int32_t* tokens_out, void* stream) {
+  TRY(check_image_loop(e, kv_start, R, n_steps, edit_region, gt_labels, tokens_out));
+  if (top_k < 0) return fail("top_k must be >= 0");
+  if (!(top_p >= 0.0 && top_p <= 1.0)) return fail("top_p must be in [0, 1], got %g", top_p);
+  return image_loop(e, x_prompt, kv_start, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, edit_region,
+                    gt_labels, tokens_out, stream, nullptr);
+}
+
+extern "C" int pg_sample_image_per_image(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
+                                         const pg_image_sampling* per_image, int rng_per_image, int greedy,
+                                         const int32_t* edit_region, const int32_t* gt_labels, int32_t* tokens_out,
+                                         void* stream) {
+  TRY(check_image_loop(e, kv_start, R, n_steps, edit_region, gt_labels, tokens_out));
+  StagedSampling ss;
+  TRY(convert_per_image(per_image, R / 2, rng_per_image, &ss));
+  return image_loop(e, x_prompt, kv_start, R, P, n_steps, 0.f, 1.f, 0, greedy, 0, 1.0, edit_region, gt_labels,
+                    tokens_out, stream, &ss);
 }
 
 // ------------------------------------------------------------------------------ f1: stage-1 text decode (x2t)

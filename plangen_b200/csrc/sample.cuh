@@ -7,7 +7,8 @@
 // u = curand_uniform4(Philox4x32-10(seed, subsequence = thread idx, offset)) where element
 // li = b*V + v of the (B,V) tensor is produced by thread idx = li % (grid*256), component
 // (li / (grid*256)) % 4, loop iteration li / (4*grid*256), grid = min(SMs * (maxThreadsPerSM/256),
-// ceil(B*V/256)) — i.e. the mapping depends on the SM count of the device, as in torch.
+// ceil(B*V/256)) — i.e. the mapping depends on the SM count of the device, as in torch.  With one
+// generator per image (rng_per_image) each image is its own (1,V) tensor: li = v, numel = V.
 #pragma once
 #include "common.cuh"
 
@@ -70,7 +71,22 @@ __device__ unsigned long long* g_sample_dbg = nullptr;   // debug timeline (tool
 // the shared-memory atomics.  The tie group at the boundary key all has the same p; its members leave in index order
 // while mass_below + j * p <= thr.  The removed e_v are zeroed and the sum recomputed over the kept set.  Greedy
 // sampling skips it (the arg-max is always kept).
+//
+// per_image != nullptr (the per-image entry points): cluster b takes cfg_weight, temperature, top_k, top_p_thr, seed
+// and a start offset (added to offset_base) from per_image[b] instead of the scalar arguments, so one batch can mix
+// requests.  rng_per_image != 0 draws image b's variates at element v of a (1, V) tensor (stride and per-step offset of
+// numel = V, chosen by the host) instead of b * V + v: the image's tokens then depend only on its own seed and offset,
+// as torch.multinomial(probs[b:b+1], 1, generator=g_b) would draw them, not on its position or the batch size.
 constexpr int SAMPLE_CLUSTER = 8;
+
+// device copy of one pg_image_sampling entry (engine.cu converts top_p to the threshold the kernel compares with)
+struct __align__(16) ImageSampling {
+  uint64_t seed, offset;
+  float cfg_weight, temperature;
+  int32_t top_k;
+  float top_p_thr;   // fp32(1 - top_p), or -1 when top-p is off for this image
+};
+static_assert(sizeof(ImageSampling) == 32, "one 32-byte entry per image");
 // order-preserving map float -> uint32 (larger value, larger key; -0 < +0 is harmless here)
 PG_DEVINL uint32_t sample_order_key(float t) {
   const uint32_t u = __float_as_uint(t);
@@ -174,7 +190,8 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
                                 int step_base, const int* __restrict__ step_ptr, int n_steps,
                                 int32_t* __restrict__ tokens_out, const T* __restrict__ embed_table, int D,
                                 float* __restrict__ x_next, const float* __restrict__ next_norm_w, T* __restrict__ xn_next,
-                                float eps, int round_resid, float* __restrict__ dbg_logits) {
+                                float eps, int round_resid, float* __restrict__ dbg_logits,
+                                const ImageSampling* __restrict__ per_image, int rng_per_image) {
   extern __shared__ __align__(16) float sh[];   // this CTA's slice of the CFG logits -> unnormalised probabilities
   // top_p_thr >= 0 (top-p on): sh is followed by the slice's logits t and the mass histograms of its radix select
   __shared__ uint32_t hist[4][256];  // top-k radix select: one histogram per pass (read by the other CTAs)
@@ -195,6 +212,13 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
   // The step counter is only written by the last kernel of a decode step; graph replays are fully ordered, and with plain
   // launches the host passes the step explicitly (step_ptr == nullptr), so reading it before the PDL wait is safe.
   const int step = step_base + (step_ptr ? *step_ptr : 0);
+  // The per-image settings are staged by a copy before the decode loop, never written by a kernel of the loop, so they
+  // are read before the PDL wait too: the Philox prefetch below needs the image's seed and offset.
+  if (per_image != nullptr) {
+    const ImageSampling s = per_image[b];
+    cfg_weight = s.cfg_weight; temperature = s.temperature; top_k = s.top_k; top_p_thr = s.top_p_thr;
+    seed = s.seed; offset_base += s.offset;
+  }
   const uint64_t offset = offset_base + offset_per_step * (uint64_t)(step - step_base);
   // The exponential variates of torch.multinomial depend on (seed, offset, element index) only - not on the logits: they
   // are drawn while the head contraction is still streaming its weights (this kernel is launched ahead of its dependency).
@@ -205,7 +229,7 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
 #pragma unroll
     for (int j = 0; j < QPRE; ++j) {
       const int v = v_lo + tid + j * SAMPLE_CL_THREADS;
-      qpre[j] = v < v_hi ? torch_exponential_at((uint64_t)b * V + v, philox_stride, seed, offset) : 1.f;
+      qpre[j] = v < v_hi ? torch_exponential_at((rng_per_image ? 0 : (uint64_t)b * V) + v, philox_stride, seed, offset) : 1.f;
     }
   }
   float bias_r[QPRE];
@@ -365,7 +389,7 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
       const float p = __fdiv_rn(sh[v - v_lo], sum);
       float score = p;
       if (!greedy) {
-        const float q = torch_exponential_at((uint64_t)b * V + v, philox_stride, seed, offset);
+        const float q = torch_exponential_at((rng_per_image ? 0 : (uint64_t)b * V) + v, philox_stride, seed, offset);
         score = __fdiv_rn(p, q);
       }
       if (score > bv || (score == bv && v < bi)) { bv = score; bi = v; }

@@ -19,7 +19,7 @@ from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass
-from typing import Dict, Optional, Sequence
+from typing import Dict, List, Optional, Sequence
 
 import torch
 
@@ -46,6 +46,82 @@ def _i64(v: int) -> int:
     """uint64 seeds through an int64 schema slot (two's complement)."""
     v = int(v) & 0xFFFFFFFFFFFFFFFF
     return v - (1 << 64) if v >= (1 << 63) else v
+
+
+def _is_seq(v) -> bool:
+    return isinstance(v, (list, tuple)) or (isinstance(v, torch.Tensor) and v.dim() > 0)
+
+
+@dataclass
+class SamplingPlan:
+    """Sampling arguments of one image batch, one entry per generated image (see sampling_plan)."""
+    per_image: bool                 # some setting or the generator differs per image: the *_per_image ops
+    rng_per_image: bool             # one generator per image
+    cfg_weight: List[float]
+    temperature: List[float]
+    top_k: List[int]
+    top_p: List[float]
+    seed: List[int]                 # batch-wide RNG: num_gen copies of the call's seed and offset
+    offset: List[int]
+    generators: List[torch.Generator]   # advanced after the call (per image, or the one batch-wide generator)
+
+
+def sampling_plan(num_gen: int, cfg_weight, temperature, top_k, top_p, generator, default_seed: int) -> SamplingPlan:
+    """Normalises the sampling arguments of sample_image / t2i / cfg_sample_embed.  Each of cfg_weight, temperature,
+    top_k and top_p is a scalar (the whole batch) or a sequence / 1-D tensor of num_gen values (image j = copy * B + b
+    under parallel_size, the reference's row-pair order).  `generator` is None (default_seed), an int seed, one CUDA
+    torch.Generator (freshly seeded, as the reference reseeds per t2i call), or a sequence of num_gen CUDA generators
+    or int seeds, one per image; a generator's current offset is honoured."""
+    def values(name, v, cast):
+        if not _is_seq(v):
+            return [cast(v.item() if isinstance(v, torch.Tensor) else v)] * num_gen, False
+        vals = v.tolist() if isinstance(v, torch.Tensor) else list(v)
+        if isinstance(v, torch.Tensor) and v.dim() != 1:
+            raise ValueError(f"`{name}` must be a scalar or a 1-D tensor, got shape {tuple(v.shape)}")
+        if len(vals) != num_gen:
+            raise ValueError(f"`{name}` has {len(vals)} values for {num_gen} generated images")
+        return [cast(x) for x in vals], True
+
+    cfg, s_cfg = values("cfg_weight", cfg_weight, float)
+    temp, s_temp = values("temperature", temperature, float)
+    ks, s_k = values("top_k", top_k, int)
+    ps, s_p = values("top_p", top_p, float)
+    if s_k:
+        for i, k in enumerate(ks):
+            if k < 0:
+                raise ValueError(f"`top_k[{i}]` has to be >= 0, but is {k}")
+    if s_p:
+        for i, p in enumerate(ps):
+            if not 0.0 <= p <= 1.0:                 # NaN fails too
+                raise ValueError(f"`top_p[{i}]` has to be a float in [0, 1], but is {p}")
+    gens: List[torch.Generator] = []
+    rng_per_image = isinstance(generator, (list, tuple))
+    if rng_per_image:
+        if len(generator) != num_gen:
+            raise ValueError(f"`generator` has {len(generator)} entries for {num_gen} generated images")
+        for i, g in enumerate(generator):
+            if isinstance(g, torch.Generator) and any(g is h for h in generator[:i]):
+                raise ValueError(f"`generator[{i}]` is passed twice; each image needs its own generator")
+        seeds, offs = [], []
+        for i, g in enumerate(generator):
+            if isinstance(g, torch.Generator):
+                if g.device.type != "cuda":
+                    raise ValueError(f"`generator[{i}]` is a {g.device.type} generator; the sampler draws as a CUDA one")
+                gens.append(g)
+                seeds.append(g.initial_seed()); offs.append(g.get_offset())
+            else:
+                seeds.append(int(g)); offs.append(0)
+    else:
+        if isinstance(generator, torch.Generator):
+            seed, off = generator.initial_seed(), generator.get_offset()
+            gens.append(generator)
+        else:
+            seed, off = int(default_seed if generator is None else generator), 0
+        if off != 0:
+            raise ValueError("generator must be freshly seeded (the reference reseeds per t2i call, :526)")
+        seeds, offs = [seed] * num_gen, [off] * num_gen
+    return SamplingPlan(rng_per_image or s_cfg or s_temp or s_k or s_p, rng_per_image, cfg, temp, ks, ps,
+                        [_i64(x) for x in seeds], offs, gens)
 
 
 def kv_start_from_mask(mask: torch.Tensor, P: int) -> torch.Tensor:
@@ -361,17 +437,28 @@ class FastJanus:
         OPS.prepare_gen_img_embeds(self.handle, ids, out)
         return out.to(self.out_dtype)
 
-    def cfg_sample_embed(self, logits: torch.Tensor, cfg_weight: float, temperature: float, seed: int, offset: int,
+    def cfg_sample_embed(self, logits: torch.Tensor, cfg_weight, temperature, seed, offset,
                          step: int, n_steps: int, tokens_out: torch.Tensor, greedy: bool = False,
                          edit_region: Optional[torch.Tensor] = None, gt_labels: Optional[torch.Tensor] = None,
-                         top_k: int = 0, top_p: float = 1.0):
+                         top_k=0, top_p=1.0):
         """plangen_base.py:580-604 in one launch; returns the next inputs_embeds (2B, D) fp32.  `top_k` / `top_p` filter the
-        CFG logits as HF's TopKLogitsWarper then TopPLogitsWarper do (0 / 1 = off)."""
+        CFG logits as HF's TopKLogitsWarper then TopPLogitsWarper do (0 / 1 = off).  cfg_weight, temperature, top_k and
+        top_p may each hold one value per image (see sampling_plan).  A sequence of B seeds (with `offset` a scalar or B
+        offsets) draws image b as torch.multinomial(probs[b:b+1], 1) on its own generator at (seed[b], offset[b])."""
         B = logits.shape[0] // 2
         lg = logits.to(device=self.device, dtype=torch.float32).contiguous()
         x_next = torch.empty(2 * B, self.dims.D, device=self.device, dtype=torch.float32)
-        OPS.cfg_sample_embed(self.handle, lg, float(cfg_weight), float(temperature), _i64(seed), int(offset), bool(greedy), int(top_k),
-                             edit_region, gt_labels, int(step), int(n_steps), tokens_out, x_next, float(top_p))
+        plan = sampling_plan(B, cfg_weight, temperature, top_k, top_p, list(seed) if _is_seq(seed) else int(seed), 0)
+        if not plan.per_image:
+            OPS.cfg_sample_embed(self.handle, lg, float(cfg_weight), float(temperature), _i64(seed), int(offset), bool(greedy),
+                                 int(top_k), edit_region, gt_labels, int(step), int(n_steps), tokens_out, x_next, float(top_p))
+            return x_next
+        offs = [int(o) for o in offset] if _is_seq(offset) else [int(offset)] * B
+        if len(offs) != B:
+            raise ValueError(f"`offset` has {len(offs)} values for {B} images")
+        OPS.cfg_sample_embed_per_image(self.handle, lg, plan.cfg_weight, plan.temperature, plan.top_k, plan.top_p, plan.seed,
+                                       offs, plan.rng_per_image, bool(greedy), edit_region, gt_labels, int(step), int(n_steps),
+                                       tokens_out, x_next)
         return x_next
 
     def philox_offset_per_step(self, B: int) -> int:
@@ -415,17 +502,18 @@ class FastJanus:
         of batch['edit_region'] - the reference's datasets emit an all-zero edit_region for non-edit samples.
         `top_k` > 0 keeps the k largest CFG logits before the softmax (north_star (4); 0 = off = the reference).
         `top_p` < 1 then keeps the nucleus, as HF's TopPLogitsWarper after TopKLogitsWarper (1 = off = the reference).
-        None: the engine's defaults."""
+        None: the engine's defaults.
+        Per image: cfg_weight, temperature, top_k and top_p may each be a sequence / 1-D tensor of num_gen values, and
+        `generator` a sequence of num_gen CUDA generators or int seeds; image j then draws as
+        torch.multinomial(probs[j:j+1], 1, generator=generator[j]) would, from the generator's current offset, and each
+        generator is advanced by n draws on a (1, img_vocab) tensor.  See sampling_plan."""
         R, P, D = inputs_embeds.shape
         if R != 2 * num_gen:
             raise ValueError("inputs_embeds rows must be 2 * num_gen (interleaved cond/uncond)")
         n = int(image_token_num_per_image)
-        if isinstance(generator, torch.Generator):
-            seed, off = generator.initial_seed(), generator.get_offset()
-        else:
-            seed, off = int(self.seed if generator is None else generator), 0
-        if off != 0:
-            raise ValueError("generator must be freshly seeded (the reference reseeds per t2i call, :526)")
+        k = self.top_k if top_k is None else top_k
+        p = self.top_p if top_p is None else top_p
+        plan = sampling_plan(num_gen, cfg_weight, temperature, k, p, generator, self.seed)
         kv_start = (kv_start_from_mask(mask.to(self.device), P) if mask is not None
                     else torch.zeros(R, dtype=torch.int32, device=self.device))
         x = inputs_embeds.to(device=self.device, dtype=torch.float32).contiguous().clone()
@@ -434,25 +522,31 @@ class FastJanus:
         er = gl = None
         if teacher:
             er, gl = self._teacher_inputs(batch, gt_labels, num_gen, n)
-        k = int(self.top_k if top_k is None else top_k)
-        p = float(self.top_p if top_p is None else top_p)
         self._keep = (kv_start, x, er, gl)        # keep alive until the stream has consumed them
-        OPS.sample_image(self.handle, x, kv_start, n, float(cfg_weight), float(temperature), _i64(seed), bool(greedy), k, er, gl, tokens, p)
+        if not plan.per_image:
+            OPS.sample_image(self.handle, x, kv_start, n, float(cfg_weight), float(temperature), plan.seed[0], bool(greedy), int(k),
+                             er, gl, tokens, float(p))
+        else:
+            OPS.sample_image_per_image(self.handle, x, kv_start, n, plan.cfg_weight, plan.temperature, plan.top_k, plan.top_p,
+                                       plan.seed, plan.offset, plan.rng_per_image, bool(greedy), er, gl, tokens)
         self._serial += 1
-        if isinstance(generator, torch.Generator):
-            generator.set_offset(off + n * self.philox_offset_per_step(num_gen))
+        per_draw = self.philox_offset_per_step(1 if plan.rng_per_image else num_gen)
+        for g in plan.generators:
+            g.set_offset(g.get_offset() + n * per_draw)
         return tokens
 
     @torch.inference_mode()
     def t2i(self, inputs_ids=None, parallel_size=1, image_token_num_per_image=None, cfg_weight=5.0, temperature=1.0,
             img_size=None, patch_size=None, gt_image=None, batch=None, mask=None, tokens=None, emb=None,
             gt_labels=None, greedy: bool = False, use_teacher_forcing: Optional[bool] = None, top_k: Optional[int] = None,
-            top_p: Optional[float] = None):
+            top_p: Optional[float] = None, generator=None):
         """System.t2i (plangen_base.py:525-565), `tokens`/`emb` branches.  Returns (dec, mask_image).
         Teacher forcing (layout-guided editing, :528-532, :593-598, :557-562) follows `use_teacher_forcing` (default: the
         engine's flag, the counterpart of `args.use_teacher_forcing`): `gt_image` is encoded with the VQ encoder as the
         reference does (or ready-made `gt_labels` are used), and `mask_image` is returned.  With the flag off `gt_image` and
-        batch['edit_region'] are ignored, exactly as in the reference."""
+        batch['edit_region'] are ignored, exactly as in the reference.
+        cfg_weight, temperature, top_k, top_p and `generator` take per-image values as sample_image does, image
+        j = copy * B + b of the `parallel_size` copies; generator None: the engine's seed."""
         n = image_token_num_per_image or self.dims.n_img_tokens
         img_size = img_size or self.dims.img_size
         patch_size = patch_size or 2 ** (len(self.dims.vq_ch_mult) - 1)      # 16 for VQ-16
@@ -469,7 +563,7 @@ class FastJanus:
             inputs_embeds = emb
         mask = torch.cat([mask.to(self.device)] * parallel_size)
         num_gen = inputs_embeds.shape[0] // 2
-        gen = self.sample_image(inputs_embeds, num_gen, n, mask, cfg_weight, temperature, None, batch, gt_labels, greedy,
+        gen = self.sample_image(inputs_embeds, num_gen, n, mask, cfg_weight, temperature, generator, batch, gt_labels, greedy,
                                 use_teacher_forcing=teacher, top_k=top_k, top_p=top_p)
         g = img_size // patch_size
         dec = self.gen_vision_model.decode_code(gen.to(dtype=torch.int), shape=[num_gen, self.dims.code_dim, g, g])

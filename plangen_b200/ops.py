@@ -5,7 +5,8 @@ Every hot-path entry point of include/plangen_b200.h is registered with `torch.l
 with their mutated arguments, run on torch's CURRENT CUDA stream and can be traced / profiled like any other operator.
 The ops take the engine as an integer handle (`FastJanus.handle`); all tensors are CUDA tensors owned by the caller.
 There is no CPU implementation: a CPU tensor fails in the dispatcher, a missing shared library fails at import of
-`_lib` - nothing falls back.
+`_lib` - nothing falls back.  The *_per_image ops take one value per image as list arguments (seeds as two's-complement
+int64) and pass them to the C-ABI as a host array of pg_image_sampling.
 
     op                          C-ABI                         reference call (plangen_base.py)
     embed_tokens                pg_embed_tokens               language_model.get_input_embeddings()(ids)      :548
@@ -14,7 +15,9 @@ There is no CPU implementation: a CPU tensor fails in the dispatcher, a missing 
     gen_head                    pg_gen_head                   gen_head(h)                                     :579
     prepare_gen_img_embeds      pg_prepare_gen_img_embeds     prepare_gen_img_embeds(ids)                     :603
     cfg_sample_embed            pg_cfg_sample_embed           CFG + softmax + multinomial + embed             :580-604
+    cfg_sample_embed_per_image  pg_cfg_sample_embed_per_image the same with per-image settings and seeds
     sample_image                pg_sample_image               System.sample_image                             :567-607
+    sample_image_per_image      pg_sample_image_per_image     the same with per-image settings and seeds
     vq_decode_code              pg_vq_decode_code             gen_vision_model.decode_code                    :555
     vq_encode                   pg_vq_encode                  gen_vision_model.encode(img)[-1][-1]            :532
     prepare_inputs_embeds       pg_prepare_inputs_embeds      prepare_inputs_embeds                           :289,366,855
@@ -24,7 +27,7 @@ from __future__ import annotations
 
 import ctypes as C
 import weakref
-from typing import Optional
+from typing import List, Optional
 
 import torch
 
@@ -64,6 +67,21 @@ def _cuda(*ts):
 def _top_p(top_p: float):
     if not 0.0 <= float(top_p) <= 1.0:          # NaN fails too
         raise ValueError(f"`top_p` has to be a float in [0, 1], but is {top_p}")
+
+
+def _per_image(B: int, cfg_weight, temperature, top_k, top_p, seed, offset):
+    """pg_image_sampling[B] (a host array) from the per-image lists; seeds arrive as two's-complement int64."""
+    if any(len(v) != B for v in (cfg_weight, temperature, top_k, top_p, seed, offset)):
+        raise ValueError(f"per-image settings need {B} entries each")
+    arr = (_lib.PgImageSampling * B)()
+    for i in range(B):
+        if not 0.0 <= float(top_p[i]) <= 1.0:          # NaN fails too
+            raise ValueError(f"image {i}: `top_p` has to be a float in [0, 1], but is {top_p[i]}")
+        if int(top_k[i]) < 0:
+            raise ValueError(f"image {i}: `top_k` has to be >= 0, but is {top_k[i]}")
+        arr[i] = _lib.PgImageSampling(int(seed[i]) & 0xFFFFFFFFFFFFFFFF, int(offset[i]), float(cfg_weight[i]),
+                                      float(temperature[i]), int(top_k[i]), float(top_p[i]))
+    return arr
 
 
 @torch.library.custom_op(f"{NS}::embed_tokens", mutates_args=("out",), device_types="cuda")
@@ -107,6 +125,18 @@ def cfg_sample_embed(handle: int, logits: torch.Tensor, cfg_weight: float, tempe
                                           int(n_steps), _p(tokens_out), _p(x_next), _st(logits)))
 
 
+@torch.library.custom_op(f"{NS}::cfg_sample_embed_per_image", mutates_args=("tokens_out", "x_next"), device_types="cuda")
+def cfg_sample_embed_per_image(handle: int, logits: torch.Tensor, cfg_weight: List[float], temperature: List[float], top_k: List[int],
+                               top_p: List[float], seed: List[int], philox_offset: List[int], rng_per_image: bool, greedy: bool,
+                               edit_region: Optional[torch.Tensor], gt_labels: Optional[torch.Tensor], step: int, n_steps: int,
+                               tokens_out: torch.Tensor, x_next: torch.Tensor) -> None:
+    e = _eng(handle); _cuda(logits, edit_region, gt_labels, tokens_out, x_next)
+    B = logits.shape[0] // 2
+    pi = _per_image(B, cfg_weight, temperature, top_k, top_p, seed, philox_offset)
+    _lib.check(e._lib.pg_cfg_sample_embed_per_image(e._h, _p(logits), B, pi, int(rng_per_image), int(greedy), _p(edit_region),
+                                                    _p(gt_labels), int(step), int(n_steps), _p(tokens_out), _p(x_next), _st(logits)))
+
+
 @torch.library.custom_op(f"{NS}::sample_image", mutates_args=("x_prompt", "tokens_out"), device_types="cuda")
 def sample_image(handle: int, x_prompt: torch.Tensor, kv_start: torch.Tensor, n_steps: int, cfg_weight: float, temperature: float,
                  seed: int, greedy: bool, top_k: int, edit_region: Optional[torch.Tensor], gt_labels: Optional[torch.Tensor],
@@ -115,6 +145,18 @@ def sample_image(handle: int, x_prompt: torch.Tensor, kv_start: torch.Tensor, n_
     R, P = x_prompt.shape[0], x_prompt.shape[1]
     _lib.check(e._lib.pg_sample_image(e._h, _p(x_prompt), _p(kv_start), R, P, int(n_steps), float(cfg_weight), float(temperature),
                                       int(seed) & 0xFFFFFFFFFFFFFFFF, int(greedy), int(top_k), float(top_p), _p(edit_region), _p(gt_labels), _p(tokens_out), _st(x_prompt)))
+
+
+@torch.library.custom_op(f"{NS}::sample_image_per_image", mutates_args=("x_prompt", "tokens_out"), device_types="cuda")
+def sample_image_per_image(handle: int, x_prompt: torch.Tensor, kv_start: torch.Tensor, n_steps: int, cfg_weight: List[float],
+                           temperature: List[float], top_k: List[int], top_p: List[float], seed: List[int], philox_offset: List[int],
+                           rng_per_image: bool, greedy: bool, edit_region: Optional[torch.Tensor], gt_labels: Optional[torch.Tensor],
+                           tokens_out: torch.Tensor) -> None:
+    e = _eng(handle); _cuda(x_prompt, kv_start, edit_region, gt_labels, tokens_out)
+    R, P = x_prompt.shape[0], x_prompt.shape[1]
+    pi = _per_image(R // 2, cfg_weight, temperature, top_k, top_p, seed, philox_offset)
+    _lib.check(e._lib.pg_sample_image_per_image(e._h, _p(x_prompt), _p(kv_start), R, P, int(n_steps), pi, int(rng_per_image),
+                                                int(greedy), _p(edit_region), _p(gt_labels), _p(tokens_out), _st(x_prompt)))
 
 
 @torch.library.custom_op(f"{NS}::vq_decode_code", mutates_args=("image_out",), device_types="cuda")
@@ -146,4 +188,5 @@ def images_to_u8(handle: int, image: torch.Tensor, out: torch.Tensor) -> None:
 
 
 OP_NAMES = ("embed_tokens", "prefill", "decode_step", "gen_head", "prepare_gen_img_embeds", "cfg_sample_embed", "sample_image",
-            "vq_decode_code", "vq_encode", "prepare_inputs_embeds", "images_to_u8")
+            "vq_decode_code", "vq_encode", "prepare_inputs_embeds", "images_to_u8", "cfg_sample_embed_per_image",
+            "sample_image_per_image")
