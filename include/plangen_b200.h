@@ -20,7 +20,7 @@
 extern "C" {
 #endif
 
-#define PG_ABI_VERSION 4
+#define PG_ABI_VERSION 5
 
 /* arithmetic regimes */
 #define PG_MODE_BF16 0 /* the reference's regime: fp32 master weights under autocast(bf16), plangen_base.py:360 */
@@ -146,6 +146,42 @@ int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_start, int 
 int pg_sample_image_per_image(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
                               const pg_image_sampling* per_image, int rng_per_image, int greedy,
                               const int32_t* edit_region, const int32_t* gt_labels, int32_t* tokens_out, void* stream);
+
+/* Image-token log-probabilities.  For image b at step i the value is log p(tok) in fp32, p being exactly the
+ * distribution the sampler draws from (CFG rounded per op in the engine dtype, /temperature, top-k, top-p, softmax; in
+ * greedy mode top-k only) and tok the token emitted at that step, sampled or forced by teacher forcing:
+ * (t_tok - max) - log(sum of the kept e), HF compute_transition_scores(..., normalize_logits=True) on the processed
+ * scores.  A forced token a filter removed gets -inf; a kept one whose exp underflows still gets its finite value.
+ * Log-probs change no token, no Philox draw and no offset.  Scalar settings: pass a uniform pg_image_sampling array with
+ * rng_per_image = 0, which samples exactly as the scalar entries do. */
+
+/* pg_cfg_sample_embed_per_image plus logprobs_out fp32 [B, n_steps] (column `step` written). */
+int pg_cfg_sample_embed_logprobs(pg_engine* e, const float* logits, int B, const pg_image_sampling* per_image,
+                                 int rng_per_image, int greedy, const int32_t* edit_region, const int32_t* gt_labels,
+                                 int step, int n_steps, int32_t* tokens_out, float* x_next, float* logprobs_out,
+                                 void* stream);
+
+/* pg_sample_image_per_image plus logprobs_out fp32 [R/2, n_steps].  The log-probs are staged in the engine inside the
+ * captured graph (its key gains a log-probs flag; the settings still do not enter it) and copied out with the tokens. */
+int pg_sample_image_logprobs(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
+                             const pg_image_sampling* per_image, int rng_per_image, int greedy,
+                             const int32_t* edit_region, const int32_t* gt_labels, int32_t* tokens_out,
+                             float* logprobs_out, void* stream);
+
+/* Teacher-forced scoring of given image tokens in one pass: logprobs_out fp32 [R/2, n] = the log-probs (as above) the
+ * image loop would report with every token forced, computed by ONE prefill over prompt + image tokens (the reference's
+ * single full-sequence forward: fp32 residual stream, the prefill's rounding points - not the decode loop's bf16
+ * residual regime, so in bf16 the two are different valid evaluations), one wide gen_head contraction over all R * n
+ * positions (in chunks that fit the prefill scratch) and the sampler's reduction in score mode.
+ * x_seq fp32 [R, P + n - 1, D] (consumed): columns < P hold the prompt embeddings (LEFT padded, kv_start as for
+ * pg_prefill); columns P .. P + n - 2 are written here from the gen_aligner(gen_embed) table, token i at column P + i
+ * on both rows of the pair.  image_tokens int32 [R/2, n] (ids clamped to [0, img_vocab)); per_image HOST [R/2]
+ * (cfg_weight, temperature, top_k, top_p; seeds and offsets are unused).  R even, n <= max_steps and
+ * P + n - 1 <= max_prompt (build the engine with a larger max_prompt to score long sequences).  Overwrites the KV cache.
+ * No allocation; the prefill's host syncs are the only ones. */
+int pg_score_image_tokens(pg_engine* e, float* x_seq, const int32_t* kv_start, int R, int P, int n,
+                          const int32_t* image_tokens, const pg_image_sampling* per_image, float* logprobs_out,
+                          void* stream);
 
 /* replaces: System.x2t (plangen_base.py:513-523) = vl_gpt.language_model.generate(inputs_embeds=,
  *           attention_mask=, pad_token_id=, eos_token_id=, max_new_tokens=, do_sample=False, use_cache=True),

@@ -59,6 +59,14 @@ EXPORTS = {
     "pg_sample_image_per_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                             C.POINTER(PgImageSampling), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                             C.c_void_p]),
+    "pg_cfg_sample_embed_logprobs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(PgImageSampling), C.c_int, C.c_int,
+                                               C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                               C.c_void_p]),
+    "pg_sample_image_logprobs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                           C.POINTER(PgImageSampling), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_void_p]),
+    "pg_score_image_tokens": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                        C.POINTER(PgImageSampling), C.c_void_p, C.c_void_p]),
     "pg_generate_greedy": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_void_p, C.POINTER(C.c_int), C.c_void_p]),
     "pg_vq_decode_code": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
@@ -99,7 +107,7 @@ def load(build_if_missing: bool = True):
         fn = getattr(lib, name)      # AttributeError if the symbol is not exported
         fn.restype = res
         fn.argtypes = args
-    if lib.pg_abi_version() != 4:
+    if lib.pg_abi_version() != 5:
         raise PgError("ABI version mismatch")
     _LIB = lib
     return lib

@@ -102,6 +102,7 @@ struct pg_engine {
   // and scalars only (the caller's tensors are fresh allocations on every call)
   int32_t *st_kv_start = nullptr, *st_edit = nullptr, *st_gt = nullptr, *st_tokens = nullptr;
   ImageSampling* st_sampling = nullptr;               // per-image entry points: [B] settings (sample.cuh)
+  float* st_logprobs = nullptr;                       // pg_sample_image_logprobs: [B][n_steps]
   // mmu front-end (SigLIP tower + aligner + scatter, vit_kernels.cuh); carved only when dims.sig_layers > 0
   int sig_chunk = 0, sig_np = 0;                      // images per pass, patches per image
   float *sig_x = nullptr, *sig_part = nullptr;
@@ -394,6 +395,7 @@ static void layout_workspace(pg_engine* e, Carve& c) {
     e->st_gt = (int32_t*)c.take(B * std::max(d.max_steps, 1) * 4);
     e->st_tokens = (int32_t*)c.take(R * (size_t)e->Tmax * 4);      // image loop: [B][n_steps]; text loop: [R][max_new]
     e->st_sampling = (ImageSampling*)c.take(B * sizeof(ImageSampling));
+    e->st_logprobs = (float*)c.take(B * std::max(d.max_steps, 1) * 4);
   }
   if (d.sig_layers > 0 && d.max_images > 0) {
     // SigLIP tower scratch for one pass of sig_chunk images; features of ALL images stay (the scatter needs them)
@@ -835,15 +837,17 @@ extern "C" int pg_host_group_rows(const int32_t* start, const uint64_t* hash, in
 
 // a3: prompt prefill.  x fp32 [R*P, D] in place.
 static int prefill_impl(pg_engine* e, float* x, const int32_t* kv_start, int R, int P, float* hidden_out, int all_positions,
-                        bool rope_rel, void* stream);
+                        bool rope_rel, void* stream, int tail = 0);
 extern "C" int pg_prefill(pg_engine* e, float* x, const int32_t* kv_start, int R, int P, float* hidden_out,
                           int all_positions, void* stream) {
   return prefill_impl(e, x, kv_start, R, P, hidden_out, all_positions, false, stream);
 }
 // rope_rel: RoPE positions = column - kv_start[row] (what HF generate() derives from the attention mask, x2t);
-// otherwise absolute columns (the image loop calls LlamaModel.forward without position_ids)
+// otherwise absolute columns (the image loop calls LlamaModel.forward without position_ids).
+// tail > 0 (pg_score_image_tokens): no last-row output; instead the final-norm'ed hidden states of the last `tail` columns
+// of every row go to hbuf in the activation type, pair-major (row ((r / 2) * tail + i) * 2 + r % 2).
 static int prefill_impl(pg_engine* e, float* x, const int32_t* kv_start, int R, int P, float* hidden_out, int all_positions,
-                        bool rope_rel, void* stream) {
+                        bool rope_rel, void* stream, int tail) {
   TRY(check_ready(e));
   const pg_dims& d = e->d;
   if (R < 1 || R > d.max_rows || P < 1 || P > d.max_prompt) return fail("prefill shape R=%d P=%d exceeds engine limits", R, P);
@@ -995,6 +999,15 @@ static int prefill_impl(pg_engine* e, float* x, const int32_t* kv_start, int R, 
   }
   // final norm: all positions -> caller's buffer; last position of every row -> hidden_t for gen_head
   const float* last_part = fuse ? nullptr : e->part;      // fused: the last down projection is already in the stream
+  if (tail > 0) {
+    TRY(k_resid_norm(e, x, last_part, S, (size_t)tok * D, normw, e->xn, nullptr, tok, 1, 0, 0, st));
+    DISPATCH_T(e,
+               launch(e, gather_tail_rows_kernel<bf16>, dim3(tail, R), dim3(256), 0, st, (const bf16*)e->xn, (bf16*)e->hbuf, row_off,
+                      (const int32_t*)e->dup_of, kv_start, P, tail, D),
+               launch(e, gather_tail_rows_kernel<float>, dim3(tail, R), dim3(256), 0, st, (const float*)e->xn, (float*)e->hbuf, row_off,
+                      (const int32_t*)e->dup_of, kv_start, P, tail, D));
+    return 0;
+  }
   if (row_off != nullptr) {
     // packed: the last real token of every row
     if (packed_dups > 0)     // rows that repeat an earlier row: their K / V strips are copies
@@ -1091,19 +1104,19 @@ extern "C" int pg_decode_step(pg_engine* e, const float* x, const int32_t* kv_st
   return 0;
 }
 
-// gen_head GEMMs: hidden_t -> head_h -> logits partials in e->part.  Returns split count / stride.
-static int head_gemms(pg_engine* e, int R, int* S_out, cudaStream_t st) {
+// gen_head GEMMs: X (hidden_t, activation type) -> H (head_h) -> logits partials in e->part.  Returns split count / stride.
+static int head_gemms(pg_engine* e, const void* X, void* H, int R, int* S_out, cudaStream_t st) {
   const pg_dims& d = e->d;
   NEED(w0, void, "head.w0");
   NEED(b0, float, "head.b0");
   NEED(w1, void, "head.w1");
   int S = 1;
-  TRY(run_gemm(e, e->hidden_t, w0, R, d.img_embed, d.D, e->part, e->part_bytes, &S, st));
+  TRY(run_gemm(e, X, w0, R, d.img_embed, d.D, e->part, e->part_bytes, &S, st));
   const size_t total = (size_t)R * d.img_embed;
   DISPATCH_T(e,
-             launch(e, bias_act_kernel<bf16>, dim3(elementwise_blocks(e, total)), dim3(256), 0, st, e->part, S, total, b0, (bf16*)e->head_h, (float*)nullptr, d.img_embed, total, 1),
-             launch(e, bias_act_kernel<float>, dim3(elementwise_blocks(e, total)), dim3(256), 0, st, e->part, S, total, b0, (float*)e->head_h, (float*)nullptr, d.img_embed, total, 1));
-  TRY(run_gemm(e, e->head_h, w1, R, d.img_vocab, d.img_embed, e->part, e->part_bytes, &S, st));
+             launch(e, bias_act_kernel<bf16>, dim3(elementwise_blocks(e, total)), dim3(256), 0, st, e->part, S, total, b0, (bf16*)H, (float*)nullptr, d.img_embed, total, 1),
+             launch(e, bias_act_kernel<float>, dim3(elementwise_blocks(e, total)), dim3(256), 0, st, e->part, S, total, b0, (float*)H, (float*)nullptr, d.img_embed, total, 1));
+  TRY(run_gemm(e, H, w1, R, d.img_vocab, d.img_embed, e->part, e->part_bytes, &S, st));
   *S_out = S;
   return 0;
 }
@@ -1121,7 +1134,7 @@ extern "C" int pg_gen_head(pg_engine* e, const float* hidden, int R, float* logi
              launch(e, bias_act_kernel<bf16>, dim3(elementwise_blocks(e, n)), dim3(256), 0, st, hidden, 1, n, (const float*)nullptr, (bf16*)e->hidden_t, (float*)nullptr, d.D, n, 0),
              launch(e, bias_act_kernel<float>, dim3(elementwise_blocks(e, n)), dim3(256), 0, st, hidden, 1, n, (const float*)nullptr, (float*)e->hidden_t, (float*)nullptr, d.D, n, 0));
   int S = 1;
-  TRY(head_gemms(e, R, &S, st));
+  TRY(head_gemms(e, e->hidden_t, e->head_h, R, &S, st));
   const size_t total = (size_t)R * d.img_vocab;
   DISPATCH_T(e,
              launch(e, bias_act_kernel<bf16>, dim3(elementwise_blocks(e, total)), dim3(256), 0, st, e->part, S, total, b1, (bf16*)nullptr, logits_out, d.img_vocab, total, 0),
@@ -1159,7 +1172,7 @@ static int k_sample(pg_engine* e, const float* part, int S, size_t sstride, cons
                     float temperature, uint64_t seed, uint64_t offset_base, int greedy, int top_k, double top_p,
                     const int32_t* edit_region, const int32_t* gt_labels, int step_base, const int* step_ptr, int n_steps,
                     int32_t* tokens_out, float* x_next, const float* next_norm_w, void* xn_next, cudaStream_t st,
-                    const PerImage* pi = nullptr) {
+                    const PerImage* pi = nullptr, float* logprobs = nullptr, int score_n = 0) {
   const pg_dims& d = e->d;
   uint64_t per_step, stride;
   philox_policy(e, philox_numel(e, B, pi), &per_step, &stride);
@@ -1176,11 +1189,11 @@ static int k_sample(pg_engine* e, const float* part, int S, size_t sstride, cons
              launch(e, cfg_sample_embed_cluster_kernel<bf16>, dim3(B * SAMPLE_CLUSTER), dim3(SAMPLE_CL_THREADS), csm, st, part, S, sstride, bias, B, d.img_vocab,
                     cfg_weight, temperature, seed, offset_base, per_step, stride, greedy, top_k, top_p_thr, edit_region, gt_labels,
                     step_base, step_ptr, n_steps, tokens_out, (const bf16*)e->embed_table, d.D, x_next, next_norm_w, (bf16*)xn_next,
-                    d.rms_eps, 1, e->dbg_logits, pi ? pi->dev : nullptr, pi ? pi->rng_per_image : 0),
+                    d.rms_eps, 1, score_n ? nullptr : e->dbg_logits, pi ? pi->dev : nullptr, pi ? pi->rng_per_image : 0, logprobs, score_n),
              launch(e, cfg_sample_embed_cluster_kernel<float>, dim3(B * SAMPLE_CLUSTER), dim3(SAMPLE_CL_THREADS), csm, st, part, S, sstride, bias, B, d.img_vocab,
                     cfg_weight, temperature, seed, offset_base, per_step, stride, greedy, top_k, top_p_thr, edit_region, gt_labels,
                     step_base, step_ptr, n_steps, tokens_out, (const float*)e->embed_table, d.D, x_next, next_norm_w, (float*)xn_next,
-                    d.rms_eps, 0, e->dbg_logits, pi ? pi->dev : nullptr, pi ? pi->rng_per_image : 0));
+                    d.rms_eps, 0, score_n ? nullptr : e->dbg_logits, pi ? pi->dev : nullptr, pi ? pi->rng_per_image : 0, logprobs, score_n));
   return 0;
 }
 
@@ -1229,10 +1242,10 @@ static int stage_per_image(pg_engine* e, const StagedSampling& ss, cudaStream_t 
   return 0;
 }
 
-extern "C" int pg_cfg_sample_embed_per_image(pg_engine* e, const float* logits, int B, const pg_image_sampling* per_image,
-                                             int rng_per_image, int greedy, const int32_t* edit_region,
-                                             const int32_t* gt_labels, int step, int n_steps, int32_t* tokens_out,
-                                             float* x_next, void* stream) {
+static int cfg_sample_embed_per_image(pg_engine* e, const float* logits, int B, const pg_image_sampling* per_image,
+                                      int rng_per_image, int greedy, const int32_t* edit_region, const int32_t* gt_labels,
+                                      int step, int n_steps, int32_t* tokens_out, float* x_next, float* logprobs_out,
+                                      void* stream) {
   TRY(check_ready(e));
   if (B < 1 || 2 * B > e->d.max_rows) return fail("sample B=%d exceeds engine limits", B);
   if (step < 0 || step >= n_steps) return fail("step %d out of range", step);
@@ -1243,7 +1256,24 @@ extern "C" int pg_cfg_sample_embed_per_image(pg_engine* e, const float* logits, 
   PerImage pi;
   TRY(stage_per_image(e, ss, st, &pi));
   return k_sample(e, logits, 1, 0, nullptr, B, 0.f, 1.f, 0, 0, greedy, 0, 1.0, edit_region, gt_labels, step, nullptr,
-                  n_steps, tokens_out, x_next, nullptr, nullptr, st, &pi);
+                  n_steps, tokens_out, x_next, nullptr, nullptr, st, &pi, logprobs_out);
+}
+
+extern "C" int pg_cfg_sample_embed_per_image(pg_engine* e, const float* logits, int B, const pg_image_sampling* per_image,
+                                             int rng_per_image, int greedy, const int32_t* edit_region,
+                                             const int32_t* gt_labels, int step, int n_steps, int32_t* tokens_out,
+                                             float* x_next, void* stream) {
+  return cfg_sample_embed_per_image(e, logits, B, per_image, rng_per_image, greedy, edit_region, gt_labels, step, n_steps,
+                                    tokens_out, x_next, nullptr, stream);
+}
+
+extern "C" int pg_cfg_sample_embed_logprobs(pg_engine* e, const float* logits, int B, const pg_image_sampling* per_image,
+                                            int rng_per_image, int greedy, const int32_t* edit_region,
+                                            const int32_t* gt_labels, int step, int n_steps, int32_t* tokens_out,
+                                            float* x_next, float* logprobs_out, void* stream) {
+  if (!logprobs_out) return fail("null argument");
+  return cfg_sample_embed_per_image(e, logits, B, per_image, rng_per_image, greedy, edit_region, gt_labels, step, n_steps,
+                                    tokens_out, x_next, logprobs_out, stream);
 }
 
 extern "C" int pg_prepare_gen_img_embeds(pg_engine* e, const int32_t* ids, int n, float* out, void* stream) {
@@ -1262,19 +1292,19 @@ extern "C" int pg_prepare_gen_img_embeds(pg_engine* e, const int32_t* ids, int n
 static int one_step(pg_engine* e, const int32_t* kv_start, int R, int P, int n_steps, float cfg_weight, float temperature,
                     uint64_t seed, int greedy, int top_k, double top_p, const int32_t* edit_region,
                     const int32_t* gt_labels, int32_t* tokens_out, bool with_lm, int step_host, cudaStream_t st,
-                    const PerImage* pi) {
+                    const PerImage* pi, float* logprobs) {
   NEED(b1, float, "head.b1");
   LayerW w0;
   TRY(layer_weights(e, 0, &w0));
   int S = 1;
-  TRY(head_gemms(e, R, &S, st));
+  TRY(head_gemms(e, e->hidden_t, e->head_h, R, &S, st));
   const bool host = step_host >= 0;
   uint64_t per_step, stride;
   philox_policy(e, philox_numel(e, R / 2, pi), &per_step, &stride);
   TRY(k_sample(e, e->part, S, (size_t)R * e->d.img_vocab, b1, R / 2, cfg_weight, temperature, seed,
                host ? per_step * (uint64_t)step_host : 0, greedy, top_k, top_p, edit_region, gt_labels, host ? step_host : 0,
                host ? nullptr : e->step_ctr, n_steps, tokens_out, with_lm ? e->x_dec : nullptr, w0.ln1,
-               with_lm ? e->xn : nullptr, st, pi));
+               with_lm ? e->xn : nullptr, st, pi, logprobs));
   if (with_lm)
     TRY(decode_layers(e, kv_start, R, host ? P + step_host : P, host ? nullptr : e->step_ctr, true, !host,
                       P + n_steps / 2, st, 0, P));
@@ -1325,7 +1355,7 @@ static int check_image_loop(pg_engine* e, const int32_t* kv_start, int R, int n_
 static int image_loop(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
                       float cfg_weight, float temperature, uint64_t seed, int greedy, int top_k, double top_p,
                       const int32_t* edit_region, const int32_t* gt_labels, int32_t* tokens_out, void* stream,
-                      const StagedSampling* per_image) {
+                      const StagedSampling* per_image, float* logprobs_out = nullptr) {
   cudaStream_t user = (cudaStream_t)stream;
   cudaStream_t st = e->own_stream;
   const int B = R / 2;
@@ -1347,6 +1377,7 @@ static int image_loop(pg_engine* e, float* x_prompt, const int32_t* kv_start, in
   const int32_t* er = edit_region ? e->st_edit : nullptr;
   const int32_t* gl = edit_region ? e->st_gt : nullptr;
   int32_t* toks = e->st_tokens;
+  float* lps = logprobs_out ? e->st_logprobs : nullptr;
   TRY(pg_prefill(e, x_prompt, kvs, R, P, nullptr, 0, (void*)st));
   CK(cudaMemsetAsync(e->step_ctr, 0, 4, st));
   if (n_steps > 1) {
@@ -1354,8 +1385,8 @@ static int image_loop(pg_engine* e, float* x_prompt, const int32_t* kv_start, in
       char key[256];
       const int prof = (e->prof_buf && e->prof_step >= 0) ? 1 : 0;
       if (pi)   // the settings are read from st_sampling: one graph serves every seed and setting of this shape
-        snprintf(key, sizeof(key), "imgpi/%d/%d/%d/%d/%d/%d/%d/%d", R, P, n_steps, greedy, edit_region ? 1 : 0,
-                 pi->rng_per_image, pi->any_top_p ? 1 : 0, prof);
+        snprintf(key, sizeof(key), "imgpi/%d/%d/%d/%d/%d/%d/%d/%d/%d", R, P, n_steps, greedy, edit_region ? 1 : 0,
+                 pi->rng_per_image, pi->any_top_p ? 1 : 0, lps ? 1 : 0, prof);
       else
         snprintf(key, sizeof(key), "img/%d/%d/%d/%a/%a/%llu/%d/%d/%a/%d/%d", R, P, n_steps, cfg_weight, temperature,
                  (unsigned long long)seed, greedy, top_k, top_p, edit_region ? 1 : 0, prof);
@@ -1363,7 +1394,7 @@ static int image_loop(pg_engine* e, float* x_prompt, const int32_t* kv_start, in
       TRY(graph_for(e, key, st, [&]() {
         e->prof_active = (e->prof_buf != nullptr && e->prof_step >= 0);
         e->prof_slot = 0;
-        int rc = one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, true, -1, st, pi);
+        int rc = one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, true, -1, st, pi, lps);
         e->prof_active = false;
         return rc;
       }, &ge));
@@ -1386,7 +1417,7 @@ static int image_loop(pg_engine* e, float* x_prompt, const int32_t* kv_start, in
           CK(cudaMemsetAsync(e->prof_buf, 0xFF, PROF_SLOTS * 8, st));
           CK(cudaMemsetAsync(e->prof_buf + PROF_SLOTS, 0, PROF_SLOTS * 8, st));
         }
-        int rc = one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, true, i, st, pi);
+        int rc = one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, true, i, st, pi, lps);
         if (e->prof_active)
           CK(cudaMemcpyAsync(e->prof_buf + 2 * PROF_SLOTS, e->prof_buf, 2 * PROF_SLOTS * 8, cudaMemcpyDeviceToDevice, st));
         e->prof_active = false;
@@ -1395,8 +1426,9 @@ static int image_loop(pg_engine* e, float* x_prompt, const int32_t* kv_start, in
     }
   }
   // last token: head + sample only (the reference computes and drops one more embed, SURVEY appendix A.12)
-  TRY(one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, false, n_steps - 1, st, pi));
+  TRY(one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, false, n_steps - 1, st, pi, lps));
   CK(cudaMemcpyAsync(tokens_out, toks, tok_bytes, cudaMemcpyDeviceToDevice, st));
+  if (lps) CK(cudaMemcpyAsync(logprobs_out, lps, tok_bytes, cudaMemcpyDeviceToDevice, st));
   CK(cudaEventRecord(e->ev_out, st));
   CK(cudaStreamWaitEvent(user, e->ev_out, 0));
   return 0;
@@ -1421,6 +1453,65 @@ extern "C" int pg_sample_image_per_image(pg_engine* e, float* x_prompt, const in
   TRY(convert_per_image(per_image, R / 2, rng_per_image, &ss));
   return image_loop(e, x_prompt, kv_start, R, P, n_steps, 0.f, 1.f, 0, greedy, 0, 1.0, edit_region, gt_labels,
                     tokens_out, stream, &ss);
+}
+
+extern "C" int pg_sample_image_logprobs(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
+                                        const pg_image_sampling* per_image, int rng_per_image, int greedy,
+                                        const int32_t* edit_region, const int32_t* gt_labels, int32_t* tokens_out,
+                                        float* logprobs_out, void* stream) {
+  TRY(check_image_loop(e, kv_start, R, n_steps, edit_region, gt_labels, tokens_out));
+  if (!logprobs_out) return fail("null argument");
+  StagedSampling ss;
+  TRY(convert_per_image(per_image, R / 2, rng_per_image, &ss));
+  return image_loop(e, x_prompt, kv_start, R, P, n_steps, 0.f, 1.f, 0, greedy, 0, 1.0, edit_region, gt_labels,
+                    tokens_out, stream, &ss, logprobs_out);
+}
+
+// ------------------------------------------------------------------------------ teacher-forced scoring
+// One prefill over prompt + image tokens, the hidden states of columns P-1 .. P+n-2 pair-major in hbuf (prefill_impl's
+// `tail`), gen_head over those R * n rows in as few wide contractions as the idle prefill scratch allows (part holds one
+// chunk's logits, qbuf its first-layer activations), and the sampler kernel in score mode per chunk.
+extern "C" int pg_score_image_tokens(pg_engine* e, float* x_seq, const int32_t* kv_start, int R, int P, int n,
+                                     const int32_t* image_tokens, const pg_image_sampling* per_image, float* logprobs_out,
+                                     void* stream) {
+  TRY(check_ready(e));
+  const pg_dims& d = e->d;
+  if (!x_seq || !kv_start || !image_tokens || !logprobs_out) return fail("null argument");
+  if (R < 2 || R % 2) return fail("score R=%d: R must be even (interleaved cond/uncond rows) and >= 2", R);
+  if (R > d.max_rows) return fail("score R=%d exceeds the engine's max_rows %d", R, d.max_rows);
+  if (P < 1) return fail("score P=%d: the prompt needs at least one column", P);
+  if (n < 1 || n > d.max_steps) return fail("score n=%d exceeds the engine's max_steps %d", n, d.max_steps);
+  const int T = P + n - 1;
+  if (T > d.max_prompt)
+    return fail("score: prompt + image tokens - 1 = %d columns exceed the engine's max_prompt %d (the prefill limit)", T,
+                d.max_prompt);
+  if (d.F < d.D) return fail("score needs F >= D (the gathered hidden states live in the prefill's MLP scratch)");
+  NEED(b1, float, "head.b1");
+  StagedSampling ss;
+  TRY(convert_per_image(per_image, R / 2, 0, &ss));
+  cudaStream_t st = (cudaStream_t)stream;
+  PerImage pi;
+  TRY(stage_per_image(e, ss, st, &pi));
+  if (n > 1)
+    DISPATCH_T(e,
+               launch(e, score_embed_kernel<bf16>, dim3(n - 1, R), dim3(256), 0, st, image_tokens, (const bf16*)e->embed_table,
+                      x_seq, P, T, n, d.D, d.img_vocab),
+               launch(e, score_embed_kernel<float>, dim3(n - 1, R), dim3(256), 0, st, image_tokens, (const float*)e->embed_table,
+                      x_seq, P, T, n, d.D, d.img_vocab));
+  TRY(prefill_impl(e, x_seq, kv_start, R, T, nullptr, 0, false, stream, n));
+  const size_t rows = (size_t)R * n;
+  size_t cap = e->part_bytes / ((size_t)std::max(d.img_vocab, d.img_embed) * 4);          // one split of logits
+  cap = std::min(cap, (size_t)d.max_rows * d.max_prompt * e->HD / d.img_embed);          // first-layer rows in qbuf
+  cap &= ~(size_t)1;
+  if (cap < 2) return fail("score: the prefill scratch holds no pair of logit rows");
+  for (size_t r0 = 0; r0 < rows; r0 += cap) {
+    const int M = (int)std::min(cap, rows - r0);
+    int S = 1;
+    TRY(head_gemms(e, (const char*)e->hbuf + r0 * d.D * e->esz, e->qbuf, M, &S, st));
+    TRY(k_sample(e, e->part, S, (size_t)M * d.img_vocab, b1, M / 2, 0.f, 1.f, 0, 0, 0, 0, 1.0, nullptr, image_tokens,
+                 (int)(r0 / 2), nullptr, n, nullptr, nullptr, nullptr, nullptr, st, &pi, logprobs_out, n));
+  }
+  return 0;
 }
 
 // ------------------------------------------------------------------------------ f1: stage-1 text decode (x2t)

@@ -520,6 +520,21 @@ gather_last_rows_kernel(const float* __restrict__ xp, float* __restrict__ out, c
   for (int i = threadIdx.x; i < D / 4; i += blockDim.x) dst[i] = src[i];
 }
 
+// teacher-forced scoring: the hidden states of the last `ncols` columns of every row (of the row it duplicates when
+// packed), pair-major: column P - ncols + i of row r -> out[((r / 2) * ncols + i) * 2 + r % 2].  grid (ncols, R)
+template <typename T>
+__global__ void __launch_bounds__(256)
+gather_tail_rows_kernel(const T* __restrict__ src, T* __restrict__ out, const int32_t* __restrict__ row_off,
+                        const int32_t* __restrict__ dup_of, const int32_t* __restrict__ kv_start, int P, int ncols, int D) {
+  pdl_launch_dependents();
+  pdl_wait();
+  const int i = blockIdx.x, r = blockIdx.y, col = P - ncols + i;
+  const size_t pos = row_off ? (size_t)row_off[dup_of[r]] + max(col - kv_start[r], 0) : (size_t)r * P + col;
+  const T* s = src + pos * D;
+  T* o = out + ((size_t)((r / 2) * ncols + i) * 2 + (r & 1)) * D;
+  for (int d = threadIdx.x; d < D; d += blockDim.x) o[d] = s[d];
+}
+
 // Prefill variant behind the contraction's fused bf16 epilogue (gemm.cuh EpiFuse): the projections arrive already
 // rounded to bf16 ([tok][3*H*128], q | k | v), so this kernel only rotates and scatters - same values as
 // qkv_rope_store_kernel<bf16> on the fp32 partials (it rounds them first), half the bytes.

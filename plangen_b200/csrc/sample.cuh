@@ -77,6 +77,13 @@ __device__ unsigned long long* g_sample_dbg = nullptr;   // debug timeline (tool
 // requests.  rng_per_image != 0 draws image b's variates at element v of a (1, V) tensor (stride and per-step offset of
 // numel = V, chosen by the host) instead of b * V + v: the image's tokens then depend only on its own seed and offset,
 // as torch.multinomial(probs[b:b+1], 1, generator=g_b) would draw them, not on its position or the batch size.
+//
+// logprobs != nullptr: log p(tok) of the distribution the draw uses (after top-k and top-p) goes to
+// logprobs[image * n_steps + step], written by the thread that visited tok in the filter loops: (t_tok - mx) - log(sum)
+// in fp32, t_tok recomputed from the partials with the same rounded ops (sh may hold e by then, and a kept e_tok may
+// underflow to 0), -inf when a filter removed tok (only a forced token can be removed).
+// score_n > 0 (teacher-forced scoring): cluster b scores the pair g = step_base + b, image g / score_n, position
+// g % score_n (n_steps == score_n); the token is always gt_labels[g], no variates are drawn and there is no arg-max.
 constexpr int SAMPLE_CLUSTER = 8;
 
 // device copy of one pg_image_sampling entry (engine.cu converts top_p to the threshold the kernel compares with)
@@ -181,6 +188,16 @@ PG_DEVINL uint32_t cluster_radix_select(W (*hist)[256], W* hsum, W* sel_w, uint3
   return prefix;
 }
 
+// t of one vocabulary entry from its cond / uncond logits (bias added): plangen_base.py:587-588, one rounded op each
+template <typename T>
+PG_DEVINL float cfg_scaled_logit(float c, float u, float cfg_weight, float temperature) {
+  c = Act<T>::rnd(c); u = Act<T>::rnd(u);
+  float t = Act<T>::rnd(__fsub_rn(c, u));
+  t = Act<T>::rnd(__fmul_rn(cfg_weight, t));
+  t = Act<T>::rnd(__fadd_rn(u, t));
+  return Act<T>::rnd(__fdiv_rn(t, temperature));
+}
+
 template <typename T>
 __global__ void __cluster_dims__(SAMPLE_CLUSTER, 1, 1) __launch_bounds__(SAMPLE_CL_THREADS)
 cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t split_stride, const float* __restrict__ bias,
@@ -191,7 +208,8 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
                                 int32_t* __restrict__ tokens_out, const T* __restrict__ embed_table, int D,
                                 float* __restrict__ x_next, const float* __restrict__ next_norm_w, T* __restrict__ xn_next,
                                 float eps, int round_resid, float* __restrict__ dbg_logits,
-                                const ImageSampling* __restrict__ per_image, int rng_per_image) {
+                                const ImageSampling* __restrict__ per_image, int rng_per_image,
+                                float* __restrict__ logprobs, int score_n) {
   extern __shared__ __align__(16) float sh[];   // this CTA's slice of the CFG logits -> unnormalised probabilities
   // top_p_thr >= 0 (top-p on): sh is followed by the slice's logits t and the mass histograms of its radix select
   __shared__ uint32_t hist[4][256];  // top-k radix select: one histogram per pass (read by the other CTAs)
@@ -211,11 +229,12 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
   const int v_lo = (int)rank * chunk, v_hi = min(V, v_lo + chunk);
   // The step counter is only written by the last kernel of a decode step; graph replays are fully ordered, and with plain
   // launches the host passes the step explicitly (step_ptr == nullptr), so reading it before the PDL wait is safe.
-  const int step = step_base + (step_ptr ? *step_ptr : 0);
+  const int step = score_n ? (step_base + b) % score_n : step_base + (step_ptr ? *step_ptr : 0);
+  const int img = score_n ? (step_base + b) / score_n : b;
   // The per-image settings are staged by a copy before the decode loop, never written by a kernel of the loop, so they
   // are read before the PDL wait too: the Philox prefetch below needs the image's seed and offset.
   if (per_image != nullptr) {
-    const ImageSampling s = per_image[b];
+    const ImageSampling s = per_image[img];
     cfg_weight = s.cfg_weight; temperature = s.temperature; top_k = s.top_k; top_p_thr = s.top_p_thr;
     seed = s.seed; offset_base += s.offset;
   }
@@ -224,7 +243,7 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
   // are drawn while the head contraction is still streaming its weights (this kernel is launched ahead of its dependency).
   constexpr int QPRE = 8;
   float qpre[QPRE];
-  const bool pre = !greedy && (v_hi - v_lo) <= QPRE * SAMPLE_CL_THREADS;
+  const bool pre = !greedy && !score_n && (v_hi - v_lo) <= QPRE * SAMPLE_CL_THREADS;
   if (pre) {
 #pragma unroll
     for (int j = 0; j < QPRE; ++j) {
@@ -243,6 +262,14 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
   }
   pdl_wait();
   SAMPLE_STAMP(1);
+  // log-probs: the token teacher forcing (or score mode) imposes, -1 if none, read again where it is needed (the kernel
+  // is at its register limit); `gone` marks it removed by a filter in the thread that visits it
+  auto forced_token = [&]() -> int {
+    const size_t at = (size_t)img * n_steps + step;
+    if (logprobs == nullptr || !(score_n || (edit_region != nullptr && __ldcg(edit_region + at) == 0))) return -1;
+    return min(max(__ldcg(gt_labels + at), 0), V - 1);
+  };
+  bool gone = false;
   const size_t rc = (size_t)(2 * b) * V, ru = (size_t)(2 * b + 1) * V;
   float mx = -INFINITY;
   for (int v0 = v_lo + tid, it = 0; v0 < v_hi; v0 += QPRE * SAMPLE_CL_THREADS, ++it) {
@@ -262,11 +289,7 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
       if (v < v_hi) {
         float c = cs[j], u = us[j];
         if (bias) { const float bb = (bias_pre && it == 0) ? bias_r[j] : bias[v]; c += bb; u += bb; }
-        c = Act<T>::rnd(c); u = Act<T>::rnd(u);
-        float t = Act<T>::rnd(__fsub_rn(c, u));           // plangen_base.py:587-588, one rounded op each
-        t = Act<T>::rnd(__fmul_rn(cfg_weight, t));
-        t = Act<T>::rnd(__fadd_rn(u, t));
-        t = Act<T>::rnd(__fdiv_rn(t, temperature));
+        const float t = cfg_scaled_logit<T>(c, u, cfg_weight, temperature);
         sh[v - v_lo] = t;
         if (dbg_logits) dbg_logits[((size_t)step * B + b) * V + v] = t;
         mx = fmaxf(mx, t);
@@ -275,6 +298,7 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
   }
   SAMPLE_STAMP(2);
   if (top_k > 0 && top_k < V) {
+    const int ftok = forced_token();
     // k-th largest CFG logit of the image = the largest key with at most V - k keys below it
     uint32_t below;
     const uint32_t kth = cluster_radix_select<uint32_t>(
@@ -284,7 +308,7 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
     mx = -INFINITY;
     for (int v = v_lo + tid; v < v_hi; v += SAMPLE_CL_THREADS) {
       float t = sh[v - v_lo];
-      if (sample_order_key(t) < kth) { t = -INFINITY; sh[v - v_lo] = t; }
+      if (sample_order_key(t) < kth) { t = -INFINITY; sh[v - v_lo] = t; gone |= v == ftok; }
       mx = fmaxf(mx, t);
     }
   }
@@ -344,6 +368,7 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
     const int lane = tid & 31, warp = tid >> 5;
     int seen = first;                                        // group members before this iteration's elements
     float kept = 0.f;
+    const int ftok = forced_token();
     for (int v0 = v_lo; v0 < v_hi; v0 += SAMPLE_CL_THREADS) {
       const int v = v0 + tid;
       const uint32_t k = v < v_hi ? sample_order_key(tsh[v - v_lo]) : 0u;
@@ -361,7 +386,7 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
       seen += all;
       if (v < v_hi) {
         float e = sh[v - v_lo];
-        if (k < kb || (tie && (u64)before < drop)) { e = 0.f; sh[v - v_lo] = e; }
+        if (k < kb || (tie && (u64)before < drop)) { e = 0.f; sh[v - v_lo] = e; gone |= v == ftok; }
         kept += e;
       }
     }
@@ -372,62 +397,77 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
 #pragma unroll
     for (uint32_t r = 0; r < SAMPLE_CLUSTER; ++r) sum += __uint_as_float(dsmem_ld_u32(&xc.sum, r));
   }
-  // argmax over p/q (first index wins ties, like torch.argmax)
-  float bv = -INFINITY;
-  int bi = 0x7fffffff;
-  if (pre) {
+  int tok = score_n ? forced_token() : 0;
+  if (!score_n) {
+    // argmax over p/q (first index wins ties, like torch.argmax)
+    float bv = -INFINITY;
+    int bi = 0x7fffffff;
+    if (pre) {
 #pragma unroll
-    for (int j = 0; j < QPRE; ++j) {
-      const int v = v_lo + tid + j * SAMPLE_CL_THREADS;
-      if (v < v_hi) {
-        const float score = __fdiv_rn(__fdiv_rn(sh[v - v_lo], sum), qpre[j]);
+      for (int j = 0; j < QPRE; ++j) {
+        const int v = v_lo + tid + j * SAMPLE_CL_THREADS;
+        if (v < v_hi) {
+          const float score = __fdiv_rn(__fdiv_rn(sh[v - v_lo], sum), qpre[j]);
+          if (score > bv || (score == bv && v < bi)) { bv = score; bi = v; }
+        }
+      }
+    } else {
+      for (int v = v_lo + tid; v < v_hi; v += SAMPLE_CL_THREADS) {
+        const float p = __fdiv_rn(sh[v - v_lo], sum);
+        float score = p;
+        if (!greedy) {
+          const float q = torch_exponential_at((rng_per_image ? 0 : (uint64_t)b * V) + v, philox_stride, seed, offset);
+          score = __fdiv_rn(p, q);
+        }
         if (score > bv || (score == bv && v < bi)) { bv = score; bi = v; }
       }
     }
-  } else {
-    for (int v = v_lo + tid; v < v_hi; v += SAMPLE_CL_THREADS) {
-      const float p = __fdiv_rn(sh[v - v_lo], sum);
-      float score = p;
-      if (!greedy) {
-        const float q = torch_exponential_at((rng_per_image ? 0 : (uint64_t)b * V) + v, philox_stride, seed, offset);
-        score = __fdiv_rn(p, q);
-      }
-      if (score > bv || (score == bv && v < bi)) { bv = score; bi = v; }
-    }
-  }
-  SAMPLE_STAMP(4);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
-    const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-    if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
-  }
-  if ((tid & 31) == 0) { bestv[tid >> 5] = bv; besti[tid >> 5] = bi; }
-  __syncthreads();
-  if (tid < 32) {
-    const bool have = tid < SAMPLE_CL_THREADS / 32;          // one entry per warp of this CTA
-    bv = have ? bestv[tid] : -INFINITY; bi = have ? besti[tid] : 0x7fffffff;
+    SAMPLE_STAMP(4);
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
       const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
       const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
       if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
     }
-    if (tid == 0) { xc.bv = bv; xc.bi = bi; }
-  }
-  cluster_sync_all();
-  bv = -INFINITY; bi = 0x7fffffff;
+    if ((tid & 31) == 0) { bestv[tid >> 5] = bv; besti[tid >> 5] = bi; }
+    __syncthreads();
+    if (tid < 32) {
+      const bool have = tid < SAMPLE_CL_THREADS / 32;          // one entry per warp of this CTA
+      bv = have ? bestv[tid] : -INFINITY; bi = have ? besti[tid] : 0x7fffffff;
 #pragma unroll
-  for (uint32_t r = 0; r < SAMPLE_CLUSTER; ++r) {
-    const float ov = __uint_as_float(dsmem_ld_u32(&xc.bv, r));
-    const int oi = (int)dsmem_ld_u32(&xc.bi, r);
-    if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+      for (int o = 16; o > 0; o >>= 1) {
+        const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+        const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+        if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+      }
+      if (tid == 0) { xc.bv = bv; xc.bi = bi; }
+    }
+    cluster_sync_all();
+    bv = -INFINITY; bi = 0x7fffffff;
+#pragma unroll
+    for (uint32_t r = 0; r < SAMPLE_CLUSTER; ++r) {
+      const float ov = __uint_as_float(dsmem_ld_u32(&xc.bv, r));
+      const int oi = (int)dsmem_ld_u32(&xc.bi, r);
+      if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+    }
+    tok = bi;
+    // teacher forcing (plangen_base.py:593-598): outside the edit region keep the ground truth
+    if (edit_region != nullptr && edit_region[(size_t)b * n_steps + step] == 0) tok = gt_labels[(size_t)b * n_steps + step];
+    tok = min(max(tok, 0), V - 1);
+    if (rank == 0 && tid == 0) tokens_out[(size_t)b * n_steps + step] = tok;
   }
-  int tok = bi;
-  // teacher forcing (plangen_base.py:593-598): outside the edit region keep the ground truth
-  if (edit_region != nullptr && edit_region[(size_t)b * n_steps + step] == 0) tok = gt_labels[(size_t)b * n_steps + step];
-  tok = min(max(tok, 0), V - 1);
-  if (rank == 0 && tid == 0) tokens_out[(size_t)b * n_steps + step] = tok;
+  if (logprobs != nullptr && tok >= v_lo && tok < v_hi && tid == (tok - v_lo) % SAMPLE_CL_THREADS) {
+    // the settings are read again rather than kept in registers across the filters (the kernel is at its register limit)
+    const float w = per_image ? __ldcg(&per_image[img].cfg_weight) : cfg_weight;
+    const float temp = per_image ? __ldcg(&per_image[img].temperature) : temperature;
+    const size_t c_at = (size_t)(2 * b) * V + tok, u_at = c_at + V;
+    float c, u;
+    if (S == 1) { c = __ldcg(part + c_at); u = __ldcg(part + u_at); }
+    else { c = reduce_splits(part, S, split_stride, c_at); u = reduce_splits(part, S, split_stride, u_at); }
+    if (bias) { c += bias[tok]; u += bias[tok]; }
+    const float t = cfg_scaled_logit<T>(c, u, w, temp);
+    logprobs[(size_t)img * n_steps + step] = gone ? -INFINITY : (t - mx) - logf(sum);
+  }
   SAMPLE_STAMP(5);
   if (x_next == nullptr) { cluster_sync_all(); return; }   // nobody may exit while its xc can still be read
   // next input = gen_aligner(gen_embed(tok)) duplicated to the cond and uncond rows (:602-604), plus
@@ -472,6 +512,18 @@ __global__ void gen_embed_gather_kernel(const int32_t* __restrict__ ids, const T
   const int i = blockIdx.x;
   const int id = min(max(ids[i], 0), V - 1);
   for (int d = threadIdx.x; d < D; d += blockDim.x) out[(size_t)i * D + d] = Act<T>::ld(table + (size_t)id * D + d);
+}
+
+// teacher-forced scoring input: image token i of pair r / 2 -> column P + i of row r of x [R][T][D] (i < n - 1)
+template <typename T>
+__global__ void score_embed_kernel(const int32_t* __restrict__ ids, const T* __restrict__ table, float* __restrict__ x,
+                                   int P, int T_cols, int n, int D, int V) {
+  pdl_launch_dependents();
+  pdl_wait();
+  const int i = blockIdx.x, r = blockIdx.y;
+  const int id = min(max(ids[(size_t)(r / 2) * n + i], 0), V - 1);
+  float* dst = x + ((size_t)r * T_cols + P + i) * D;
+  for (int d = threadIdx.x; d < D; d += blockDim.x) dst[d] = Act<T>::ld(table + (size_t)id * D + d);
 }
 
 // first Linear of gen_aligner on the 8-wide codes: h[v][n] = gelu(rnd(sum_k rnd(E[v][k]) * W0[n][k] + b0[n]))

@@ -124,6 +124,28 @@ def sampling_plan(num_gen: int, cfg_weight, temperature, top_k, top_p, generator
                         [_i64(x) for x in seeds], offs, gens)
 
 
+def check_score_args(num_gen: int, P: int, image_tokens: torch.Tensor, mask: Optional[torch.Tensor], img_vocab: int,
+                     max_steps: int) -> int:
+    """Validates the arguments of FastJanus.score_image_tokens (prompt rows 2 * num_gen of P columns) and returns n, the
+    image tokens per image.  image_tokens (num_gen, n) ids in [0, img_vocab); mask (2 * num_gen, P + n) as t2i takes it."""
+    if not isinstance(image_tokens, torch.Tensor) or image_tokens.dim() != 2:
+        raise ValueError("`image_tokens` must be a (num_images, n) tensor")
+    if image_tokens.dtype.is_floating_point or image_tokens.dtype == torch.bool:
+        raise ValueError(f"`image_tokens` must hold integer ids, got {image_tokens.dtype}")
+    if image_tokens.shape[0] != num_gen:
+        raise ValueError(f"`image_tokens` has {image_tokens.shape[0]} rows for {num_gen} images (the prompt has {2 * num_gen} rows)")
+    n = int(image_tokens.shape[1])
+    if not 1 <= n <= max_steps:
+        raise ValueError(f"`image_tokens` has n = {n} tokens per image; the engine takes 1 .. max_steps = {max_steps}")
+    if image_tokens.numel():
+        lo, hi = int(image_tokens.min()), int(image_tokens.max())
+        if lo < 0 or hi >= img_vocab:
+            raise ValueError(f"`image_tokens` ids must be in [0, {img_vocab}), got [{lo}, {hi}]")
+    if mask is not None and tuple(mask.shape) != (2 * num_gen, P + n):
+        raise ValueError(f"`mask` must be (2B, P + n) = {(2 * num_gen, P + n)}, got {tuple(mask.shape)}")
+    return n
+
+
 def kv_start_from_mask(mask: torch.Tensor, P: int) -> torch.Tensor:
     """Lossless encoding of the reference's 0/1 mask (LEFT padding only, image part all ones;
     plangen_base.py:708-712,668,686): number of leading pad columns per row.  Any other mask shape is
@@ -440,22 +462,29 @@ class FastJanus:
     def cfg_sample_embed(self, logits: torch.Tensor, cfg_weight, temperature, seed, offset,
                          step: int, n_steps: int, tokens_out: torch.Tensor, greedy: bool = False,
                          edit_region: Optional[torch.Tensor] = None, gt_labels: Optional[torch.Tensor] = None,
-                         top_k=0, top_p=1.0):
+                         top_k=0, top_p=1.0, logprobs_out: Optional[torch.Tensor] = None):
         """plangen_base.py:580-604 in one launch; returns the next inputs_embeds (2B, D) fp32.  `top_k` / `top_p` filter the
         CFG logits as HF's TopKLogitsWarper then TopPLogitsWarper do (0 / 1 = off).  cfg_weight, temperature, top_k and
         top_p may each hold one value per image (see sampling_plan).  A sequence of B seeds (with `offset` a scalar or B
-        offsets) draws image b as torch.multinomial(probs[b:b+1], 1) on its own generator at (seed[b], offset[b])."""
+        offsets) draws image b as torch.multinomial(probs[b:b+1], 1) on its own generator at (seed[b], offset[b]).
+        logprobs_out: fp32 (B, n_steps) whose column `step` receives log p(token) under the distribution drawn from
+        (see sample_image); the tokens are the same as without it."""
         B = logits.shape[0] // 2
         lg = logits.to(device=self.device, dtype=torch.float32).contiguous()
         x_next = torch.empty(2 * B, self.dims.D, device=self.device, dtype=torch.float32)
         plan = sampling_plan(B, cfg_weight, temperature, top_k, top_p, list(seed) if _is_seq(seed) else int(seed), 0)
-        if not plan.per_image:
+        if not plan.per_image and logprobs_out is None:
             OPS.cfg_sample_embed(self.handle, lg, float(cfg_weight), float(temperature), _i64(seed), int(offset), bool(greedy),
                                  int(top_k), edit_region, gt_labels, int(step), int(n_steps), tokens_out, x_next, float(top_p))
             return x_next
         offs = [int(o) for o in offset] if _is_seq(offset) else [int(offset)] * B
         if len(offs) != B:
             raise ValueError(f"`offset` has {len(offs)} values for {B} images")
+        if logprobs_out is not None:     # all-scalar settings too: uniform lists sample exactly as the scalar op
+            OPS.cfg_sample_embed_logprobs(self.handle, lg, plan.cfg_weight, plan.temperature, plan.top_k, plan.top_p, plan.seed,
+                                          offs, plan.rng_per_image, bool(greedy), edit_region, gt_labels, int(step),
+                                          int(n_steps), tokens_out, x_next, logprobs_out)
+            return x_next
         OPS.cfg_sample_embed_per_image(self.handle, lg, plan.cfg_weight, plan.temperature, plan.top_k, plan.top_p, plan.seed,
                                        offs, plan.rng_per_image, bool(greedy), edit_region, gt_labels, int(step), int(n_steps),
                                        tokens_out, x_next)
@@ -495,7 +524,7 @@ class FastJanus:
     def sample_image(self, inputs_embeds, num_gen, image_token_num_per_image, mask, cfg_weight, temperature,
                      generator=None, batch=None, gt_labels=None, greedy: bool = False,
                      use_teacher_forcing: Optional[bool] = None, top_k: Optional[int] = None,
-                     top_p: Optional[float] = None):
+                     top_p: Optional[float] = None, return_logprobs: bool = False):
         """System.sample_image (plangen_base.py:567-607).  `generator`: torch CUDA generator (its seed and
         philox offset are honoured and advanced) or an int seed.  Teacher forcing (:593-598) is gated on
         `use_teacher_forcing` (default: the engine's flag = `args.use_teacher_forcing`), never on the mere presence
@@ -506,7 +535,10 @@ class FastJanus:
         Per image: cfg_weight, temperature, top_k and top_p may each be a sequence / 1-D tensor of num_gen values, and
         `generator` a sequence of num_gen CUDA generators or int seeds; image j then draws as
         torch.multinomial(probs[j:j+1], 1, generator=generator[j]) would, from the generator's current offset, and each
-        generator is advanced by n draws on a (1, img_vocab) tensor.  See sampling_plan."""
+        generator is advanced by n draws on a (1, img_vocab) tensor.  See sampling_plan.
+        return_logprobs: returns (tokens, logprobs), logprobs fp32 (num_gen, n) = log p(token) of every step under the
+        distribution the draw used (CFG, temperature, top-k, top-p; greedy: top-k only), forced tokens included (-inf
+        where a filter removed one).  Tokens, draws and generator offsets are the same as without it."""
         R, P, D = inputs_embeds.shape
         if R != 2 * num_gen:
             raise ValueError("inputs_embeds rows must be 2 * num_gen (interleaved cond/uncond)")
@@ -523,7 +555,12 @@ class FastJanus:
         if teacher:
             er, gl = self._teacher_inputs(batch, gt_labels, num_gen, n)
         self._keep = (kv_start, x, er, gl)        # keep alive until the stream has consumed them
-        if not plan.per_image:
+        logprobs = None
+        if return_logprobs:              # all-scalar settings too: uniform lists sample exactly as the scalar op
+            logprobs = torch.empty(num_gen, n, dtype=torch.float32, device=self.device)
+            OPS.sample_image_logprobs(self.handle, x, kv_start, n, plan.cfg_weight, plan.temperature, plan.top_k, plan.top_p,
+                                      plan.seed, plan.offset, plan.rng_per_image, bool(greedy), er, gl, tokens, logprobs)
+        elif not plan.per_image:
             OPS.sample_image(self.handle, x, kv_start, n, float(cfg_weight), float(temperature), plan.seed[0], bool(greedy), int(k),
                              er, gl, tokens, float(p))
         else:
@@ -533,20 +570,21 @@ class FastJanus:
         per_draw = self.philox_offset_per_step(1 if plan.rng_per_image else num_gen)
         for g in plan.generators:
             g.set_offset(g.get_offset() + n * per_draw)
-        return tokens
+        return (tokens, logprobs) if return_logprobs else tokens
 
     @torch.inference_mode()
     def t2i(self, inputs_ids=None, parallel_size=1, image_token_num_per_image=None, cfg_weight=5.0, temperature=1.0,
             img_size=None, patch_size=None, gt_image=None, batch=None, mask=None, tokens=None, emb=None,
             gt_labels=None, greedy: bool = False, use_teacher_forcing: Optional[bool] = None, top_k: Optional[int] = None,
-            top_p: Optional[float] = None, generator=None):
+            top_p: Optional[float] = None, generator=None, return_logprobs: bool = False):
         """System.t2i (plangen_base.py:525-565), `tokens`/`emb` branches.  Returns (dec, mask_image).
         Teacher forcing (layout-guided editing, :528-532, :593-598, :557-562) follows `use_teacher_forcing` (default: the
         engine's flag, the counterpart of `args.use_teacher_forcing`): `gt_image` is encoded with the VQ encoder as the
         reference does (or ready-made `gt_labels` are used), and `mask_image` is returned.  With the flag off `gt_image` and
         batch['edit_region'] are ignored, exactly as in the reference.
         cfg_weight, temperature, top_k, top_p and `generator` take per-image values as sample_image does, image
-        j = copy * B + b of the `parallel_size` copies; generator None: the engine's seed."""
+        j = copy * B + b of the `parallel_size` copies; generator None: the engine's seed.
+        return_logprobs: returns (dec, mask_image, logprobs) with the per-step log-probs of sample_image."""
         n = image_token_num_per_image or self.dims.n_img_tokens
         img_size = img_size or self.dims.img_size
         patch_size = patch_size or 2 ** (len(self.dims.vq_ch_mult) - 1)      # 16 for VQ-16
@@ -564,7 +602,10 @@ class FastJanus:
         mask = torch.cat([mask.to(self.device)] * parallel_size)
         num_gen = inputs_embeds.shape[0] // 2
         gen = self.sample_image(inputs_embeds, num_gen, n, mask, cfg_weight, temperature, generator, batch, gt_labels, greedy,
-                                use_teacher_forcing=teacher, top_k=top_k, top_p=top_p)
+                                use_teacher_forcing=teacher, top_k=top_k, top_p=top_p, return_logprobs=return_logprobs)
+        logprobs = None
+        if return_logprobs:
+            gen, logprobs = gen
         g = img_size // patch_size
         dec = self.gen_vision_model.decode_code(gen.to(dtype=torch.int), shape=[num_gen, self.dims.code_dim, g, g])
         self.last_tokens = gen
@@ -576,7 +617,42 @@ class FastJanus:
             er = batch["edit_region"].to(self.device).reshape(-1, 1, g, g).repeat(1, 3, 1, 1).float()
             mask_image = torch.nn.functional.interpolate(er, size=(img_size, img_size), mode="bilinear",
                                                          align_corners=False).round().to(dec)
-        return dec, mask_image
+        return (dec, mask_image, logprobs) if return_logprobs else (dec, mask_image)
+
+    @torch.inference_mode()
+    def score_image_tokens(self, tokens=None, mask=None, image_tokens=None, cfg_weight=5.0, temperature=1.0, top_k=0,
+                           top_p=1.0, emb=None) -> torch.Tensor:
+        """Log-probabilities of GIVEN image tokens: fp32 (B, n), entry (b, i) = log p(image_tokens[b, i]) under the
+        distribution the image loop would sample step i from with every earlier token forced (CFG, temperature, top-k,
+        top-p as in sample_image; -inf where a filter removes the token).  One prefill over prompt + image tokens, one wide
+        gen_head contraction and the sampler's reduction (pg_score_image_tokens) instead of n decode steps.  The LM runs as
+        the reference's single full-sequence forward (fp32 residual stream); the decode loop keeps a bf16 residual stream,
+        so in bf16 the two are different valid evaluations, equal within fp32 noise in fp32 check mode.
+        `tokens` (2B, P) ids or `emb` (2B, P, D), and `mask` (2B, P + n), as t2i takes them; image_tokens (B, n) ids in
+        [0, img_vocab); settings scalar or per image.  P + n - 1 must fit the engine's max_prompt."""
+        if tokens is None and emb is None:
+            raise ValueError("pass `tokens` (2B, P) or `emb` (2B, P, D)")
+        if mask is None:
+            raise ValueError("`mask` (2B, P + n) is required")
+        if tokens is not None:
+            emb = self.language_model.get_input_embeddings()(tokens.to(self.device))
+        R, P, D = emb.shape
+        if R % 2 or R == 0:
+            raise ValueError(f"the prompt needs 2B rows (interleaved cond/uncond), got {R}")
+        B = R // 2
+        if image_tokens is None:
+            raise ValueError("`image_tokens` (B, n) is required")
+        n = check_score_args(B, P, image_tokens, mask, self.dims.img_vocab, self.max_steps)
+        plan = sampling_plan(B, cfg_weight, temperature, top_k, top_p, None, self.seed)
+        kv_start = kv_start_from_mask(mask.to(self.device), P)
+        x = torch.empty(R, P + n - 1, D, dtype=torch.float32, device=self.device)
+        x[:, :P] = emb.to(device=self.device, dtype=torch.float32)
+        ids = image_tokens.to(device=self.device, dtype=torch.int32).contiguous()
+        out = torch.empty(B, n, dtype=torch.float32, device=self.device)
+        self._keep = (kv_start, x, ids)
+        OPS.score_image_tokens(self.handle, x, kv_start, P, ids, plan.cfg_weight, plan.temperature, plan.top_k, plan.top_p, out)
+        self._serial += 1                # the KV cache now holds the scored sequence
+        return out
 
     def images_to_uint8(self, dec: torch.Tensor) -> torch.Tensor:
         """denorm_pt (src/utils/funcs.py:511-512) then `(x*255).astype(np.uint8)` (funcs.py:497-498, truncation) on the

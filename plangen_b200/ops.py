@@ -18,6 +18,9 @@ int64) and pass them to the C-ABI as a host array of pg_image_sampling.
     cfg_sample_embed_per_image  pg_cfg_sample_embed_per_image the same with per-image settings and seeds
     sample_image                pg_sample_image               System.sample_image                             :567-607
     sample_image_per_image      pg_sample_image_per_image     the same with per-image settings and seeds
+    cfg_sample_embed_logprobs   pg_cfg_sample_embed_logprobs  cfg_sample_embed_per_image + log p(token) per image
+    sample_image_logprobs       pg_sample_image_logprobs      sample_image_per_image + log p(token) per image and step
+    score_image_tokens          pg_score_image_tokens         log p(given tokens): one teacher-forced prefill + gen_head
     vq_decode_code              pg_vq_decode_code             gen_vision_model.decode_code                    :555
     vq_encode                   pg_vq_encode                  gen_vision_model.encode(img)[-1][-1]            :532
     prepare_inputs_embeds       pg_prepare_inputs_embeds      prepare_inputs_embeds                           :289,366,855
@@ -159,6 +162,46 @@ def sample_image_per_image(handle: int, x_prompt: torch.Tensor, kv_start: torch.
                                                 int(greedy), _p(edit_region), _p(gt_labels), _p(tokens_out), _st(x_prompt)))
 
 
+@torch.library.custom_op(f"{NS}::cfg_sample_embed_logprobs", mutates_args=("tokens_out", "x_next", "logprobs_out"),
+                         device_types="cuda")
+def cfg_sample_embed_logprobs(handle: int, logits: torch.Tensor, cfg_weight: List[float], temperature: List[float], top_k: List[int],
+                              top_p: List[float], seed: List[int], philox_offset: List[int], rng_per_image: bool, greedy: bool,
+                              edit_region: Optional[torch.Tensor], gt_labels: Optional[torch.Tensor], step: int, n_steps: int,
+                              tokens_out: torch.Tensor, x_next: torch.Tensor, logprobs_out: torch.Tensor) -> None:
+    e = _eng(handle); _cuda(logits, edit_region, gt_labels, tokens_out, x_next, logprobs_out)
+    B = logits.shape[0] // 2
+    pi = _per_image(B, cfg_weight, temperature, top_k, top_p, seed, philox_offset)
+    _lib.check(e._lib.pg_cfg_sample_embed_logprobs(e._h, _p(logits), B, pi, int(rng_per_image), int(greedy), _p(edit_region),
+                                                   _p(gt_labels), int(step), int(n_steps), _p(tokens_out), _p(x_next),
+                                                   _p(logprobs_out), _st(logits)))
+
+
+@torch.library.custom_op(f"{NS}::sample_image_logprobs", mutates_args=("x_prompt", "tokens_out", "logprobs_out"),
+                         device_types="cuda")
+def sample_image_logprobs(handle: int, x_prompt: torch.Tensor, kv_start: torch.Tensor, n_steps: int, cfg_weight: List[float],
+                          temperature: List[float], top_k: List[int], top_p: List[float], seed: List[int], philox_offset: List[int],
+                          rng_per_image: bool, greedy: bool, edit_region: Optional[torch.Tensor], gt_labels: Optional[torch.Tensor],
+                          tokens_out: torch.Tensor, logprobs_out: torch.Tensor) -> None:
+    e = _eng(handle); _cuda(x_prompt, kv_start, edit_region, gt_labels, tokens_out, logprobs_out)
+    R, P = x_prompt.shape[0], x_prompt.shape[1]
+    pi = _per_image(R // 2, cfg_weight, temperature, top_k, top_p, seed, philox_offset)
+    _lib.check(e._lib.pg_sample_image_logprobs(e._h, _p(x_prompt), _p(kv_start), R, P, int(n_steps), pi, int(rng_per_image),
+                                               int(greedy), _p(edit_region), _p(gt_labels), _p(tokens_out), _p(logprobs_out),
+                                               _st(x_prompt)))
+
+
+@torch.library.custom_op(f"{NS}::score_image_tokens", mutates_args=("x_seq", "logprobs_out"), device_types="cuda")
+def score_image_tokens(handle: int, x_seq: torch.Tensor, kv_start: torch.Tensor, P: int, image_tokens: torch.Tensor,
+                       cfg_weight: List[float], temperature: List[float], top_k: List[int], top_p: List[float],
+                       logprobs_out: torch.Tensor) -> None:
+    e = _eng(handle); _cuda(x_seq, kv_start, image_tokens, logprobs_out)
+    R, n = x_seq.shape[0], image_tokens.shape[1]
+    B = R // 2
+    pi = _per_image(B, cfg_weight, temperature, top_k, top_p, [0] * B, [0] * B)
+    _lib.check(e._lib.pg_score_image_tokens(e._h, _p(x_seq), _p(kv_start), R, int(P), n, _p(image_tokens), pi,
+                                            _p(logprobs_out), _st(x_seq)))
+
+
 @torch.library.custom_op(f"{NS}::vq_decode_code", mutates_args=("image_out",), device_types="cuda")
 def vq_decode_code(handle: int, codes: torch.Tensor, gh: int, gw: int, image_out: torch.Tensor) -> None:
     e = _eng(handle); _cuda(codes, image_out)
@@ -189,4 +232,4 @@ def images_to_u8(handle: int, image: torch.Tensor, out: torch.Tensor) -> None:
 
 OP_NAMES = ("embed_tokens", "prefill", "decode_step", "gen_head", "prepare_gen_img_embeds", "cfg_sample_embed", "sample_image",
             "vq_decode_code", "vq_encode", "prepare_inputs_embeds", "images_to_u8", "cfg_sample_embed_per_image",
-            "sample_image_per_image")
+            "sample_image_per_image", "cfg_sample_embed_logprobs", "sample_image_logprobs", "score_image_tokens")
