@@ -20,7 +20,7 @@
 extern "C" {
 #endif
 
-#define PG_ABI_VERSION 5
+#define PG_ABI_VERSION 6
 
 /* arithmetic regimes */
 #define PG_MODE_BF16 0 /* the reference's regime: fp32 master weights under autocast(bf16), plangen_base.py:360 */
@@ -239,6 +239,25 @@ int pg_debug_copy(pg_engine* e, const char* name, void* dst_dev, size_t nbytes, 
  * buffer must have been zeroed with pg_debug_zero_part. */
 int pg_test_attn_decode(pg_engine* e, const int32_t* kv_start, int R, int pos, int layer, void* stream);
 int pg_debug_zero_part(pg_engine* e, size_t nbytes, void* stream);
+
+/* One decode-attention launch exactly as the decode step issues it (same kernel, block, shared memory and cut for a
+ * given CTA count; PDL off), on caller-owned operands, for unit tests of the kernel's own operation.
+ *   impl 3: attn_decode_v5_kernel (bf16 engines); impl 0: the plain kernel in the engine's dtype with `splits`
+ *           T-splits (0 = the engine's rule); it uses the engine's split workspace and takes no src_row.
+ *   part: fp32 QKV split-K partials [S][R][3*H*128], S <= 64.
+ *   kcache / vcache: [R][H][Tmax][128] in the engine's dtype; the kernel writes column pos (the new k / v).
+ *   kv_start[R] (<= pos), src_row[R] or NULL, alias_P: cached columns below alias_P of row r are read from row
+ *           src_row[r] (impl 3 only).
+ *   pos, step_ptr: the position is pos + *step_ptr when step_ptr is not NULL (read once on the host for the
+ *           bounds check, which synchronises `stream`); it must be below Tmax and the engine's Tmax (RoPE tables).
+ *   rope_flags: 1 = bf16 trig with absolute positions (image decode), 0 = fp32 trig, 2 = fp32 trig with positions
+ *           relative to kv_start (text decode).
+ *   ctas: grid of impl 3, 0 = number of SMs, never more (a contributor waits for lower-numbered CTAs).
+ *   H: any head count.  out: [R][H*128] in the engine's dtype.
+ *   ws: impl 3's hand-off records, R*H*64*130 64-bit words, zero on entry and zero again on return. */
+int pg_test_attn_decode_io(pg_engine* e, int impl, int splits, const float* part, int S, int R, int H, void* kcache,
+                           void* vcache, int Tmax, const int32_t* kv_start, const int32_t* src_row, int alias_P, int pos,
+                           const int32_t* step_ptr, int rope_flags, int ctas, void* out, uint64_t* ws, void* stream);
 
 /* Host-only helper of the prefill (no device work, callable without a GPU): proposes, for every prompt row, the FIRST
  * row of the batch with the same left padding `start[r]` and the same 64-bit content hash (itself when there is none).

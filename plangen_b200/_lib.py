@@ -80,6 +80,9 @@ EXPORTS = {
     "pg_debug_copy": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "pg_test_attn_decode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "pg_debug_zero_part": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p]),
+    "pg_test_attn_decode_io": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                         C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int,
+                                         C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pg_host_group_rows": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "pg_test_gemm": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                C.c_int, C.c_void_p, C.c_void_p]),
@@ -107,7 +110,7 @@ def load(build_if_missing: bool = True):
         fn = getattr(lib, name)      # AttributeError if the symbol is not exported
         fn.restype = res
         fn.argtypes = args
-    if lib.pg_abi_version() != 5:
+    if lib.pg_abi_version() != 6:
         raise PgError("ABI version mismatch")
     _LIB = lib
     return lib

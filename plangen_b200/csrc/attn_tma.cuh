@@ -64,18 +64,21 @@ PG_DEVINL void at_stamp(unsigned long long* dbg, int g, int k) {
   if (dbg) dbg[((size_t)blockIdx.x * AT_NG + g) * 16 + k] = global_timer_ns();
 }
 
-// units of one row: tiles covering cached tokens [start, pos) on a 32-token grid, plus the new token
+// tiles covering cached tokens [start, pos) on a 32-token grid
 PG_DEVINL int row_tiles(int start, int pos) { return pos > start ? ((pos - 1) / AT_TILE - start / AT_TILE + 1) : 0; }
 
-// exclusive prefix of units per row into row_units[0..R] (one warp)
-PG_DEVINL void build_row_units(int* row_units, const int32_t* kv_start, int R, int pos, int lane,
-                                int* row_start = nullptr, int new_token_unit = 1) {
-  int carry = 0;
+// exclusive prefix of units per row into row_units[0..R], and the largest row's unit count into *u_max (one warp).
+// A row's units are its tiles; the token being decoded rides on the last one.  A row without cached tokens
+// (kv_start == pos: an all-padding prompt) still gets one unit, which carries only the new token.
+PG_DEVINL void build_row_units(int* row_units, const int32_t* kv_start, int R, int pos, int lane, int* row_start,
+                                int* u_max) {
+  int carry = 0, mx = 0;
   for (int r0 = 0; r0 < R; r0 += 32) {
     const int r = r0 + lane;
     const int st = (r < R) ? kv_start[r] : 0;
-    if (row_start && r < R) row_start[r] = st;
-    int u = (r < R) ? row_tiles(st, pos) + new_token_unit : 0;
+    if (r < R) row_start[r] = st;
+    int u = (r < R) ? max(row_tiles(st, pos), 1) : 0;
+    mx = max(mx, u);
     int incl = u;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
@@ -85,12 +88,36 @@ PG_DEVINL void build_row_units(int* row_units, const int32_t* kv_start, int R, i
     if (r < R) row_units[r] = carry + incl - u;
     carry += __shfl_sync(0xffffffffu, incl, 31);
   }
-  if (lane == 0) row_units[R] = carry;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) mx = max(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  if (lane == 0) { row_units[R] = carry; *u_max = mx; }
 }
 
 // How the flat unit space is cut: CTA c gets [c*per, (c+1)*per), its group g gets [.. + g*sub, .. + (g+1)*sub)
+// Invariant: no item gets more than AT_MAX_SLOTS contributors (non-empty group slots intersecting its units), because an
+// item owns AT_MAX_SLOTS hand-off records.  The even cut keeps it unless few long items meet many CTAs: when bound() says
+// an item of u_max units could meet more slots, sub is widened to at least ceil((u_max - 1) / (AT_MAX_SLOTS - 1)) and per
+// to 4 * sub.  Every slot then holds sub units, so an item meets at most 1 + ceil((u - 1) / sub) <= AT_MAX_SLOTS slots,
+// and per only grows, so the CTAs still cover U.  Elsewhere (every Janus shape) the cut is the even cut.
 struct AttnCut {
   int U, per, sub;
+  PG_DEVINL void init(int units, int ctas, int u_max) {
+    U = units;
+    per = max(1, (U + ctas - 1) / ctas);
+    sub = (per + AT_NG - 1) / AT_NG;
+    if (bound(u_max) > AT_MAX_SLOTS) {
+      sub = max(sub, (u_max + AT_MAX_SLOTS - 3) / (AT_MAX_SLOTS - 1));
+      per = AT_NG * sub;
+    }
+  }
+  // the most slots an item of u >= 1 units can meet, over every alignment: 1 + the slot starts strictly inside it.  A
+  // whole CTA has k non-empty slots, the last one of g <= sub units; starts repeat with period per.
+  PG_DEVINL int bound(int u) const {
+    const int k = (per + sub - 1) / sub, g = per - (k - 1) * sub;
+    const int m = (u - 1) / per, rem = (u - 1) % per;
+    const int inner = rem == 0 ? 0 : min(k, rem - 1 >= g ? 2 + (rem - 1 - g) / sub : 1);
+    return 1 + k * m + inner;
+  }
   PG_DEVINL void group_range(int c, int g, int& lo, int& hi) const {
     const int cb = min(c * per, U), ce = min(cb + per, U);
     lo = min(cb + g * sub, ce);
@@ -135,12 +162,15 @@ PG_DEVINL void attn_produce_group(int gb, int ge, const int* row_units, int R, i
       const int t0k = (st / AT_TILE + k) * AT_TILE;
       const int a = k == 0 ? (st & (AT_TILE - 1)) : 0;                 // first valid token slot of the tile
       const int b = min(AT_TILE, pos - t0k);                           // one past the last cached token slot
-      const uint32_t bytes = (uint32_t)(b - a) * (HEAD_DIM * 2);
+      const uint32_t bytes = (uint32_t)max(b - a, 0) * (HEAD_DIM * 2);
+      // a row without cached tokens copies nothing: its arrive with 0 bytes expected completes the stage's phase
       mbar_expect_tx(&full_bar[s], 2 * bytes);
       const size_t off = (((size_t)r * H + h) * Tmax + t0k + a) * HEAD_DIM;
       uint8_t* dst = ring + (size_t)s * stage_stride_bytes + (size_t)a * (HEAD_DIM * 2);
       const int rs = (src_row != nullptr && t0k + a < alias_P) ? src_row[r] : r;
-      if (rs != r) {
+      if (bytes == 0) {
+        // no bulk copy of zero bytes
+      } else if (rs != r) {
         // tokens [t0k + a, min(t0k + b, alias_P)) from the source row, the rest (generated tokens) from the row itself
         const int nb = min(b, alias_P - t0k) - a;
         const uint32_t sb = (uint32_t)nb * (HEAD_DIM * 2);

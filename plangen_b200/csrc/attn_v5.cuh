@@ -10,7 +10,8 @@
 // new-token unit paid two boundaries before their first tile and finished last.
 //
 // Hence, on the consumer side:
-//   * the token being decoded rides on the item's last tile (no unit of its own): no empty segments;
+//   * the token being decoded rides on the item's last tile (no unit of its own): no empty segments.  A row
+//     without cached tokens has one unit that carries only the new token (build_row_units);
 //   * the partials of the NEXT segment's q / k / v are loaded into registers before the current segment's
 //     tile loop and only consumed at the boundary: the round trip overlaps the stream;
 //   * hand-off without waiting: a contributor stores its record as 64-bit words {value, valid flag} (one
@@ -292,8 +293,9 @@ PG_DEVINL void a5_group_stream(int tg, int gb, int ge, int r0, const AttnCut& cu
   }
   // ---- deferred merge: take the records of ranks 0 .. n-2 as they become valid, combine in rank order
   //      (own record last), clear the words for the next launch.  With few rows an item is cut over many
-  //      groups (n-1 up to 63): the (M, L) words are fetched by 2(n-1) threads at once into shared memory and
-  //      the output words eight records at a time, instead of one dependent round trip per record.
+  //      groups (n <= AT_MAX_SLOTS by the AttnCut invariant, so n-1 <= 63 and 2(n-1) < AT_GT): the (M, L) words are
+  //      fetched by 2(n-1) threads at once into shared memory and the output words eight records at a time, instead
+  //      of one dependent round trip per record.
   if (df_it >= 0) {
     const int n_other = df_n - 1;
     unsigned long long* wb = ws_ll + (size_t)df_it * AT_MAX_SLOTS * A5_REC;
@@ -358,7 +360,7 @@ attn_decode_v5_kernel(const float* __restrict__ part, int S, size_t split_stride
   unsigned long long* ws_ll = reinterpret_cast<unsigned long long*>(ws_ll_f);   // zero-initialised {flag, value} words
   uint8_t* ring = (uint8_t*)(((uintptr_t)smem_raw + 127) & ~(uintptr_t)127);
   __shared__ uint64_t full_bar[A5_STAGES], empty_bar[A5_STAGES];
-  __shared__ int row_units[AT_MAX_ROWS + 1], row_start[AT_MAX_ROWS];
+  __shared__ int row_units[AT_MAX_ROWS + 1], row_start[AT_MAX_ROWS], u_max;
   __shared__ A5GroupSmem gsm[AT_NG];
   __shared__ int stage_tab[AT_NG * A5_SPG];
 
@@ -381,13 +383,11 @@ attn_decode_v5_kernel(const float* __restrict__ part, int S, size_t split_stride
   for (int i = tid; i < A5_STAGES * 2 * AT_TILE_BYTES / 16; i += AT_THREADS)
     asm volatile("st.shared.v4.u32 [%0], {%1, %1, %1, %1};" ::"r"(smem_u32(ring) + (uint32_t)i * 16u), "r"(0u) : "memory");
   fence_proxy_async();
-  if (warp == 0) build_row_units(row_units, kv_start, R, pos, lane, row_start, 0);
+  if (warp == 0) build_row_units(row_units, kv_start, R, pos, lane, row_start, &u_max);
   __syncthreads();
   if (tid < AT_NG) at_stamp(dbg, tid, 1);
   AttnCut cut;
-  cut.U = row_units[R] * H;
-  cut.per = max(1, (cut.U + (int)gridDim.x - 1) / (int)gridDim.x);
-  cut.sub = (cut.per + AT_NG - 1) / AT_NG;
+  cut.init(row_units[R] * H, (int)gridDim.x, u_max);
   const int c = blockIdx.x;
   const int g = (warp >= AT_NW) ? warp - AT_NW : warp / AT_GW;
   int gb, ge;

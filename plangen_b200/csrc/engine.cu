@@ -2137,6 +2137,70 @@ extern "C" int pg_test_attn_decode(pg_engine* e, const int32_t* kv_start, int R,
   e->use_pdl = saved;
   return rc;
 }
+// One decode-attention launch as decode_layers issues it (same kernel, block, shared memory and cut for a CTA count),
+// on caller-owned operands and with PDL off, so a test can compare the kernel with a reference of its own operation.
+extern "C" int pg_test_attn_decode_io(pg_engine* e, int impl, int splits, const float* part, int S, int R, int H,
+                                      void* kcache, void* vcache, int Tmax, const int32_t* kv_start,
+                                      const int32_t* src_row, int alias_P, int pos, const int32_t* step_ptr,
+                                      int rope_flags, int ctas, void* out, uint64_t* ws, void* stream) {
+  TRY(check_ready(e));
+  cudaStream_t st = (cudaStream_t)stream;
+  if (impl != 0 && impl != 3) return fail("pg_test_attn_decode_io: impl must be 0 (plain kernel) or 3 (v5)");
+  if (impl == 3 && !e->bf16) return fail("pg_test_attn_decode_io: impl 3 needs a bf16 engine");
+  if (!part || !kcache || !vcache || !kv_start || !out) return fail("pg_test_attn_decode_io: null operand");
+  if (S < 1 || S > 64) return fail("pg_test_attn_decode_io: S=%d must be in [1, 64]", S);
+  if (H < 1) return fail("pg_test_attn_decode_io: H=%d must be >= 1", H);
+  if (R < 1 || (impl == 3 && R > AT_MAX_ROWS)) return fail("pg_test_attn_decode_io: R=%d must be in [1, %d]", R, AT_MAX_ROWS);
+  if (Tmax < 1) return fail("pg_test_attn_decode_io: Tmax=%d must be >= 1", Tmax);
+  if (rope_flags != 0 && rope_flags != 1 && rope_flags != ROPE_REL)
+    return fail("pg_test_attn_decode_io: rope_flags=%d must be 0, 1 or %d", rope_flags, ROPE_REL);
+  if (ctas < 0 || ctas > e->num_sms) return fail("pg_test_attn_decode_io: ctas=%d must be in [0, num_sms=%d]", ctas, e->num_sms);
+  if (splits < 0 || splits > 64) return fail("pg_test_attn_decode_io: splits=%d must be in [0, 64]", splits);
+  // the position the kernel will use: with step_ptr it is pos + *step_ptr, read here to check its bounds
+  int pos_eff = pos;
+  if (step_ptr) {
+    int32_t step = 0;
+    CK(cudaMemcpyAsync(&step, step_ptr, 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    pos_eff = pos + step;
+  }
+  if (pos_eff < 0 || pos_eff >= Tmax) return fail("pg_test_attn_decode_io: pos=%d must be in [0, Tmax=%d)", pos_eff, Tmax);
+  if (pos_eff >= e->Tmax) return fail("pg_test_attn_decode_io: pos=%d must be below the engine's Tmax=%d (RoPE tables)", pos_eff, e->Tmax);
+  NEED(cosT, float, "rope_cos");
+  NEED(sinT, float, "rope_sin");
+  const float scale = 1.0f / sqrtf((float)HEAD_DIM);
+  const size_t split_stride = (size_t)R * 3 * H * HEAD_DIM;
+  const int saved = e->use_pdl;
+  e->use_pdl = 0;
+  int rc = 0;
+  if (impl == 3) {
+    if (!ws) rc = fail("pg_test_attn_decode_io: ws (R*H*%d*%d zeroed words) is required for impl 3", AT_MAX_SLOTS, A5_REC);
+    if (!src_row && alias_P != 0) rc = fail("pg_test_attn_decode_io: alias_P=%d without src_row", alias_P);
+    if (!rc)
+      rc = launch(e, attn_decode_v5_kernel, dim3(ctas > 0 ? ctas : e->num_sms), dim3(AT_THREADS), A5_SMEM, st, part, S,
+                  split_stride, cosT, sinT, (bf16*)kcache, (bf16*)vcache, kv_start, (bf16*)out, (float*)ws, R, H, Tmax, pos,
+                  (const int*)step_ptr, scale, rope_flags, 1, next_prof(e), (unsigned long long*)nullptr, src_row, alias_P);
+  } else {
+    const int nsp = splits > 0 ? splits : attn_split_count(e, R, pos_eff + 1);
+    if (src_row || alias_P != 0) rc = fail("pg_test_attn_decode_io: the plain kernel reads every row's own cache (src_row, alias_P)");
+    else if ((size_t)R * H * nsp > (size_t)e->d.max_rows * e->d.H * 64)
+      rc = fail("pg_test_attn_decode_io: R*H*splits=%zu exceeds the split workspace (%zu)", (size_t)R * H * nsp,
+                (size_t)e->d.max_rows * e->d.H * 64);
+    else if ((size_t)R * H > (size_t)e->d.max_rows * e->d.H)
+      rc = fail("pg_test_attn_decode_io: R*H=%d exceeds the split counters (%d)", R * H, e->d.max_rows * e->d.H);
+    else if (e->bf16)
+      rc = launch(e, attn_decode_kernel<bf16>, dim3(H, R, nsp), dim3(128), 0, st, part, S, split_stride, cosT, sinT,
+                  (bf16*)kcache, (bf16*)vcache, kv_start, (bf16*)out, e->attn_ws, e->attn_cnt, H, Tmax, pos,
+                  (const int*)step_ptr, scale, rope_flags);
+    else
+      rc = launch(e, attn_decode_kernel<float>, dim3(H, R, nsp), dim3(128), 0, st, part, S, split_stride, cosT, sinT,
+                  (float*)kcache, (float*)vcache, kv_start, (float*)out, e->attn_ws, e->attn_cnt, H, Tmax, pos,
+                  (const int*)step_ptr, scale, rope_flags);
+  }
+  e->use_pdl = saved;
+  return rc;
+}
+
 extern "C" int pg_debug_zero_part(pg_engine* e, size_t nbytes, void* stream) {
   if (!e || !e->part) return fail("null engine");
   CK(cudaMemsetAsync(e->part, 0, std::min(nbytes, e->part_bytes), (cudaStream_t)stream));
