@@ -20,7 +20,7 @@
 extern "C" {
 #endif
 
-#define PG_ABI_VERSION 6
+#define PG_ABI_VERSION 7
 
 /* arithmetic regimes */
 #define PG_MODE_BF16 0 /* the reference's regime: fp32 master weights under autocast(bf16), plangen_base.py:360 */
@@ -269,6 +269,61 @@ int pg_host_group_rows(const int32_t* start, const uint64_t* hash, int R, int32_
  * impl 0 = SIMT (fp32 or bf16 inputs), 1 = tcgen05 (bf16 inputs).  C fp32 [splits][M][N]. */
 int pg_test_gemm(pg_engine* e, int impl, int is_bf16, const void* X, const void* W, int M, int N,
                  int K, int splits, float* C, void* stream);
+
+/* One tcgen05 contraction exactly as the engine issues it (run_gemm, run_conv_gemm, the stream-K gate|up launch; PDL
+ * off) on caller-owned bf16 operands, for unit tests of the fused epilogues.  bf16 engines only.
+ *   X [M][K] (conv: NHWC activation [img_b][img_h][img_w][K / 9]), W [N][K] row-major (conv: [Cout = N][9 * Cin]).
+ *   weights 1: W is first copied tile-major (tile_weight_kernel, as pg_engine_finalize does) into w_tiled, which the
+ *   contraction then streams; the copy stays there for inspection.  Read by gemm_tc and stream-K only.
+ *   mode:
+ *     PG_TC_PLAIN   C fp32 [splits][M][N] split-K partials (splits >= 1; fewer may be used, as pg_test_gemm);
+ *     PG_TC_ROWS    out bf16 [M][N] = bf16(act(bf16(acc + bias))) or bf16(bf16(acc + bias) + add16) (add16 may be out),
+ *                   act = GELU when gelu == 1; bias may be NULL;
+ *     PG_TC_RESID   resid fp32 [M][N] += bf16(acc + bias);
+ *     PG_TC_SWIGLU  out bf16 [M][N / 2]: W rows interleaved by 64 (weights.py), N % 128 == 0;
+ *     PG_TC_QKV     q_out [M][H*128], kcache / vcache [R][H][Tmax][128]; N == 3*H*128, M > 128 (CTA pair); row_off[R]
+ *                   (packed stream, positions kv_start[r] + t - row_off[r]) or NULL (padded [R][P] block, position t % P);
+ *                   rope_start[R] or NULL.  Positions must be below Tmax and the engine's Tmax (RoPE tables);
+ *     PG_TC_SWIGLU_SK  stream-K gate|up + SwiGLU (M <= 64, tile-major weights): out as PG_TC_SWIGLU, ctas (0 = the
+ *                   production rule), scratch fp32 and counters (zero on entry, zero again on return) of the caller;
+ *     PG_TC_CONV    3x3 implicit convolution, pad 1: C fp32 [pixels][N], or with out set the fused bias / add16 bf16 store.
+ *   path / path_nt (out): the kernel that ran (PG_PATH_*), and its token-tile width. */
+#define PG_TC_PLAIN 0
+#define PG_TC_ROWS 1
+#define PG_TC_RESID 2
+#define PG_TC_SWIGLU 3
+#define PG_TC_QKV 4
+#define PG_TC_SWIGLU_SK 5
+#define PG_TC_CONV 6
+#define PG_PATH_NONE 0
+#define PG_PATH_SIMT 1
+#define PG_PATH_TC 2      /* gemm_tc_kernel<path_nt> */
+#define PG_PATH_TC2 3     /* gemm_tc2_kernel (CTA pair) */
+#define PG_PATH_SK 4      /* gemm_swiglu_sk_kernel<path_nt> */
+#define PG_PATH_CONV 5    /* gemm_tc_kernel<192> as implicit convolution */
+#define PG_PATH_IM2COL 6  /* the convolution does not qualify: the engine would use im2col (nothing launched) */
+typedef struct pg_test_contraction {
+  int mode, weights;
+  int M, N, K, splits;
+  const void* X;
+  const void* W;
+  void* w_tiled; size_t w_tiled_bytes;
+  float* C; size_t c_bytes;
+  void* out;
+  const float* bias;
+  int gelu;
+  const void* add16;
+  float* resid;
+  void* q_out; void* kcache; void* vcache;
+  const int32_t* row_off; const int32_t* kv_start; const int32_t* rope_start;
+  int R, P, H, Tmax;
+  int ctas;
+  float* scratch; size_t scratch_bytes;
+  int* counters; int n_counters;
+  int img_b, img_h, img_w;
+  int path, path_nt;
+} pg_test_contraction;
+int pg_test_contraction_run(pg_engine* e, pg_test_contraction* p, void* stream);
 
 #ifdef __cplusplus
 }

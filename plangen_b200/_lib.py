@@ -31,6 +31,20 @@ class PgImageSampling(C.Structure):
                 ("top_k", C.c_int32), ("top_p", C.c_double)]
 
 
+class PgTestContraction(C.Structure):
+    """pg_test_contraction: one contraction of pg_test_contraction_run (include/plangen_b200.h)."""
+    _fields_ = [
+        ("mode", C.c_int32), ("weights", C.c_int32), ("M", C.c_int32), ("N", C.c_int32), ("K", C.c_int32), ("splits", C.c_int32),
+        ("X", C.c_void_p), ("W", C.c_void_p), ("w_tiled", C.c_void_p), ("w_tiled_bytes", C.c_size_t),
+        ("C", C.c_void_p), ("c_bytes", C.c_size_t), ("out", C.c_void_p), ("bias", C.c_void_p), ("gelu", C.c_int32),
+        ("add16", C.c_void_p), ("resid", C.c_void_p), ("q_out", C.c_void_p), ("kcache", C.c_void_p), ("vcache", C.c_void_p),
+        ("row_off", C.c_void_p), ("kv_start", C.c_void_p), ("rope_start", C.c_void_p),
+        ("R", C.c_int32), ("P", C.c_int32), ("H", C.c_int32), ("Tmax", C.c_int32), ("ctas", C.c_int32),
+        ("scratch", C.c_void_p), ("scratch_bytes", C.c_size_t), ("counters", C.c_void_p), ("n_counters", C.c_int32),
+        ("img_b", C.c_int32), ("img_h", C.c_int32), ("img_w", C.c_int32), ("path", C.c_int32), ("path_nt", C.c_int32),
+    ]
+
+
 class PgError(RuntimeError):
     pass
 
@@ -86,6 +100,7 @@ EXPORTS = {
     "pg_host_group_rows": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "pg_test_gemm": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                C.c_int, C.c_void_p, C.c_void_p]),
+    "pg_test_contraction_run": (C.c_int, [C.c_void_p, C.POINTER(PgTestContraction), C.c_void_p]),
 }
 
 
@@ -110,7 +125,7 @@ def load(build_if_missing: bool = True):
         fn = getattr(lib, name)      # AttributeError if the symbol is not exported
         fn.restype = res
         fn.argtypes = args
-    if lib.pg_abi_version() != 6:
+    if lib.pg_abi_version() != 7:
         raise PgError("ABI version mismatch")
     _LIB = lib
     return lib

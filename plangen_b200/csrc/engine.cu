@@ -122,6 +122,7 @@ struct pg_engine {
   float* xpack = nullptr; float* x_last = nullptr; int32_t* row_off = nullptr; int32_t* row_off_host = nullptr;
   int gu_streamk = 1;                                 // decode gate|up + SwiGLU as a stream-K launch over all SMs (gemm_sk.cuh)
   int* sk_counters = nullptr;
+  int last_path = PG_PATH_NONE, last_nt = 0;          // kernel the last run_gemm / run_conv_gemm launched (pg_test_contraction_run)
   int prefill_qkv_fuse = 1;                           // prefill QKV: RoPE + q / cache stores in the CTA-pair contraction's epilogue
   QkvEpi qkv_epi_next = {};                           // consumed (and cleared) by the next CTA-pair launch
   int sig_attn_tc = 1;                                // tcgen05 attention (bf16, head_dim 64); 0 = CUDA-core kernel
@@ -233,6 +234,7 @@ constexpr int CONV_NT = 192;
 static int run_conv_gemm(pg_engine* e, const void* act, const void* Wc, int B, int H, int W, int Cin, int Cout, float* C,
                          size_t c_bytes, cudaStream_t st, int* taken, const EpiFuse* epi = nullptr) {
   *taken = 0;
+  e->last_path = PG_PATH_IM2COL; e->last_nt = 0;
   if (!e->bf16 || !e->use_tc || Cin % TC_BK != 0) return 0;
   if ((((uintptr_t)act) & 15) || (((uintptr_t)Wc) & 15)) return 0;
   int bw = 0;
@@ -258,9 +260,14 @@ static int run_conv_gemm(pg_engine* e, const void* act, const void* Wc, int B, i
   const int num_kb = 9 * Cin / TC_BK;
   TRY(launch_tc<CONV_NT>(e, mw, mx, C, (int)pixels, Cout, 9 * Cin, 1, num_kb, true, nullptr, nullptr, st, &cg,
                          B * cg.tiles_x * cg.tiles_y, epi));
+  e->last_path = PG_PATH_CONV; e->last_nt = CONV_NT;
   *taken = 1;
   return 0;
 }
+
+// the tcgen05 contraction runs on CTA pairs (gemm_tc2.cuh) for 256-token tiles without split-K, SwiGLU-to-hbuf or a lone
+// weight tile
+static bool tc_pair_taken(int M, int N, int splits, bool swiglu_out) { return M > 128 && splits == 1 && !swiglu_out && N > TC_BM; }
 
 // C[splits][M][N] fp32 = X[M][K] * W[N][K]^T.  Returns the number of splits used through *splits_out.
 static int run_gemm(pg_engine* e, const void* X, const void* W, int M, int N, int K, float* C, size_t c_bytes,
@@ -302,7 +309,7 @@ static int run_gemm(pg_engine* e, const void* X, const void* W, int M, int N, in
     }
     CUtensorMap mw, mx;
     TRY(make_map_2d(e, &mw, W, (uint64_t)N, (uint64_t)K, TC_BM));
-    if (NT == 256 && splits == 1 && !swiglu_out && N > TC_BM) {
+    if (tc_pair_taken(M, N, splits, swiglu_out != nullptr)) {
       // tensor-bound shape: CTA pairs, one 256 x 256 x 16 MMA per pair and k-step (gemm_tc2.cuh)
       TRY(make_map_2d(e, &mx, X, (uint64_t)M, (uint64_t)K, (uint32_t)(TC2_NT / 2)));
       EpiFuse ep2 = {};
@@ -314,6 +321,7 @@ static int run_gemm(pg_engine* e, const void* X, const void* W, int M, int N, in
       if (ep2.gelu == 3 && (qe.q_out == nullptr || N != 3 * qe.H * HEAD_DIM)) return fail("internal: QKV epilogue without its destinations");
       TRY(launch(e, gemm_tc2_kernel, dim3(2 * pairs, 1, 1), dim3(TC2_THREADS), (size_t)tc2p_smem_bytes(e->tc2_stages), st, mw, mx, C, M,
                  N, K, e->tc2_stages, e->use_pdl, next_prof(e), ep2, qe));
+      e->last_path = PG_PATH_TC2; e->last_nt = TC2_NT;
       *splits_out = 1;
       return 0;
     }
@@ -326,6 +334,7 @@ static int run_gemm(pg_engine* e, const void* X, const void* W, int M, int N, in
       case 128: TRY(launch_tc<128>(e, mw, mx, C, M, N, K, splits, kb_per_split, w_const, w_tiled, swiglu_out, st, nullptr, 0, epi)); break;
       default: TRY(launch_tc<256>(e, mw, mx, C, M, N, K, splits, kb_per_split, w_const, w_tiled, swiglu_out, st, nullptr, 0, epi)); break;
     }
+    e->last_path = PG_PATH_TC; e->last_nt = NT;
   } else {
     if (swiglu_out || epi) return fail("internal: fused epilogues need the tcgen05 path");
     if (K % 4 != 0) return fail("SIMT GEMM needs K %% 4 == 0 (K=%d)", K);
@@ -341,8 +350,20 @@ static int run_gemm(pg_engine* e, const void* X, const void* W, int M, int N, in
       TRY(launch(e, gemm_simt_kernel<bf16>, grid, dim3(256), 0, st, (const bf16*)X, (const bf16*)W, C, M, N, K, k_per_split));
     else
       TRY(launch(e, gemm_simt_kernel<float>, grid, dim3(256), 0, st, (const float*)X, (const float*)W, C, M, N, K, k_per_split));
+    e->last_path = PG_PATH_SIMT; e->last_nt = 0;
   }
   *splits_out = splits;
+  return 0;
+}
+
+// Tile-major, pre-swizzled copy of a row-major bf16 weight [N][K] (tile_weight_kernel): ceil(N/128) x ceil(K/64) tiles of
+// 16 KB, zero-padded at the edges.
+static size_t tile_major_bytes(int N, int K) { return (size_t)((N + TC_BM - 1) / TC_BM) * ((K + TC_BK - 1) / TC_BK) * TC_A_BYTES; }
+static int build_tile_major(pg_engine* e, const void* W, int N, int K, uint8_t* dst, cudaStream_t st) {
+  const size_t n_chunks = tile_major_bytes(N, K) / 16;
+  const int blocks = (int)std::min<size_t>((n_chunks + 255) / 256, (size_t)e->num_sms * 16);
+  tile_weight_kernel<<<blocks, 256, 0, st>>>((const bf16*)W, dst, N, K, (K + TC_BK - 1) / TC_BK, n_chunks);
+  CK(cudaGetLastError());
   return 0;
 }
 
@@ -743,18 +764,14 @@ extern "C" int pg_engine_finalize(pg_engine* e, void* stream) {
     if (const void* hw1 = T_(e, "head.w1")) items.push_back({hw1, d.img_vocab, d.img_embed});
     if (const void* lmh = T_(e, "lm_head")) items.push_back({lmh, d.vocab, d.D});      // stage-1 text decode (optional)
     size_t total_bytes = 0;
-    auto tiles_of = [](const Item& it) { return (size_t)((it.N + TC_BM - 1) / TC_BM) * ((it.K + TC_BK - 1) / TC_BK); };
-    for (const Item& it : items) if (it.K % 8 == 0) total_bytes += tiles_of(it) * TC_A_BYTES;
+    for (const Item& it : items) if (it.K % 8 == 0) total_bytes += tile_major_bytes(it.N, it.K);
     CK(cudaMalloc(&e->tiled_buf, std::max<size_t>(total_bytes, 16)));
     size_t off = 0;
     for (const Item& it : items) {
       if (it.K % 8 != 0 || (((uintptr_t)it.w) & 15) != 0) continue;
-      const size_t n_chunks = tiles_of(it) * (TC_A_BYTES / 16);
-      const int blocks = (int)std::min<size_t>((n_chunks + 255) / 256, (size_t)e->num_sms * 16);
-      tile_weight_kernel<<<blocks, 256, 0, st>>>((const bf16*)it.w, e->tiled_buf + off, it.N, it.K, (it.K + TC_BK - 1) / TC_BK, n_chunks);
-      CK(cudaGetLastError());
+      TRY(build_tile_major(e, it.w, it.N, it.K, e->tiled_buf + off, st));
       e->tiled[it.w] = {e->tiled_buf + off, it.N, it.K};
-      off += tiles_of(it) * TC_A_BYTES;
+      off += tile_major_bytes(it.N, it.K);
     }
   }
   CK(cudaStreamSynchronize(st));
@@ -779,6 +796,49 @@ static int elementwise_blocks(pg_engine* e, size_t total) {
 // otherwise the contraction followed by swiglu_kernel.
 // (decode-sized token counts only: with 256-token tiles the two gate warps' expf work would outlast the MMAs)
 static bool fused_swiglu_ok(const pg_engine* e, int tok) { return e->bf16 && e->use_tc && e->d.F % 64 == 0 && tok <= 128; }
+
+// Stream-K gate|up + SwiGLU (gemm_sk.cuh) of X [tok][D] (tok <= 64) against the tile-major gate|up weight [2F][D] into
+// h [tok][F].  ctas: the grid, 0 = one CTA per SM (at most one per unit).  scratch holds n_tiles x max_contrib partial
+// tiles; counters[n_tiles] are zero on entry and zero again once the launch completes.
+static int launch_swiglu_sk(pg_engine* e, const void* X, const uint8_t* w_tiled, int tok, int F, int D, int ctas, float* scratch,
+                            size_t scratch_bytes, int* counters, int n_counters, bf16* h_out, cudaStream_t st) {
+  if (tok < 1 || tok > 64) return fail("stream-K SwiGLU: M=%d must be in [1, 64]", tok);
+  if (F % 64 != 0 || D % TC_BK != 0) return fail("stream-K SwiGLU: F=%d must be a multiple of 64 and D=%d of %d", F, D, TC_BK);
+  const int NT = tok <= 16 ? 16 : tok <= 32 ? 32 : 64;
+  const int n_tiles = 2 * F / TC_BM, num_kb = D / TC_BK;
+  const long U = (long)n_tiles * num_kb;
+  if (ctas < 0 || ctas > e->num_sms) return fail("stream-K SwiGLU: ctas=%d must be in [0, num_sms=%d]", ctas, e->num_sms);
+  const int G = (int)std::min<long>(ctas > 0 ? ctas : e->num_sms, U);
+  const int per_min = (int)std::max<long>(1, U / G);
+  const int max_contrib = (num_kb + per_min - 1) / per_min + 1;
+  // a CTA keeps at most SKG_MAX_FRAGS fragments; one whose range touched more tiles would drop the rest, and their
+  // finishers would wait for partials nobody publishes
+  for (int c = 0; c < G; ++c) {
+    const long u0 = ((long)c * U) / G, u1 = ((long)(c + 1) * U) / G;
+    if (u1 > u0 && (u1 - 1) / num_kb - u0 / num_kb + 1 > SKG_MAX_FRAGS)
+      return fail("stream-K SwiGLU: CTA %d of %d spans %ld tiles (at most %d fragments per CTA; %ld units of %d k-blocks)", c, G,
+                  (u1 - 1) / num_kb - u0 / num_kb + 1, SKG_MAX_FRAGS, U, num_kb);
+  }
+  if ((size_t)n_tiles * max_contrib * NT * TC_BM * 4 > scratch_bytes)
+    return fail("stream-K SwiGLU: scratch of %zu bytes holds fewer than %d tiles x %d contributors x %d x %d fp32", scratch_bytes, n_tiles,
+                max_contrib, NT, TC_BM);
+  if (n_counters < n_tiles) return fail("stream-K SwiGLU: %d counters for %d tiles", n_counters, n_tiles);
+  CUtensorMap mx;
+  TRY(make_map_2d(e, &mx, X, (uint64_t)tok, (uint64_t)D, (uint32_t)NT));
+  const int stage_bytes = TC_A_BYTES + NT * TC_BK * 2;
+  int stages = std::min(12, (200 * 1024) / stage_bytes) & ~1;
+  const size_t smem = (size_t)stages * stage_bytes + SKG_XCH_BYTES + 1024 + 512;
+  e->last_path = PG_PATH_SK; e->last_nt = NT;
+  if (NT == 64)
+    return launch(e, gemm_swiglu_sk_kernel<64>, dim3(G), dim3(SKG_THREADS), smem, st, mx, w_tiled, tok, F, n_tiles, num_kb, stages,
+                  e->use_pdl, scratch, max_contrib, counters, h_out, next_prof(e));
+  if (NT == 16)
+    return launch(e, gemm_swiglu_sk_kernel<16>, dim3(G), dim3(SKG_THREADS), smem, st, mx, w_tiled, tok, F, n_tiles, num_kb, stages,
+                  e->use_pdl, scratch, max_contrib, counters, h_out, next_prof(e));
+  return launch(e, gemm_swiglu_sk_kernel<32>, dim3(G), dim3(SKG_THREADS), smem, st, mx, w_tiled, tok, F, n_tiles, num_kb, stages,
+                e->use_pdl, scratch, max_contrib, counters, h_out, next_prof(e));
+}
+
 static int k_gate_up(pg_engine* e, const LayerW& w, int tok, cudaStream_t st) {
   const pg_dims& d = e->d;
   const int F = d.F, D = d.D;
@@ -790,28 +850,9 @@ static int k_gate_up(pg_engine* e, const LayerW& w, int tok, cudaStream_t st) {
   if (fused_swiglu_ok(e, tok) && tok <= 64 && D % TC_BK == 0 &&
       (e->gu_streamk == 2 || (e->gu_streamk == 1 && 2 * F / TC_BM > e->num_sms))) {
     auto it = e->tiled.find(w.wgu);
-    if (it != e->tiled.end() && it->second.N == 2 * F && it->second.K == D) {
-      const int NT = tok <= 16 ? 16 : tok <= 32 ? 32 : 64;
-      const int n_tiles = 2 * F / TC_BM, num_kb = D / TC_BK;
-      const long U = (long)n_tiles * num_kb;
-      const int G = (int)std::min<long>(e->num_sms, U);
-      const int per_min = (int)std::max<long>(1, U / G);
-      const int max_contrib = (num_kb + per_min - 1) / per_min + 1;
-      if ((size_t)n_tiles * max_contrib * NT * TC_BM * 4 > e->part_bytes) return fail("internal: stream-K scratch does not fit the partial buffer");
-      CUtensorMap mx;
-      TRY(make_map_2d(e, &mx, e->xn, (uint64_t)tok, (uint64_t)D, (uint32_t)NT));
-      const int stage_bytes = TC_A_BYTES + NT * TC_BK * 2;
-      int stages = std::min(12, (200 * 1024) / stage_bytes) & ~1;
-      const size_t smem = (size_t)stages * stage_bytes + SKG_XCH_BYTES + 1024 + 512;
-      if (NT == 64)
-        return launch(e, gemm_swiglu_sk_kernel<64>, dim3(G), dim3(SKG_THREADS), smem, st, mx, it->second.ptr, tok, F, n_tiles, num_kb, stages,
-                      e->use_pdl, e->part, max_contrib, e->sk_counters, (bf16*)e->hbuf, next_prof(e));
-      if (NT == 16)
-        return launch(e, gemm_swiglu_sk_kernel<16>, dim3(G), dim3(SKG_THREADS), smem, st, mx, it->second.ptr, tok, F, n_tiles, num_kb, stages,
-                      e->use_pdl, e->part, max_contrib, e->sk_counters, (bf16*)e->hbuf, next_prof(e));
-      return launch(e, gemm_swiglu_sk_kernel<32>, dim3(G), dim3(SKG_THREADS), smem, st, mx, it->second.ptr, tok, F, n_tiles, num_kb, stages,
-                    e->use_pdl, e->part, max_contrib, e->sk_counters, (bf16*)e->hbuf, next_prof(e));
-    }
+    if (it != e->tiled.end() && it->second.N == 2 * F && it->second.K == D)
+      return launch_swiglu_sk(e, e->xn, it->second.ptr, tok, F, D, 0, e->part, e->part_bytes, e->sk_counters, 2 * F / TC_BM,
+                              (bf16*)e->hbuf, st);
   }
   if (fused_swiglu_ok(e, tok)) return run_gemm(e, e->xn, w.wgu, tok, 2 * F, D, e->part, e->part_bytes, &S, st, -1, 0, true, nullptr, e->hbuf);
   TRY(run_gemm(e, e->xn, w.wgu, tok, 2 * F, D, e->part, e->part_bytes, &S, st));
@@ -2235,4 +2276,134 @@ extern "C" int pg_test_gemm(pg_engine* e, int impl, int is_bf16, const void* X, 
     CK(cudaMemsetAsync(C + (size_t)S * M * N, 0, (size_t)(std::max(splits, 1) - S) * M * N * 4, (cudaStream_t)stream));
   }
   return 0;
+}
+
+// One contraction as the engine issues it (run_gemm / run_conv_gemm / launch_swiglu_sk, PDL off) on caller-owned operands,
+// reporting the kernel that ran, so a test can compare each fused epilogue with a restatement of its rounding points.
+extern "C" int pg_test_contraction_run(pg_engine* e, pg_test_contraction* p, void* stream) {
+  TRY(check_ready(e));
+  if (!p) return fail("pg_test_contraction_run: null parameters");
+  p->path = PG_PATH_NONE; p->path_nt = 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (!e->bf16 || !e->use_tc) return fail("pg_test_contraction_run: needs a bf16 engine with use_tc");
+  const int M = p->M, N = p->N, K = p->K, mode = p->mode;
+  if (mode < PG_TC_PLAIN || mode > PG_TC_CONV) return fail("pg_test_contraction_run: mode=%d must be in [0, 6]", mode);
+  if (M < 1 || N < 1 || K < 1) return fail("pg_test_contraction_run: M=%d N=%d K=%d must be >= 1", M, N, K);
+  if (K % 8 != 0) return fail("pg_test_contraction_run: K=%d must be a multiple of 8", K);
+  if (!p->X || !p->W) return fail("pg_test_contraction_run: null X or W");
+  if ((((uintptr_t)p->X) | ((uintptr_t)p->W)) & 15) return fail("pg_test_contraction_run: X and W must be 16-byte aligned");
+  if (p->weights != 0 && p->weights != 1) return fail("pg_test_contraction_run: weights=%d must be 0 (row-major) or 1 (tile-major)", p->weights);
+  const bool out_mode = mode == PG_TC_ROWS || mode == PG_TC_SWIGLU || mode == PG_TC_SWIGLU_SK || (mode == PG_TC_CONV && p->out);
+  if (out_mode && !p->out) return fail("pg_test_contraction_run: out is required for mode %d", mode);
+  if ((mode == PG_TC_PLAIN || (mode == PG_TC_CONV && !p->out)) && !p->C) return fail("pg_test_contraction_run: C is required for mode %d", mode);
+  if (mode == PG_TC_RESID && !p->resid) return fail("pg_test_contraction_run: resid is required for mode %d", mode);
+  if ((p->gelu != 0 && p->gelu != 1) || (p->gelu && mode != PG_TC_ROWS)) return fail("pg_test_contraction_run: gelu=%d is 0, or 1 in PG_TC_ROWS", p->gelu);
+  if (p->add16 && p->gelu) return fail("pg_test_contraction_run: add16 and gelu are exclusive");
+  if (p->add16 && mode != PG_TC_ROWS && mode != PG_TC_CONV) return fail("pg_test_contraction_run: add16 needs PG_TC_ROWS or PG_TC_CONV");
+  if (p->bias && mode != PG_TC_ROWS && mode != PG_TC_RESID && mode != PG_TC_CONV) return fail("pg_test_contraction_run: bias needs PG_TC_ROWS, PG_TC_RESID or PG_TC_CONV");
+  if ((mode == PG_TC_SWIGLU || mode == PG_TC_SWIGLU_SK) && N % TC_BM != 0) return fail("pg_test_contraction_run: SwiGLU needs N %% 128 == 0 (N=%d)", N);
+  if (mode == PG_TC_SWIGLU && M > 128 && N <= TC_BM) return fail("pg_test_contraction_run: SwiGLU with M=%d > 128 runs on the CTA pair, which needs N > 128", M);
+  if ((mode == PG_TC_ROWS || mode == PG_TC_RESID) && N % 8 != 0) return fail("pg_test_contraction_run: fused epilogues need N %% 8 == 0 (N=%d)", N);
+  if (mode != PG_TC_PLAIN && p->splits > 1) return fail("pg_test_contraction_run: splits=%d: only PG_TC_PLAIN splits K", p->splits);
+  // weights: tile-major copy into the caller's buffer (the kernel pg_engine_finalize uses)
+  const uint8_t* w_tiled = nullptr;
+  if (p->weights == 1) {
+    if (mode == PG_TC_CONV) return fail("pg_test_contraction_run: the implicit convolution reads row-major weights only");
+    if (tc_pair_taken(M, N, mode == PG_TC_PLAIN ? std::max(p->splits, 1) : 1, mode == PG_TC_SWIGLU && M <= 128) && mode != PG_TC_SWIGLU_SK)
+      return fail("pg_test_contraction_run: M=%d N=%d runs on the CTA pair, which streams row-major weights (weights=1)", M, N);
+    if (!p->w_tiled || p->w_tiled_bytes < tile_major_bytes(N, K))
+      return fail("pg_test_contraction_run: w_tiled needs %zu bytes (has %zu)", tile_major_bytes(N, K), p->w_tiled_bytes);
+    TRY(build_tile_major(e, p->W, N, K, (uint8_t*)p->w_tiled, st));
+    w_tiled = (const uint8_t*)p->w_tiled;
+  } else if (mode == PG_TC_SWIGLU_SK) {
+    return fail("pg_test_contraction_run: stream-K streams tile-major weights (weights=1)");
+  }
+  QkvEpi qe = {};
+  if (mode == PG_TC_QKV) {
+    const int R = p->R, P = p->P, H = p->H, Tmax = p->Tmax;
+    if (H < 1 || N != 3 * H * HEAD_DIM) return fail("pg_test_contraction_run: QKV needs N == 3*H*128 (N=%d H=%d)", N, H);
+    if (!tc_pair_taken(M, N, 1, false)) return fail("pg_test_contraction_run: the QKV epilogue runs on the CTA pair only (M=%d must be > 128)", M);
+    if (!p->q_out || !p->kcache || !p->vcache || !p->kv_start) return fail("pg_test_contraction_run: QKV needs q_out, kcache, vcache and kv_start");
+    if (R < 1 || Tmax < 1) return fail("pg_test_contraction_run: QKV needs R=%d >= 1 and Tmax=%d >= 1", R, Tmax);
+    // every token's cache column and RoPE position, restated on the host for the bounds
+    std::vector<int32_t> ks(R), ro(R), rs(R, 0);
+    CK(cudaMemcpyAsync(ks.data(), p->kv_start, (size_t)R * 4, cudaMemcpyDeviceToHost, st));
+    if (p->row_off) CK(cudaMemcpyAsync(ro.data(), p->row_off, (size_t)R * 4, cudaMemcpyDeviceToHost, st));
+    if (p->rope_start) CK(cudaMemcpyAsync(rs.data(), p->rope_start, (size_t)R * 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (!p->row_off && (P < 1 || (size_t)M > (size_t)R * P)) return fail("pg_test_contraction_run: QKV padded block needs M=%d <= R*P (R=%d P=%d)", M, R, P);
+    for (int m = 0; m < M; ++m) {
+      int rw = 0, col = 0;
+      if (p->row_off) {
+        int lo = 0, hi = R - 1;
+        while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (ro[mid] <= m) lo = mid; else hi = mid - 1; }
+        rw = lo; col = ks[rw] + (m - ro[rw]);
+        if (m < ro[rw]) return fail("pg_test_contraction_run: QKV token %d lies before row_off[0]=%d", m, ro[0]);
+      } else {
+        rw = m / P; col = m % P;
+      }
+      const int pr = p->rope_start ? std::max(col - rs[rw], 0) : col;
+      if (col < 0 || col >= Tmax) return fail("pg_test_contraction_run: QKV token %d: cache column %d must be in [0, Tmax=%d)", m, col, Tmax);
+      if (pr >= e->Tmax) return fail("pg_test_contraction_run: QKV token %d: RoPE position %d must be below the engine's Tmax=%d", m, pr, e->Tmax);
+    }
+    NEED(cosT, float, "rope_cos");
+    NEED(sinT, float, "rope_sin");
+    qe = QkvEpi{cosT, sinT, (bf16*)p->q_out, (bf16*)p->kcache, (bf16*)p->vcache, p->row_off, p->kv_start, p->rope_start, R, P, H, Tmax};
+  }
+  const int saved_pdl = e->use_pdl;
+  e->use_pdl = 0;
+  int rc = 0;
+  int S = 1;
+  const size_t fused_bytes = (size_t)M * N * 4;   // the fused epilogues write no partials; run_gemm only checks the size
+  EpiFuse ep = {p->bias, (bf16*)p->out, nullptr, p->gelu, (const bf16*)p->add16};
+  switch (mode) {
+    case PG_TC_PLAIN: {
+      const int sp = std::max(p->splits, 1);
+      if (!p->C || p->c_bytes < (size_t)sp * M * N * 4) { rc = fail("pg_test_contraction_run: C needs splits*M*N*4 = %zu bytes", (size_t)sp * M * N * 4); break; }
+      rc = run_gemm(e, p->X, p->W, M, N, K, p->C, (size_t)sp * M * N * 4, &S, st, 1, sp, false, w_tiled);
+      if (!rc && S != sp) rc = cudaMemsetAsync(p->C + (size_t)S * M * N, 0, (size_t)(sp - S) * M * N * 4, st) == cudaSuccess ? 0 : fail("memset of unused splits failed");
+      break;
+    }
+    case PG_TC_ROWS:
+      rc = run_gemm(e, p->X, p->W, M, N, K, nullptr, fused_bytes, &S, st, 1, 1, false, w_tiled, nullptr, &ep);
+      break;
+    case PG_TC_RESID: {
+      const EpiFuse er = {p->bias, nullptr, p->resid, 0, nullptr};
+      rc = run_gemm(e, p->X, p->W, M, N, K, nullptr, fused_bytes, &S, st, 1, 1, false, w_tiled, nullptr, &er);
+      break;
+    }
+    case PG_TC_SWIGLU:
+      if (M <= 128) {
+        rc = run_gemm(e, p->X, p->W, M, N, K, nullptr, fused_bytes, &S, st, 1, 1, false, w_tiled, p->out);
+      } else {
+        const EpiFuse eg = {nullptr, (bf16*)p->out, nullptr, 2, nullptr};
+        rc = run_gemm(e, p->X, p->W, M, N, K, nullptr, fused_bytes, &S, st, 1, 1, false, nullptr, nullptr, &eg);
+      }
+      break;
+    case PG_TC_QKV: {
+      const EpiFuse eq = {nullptr, (bf16*)p->q_out, nullptr, 3, nullptr};
+      e->qkv_epi_next = qe;
+      rc = run_gemm(e, p->X, p->W, M, N, K, nullptr, fused_bytes, &S, st, 1, 1, false, nullptr, nullptr, &eq);
+      e->qkv_epi_next = QkvEpi{};
+      break;
+    }
+    case PG_TC_SWIGLU_SK:
+      if (!p->scratch || !p->counters) { rc = fail("pg_test_contraction_run: stream-K needs scratch and counters"); break; }
+      rc = launch_swiglu_sk(e, p->X, w_tiled, M, N / 2, K, p->ctas, p->scratch, p->scratch_bytes, p->counters, p->n_counters, (bf16*)p->out, st);
+      break;
+    case PG_TC_CONV: {
+      const int B = p->img_b, H = p->img_h, W = p->img_w, Cin = K / 9;
+      if (K % 9 != 0 || B < 1 || H < 1 || W < 1 || (size_t)M != (size_t)B * H * W) {
+        rc = fail("pg_test_contraction_run: conv needs K = 9*Cin and M = img_b*img_h*img_w (M=%d K=%d B=%d H=%d W=%d)", M, K, B, H, W);
+        break;
+      }
+      if (p->out && N % 8 != 0) { rc = fail("pg_test_contraction_run: the fused conv epilogue needs N %% 8 == 0 (N=%d)", N); break; }
+      int taken = 0;
+      rc = run_conv_gemm(e, p->X, p->W, B, H, W, Cin, N, p->C, p->C ? p->c_bytes : (size_t)M * N * 4, st, &taken, p->out ? &ep : nullptr);
+      break;
+    }
+  }
+  e->use_pdl = saved_pdl;
+  if (!rc) { p->path = e->last_path; p->path_nt = e->last_nt; }
+  return rc;
 }
