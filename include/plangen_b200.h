@@ -20,7 +20,7 @@
 extern "C" {
 #endif
 
-#define PG_ABI_VERSION 7
+#define PG_ABI_VERSION 8
 
 /* arithmetic regimes */
 #define PG_MODE_BF16 0 /* the reference's regime: fp32 master weights under autocast(bf16), plangen_base.py:360 */
@@ -182,6 +182,30 @@ int pg_sample_image_logprobs(pg_engine* e, float* x_prompt, const int32_t* kv_st
 int pg_score_image_tokens(pg_engine* e, float* x_seq, const int32_t* kv_start, int R, int P, int n,
                           const int32_t* image_tokens, const pg_image_sampling* per_image, float* logprobs_out,
                           void* stream);
+
+/* Guidance schedules: a guidance weight per image AND per step (LlamaGen's cfg_interval, MAR's linear ramp).
+ * cfg_schedule_host = HOST fp32 array [R/2][n] (row-major; copied at entry, reusable when the call returns): at step i
+ * image b is sampled exactly as the per-image entry points sample it with per_image[b].cfg_weight = cfg_schedule[b][i]
+ * (same rounding per op in the engine dtype, /temperature, top-k, top-p, softmax, Philox draws and offsets); its
+ * log-probs are taken under that distribution.  per_image[b].cfg_weight is IGNORED (it may hold anything, NaN
+ * included); every other field keeps its meaning.  Every entry must be finite: a failure names the image and the step
+ * ("image b, step i"), checked on the host without a device sync.
+ * A weight of 1 is u + 1 * (c - u) rounded per op, not the conditional logits alone: in bf16 the two can differ by a
+ * rounding, so an interval schedule (w, then 1) reproduces "guidance off" in distribution, not bit for bit.  The
+ * unconditional rows are computed on every step, also after the last step whose weight differs from 1. */
+
+/* pg_sample_image_per_image with a guidance schedule [R/2][n_steps]; logprobs_out fp32 [R/2, n_steps] as for
+ * pg_sample_image_logprobs, or NULL for none.  The schedule is staged in the engine and read on the device: the captured
+ * decode-step graph's key gains a schedule flag but not the values, so new schedules replay the same graph. */
+int pg_sample_image_scheduled(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
+                              const pg_image_sampling* per_image, int rng_per_image, int greedy,
+                              const int32_t* edit_region, const int32_t* gt_labels, const float* cfg_schedule_host,
+                              int32_t* tokens_out, float* logprobs_out, void* stream);
+
+/* pg_score_image_tokens with a guidance schedule [R/2][n]: position i of image b is scored with cfg_schedule[b][i]. */
+int pg_score_image_tokens_scheduled(pg_engine* e, float* x_seq, const int32_t* kv_start, int R, int P, int n,
+                                    const int32_t* image_tokens, const pg_image_sampling* per_image,
+                                    const float* cfg_schedule_host, float* logprobs_out, void* stream);
 
 /* replaces: System.x2t (plangen_base.py:513-523) = vl_gpt.language_model.generate(inputs_embeds=,
  *           attention_mask=, pad_token_id=, eos_token_id=, max_new_tokens=, do_sample=False, use_cache=True),

@@ -81,6 +81,11 @@ EXPORTS = {
                                            C.c_void_p, C.c_void_p]),
     "pg_score_image_tokens": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                         C.POINTER(PgImageSampling), C.c_void_p, C.c_void_p]),
+    "pg_sample_image_scheduled": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                            C.POINTER(PgImageSampling), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_void_p, C.c_void_p, C.c_void_p]),
+    "pg_score_image_tokens_scheduled": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                                  C.POINTER(PgImageSampling), C.c_void_p, C.c_void_p, C.c_void_p]),
     "pg_generate_greedy": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_void_p, C.POINTER(C.c_int), C.c_void_p]),
     "pg_vq_decode_code": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
@@ -125,7 +130,7 @@ def load(build_if_missing: bool = True):
         fn = getattr(lib, name)      # AttributeError if the symbol is not exported
         fn.restype = res
         fn.argtypes = args
-    if lib.pg_abi_version() != 7:
+    if lib.pg_abi_version() != 8:
         raise PgError("ABI version mismatch")
     _LIB = lib
     return lib

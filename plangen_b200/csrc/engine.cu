@@ -103,6 +103,7 @@ struct pg_engine {
   int32_t *st_kv_start = nullptr, *st_edit = nullptr, *st_gt = nullptr, *st_tokens = nullptr;
   ImageSampling* st_sampling = nullptr;               // per-image entry points: [B] settings (sample.cuh)
   float* st_logprobs = nullptr;                       // pg_sample_image_logprobs: [B][n_steps]
+  float* st_cfg = nullptr;                            // the *_scheduled entry points: guidance schedule [B][n_steps]
   // mmu front-end (SigLIP tower + aligner + scatter, vit_kernels.cuh); carved only when dims.sig_layers > 0
   int sig_chunk = 0, sig_np = 0;                      // images per pass, patches per image
   float *sig_x = nullptr, *sig_part = nullptr;
@@ -417,6 +418,7 @@ static void layout_workspace(pg_engine* e, Carve& c) {
     e->st_tokens = (int32_t*)c.take(R * (size_t)e->Tmax * 4);      // image loop: [B][n_steps]; text loop: [R][max_new]
     e->st_sampling = (ImageSampling*)c.take(B * sizeof(ImageSampling));
     e->st_logprobs = (float*)c.take(B * std::max(d.max_steps, 1) * 4);
+    e->st_cfg = (float*)c.take(B * std::max(d.max_steps, 1) * 4);
   }
   if (d.sig_layers > 0 && d.max_images > 0) {
     // SigLIP tower scratch for one pass of sig_chunk images; features of ALL images stay (the scatter needs them)
@@ -1195,10 +1197,12 @@ static void philox_policy(pg_engine* e, size_t numel, uint64_t* counter_offset, 
 
 // Per-image settings of one sampler launch or decode loop (the per-image entry points; nullptr everywhere else):
 // `dev` holds B staged entries; the scalar settings arguments are then ignored.  any_top_p: some image has top_p < 1.
+// cfg_sched: the staged guidance schedule [B][n_steps] of the *_scheduled entry points (nullptr: dev's cfg_weight).
 struct PerImage {
   const ImageSampling* dev;
   int rng_per_image;
   bool any_top_p;
+  const float* cfg_sched;
 };
 
 // Philox element count of one draw: the whole (B, V) tensor, or one image's (1, V) row with per-image generators
@@ -1230,11 +1234,13 @@ static int k_sample(pg_engine* e, const float* part, int S, size_t sstride, cons
              launch(e, cfg_sample_embed_cluster_kernel<bf16>, dim3(B * SAMPLE_CLUSTER), dim3(SAMPLE_CL_THREADS), csm, st, part, S, sstride, bias, B, d.img_vocab,
                     cfg_weight, temperature, seed, offset_base, per_step, stride, greedy, top_k, top_p_thr, edit_region, gt_labels,
                     step_base, step_ptr, n_steps, tokens_out, (const bf16*)e->embed_table, d.D, x_next, next_norm_w, (bf16*)xn_next,
-                    d.rms_eps, 1, score_n ? nullptr : e->dbg_logits, pi ? pi->dev : nullptr, pi ? pi->rng_per_image : 0, logprobs, score_n),
+                    d.rms_eps, 1, score_n ? nullptr : e->dbg_logits, pi ? pi->dev : nullptr, pi ? pi->rng_per_image : 0, logprobs, score_n,
+                    pi ? pi->cfg_sched : nullptr),
              launch(e, cfg_sample_embed_cluster_kernel<float>, dim3(B * SAMPLE_CLUSTER), dim3(SAMPLE_CL_THREADS), csm, st, part, S, sstride, bias, B, d.img_vocab,
                     cfg_weight, temperature, seed, offset_base, per_step, stride, greedy, top_k, top_p_thr, edit_region, gt_labels,
                     step_base, step_ptr, n_steps, tokens_out, (const float*)e->embed_table, d.D, x_next, next_norm_w, (float*)xn_next,
-                    d.rms_eps, 0, score_n ? nullptr : e->dbg_logits, pi ? pi->dev : nullptr, pi ? pi->rng_per_image : 0, logprobs, score_n));
+                    d.rms_eps, 0, score_n ? nullptr : e->dbg_logits, pi ? pi->dev : nullptr, pi ? pi->rng_per_image : 0, logprobs, score_n,
+                    pi ? pi->cfg_sched : nullptr));
   return 0;
 }
 
@@ -1254,11 +1260,12 @@ extern "C" int pg_cfg_sample_embed(pg_engine* e, const float* logits, int B, flo
 }
 
 // The caller's per-image settings, validated (naming the image) and converted to the kernel's entries.  Batch-wide RNG:
-// every entry takes image 0's seed and offset.
+// every entry takes image 0's seed and offset.  cfg_sched: the guidance schedule [B][n_steps] (empty: none).
 struct StagedSampling {
   std::vector<ImageSampling> dev;
   int rng_per_image = 0;
   bool any_top_p = false;
+  std::vector<float> cfg_sched;
 };
 
 static int convert_per_image(const pg_image_sampling* h, int B, int rng_per_image, StagedSampling* out) {
@@ -1276,10 +1283,25 @@ static int convert_per_image(const pg_image_sampling* h, int B, int rng_per_imag
   return 0;
 }
 
-// copy into st_sampling on `st` (a plain copy from pageable memory: `ss` may go when it returns)
+// The caller's guidance schedule (HOST [B][n]), checked on the host (no device sync; a failure names the entry) and kept
+// in `out` for stage_per_image.
+static int convert_schedule(const float* h, int B, int n, StagedSampling* out) {
+  if (!h) return fail("null argument");
+  for (int b = 0; b < B; ++b)
+    for (int i = 0; i < n; ++i)
+      if (!std::isfinite(h[(size_t)b * n + i]))
+        return fail("image %d, step %d: cfg_schedule must be finite, got %g", b, i, h[(size_t)b * n + i]);
+  out->cfg_sched.assign(h, h + (size_t)B * n);
+  return 0;
+}
+
+// copy into st_sampling (and st_cfg) on `st` (plain copies from pageable memory: `ss` may go when it returns)
 static int stage_per_image(pg_engine* e, const StagedSampling& ss, cudaStream_t st, PerImage* out) {
   CK(cudaMemcpyAsync(e->st_sampling, ss.dev.data(), ss.dev.size() * sizeof(ImageSampling), cudaMemcpyHostToDevice, st));
-  *out = {e->st_sampling, ss.rng_per_image, ss.any_top_p};
+  const bool sched = !ss.cfg_sched.empty();
+  if (sched)
+    CK(cudaMemcpyAsync(e->st_cfg, ss.cfg_sched.data(), ss.cfg_sched.size() * 4, cudaMemcpyHostToDevice, st));
+  *out = {e->st_sampling, ss.rng_per_image, ss.any_top_p, sched ? e->st_cfg : nullptr};
   return 0;
 }
 
@@ -1425,9 +1447,9 @@ static int image_loop(pg_engine* e, float* x_prompt, const int32_t* kv_start, in
     if (e->use_graph) {
       char key[256];
       const int prof = (e->prof_buf && e->prof_step >= 0) ? 1 : 0;
-      if (pi)   // the settings are read from st_sampling: one graph serves every seed and setting of this shape
-        snprintf(key, sizeof(key), "imgpi/%d/%d/%d/%d/%d/%d/%d/%d/%d", R, P, n_steps, greedy, edit_region ? 1 : 0,
-                 pi->rng_per_image, pi->any_top_p ? 1 : 0, lps ? 1 : 0, prof);
+      if (pi)   // settings and schedule are read from st_sampling / st_cfg: one graph serves every value of this shape
+        snprintf(key, sizeof(key), "imgpi/%d/%d/%d/%d/%d/%d/%d/%d/%d/%d", R, P, n_steps, greedy, edit_region ? 1 : 0,
+                 pi->rng_per_image, pi->any_top_p ? 1 : 0, lps ? 1 : 0, pi->cfg_sched ? 1 : 0, prof);
       else
         snprintf(key, sizeof(key), "img/%d/%d/%d/%a/%a/%llu/%d/%d/%a/%d/%d", R, P, n_steps, cfg_weight, temperature,
                  (unsigned long long)seed, greedy, top_k, top_p, edit_region ? 1 : 0, prof);
@@ -1508,13 +1530,26 @@ extern "C" int pg_sample_image_logprobs(pg_engine* e, float* x_prompt, const int
                     tokens_out, stream, &ss, logprobs_out);
 }
 
+extern "C" int pg_sample_image_scheduled(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
+                                         const pg_image_sampling* per_image, int rng_per_image, int greedy,
+                                         const int32_t* edit_region, const int32_t* gt_labels, const float* cfg_schedule_host,
+                                         int32_t* tokens_out, float* logprobs_out, void* stream) {
+  TRY(check_image_loop(e, kv_start, R, n_steps, edit_region, gt_labels, tokens_out));
+  StagedSampling ss;
+  TRY(convert_per_image(per_image, R / 2, rng_per_image, &ss));
+  TRY(convert_schedule(cfg_schedule_host, R / 2, n_steps, &ss));
+  return image_loop(e, x_prompt, kv_start, R, P, n_steps, 0.f, 1.f, 0, greedy, 0, 1.0, edit_region, gt_labels,
+                    tokens_out, stream, &ss, logprobs_out);
+}
+
 // ------------------------------------------------------------------------------ teacher-forced scoring
 // One prefill over prompt + image tokens, the hidden states of columns P-1 .. P+n-2 pair-major in hbuf (prefill_impl's
 // `tail`), gen_head over those R * n rows in as few wide contractions as the idle prefill scratch allows (part holds one
 // chunk's logits, qbuf its first-layer activations), and the sampler kernel in score mode per chunk.
-extern "C" int pg_score_image_tokens(pg_engine* e, float* x_seq, const int32_t* kv_start, int R, int P, int n,
-                                     const int32_t* image_tokens, const pg_image_sampling* per_image, float* logprobs_out,
-                                     void* stream) {
+// cfg_schedule_host: the guidance schedule [R/2][n] of pg_score_image_tokens_scheduled, nullptr for pg_score_image_tokens.
+static int score_image_tokens(pg_engine* e, float* x_seq, const int32_t* kv_start, int R, int P, int n,
+                              const int32_t* image_tokens, const pg_image_sampling* per_image,
+                              const float* cfg_schedule_host, float* logprobs_out, void* stream) {
   TRY(check_ready(e));
   const pg_dims& d = e->d;
   if (!x_seq || !kv_start || !image_tokens || !logprobs_out) return fail("null argument");
@@ -1530,6 +1565,7 @@ extern "C" int pg_score_image_tokens(pg_engine* e, float* x_seq, const int32_t* 
   NEED(b1, float, "head.b1");
   StagedSampling ss;
   TRY(convert_per_image(per_image, R / 2, 0, &ss));
+  if (cfg_schedule_host) TRY(convert_schedule(cfg_schedule_host, R / 2, n, &ss));
   cudaStream_t st = (cudaStream_t)stream;
   PerImage pi;
   TRY(stage_per_image(e, ss, st, &pi));
@@ -1553,6 +1589,19 @@ extern "C" int pg_score_image_tokens(pg_engine* e, float* x_seq, const int32_t* 
                  (int)(r0 / 2), nullptr, n, nullptr, nullptr, nullptr, nullptr, st, &pi, logprobs_out, n));
   }
   return 0;
+}
+
+extern "C" int pg_score_image_tokens(pg_engine* e, float* x_seq, const int32_t* kv_start, int R, int P, int n,
+                                     const int32_t* image_tokens, const pg_image_sampling* per_image, float* logprobs_out,
+                                     void* stream) {
+  return score_image_tokens(e, x_seq, kv_start, R, P, n, image_tokens, per_image, nullptr, logprobs_out, stream);
+}
+
+extern "C" int pg_score_image_tokens_scheduled(pg_engine* e, float* x_seq, const int32_t* kv_start, int R, int P, int n,
+                                               const int32_t* image_tokens, const pg_image_sampling* per_image,
+                                               const float* cfg_schedule_host, float* logprobs_out, void* stream) {
+  if (!cfg_schedule_host) return fail("null argument");
+  return score_image_tokens(e, x_seq, kv_start, R, P, n, image_tokens, per_image, cfg_schedule_host, logprobs_out, stream);
 }
 
 // ------------------------------------------------------------------------------ f1: stage-1 text decode (x2t)

@@ -84,6 +84,8 @@ __device__ unsigned long long* g_sample_dbg = nullptr;   // debug timeline (tool
 // underflow to 0), -inf when a filter removed tok (only a forced token can be removed).
 // score_n > 0 (teacher-forced scoring): cluster b scores the pair g = step_base + b, image g / score_n, position
 // g % score_n (n_steps == score_n); the token is always gt_labels[g], no variates are drawn and there is no arg-max.
+// cfg_sched != nullptr (guidance schedules): the guidance weight is cfg_sched[image * n_steps + step] instead of the
+// scalar or per-image one, read wherever the weight is read; in score mode that index is g.
 constexpr int SAMPLE_CLUSTER = 8;
 
 // device copy of one pg_image_sampling entry (engine.cu converts top_p to the threshold the kernel compares with)
@@ -209,7 +211,7 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
                                 float* __restrict__ x_next, const float* __restrict__ next_norm_w, T* __restrict__ xn_next,
                                 float eps, int round_resid, float* __restrict__ dbg_logits,
                                 const ImageSampling* __restrict__ per_image, int rng_per_image,
-                                float* __restrict__ logprobs, int score_n) {
+                                float* __restrict__ logprobs, int score_n, const float* __restrict__ cfg_sched) {
   extern __shared__ __align__(16) float sh[];   // this CTA's slice of the CFG logits -> unnormalised probabilities
   // top_p_thr >= 0 (top-p on): sh is followed by the slice's logits t and the mass histograms of its radix select
   __shared__ uint32_t hist[4][256];  // top-k radix select: one histogram per pass (read by the other CTAs)
@@ -231,13 +233,15 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
   // launches the host passes the step explicitly (step_ptr == nullptr), so reading it before the PDL wait is safe.
   const int step = score_n ? (step_base + b) % score_n : step_base + (step_ptr ? *step_ptr : 0);
   const int img = score_n ? (step_base + b) / score_n : b;
-  // The per-image settings are staged by a copy before the decode loop, never written by a kernel of the loop, so they
-  // are read before the PDL wait too: the Philox prefetch below needs the image's seed and offset.
+  // The per-image settings and the guidance schedule are staged by a copy before the decode loop, never written by a
+  // kernel of the loop, so they are read before the PDL wait too: the Philox prefetch below needs the image's seed and
+  // offset.
   if (per_image != nullptr) {
     const ImageSampling s = per_image[img];
     cfg_weight = s.cfg_weight; temperature = s.temperature; top_k = s.top_k; top_p_thr = s.top_p_thr;
     seed = s.seed; offset_base += s.offset;
   }
+  if (cfg_sched != nullptr) cfg_weight = cfg_sched[(size_t)img * n_steps + step];
   const uint64_t offset = offset_base + offset_per_step * (uint64_t)(step - step_base);
   // The exponential variates of torch.multinomial depend on (seed, offset, element index) only - not on the logits: they
   // are drawn while the head contraction is still streaming its weights (this kernel is launched ahead of its dependency).
@@ -458,7 +462,8 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
   }
   if (logprobs != nullptr && tok >= v_lo && tok < v_hi && tid == (tok - v_lo) % SAMPLE_CL_THREADS) {
     // the settings are read again rather than kept in registers across the filters (the kernel is at its register limit)
-    const float w = per_image ? __ldcg(&per_image[img].cfg_weight) : cfg_weight;
+    const float w = cfg_sched ? __ldcg(cfg_sched + (size_t)img * n_steps + step)
+                              : per_image ? __ldcg(&per_image[img].cfg_weight) : cfg_weight;
     const float temp = per_image ? __ldcg(&per_image[img].temperature) : temperature;
     const size_t c_at = (size_t)(2 * b) * V + tok, u_at = c_at + V;
     float c, u;

@@ -124,6 +124,42 @@ def sampling_plan(num_gen: int, cfg_weight, temperature, top_k, top_p, generator
                         [_i64(x) for x in seeds], offs, gens)
 
 
+def guidance_schedule(cfg_weight, num_gen: int, n: int) -> Optional[torch.Tensor]:
+    """A guidance schedule: cfg_weight as a 2-D tensor or nested sequence of shape (num_gen, n), entry [j, i] the weight
+    of image j at step i (image j = copy * B + b under t2i's parallel_size), returned as the CPU fp32 table the
+    *_scheduled ops take.  None for a scalar or 1-D cfg_weight, which sampling_plan handles as before.  A wrong shape,
+    more than two dimensions or a non-finite entry raises ValueError naming the entry."""
+    if isinstance(cfg_weight, torch.Tensor):
+        if cfg_weight.dim() < 2:
+            return None
+        if cfg_weight.dim() != 2:
+            raise ValueError(f"`cfg_weight` must be a scalar, one value per image or an (images, steps) schedule, "
+                             f"got shape {tuple(cfg_weight.shape)}")
+        rows = cfg_weight.tolist()
+    elif isinstance(cfg_weight, (list, tuple)) and any(_is_seq(r) for r in cfg_weight):
+        rows = []
+        for j, r in enumerate(cfg_weight):
+            if not _is_seq(r):
+                raise ValueError(f"`cfg_weight[{j}]` is a scalar; a schedule needs a sequence of {n} steps per image")
+            rows.append(r.tolist() if isinstance(r, torch.Tensor) else list(r))
+    else:
+        return None
+    if len(rows) != num_gen:
+        raise ValueError(f"`cfg_weight` schedule has {len(rows)} rows for {num_gen} generated images")
+    for j, r in enumerate(rows):
+        if len(r) != n:
+            raise ValueError(f"`cfg_weight[{j}]` has {len(r)} steps for {n} image tokens")
+        for i, w in enumerate(r):
+            if _is_seq(w):
+                raise ValueError(f"`cfg_weight[{j}, {i}]` is a sequence; a schedule has two dimensions (images, steps)")
+    table = torch.tensor(rows, dtype=torch.float32).reshape(num_gen, n)
+    bad = (~torch.isfinite(table)).nonzero()
+    if len(bad):
+        j, i = (int(v) for v in bad[0])
+        raise ValueError(f"`cfg_weight[{j}, {i}]` must be finite, got {rows[j][i]}")
+    return table
+
+
 def check_score_args(num_gen: int, P: int, image_tokens: torch.Tensor, mask: Optional[torch.Tensor], img_vocab: int,
                      max_steps: int) -> int:
     """Validates the arguments of FastJanus.score_image_tokens (prompt rows 2 * num_gen of P columns) and returns n, the
@@ -538,14 +574,20 @@ class FastJanus:
         generator is advanced by n draws on a (1, img_vocab) tensor.  See sampling_plan.
         return_logprobs: returns (tokens, logprobs), logprobs fp32 (num_gen, n) = log p(token) of every step under the
         distribution the draw used (CFG, temperature, top-k, top-p; greedy: top-k only), forced tokens included (-inf
-        where a filter removed one).  Tokens, draws and generator offsets are the same as without it."""
+        where a filter removed one).  Tokens, draws and generator offsets are the same as without it.
+        Guidance schedule: cfg_weight may also be a 2-D tensor or nested sequence (num_gen, n), entry [j, i] the weight
+        of image j at step i (see guidance_schedule); step i of image j is then sampled exactly as with the per-image
+        cfg_weight[j] = cfg_weight[j, i], and the log-probs are taken under that distribution.  A weight of 1 is
+        u + 1 * (c - u) rounded per op, not the conditional logits alone (in bf16 they can differ by a rounding), and the
+        unconditional rows are computed on every step."""
         R, P, D = inputs_embeds.shape
         if R != 2 * num_gen:
             raise ValueError("inputs_embeds rows must be 2 * num_gen (interleaved cond/uncond)")
         n = int(image_token_num_per_image)
         k = self.top_k if top_k is None else top_k
         p = self.top_p if top_p is None else top_p
-        plan = sampling_plan(num_gen, cfg_weight, temperature, k, p, generator, self.seed)
+        sched = guidance_schedule(cfg_weight, num_gen, n)
+        plan = sampling_plan(num_gen, 1.0 if sched is not None else cfg_weight, temperature, k, p, generator, self.seed)
         kv_start = (kv_start_from_mask(mask.to(self.device), P) if mask is not None
                     else torch.zeros(R, dtype=torch.int32, device=self.device))
         x = inputs_embeds.to(device=self.device, dtype=torch.float32).contiguous().clone()
@@ -556,8 +598,12 @@ class FastJanus:
             er, gl = self._teacher_inputs(batch, gt_labels, num_gen, n)
         self._keep = (kv_start, x, er, gl)        # keep alive until the stream has consumed them
         logprobs = None
-        if return_logprobs:              # all-scalar settings too: uniform lists sample exactly as the scalar op
+        if return_logprobs:
             logprobs = torch.empty(num_gen, n, dtype=torch.float32, device=self.device)
+        if sched is not None:            # the schedule replaces the per-image cfg_weight
+            OPS.sample_image_scheduled(self.handle, x, kv_start, n, sched, plan.temperature, plan.top_k, plan.top_p, plan.seed,
+                                       plan.offset, plan.rng_per_image, bool(greedy), er, gl, tokens, logprobs)
+        elif return_logprobs:            # all-scalar settings too: uniform lists sample exactly as the scalar op
             OPS.sample_image_logprobs(self.handle, x, kv_start, n, plan.cfg_weight, plan.temperature, plan.top_k, plan.top_p,
                                       plan.seed, plan.offset, plan.rng_per_image, bool(greedy), er, gl, tokens, logprobs)
         elif not plan.per_image:
@@ -583,7 +629,8 @@ class FastJanus:
         reference does (or ready-made `gt_labels` are used), and `mask_image` is returned.  With the flag off `gt_image` and
         batch['edit_region'] are ignored, exactly as in the reference.
         cfg_weight, temperature, top_k, top_p and `generator` take per-image values as sample_image does, image
-        j = copy * B + b of the `parallel_size` copies; generator None: the engine's seed.
+        j = copy * B + b of the `parallel_size` copies; generator None: the engine's seed.  A 2-D cfg_weight
+        (parallel_size * B, n) is a guidance schedule, row j for image j (see sample_image).
         return_logprobs: returns (dec, mask_image, logprobs) with the per-step log-probs of sample_image."""
         n = image_token_num_per_image or self.dims.n_img_tokens
         img_size = img_size or self.dims.img_size
@@ -629,7 +676,8 @@ class FastJanus:
         the reference's single full-sequence forward (fp32 residual stream); the decode loop keeps a bf16 residual stream,
         so in bf16 the two are different valid evaluations, equal within fp32 noise in fp32 check mode.
         `tokens` (2B, P) ids or `emb` (2B, P, D), and `mask` (2B, P + n), as t2i takes them; image_tokens (B, n) ids in
-        [0, img_vocab); settings scalar or per image.  P + n - 1 must fit the engine's max_prompt."""
+        [0, img_vocab); settings scalar or per image, and cfg_weight also a (B, n) guidance schedule as sample_image takes
+        it (position i of image b scored with cfg_weight[b, i]).  P + n - 1 must fit the engine's max_prompt."""
         if tokens is None and emb is None:
             raise ValueError("pass `tokens` (2B, P) or `emb` (2B, P, D)")
         if mask is None:
@@ -643,14 +691,20 @@ class FastJanus:
         if image_tokens is None:
             raise ValueError("`image_tokens` (B, n) is required")
         n = check_score_args(B, P, image_tokens, mask, self.dims.img_vocab, self.max_steps)
-        plan = sampling_plan(B, cfg_weight, temperature, top_k, top_p, None, self.seed)
+        sched = guidance_schedule(cfg_weight, B, n)
+        plan = sampling_plan(B, 1.0 if sched is not None else cfg_weight, temperature, top_k, top_p, None, self.seed)
         kv_start = kv_start_from_mask(mask.to(self.device), P)
         x = torch.empty(R, P + n - 1, D, dtype=torch.float32, device=self.device)
         x[:, :P] = emb.to(device=self.device, dtype=torch.float32)
         ids = image_tokens.to(device=self.device, dtype=torch.int32).contiguous()
         out = torch.empty(B, n, dtype=torch.float32, device=self.device)
         self._keep = (kv_start, x, ids)
-        OPS.score_image_tokens(self.handle, x, kv_start, P, ids, plan.cfg_weight, plan.temperature, plan.top_k, plan.top_p, out)
+        if sched is not None:
+            OPS.score_image_tokens_scheduled(self.handle, x, kv_start, P, ids, sched, plan.temperature, plan.top_k,
+                                             plan.top_p, out)
+        else:
+            OPS.score_image_tokens(self.handle, x, kv_start, P, ids, plan.cfg_weight, plan.temperature, plan.top_k,
+                                   plan.top_p, out)
         self._serial += 1                # the KV cache now holds the scored sequence
         return out
 
