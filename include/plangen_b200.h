@@ -20,7 +20,7 @@
 extern "C" {
 #endif
 
-#define PG_ABI_VERSION 8
+#define PG_ABI_VERSION 9
 
 /* arithmetic regimes */
 #define PG_MODE_BF16 0 /* the reference's regime: fp32 master weights under autocast(bf16), plangen_base.py:360 */
@@ -84,34 +84,23 @@ int pg_decode_step(pg_engine* e, const float* x, const int32_t* kv_start, int R,
  * hidden fp32 [R,D] -> logits fp32 [R,img_vocab] (bf16-rounded values in PG_MODE_BF16). */
 int pg_gen_head(pg_engine* e, const float* hidden, int R, float* logits_out, void* stream);
 
-/* replaces: plangen_base.py:580-604 — CFG combine, /temperature, softmax,
- * torch.multinomial(1) (Philox4x32-10, bit-compatible with torch's CUDA generator at
- * (seed, philox_offset)), teacher-forcing override (:593-598), token duplication and
- * prepare_gen_img_embeds.  logits fp32 [2B, V] (rows interleaved cond/uncond).
- * edit_region / gt_labels: int32 [B, n_steps], both or neither (NULL = no teacher forcing; the caller gates them on
- * args.use_teacher_forcing as the reference does, :593).  greedy != 0 -> argmax.
- * top_k > 0: only CFG logits >= the k-th largest survive (`logits[logits < topk(logits,k)[..., -1:]] = -inf`) before
- * the softmax; 0 = off = the reference (it has no top-k; north_star names the option).
- * top_p in [0, 1) (after top-k): HF TopPLogitsWarper with min_tokens_to_keep = 1 - in ascending (logit, index) order
- * the longest prefix whose cumulative probability is <= fp32(1 - top_p) is removed, the largest logit always stays;
- * 1 = off (the default, the unfiltered path).  Outside [0, 1] or NaN: failure.  Ignored when greedy != 0.
- * tokens_out int32 [B, n_steps] (column `step` written); x_next fp32 [2B, D]. */
-int pg_cfg_sample_embed(pg_engine* e, const float* logits, int B, float cfg_weight,
-                        float temperature, uint64_t seed, uint64_t philox_offset, int greedy, int top_k,
-                        double top_p, const int32_t* edit_region, const int32_t* gt_labels, int step,
-                        int n_steps, int32_t* tokens_out, float* x_next, void* stream);
-
-/* Sampling settings of one image for the *_per_image entry points, passed as a HOST array of B entries (copied at entry;
- * the array may be reused when the call returns).  Image b is sampled exactly as the scalar entry points sample a whole
- * batch run with (cfg_weight, temperature, top_k, top_p): CFG per op in the engine dtype, a correctly rounded
- * /temperature, top-k, top-p, softmax.  top_k >= 0 and top_p in [0, 1] (NaN fails) are checked per image and a failure
- * names the image.  top_p is a double, like the scalar entries' argument: the kernel compares against fp32(1 - top_p)
- * with 1 - top_p in double, as torch does.
- * seed / offset: rng_per_image != 0 - image b draws as torch.multinomial(probs[b:b+1], 1, generator=g_b) with g_b at
- * (seed, offset): element v of a (1, V) tensor, so its tokens depend neither on b nor on B; each step advances its
- * offset by torch's per-draw increment for numel = V (4 at V = 16384).  rng_per_image == 0 - entry 0's seed and offset
- * serve the whole call with the scalar path's mapping (element b * V + v of one (B, V) draw); the other entries' seed
- * and offset are ignored. */
+/* Sampling settings of one image, passed to the three sampling entry points below as a HOST array of B entries (copied at
+ * entry; the array may be reused when the call returns).  One batch can serve requests with different seeds, guidance
+ * scales, temperatures, top-k and top-p; batch-wide settings are the same entry repeated.
+ * Image b is sampled with its (cfg_weight, temperature, top_k, top_p): CFG rounded per op in the engine dtype, a
+ * correctly rounded /temperature, top-k, top-p, softmax.
+ *   top_k > 0: only CFG logits >= the k-th largest survive (`logits[logits < topk(logits,k)[..., -1:]] = -inf`) before
+ *     the softmax; 0 = off = the reference (it has no top-k; north_star names the option).
+ *   top_p in [0, 1) (after top-k): HF TopPLogitsWarper with min_tokens_to_keep = 1 - in ascending (logit, index) order
+ *     the longest prefix whose cumulative probability is <= fp32(1 - top_p) is removed, the largest logit always stays;
+ *     1 = off (the unfiltered path).  top_p is a double: the kernel compares against fp32(1 - top_p) with 1 - top_p in
+ *     double, as torch does.  Ignored when greedy != 0.
+ *   top_k >= 0 and top_p in [0, 1] (NaN fails) are checked per image, and a failure names the image.
+ * seed / offset: torch.multinomial(1) with Philox4x32-10, bit-compatible with torch's CUDA generator at (seed, offset).
+ *   rng_per_image != 0 - image b draws as torch.multinomial(probs[b:b+1], 1, generator=g_b) with g_b at (seed, offset):
+ *   element v of a (1, V) tensor, so its tokens depend neither on b nor on B; each step advances its offset by torch's
+ *   per-draw increment for numel = V (4 at V = 16384).  rng_per_image == 0 - entry 0's seed and offset serve the whole
+ *   call as one generator drawing a (B, V) tensor (element b * V + v); the other entries' seed and offset are ignored. */
 typedef struct pg_image_sampling {
   uint64_t seed, offset;
   float cfg_weight, temperature;
@@ -119,11 +108,35 @@ typedef struct pg_image_sampling {
   double top_p;
 } pg_image_sampling;
 
-/* pg_cfg_sample_embed with per-image settings: per_image = HOST array [B] (see pg_image_sampling; its offsets are the
- * offsets of this draw).  greedy, teacher forcing, step, n_steps and the outputs as for pg_cfg_sample_embed. */
-int pg_cfg_sample_embed_per_image(pg_engine* e, const float* logits, int B, const pg_image_sampling* per_image,
-                                  int rng_per_image, int greedy, const int32_t* edit_region, const int32_t* gt_labels,
-                                  int step, int n_steps, int32_t* tokens_out, float* x_next, void* stream);
+/* Image-token log-probabilities (logprobs_out; NULL: none).  For image b at step i the value is log p(tok) in fp32, p
+ * being exactly the distribution the sampler draws from (CFG rounded per op in the engine dtype, /temperature, top-k,
+ * top-p, softmax; in greedy mode top-k only) and tok the token emitted at that step, sampled or forced by teacher forcing:
+ * (t_tok - max) - log(sum of the kept e), HF compute_transition_scores(..., normalize_logits=True) on the processed
+ * scores.  A forced token a filter removed gets -inf; a kept one whose exp underflows still gets its finite value.
+ * Log-probs change no token, no Philox draw and no offset.
+ *
+ * Guidance schedules (cfg_schedule_host; NULL: per_image[b].cfg_weight): a guidance weight per image AND per step
+ * (LlamaGen's cfg_interval, MAR's linear ramp), a HOST fp32 array [R/2][n] (row-major; copied at entry, reusable when the
+ * call returns).  At step i image b is sampled exactly as with per_image[b].cfg_weight = cfg_schedule[b][i] (same
+ * rounding per op, /temperature, top-k, top-p, softmax, Philox draws and offsets); its log-probs are taken under that
+ * distribution.  per_image[b].cfg_weight is then IGNORED (it may hold anything, NaN included); every other field keeps
+ * its meaning.  Every entry must be finite: a failure names the image and the step ("image b, step i"), checked on the
+ * host without a device sync.  A weight of 1 is u + 1 * (c - u) rounded per op, not the conditional logits alone: in
+ * bf16 the two can differ by a rounding, so an interval schedule (w, then 1) reproduces "guidance off" in distribution,
+ * not bit for bit.  The unconditional rows are computed on every step, also after the last step whose weight differs
+ * from 1. */
+
+/* replaces: plangen_base.py:580-604 — CFG combine, /temperature, softmax, torch.multinomial(1), teacher-forcing override
+ * (:593-598), token duplication and prepare_gen_img_embeds.  logits fp32 [2B, V] (rows interleaved cond/uncond).
+ * per_image HOST [B] (see pg_image_sampling; its offsets are the offsets of this draw).
+ * edit_region / gt_labels: int32 [B, n_steps], both or neither (NULL = no teacher forcing; the caller gates them on
+ * args.use_teacher_forcing as the reference does, :593).  greedy != 0 -> argmax.
+ * tokens_out int32 [B, n_steps] (column `step` written); x_next fp32 [2B, D]; logprobs_out fp32 [B, n_steps] (column
+ * `step` written) or NULL.  The settings are staged in engine memory on `stream`: like every entry point, calls on one
+ * engine must be made in order. */
+int pg_cfg_sample_embed(pg_engine* e, const float* logits, int B, const pg_image_sampling* per_image, int rng_per_image,
+                        int greedy, const int32_t* edit_region, const int32_t* gt_labels, int step, int n_steps,
+                        int32_t* tokens_out, float* x_next, float* logprobs_out, void* stream);
 
 /* replaces: vl_gpt.prepare_gen_img_embeds(ids)     modeling_vlm.py:270-271
  * ids int32 [n] -> fp32 [n, D] */
@@ -131,42 +144,17 @@ int pg_prepare_gen_img_embeds(pg_engine* e, const int32_t* ids, int n, float* ou
 
 /* replaces: System.sample_image (plangen_base.py:567-607), whole loop on the device:
  * prefill + n_steps x (gen_head, CFG, sample, embed, decode step) with no host sync.
- * x_prompt fp32 [R,P,D] (consumed).  tokens_out int32 [R/2, n_steps].  kv_start / edit_region / gt_labels are copied
- * into engine-owned buffers at entry (captured graphs are keyed on shapes and scalars, not on caller addresses).
- * top_k / top_p as for pg_cfg_sample_embed.  pg_sample_image_per_image below takes these settings per image. */
-int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P,
-                    int n_steps, float cfg_weight, float temperature, uint64_t seed, int greedy, int top_k,
-                    double top_p, const int32_t* edit_region, const int32_t* gt_labels,
-                    int32_t* tokens_out, void* stream);
-
-/* pg_sample_image with per-image settings: per_image = HOST array [R/2] (see pg_image_sampling), so one batch can serve
- * requests with different seeds, guidance scales, temperatures, top-k and top-p.  The settings are staged in the engine
- * and read on the device, so the captured decode-step graph depends on the shape, greedy, teacher forcing,
- * rng_per_image and whether any image uses top-p - not on the values: new seeds and settings replay the same graph. */
-int pg_sample_image_per_image(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
-                              const pg_image_sampling* per_image, int rng_per_image, int greedy,
-                              const int32_t* edit_region, const int32_t* gt_labels, int32_t* tokens_out, void* stream);
-
-/* Image-token log-probabilities.  For image b at step i the value is log p(tok) in fp32, p being exactly the
- * distribution the sampler draws from (CFG rounded per op in the engine dtype, /temperature, top-k, top-p, softmax; in
- * greedy mode top-k only) and tok the token emitted at that step, sampled or forced by teacher forcing:
- * (t_tok - max) - log(sum of the kept e), HF compute_transition_scores(..., normalize_logits=True) on the processed
- * scores.  A forced token a filter removed gets -inf; a kept one whose exp underflows still gets its finite value.
- * Log-probs change no token, no Philox draw and no offset.  Scalar settings: pass a uniform pg_image_sampling array with
- * rng_per_image = 0, which samples exactly as the scalar entries do. */
-
-/* pg_cfg_sample_embed_per_image plus logprobs_out fp32 [B, n_steps] (column `step` written). */
-int pg_cfg_sample_embed_logprobs(pg_engine* e, const float* logits, int B, const pg_image_sampling* per_image,
-                                 int rng_per_image, int greedy, const int32_t* edit_region, const int32_t* gt_labels,
-                                 int step, int n_steps, int32_t* tokens_out, float* x_next, float* logprobs_out,
-                                 void* stream);
-
-/* pg_sample_image_per_image plus logprobs_out fp32 [R/2, n_steps].  The log-probs are staged in the engine inside the
- * captured graph (its key gains a log-probs flag; the settings still do not enter it) and copied out with the tokens. */
-int pg_sample_image_logprobs(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
-                             const pg_image_sampling* per_image, int rng_per_image, int greedy,
-                             const int32_t* edit_region, const int32_t* gt_labels, int32_t* tokens_out,
-                             float* logprobs_out, void* stream);
+ * x_prompt fp32 [R,P,D] (consumed).  per_image HOST [R/2]; cfg_schedule_host HOST [R/2][n_steps] or NULL.
+ * tokens_out int32 [R/2, n_steps]; logprobs_out fp32 [R/2, n_steps] or NULL.  kv_start / edit_region / gt_labels, the
+ * settings and the schedule are copied into engine-owned buffers at entry and read on the device, so the captured
+ * decode-step graph is keyed on the shape, greedy, teacher forcing, rng_per_image, whether any image uses top-p, whether
+ * log-probs are asked for and whether there is a schedule - not on caller addresses nor on the values: new seeds,
+ * settings and schedules replay the same graph.  The log-probs are staged in the engine inside the captured graph and
+ * copied out with the tokens. */
+int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
+                    const pg_image_sampling* per_image, int rng_per_image, int greedy, const int32_t* edit_region,
+                    const int32_t* gt_labels, const float* cfg_schedule_host, int32_t* tokens_out, float* logprobs_out,
+                    void* stream);
 
 /* Teacher-forced scoring of given image tokens in one pass: logprobs_out fp32 [R/2, n] = the log-probs (as above) the
  * image loop would report with every token forced, computed by ONE prefill over prompt + image tokens (the reference's
@@ -176,36 +164,13 @@ int pg_sample_image_logprobs(pg_engine* e, float* x_prompt, const int32_t* kv_st
  * x_seq fp32 [R, P + n - 1, D] (consumed): columns < P hold the prompt embeddings (LEFT padded, kv_start as for
  * pg_prefill); columns P .. P + n - 2 are written here from the gen_aligner(gen_embed) table, token i at column P + i
  * on both rows of the pair.  image_tokens int32 [R/2, n] (ids clamped to [0, img_vocab)); per_image HOST [R/2]
- * (cfg_weight, temperature, top_k, top_p; seeds and offsets are unused).  R even, n <= max_steps and
- * P + n - 1 <= max_prompt (build the engine with a larger max_prompt to score long sequences).  Overwrites the KV cache.
- * No allocation; the prefill's host syncs are the only ones. */
+ * (cfg_weight, temperature, top_k, top_p; seeds and offsets are unused); cfg_schedule_host HOST [R/2][n] or NULL:
+ * position i of image b is scored with cfg_schedule[b][i].  R even, n <= max_steps and P + n - 1 <= max_prompt (build
+ * the engine with a larger max_prompt to score long sequences).  Overwrites the KV cache.  No allocation; the prefill's
+ * host syncs are the only ones. */
 int pg_score_image_tokens(pg_engine* e, float* x_seq, const int32_t* kv_start, int R, int P, int n,
-                          const int32_t* image_tokens, const pg_image_sampling* per_image, float* logprobs_out,
-                          void* stream);
-
-/* Guidance schedules: a guidance weight per image AND per step (LlamaGen's cfg_interval, MAR's linear ramp).
- * cfg_schedule_host = HOST fp32 array [R/2][n] (row-major; copied at entry, reusable when the call returns): at step i
- * image b is sampled exactly as the per-image entry points sample it with per_image[b].cfg_weight = cfg_schedule[b][i]
- * (same rounding per op in the engine dtype, /temperature, top-k, top-p, softmax, Philox draws and offsets); its
- * log-probs are taken under that distribution.  per_image[b].cfg_weight is IGNORED (it may hold anything, NaN
- * included); every other field keeps its meaning.  Every entry must be finite: a failure names the image and the step
- * ("image b, step i"), checked on the host without a device sync.
- * A weight of 1 is u + 1 * (c - u) rounded per op, not the conditional logits alone: in bf16 the two can differ by a
- * rounding, so an interval schedule (w, then 1) reproduces "guidance off" in distribution, not bit for bit.  The
- * unconditional rows are computed on every step, also after the last step whose weight differs from 1. */
-
-/* pg_sample_image_per_image with a guidance schedule [R/2][n_steps]; logprobs_out fp32 [R/2, n_steps] as for
- * pg_sample_image_logprobs, or NULL for none.  The schedule is staged in the engine and read on the device: the captured
- * decode-step graph's key gains a schedule flag but not the values, so new schedules replay the same graph. */
-int pg_sample_image_scheduled(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
-                              const pg_image_sampling* per_image, int rng_per_image, int greedy,
-                              const int32_t* edit_region, const int32_t* gt_labels, const float* cfg_schedule_host,
-                              int32_t* tokens_out, float* logprobs_out, void* stream);
-
-/* pg_score_image_tokens with a guidance schedule [R/2][n]: position i of image b is scored with cfg_schedule[b][i]. */
-int pg_score_image_tokens_scheduled(pg_engine* e, float* x_seq, const int32_t* kv_start, int R, int P, int n,
-                                    const int32_t* image_tokens, const pg_image_sampling* per_image,
-                                    const float* cfg_schedule_host, float* logprobs_out, void* stream);
+                          const int32_t* image_tokens, const pg_image_sampling* per_image,
+                          const float* cfg_schedule_host, float* logprobs_out, void* stream);
 
 /* replaces: System.x2t (plangen_base.py:513-523) = vl_gpt.language_model.generate(inputs_embeds=,
  *           attention_mask=, pad_token_id=, eos_token_id=, max_new_tokens=, do_sample=False, use_cache=True),

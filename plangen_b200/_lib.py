@@ -26,7 +26,7 @@ class PgDims(C.Structure):
 
 
 class PgImageSampling(C.Structure):
-    """pg_image_sampling: one image's settings for the *_per_image entry points."""
+    """pg_image_sampling: one image's sampling settings (include/plangen_b200.h)."""
     _fields_ = [("seed", C.c_uint64), ("offset", C.c_uint64), ("cfg_weight", C.c_float), ("temperature", C.c_float),
                 ("top_k", C.c_int32), ("top_p", C.c_double)]
 
@@ -62,30 +62,13 @@ EXPORTS = {
     "pg_prefill": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
     "pg_decode_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "pg_gen_head": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
-    "pg_cfg_sample_embed": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_float, C.c_float, C.c_uint64, C.c_uint64,
-                                      C.c_int, C.c_int, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
-                                      C.c_void_p]),
-    "pg_cfg_sample_embed_per_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(PgImageSampling), C.c_int, C.c_int,
-                                                C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "pg_cfg_sample_embed": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(PgImageSampling), C.c_int, C.c_int, C.c_void_p,
+                                      C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pg_prepare_gen_img_embeds": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
-    "pg_sample_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float,
-                                  C.c_uint64, C.c_int, C.c_int, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
-    "pg_sample_image_per_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
-                                            C.POINTER(PgImageSampling), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
-                                            C.c_void_p]),
-    "pg_cfg_sample_embed_logprobs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(PgImageSampling), C.c_int, C.c_int,
-                                               C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
-                                               C.c_void_p]),
-    "pg_sample_image_logprobs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
-                                           C.POINTER(PgImageSampling), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
-                                           C.c_void_p, C.c_void_p]),
+    "pg_sample_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(PgImageSampling),
+                                  C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pg_score_image_tokens": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p,
-                                        C.POINTER(PgImageSampling), C.c_void_p, C.c_void_p]),
-    "pg_sample_image_scheduled": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
-                                            C.POINTER(PgImageSampling), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
-                                            C.c_void_p, C.c_void_p, C.c_void_p]),
-    "pg_score_image_tokens_scheduled": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p,
-                                                  C.POINTER(PgImageSampling), C.c_void_p, C.c_void_p, C.c_void_p]),
+                                        C.POINTER(PgImageSampling), C.c_void_p, C.c_void_p, C.c_void_p]),
     "pg_generate_greedy": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_void_p, C.POINTER(C.c_int), C.c_void_p]),
     "pg_vq_decode_code": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
@@ -130,7 +113,7 @@ def load(build_if_missing: bool = True):
         fn = getattr(lib, name)      # AttributeError if the symbol is not exported
         fn.restype = res
         fn.argtypes = args
-    if lib.pg_abi_version() != 8:
+    if lib.pg_abi_version() != 9:
         raise PgError("ABI version mismatch")
     _LIB = lib
     return lib

@@ -101,9 +101,9 @@ struct pg_engine {
   // engine-owned staging of the per-call inputs / outputs of the fused loops, so captured graphs depend on shapes
   // and scalars only (the caller's tensors are fresh allocations on every call)
   int32_t *st_kv_start = nullptr, *st_edit = nullptr, *st_gt = nullptr, *st_tokens = nullptr;
-  ImageSampling* st_sampling = nullptr;               // per-image entry points: [B] settings (sample.cuh)
-  float* st_logprobs = nullptr;                       // pg_sample_image_logprobs: [B][n_steps]
-  float* st_cfg = nullptr;                            // the *_scheduled entry points: guidance schedule [B][n_steps]
+  ImageSampling* st_sampling = nullptr;               // sampling settings of every image: [B] (sample.cuh)
+  float* st_logprobs = nullptr;                       // image loop log-probs: [B][n_steps]
+  float* st_cfg = nullptr;                            // guidance schedule: [B][n_steps] (loop) or [B][n] (scorer)
   // mmu front-end (SigLIP tower + aligner + scatter, vit_kernels.cuh); carved only when dims.sig_layers > 0
   int sig_chunk = 0, sig_np = 0;                      // images per pass, patches per image
   float *sig_x = nullptr, *sig_part = nullptr;
@@ -1195,9 +1195,8 @@ static void philox_policy(pg_engine* e, size_t numel, uint64_t* counter_offset, 
   *stride = grid * block;
 }
 
-// Per-image settings of one sampler launch or decode loop (the per-image entry points; nullptr everywhere else):
-// `dev` holds B staged entries; the scalar settings arguments are then ignored.  any_top_p: some image has top_p < 1.
-// cfg_sched: the staged guidance schedule [B][n_steps] of the *_scheduled entry points (nullptr: dev's cfg_weight).
+// The sampling settings of one sampler launch or decode loop, staged in engine memory (stage_per_image):
+// `dev` = st_sampling [B], cfg_sched = st_cfg [B][n] or nullptr (dev's cfg_weight).  any_top_p: some image has top_p < 1.
 struct PerImage {
   const ImageSampling* dev;
   int rng_per_image;
@@ -1206,18 +1205,17 @@ struct PerImage {
 };
 
 // Philox element count of one draw: the whole (B, V) tensor, or one image's (1, V) row with per-image generators
-static size_t philox_numel(const pg_engine* e, int B, const PerImage* pi) {
-  return (pi && pi->rng_per_image ? 1 : (size_t)B) * e->d.img_vocab;
+static size_t philox_numel(const pg_engine* e, int B, const PerImage& pi) {
+  return (pi.rng_per_image ? 1 : (size_t)B) * e->d.img_vocab;
 }
 
 // top-p threshold: what torch compares the fp32 cumulative sum with, fp32(1 - top_p) with 1 - top_p in double; -1 = off
 static float top_p_threshold(double top_p) { return top_p < 1.0 ? (float)(1.0 - top_p) : -1.f; }
 
-static int k_sample(pg_engine* e, const float* part, int S, size_t sstride, const float* bias, int B, float cfg_weight,
-                    float temperature, uint64_t seed, uint64_t offset_base, int greedy, int top_k, double top_p,
-                    const int32_t* edit_region, const int32_t* gt_labels, int step_base, const int* step_ptr, int n_steps,
-                    int32_t* tokens_out, float* x_next, const float* next_norm_w, void* xn_next, cudaStream_t st,
-                    const PerImage* pi = nullptr, float* logprobs = nullptr, int score_n = 0) {
+static int k_sample(pg_engine* e, const float* part, int S, size_t sstride, const float* bias, int B, uint64_t offset_base,
+                    int greedy, const int32_t* edit_region, const int32_t* gt_labels, int step_base, const int* step_ptr,
+                    int n_steps, int32_t* tokens_out, float* x_next, const float* next_norm_w, void* xn_next, cudaStream_t st,
+                    const PerImage& pi, float* logprobs = nullptr, int score_n = 0) {
   const pg_dims& d = e->d;
   uint64_t per_step, stride;
   philox_policy(e, philox_numel(e, B, pi), &per_step, &stride);
@@ -1225,42 +1223,25 @@ static int k_sample(pg_engine* e, const float* part, int S, size_t sstride, cons
   size_t csm = chunk * 4;
   // top-p: the kernel keeps the logits and the select's 5 x 256 fixed-point mass histograms in dynamic shared memory
   // (per image: sized when any image uses it; the others skip the select)
-  const float top_p_thr = top_p_threshold(top_p);
-  if (pi ? pi->any_top_p : top_p < 1.0) {
+  if (pi.any_top_p) {
     csm = ((chunk + 1) & ~(size_t)1) * 8 + 5 * 256 * 8;
     if (csm > 48 * 1024) return fail("top_p needs %zu B of shared memory per CTA at img_vocab %d (48 KB available)", csm, d.img_vocab);
   }
   DISPATCH_T(e,
              launch(e, cfg_sample_embed_cluster_kernel<bf16>, dim3(B * SAMPLE_CLUSTER), dim3(SAMPLE_CL_THREADS), csm, st, part, S, sstride, bias, B, d.img_vocab,
-                    cfg_weight, temperature, seed, offset_base, per_step, stride, greedy, top_k, top_p_thr, edit_region, gt_labels,
-                    step_base, step_ptr, n_steps, tokens_out, (const bf16*)e->embed_table, d.D, x_next, next_norm_w, (bf16*)xn_next,
-                    d.rms_eps, 1, score_n ? nullptr : e->dbg_logits, pi ? pi->dev : nullptr, pi ? pi->rng_per_image : 0, logprobs, score_n,
-                    pi ? pi->cfg_sched : nullptr),
+                    offset_base, per_step, stride, greedy, edit_region, gt_labels, step_base, step_ptr, n_steps, tokens_out,
+                    (const bf16*)e->embed_table, d.D, x_next, next_norm_w, (bf16*)xn_next, d.rms_eps, 1,
+                    score_n ? nullptr : e->dbg_logits, pi.dev, pi.rng_per_image, logprobs, score_n, pi.cfg_sched),
              launch(e, cfg_sample_embed_cluster_kernel<float>, dim3(B * SAMPLE_CLUSTER), dim3(SAMPLE_CL_THREADS), csm, st, part, S, sstride, bias, B, d.img_vocab,
-                    cfg_weight, temperature, seed, offset_base, per_step, stride, greedy, top_k, top_p_thr, edit_region, gt_labels,
-                    step_base, step_ptr, n_steps, tokens_out, (const float*)e->embed_table, d.D, x_next, next_norm_w, (float*)xn_next,
-                    d.rms_eps, 0, score_n ? nullptr : e->dbg_logits, pi ? pi->dev : nullptr, pi ? pi->rng_per_image : 0, logprobs, score_n,
-                    pi ? pi->cfg_sched : nullptr));
+                    offset_base, per_step, stride, greedy, edit_region, gt_labels, step_base, step_ptr, n_steps, tokens_out,
+                    (const float*)e->embed_table, d.D, x_next, next_norm_w, (float*)xn_next, d.rms_eps, 0,
+                    score_n ? nullptr : e->dbg_logits, pi.dev, pi.rng_per_image, logprobs, score_n, pi.cfg_sched));
   return 0;
 }
 
-// a6-a8
-extern "C" int pg_cfg_sample_embed(pg_engine* e, const float* logits, int B, float cfg_weight, float temperature,
-                                   uint64_t seed, uint64_t philox_offset, int greedy, int top_k, double top_p,
-                                   const int32_t* edit_region, const int32_t* gt_labels, int step, int n_steps,
-                                   int32_t* tokens_out, float* x_next, void* stream) {
-  TRY(check_ready(e));
-  if (B < 1 || 2 * B > e->d.max_rows) return fail("sample B=%d exceeds engine limits", B);
-  if (step < 0 || step >= n_steps) return fail("step %d out of range", step);
-  if (top_k < 0) return fail("top_k must be >= 0");
-  if (!(top_p >= 0.0 && top_p <= 1.0)) return fail("top_p must be in [0, 1], got %g", top_p);
-  if ((edit_region == nullptr) != (gt_labels == nullptr)) return fail("edit_region and gt_labels go together");
-  return k_sample(e, logits, 1, 0, nullptr, B, cfg_weight, temperature, seed, philox_offset, greedy, top_k, top_p, edit_region,
-                  gt_labels, step, nullptr, n_steps, tokens_out, x_next, nullptr, nullptr, (cudaStream_t)stream);
-}
-
-// The caller's per-image settings, validated (naming the image) and converted to the kernel's entries.  Batch-wide RNG:
-// every entry takes image 0's seed and offset.  cfg_sched: the guidance schedule [B][n_steps] (empty: none).
+// The caller's sampling settings, validated (naming the image) and converted to the kernel's entries on the host, the
+// only place they are checked.  Batch-wide RNG: every entry takes image 0's seed and offset.  cfg_sched: the guidance
+// schedule [B][n] (empty: none).
 struct StagedSampling {
   std::vector<ImageSampling> dev;
   int rng_per_image = 0;
@@ -1305,10 +1286,11 @@ static int stage_per_image(pg_engine* e, const StagedSampling& ss, cudaStream_t 
   return 0;
 }
 
-static int cfg_sample_embed_per_image(pg_engine* e, const float* logits, int B, const pg_image_sampling* per_image,
-                                      int rng_per_image, int greedy, const int32_t* edit_region, const int32_t* gt_labels,
-                                      int step, int n_steps, int32_t* tokens_out, float* x_next, float* logprobs_out,
-                                      void* stream) {
+// a6-a8
+extern "C" int pg_cfg_sample_embed(pg_engine* e, const float* logits, int B, const pg_image_sampling* per_image,
+                                   int rng_per_image, int greedy, const int32_t* edit_region, const int32_t* gt_labels,
+                                   int step, int n_steps, int32_t* tokens_out, float* x_next, float* logprobs_out,
+                                   void* stream) {
   TRY(check_ready(e));
   if (B < 1 || 2 * B > e->d.max_rows) return fail("sample B=%d exceeds engine limits", B);
   if (step < 0 || step >= n_steps) return fail("step %d out of range", step);
@@ -1318,25 +1300,8 @@ static int cfg_sample_embed_per_image(pg_engine* e, const float* logits, int B, 
   cudaStream_t st = (cudaStream_t)stream;
   PerImage pi;
   TRY(stage_per_image(e, ss, st, &pi));
-  return k_sample(e, logits, 1, 0, nullptr, B, 0.f, 1.f, 0, 0, greedy, 0, 1.0, edit_region, gt_labels, step, nullptr,
-                  n_steps, tokens_out, x_next, nullptr, nullptr, st, &pi, logprobs_out);
-}
-
-extern "C" int pg_cfg_sample_embed_per_image(pg_engine* e, const float* logits, int B, const pg_image_sampling* per_image,
-                                             int rng_per_image, int greedy, const int32_t* edit_region,
-                                             const int32_t* gt_labels, int step, int n_steps, int32_t* tokens_out,
-                                             float* x_next, void* stream) {
-  return cfg_sample_embed_per_image(e, logits, B, per_image, rng_per_image, greedy, edit_region, gt_labels, step, n_steps,
-                                    tokens_out, x_next, nullptr, stream);
-}
-
-extern "C" int pg_cfg_sample_embed_logprobs(pg_engine* e, const float* logits, int B, const pg_image_sampling* per_image,
-                                            int rng_per_image, int greedy, const int32_t* edit_region,
-                                            const int32_t* gt_labels, int step, int n_steps, int32_t* tokens_out,
-                                            float* x_next, float* logprobs_out, void* stream) {
-  if (!logprobs_out) return fail("null argument");
-  return cfg_sample_embed_per_image(e, logits, B, per_image, rng_per_image, greedy, edit_region, gt_labels, step, n_steps,
-                                    tokens_out, x_next, logprobs_out, stream);
+  return k_sample(e, logits, 1, 0, nullptr, B, 0, greedy, edit_region, gt_labels, step, nullptr, n_steps, tokens_out, x_next,
+                  nullptr, nullptr, st, pi, logprobs_out);
 }
 
 extern "C" int pg_prepare_gen_img_embeds(pg_engine* e, const int32_t* ids, int n, float* out, void* stream) {
@@ -1352,10 +1317,9 @@ extern "C" int pg_prepare_gen_img_embeds(pg_engine* e, const int32_t* ids, int n
 // step_host >= 0: the host supplies the step index (plain launches); < 0: read the device-side counter
 // (graph replays; consecutive graph launches are fully ordered, so kernels may read it before their
 // PDL wait).
-static int one_step(pg_engine* e, const int32_t* kv_start, int R, int P, int n_steps, float cfg_weight, float temperature,
-                    uint64_t seed, int greedy, int top_k, double top_p, const int32_t* edit_region,
+static int one_step(pg_engine* e, const int32_t* kv_start, int R, int P, int n_steps, int greedy, const int32_t* edit_region,
                     const int32_t* gt_labels, int32_t* tokens_out, bool with_lm, int step_host, cudaStream_t st,
-                    const PerImage* pi, float* logprobs) {
+                    const PerImage& pi, float* logprobs) {
   NEED(b1, float, "head.b1");
   LayerW w0;
   TRY(layer_weights(e, 0, &w0));
@@ -1364,10 +1328,9 @@ static int one_step(pg_engine* e, const int32_t* kv_start, int R, int P, int n_s
   const bool host = step_host >= 0;
   uint64_t per_step, stride;
   philox_policy(e, philox_numel(e, R / 2, pi), &per_step, &stride);
-  TRY(k_sample(e, e->part, S, (size_t)R * e->d.img_vocab, b1, R / 2, cfg_weight, temperature, seed,
-               host ? per_step * (uint64_t)step_host : 0, greedy, top_k, top_p, edit_region, gt_labels, host ? step_host : 0,
-               host ? nullptr : e->step_ctr, n_steps, tokens_out, with_lm ? e->x_dec : nullptr, w0.ln1,
-               with_lm ? e->xn : nullptr, st, pi, logprobs));
+  TRY(k_sample(e, e->part, S, (size_t)R * e->d.img_vocab, b1, R / 2, host ? per_step * (uint64_t)step_host : 0, greedy,
+               edit_region, gt_labels, host ? step_host : 0, host ? nullptr : e->step_ctr, n_steps, tokens_out,
+               with_lm ? e->x_dec : nullptr, w0.ln1, with_lm ? e->xn : nullptr, st, pi, logprobs));
   if (with_lm)
     TRY(decode_layers(e, kv_start, R, host ? P + step_host : P, host ? nullptr : e->step_ctr, true, !host,
                       P + n_steps / 2, st, 0, P));
@@ -1402,26 +1365,22 @@ static int graph_for(pg_engine* e, const std::string& key, cudaStream_t st, F&& 
   return 0;
 }
 
-static int check_image_loop(pg_engine* e, const int32_t* kv_start, int R, int n_steps, const int32_t* edit_region,
-                            const int32_t* gt_labels, int32_t* tokens_out) {
+extern "C" int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
+                               const pg_image_sampling* per_image, int rng_per_image, int greedy, const int32_t* edit_region,
+                               const int32_t* gt_labels, const float* cfg_schedule_host, int32_t* tokens_out,
+                               float* logprobs_out, void* stream) {
   TRY(check_ready(e));
   if (R % 2) return fail("R must be even (interleaved cond/uncond rows)");
   if (R < 2 || R > e->d.max_rows) return fail("sample_image R=%d exceeds engine limits", R);
   if (n_steps < 1 || n_steps > e->d.max_steps) return fail("n_steps %d exceeds engine limit %d", n_steps, e->d.max_steps);
   if ((edit_region == nullptr) != (gt_labels == nullptr)) return fail("edit_region and gt_labels go together ([R/2][n_steps] each)");
   if (!kv_start || !tokens_out) return fail("null argument");
-  return 0;
-}
-
-// The image loop of pg_sample_image (pi == nullptr: the scalar settings) and pg_sample_image_per_image (per_image:
-// the caller's settings, staged here).  Arguments are checked by the callers.
-static int image_loop(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
-                      float cfg_weight, float temperature, uint64_t seed, int greedy, int top_k, double top_p,
-                      const int32_t* edit_region, const int32_t* gt_labels, int32_t* tokens_out, void* stream,
-                      const StagedSampling* per_image, float* logprobs_out = nullptr) {
+  const int B = R / 2;
+  StagedSampling ss;
+  TRY(convert_per_image(per_image, B, rng_per_image, &ss));
+  if (cfg_schedule_host) TRY(convert_schedule(cfg_schedule_host, B, n_steps, &ss));
   cudaStream_t user = (cudaStream_t)stream;
   cudaStream_t st = e->own_stream;
-  const int B = R / 2;
   const size_t tok_bytes = (size_t)B * n_steps * 4;
   CK(cudaEventRecord(e->ev_in, user));
   CK(cudaStreamWaitEvent(st, e->ev_in, 0));
@@ -1430,12 +1389,8 @@ static int image_loop(pg_engine* e, float* x_prompt, const int32_t* kv_start, in
     CK(cudaMemcpyAsync(e->st_edit, edit_region, tok_bytes, cudaMemcpyDeviceToDevice, st));
     CK(cudaMemcpyAsync(e->st_gt, gt_labels, tok_bytes, cudaMemcpyDeviceToDevice, st));
   }
-  PerImage pi_v = {};
-  const PerImage* pi = nullptr;
-  if (per_image) {
-    TRY(stage_per_image(e, *per_image, st, &pi_v));
-    pi = &pi_v;
-  }
+  PerImage pi;
+  TRY(stage_per_image(e, ss, st, &pi));
   const int32_t* kvs = e->st_kv_start;
   const int32_t* er = edit_region ? e->st_edit : nullptr;
   const int32_t* gl = edit_region ? e->st_gt : nullptr;
@@ -1445,19 +1400,16 @@ static int image_loop(pg_engine* e, float* x_prompt, const int32_t* kv_start, in
   CK(cudaMemsetAsync(e->step_ctr, 0, 4, st));
   if (n_steps > 1) {
     if (e->use_graph) {
+      // settings and schedule are read from st_sampling / st_cfg: one graph serves every value of this shape
       char key[256];
       const int prof = (e->prof_buf && e->prof_step >= 0) ? 1 : 0;
-      if (pi)   // settings and schedule are read from st_sampling / st_cfg: one graph serves every value of this shape
-        snprintf(key, sizeof(key), "imgpi/%d/%d/%d/%d/%d/%d/%d/%d/%d/%d", R, P, n_steps, greedy, edit_region ? 1 : 0,
-                 pi->rng_per_image, pi->any_top_p ? 1 : 0, lps ? 1 : 0, pi->cfg_sched ? 1 : 0, prof);
-      else
-        snprintf(key, sizeof(key), "img/%d/%d/%d/%a/%a/%llu/%d/%d/%a/%d/%d", R, P, n_steps, cfg_weight, temperature,
-                 (unsigned long long)seed, greedy, top_k, top_p, edit_region ? 1 : 0, prof);
+      snprintf(key, sizeof(key), "imgpi/%d/%d/%d/%d/%d/%d/%d/%d/%d/%d", R, P, n_steps, greedy, edit_region ? 1 : 0,
+               pi.rng_per_image, pi.any_top_p ? 1 : 0, lps ? 1 : 0, pi.cfg_sched ? 1 : 0, prof);
       pg_engine::GraphEntry* ge = nullptr;
       TRY(graph_for(e, key, st, [&]() {
         e->prof_active = (e->prof_buf != nullptr && e->prof_step >= 0);
         e->prof_slot = 0;
-        int rc = one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, true, -1, st, pi, lps);
+        int rc = one_step(e, kvs, R, P, n_steps, greedy, er, gl, toks, true, -1, st, pi, lps);
         e->prof_active = false;
         return rc;
       }, &ge));
@@ -1480,7 +1432,7 @@ static int image_loop(pg_engine* e, float* x_prompt, const int32_t* kv_start, in
           CK(cudaMemsetAsync(e->prof_buf, 0xFF, PROF_SLOTS * 8, st));
           CK(cudaMemsetAsync(e->prof_buf + PROF_SLOTS, 0, PROF_SLOTS * 8, st));
         }
-        int rc = one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, true, i, st, pi, lps);
+        int rc = one_step(e, kvs, R, P, n_steps, greedy, er, gl, toks, true, i, st, pi, lps);
         if (e->prof_active)
           CK(cudaMemcpyAsync(e->prof_buf + 2 * PROF_SLOTS, e->prof_buf, 2 * PROF_SLOTS * 8, cudaMemcpyDeviceToDevice, st));
         e->prof_active = false;
@@ -1489,7 +1441,7 @@ static int image_loop(pg_engine* e, float* x_prompt, const int32_t* kv_start, in
     }
   }
   // last token: head + sample only (the reference computes and drops one more embed, SURVEY appendix A.12)
-  TRY(one_step(e, kvs, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, er, gl, toks, false, n_steps - 1, st, pi, lps));
+  TRY(one_step(e, kvs, R, P, n_steps, greedy, er, gl, toks, false, n_steps - 1, st, pi, lps));
   CK(cudaMemcpyAsync(tokens_out, toks, tok_bytes, cudaMemcpyDeviceToDevice, st));
   if (lps) CK(cudaMemcpyAsync(logprobs_out, lps, tok_bytes, cudaMemcpyDeviceToDevice, st));
   CK(cudaEventRecord(e->ev_out, st));
@@ -1497,59 +1449,13 @@ static int image_loop(pg_engine* e, float* x_prompt, const int32_t* kv_start, in
   return 0;
 }
 
-extern "C" int pg_sample_image(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
-                               float cfg_weight, float temperature, uint64_t seed, int greedy, int top_k, double top_p,
-                               const int32_t* edit_region, const int32_t* gt_labels, int32_t* tokens_out, void* stream) {
-  TRY(check_image_loop(e, kv_start, R, n_steps, edit_region, gt_labels, tokens_out));
-  if (top_k < 0) return fail("top_k must be >= 0");
-  if (!(top_p >= 0.0 && top_p <= 1.0)) return fail("top_p must be in [0, 1], got %g", top_p);
-  return image_loop(e, x_prompt, kv_start, R, P, n_steps, cfg_weight, temperature, seed, greedy, top_k, top_p, edit_region,
-                    gt_labels, tokens_out, stream, nullptr);
-}
-
-extern "C" int pg_sample_image_per_image(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
-                                         const pg_image_sampling* per_image, int rng_per_image, int greedy,
-                                         const int32_t* edit_region, const int32_t* gt_labels, int32_t* tokens_out,
-                                         void* stream) {
-  TRY(check_image_loop(e, kv_start, R, n_steps, edit_region, gt_labels, tokens_out));
-  StagedSampling ss;
-  TRY(convert_per_image(per_image, R / 2, rng_per_image, &ss));
-  return image_loop(e, x_prompt, kv_start, R, P, n_steps, 0.f, 1.f, 0, greedy, 0, 1.0, edit_region, gt_labels,
-                    tokens_out, stream, &ss);
-}
-
-extern "C" int pg_sample_image_logprobs(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
-                                        const pg_image_sampling* per_image, int rng_per_image, int greedy,
-                                        const int32_t* edit_region, const int32_t* gt_labels, int32_t* tokens_out,
-                                        float* logprobs_out, void* stream) {
-  TRY(check_image_loop(e, kv_start, R, n_steps, edit_region, gt_labels, tokens_out));
-  if (!logprobs_out) return fail("null argument");
-  StagedSampling ss;
-  TRY(convert_per_image(per_image, R / 2, rng_per_image, &ss));
-  return image_loop(e, x_prompt, kv_start, R, P, n_steps, 0.f, 1.f, 0, greedy, 0, 1.0, edit_region, gt_labels,
-                    tokens_out, stream, &ss, logprobs_out);
-}
-
-extern "C" int pg_sample_image_scheduled(pg_engine* e, float* x_prompt, const int32_t* kv_start, int R, int P, int n_steps,
-                                         const pg_image_sampling* per_image, int rng_per_image, int greedy,
-                                         const int32_t* edit_region, const int32_t* gt_labels, const float* cfg_schedule_host,
-                                         int32_t* tokens_out, float* logprobs_out, void* stream) {
-  TRY(check_image_loop(e, kv_start, R, n_steps, edit_region, gt_labels, tokens_out));
-  StagedSampling ss;
-  TRY(convert_per_image(per_image, R / 2, rng_per_image, &ss));
-  TRY(convert_schedule(cfg_schedule_host, R / 2, n_steps, &ss));
-  return image_loop(e, x_prompt, kv_start, R, P, n_steps, 0.f, 1.f, 0, greedy, 0, 1.0, edit_region, gt_labels,
-                    tokens_out, stream, &ss, logprobs_out);
-}
-
 // ------------------------------------------------------------------------------ teacher-forced scoring
 // One prefill over prompt + image tokens, the hidden states of columns P-1 .. P+n-2 pair-major in hbuf (prefill_impl's
 // `tail`), gen_head over those R * n rows in as few wide contractions as the idle prefill scratch allows (part holds one
 // chunk's logits, qbuf its first-layer activations), and the sampler kernel in score mode per chunk.
-// cfg_schedule_host: the guidance schedule [R/2][n] of pg_score_image_tokens_scheduled, nullptr for pg_score_image_tokens.
-static int score_image_tokens(pg_engine* e, float* x_seq, const int32_t* kv_start, int R, int P, int n,
-                              const int32_t* image_tokens, const pg_image_sampling* per_image,
-                              const float* cfg_schedule_host, float* logprobs_out, void* stream) {
+extern "C" int pg_score_image_tokens(pg_engine* e, float* x_seq, const int32_t* kv_start, int R, int P, int n,
+                                     const int32_t* image_tokens, const pg_image_sampling* per_image,
+                                     const float* cfg_schedule_host, float* logprobs_out, void* stream) {
   TRY(check_ready(e));
   const pg_dims& d = e->d;
   if (!x_seq || !kv_start || !image_tokens || !logprobs_out) return fail("null argument");
@@ -1585,23 +1491,10 @@ static int score_image_tokens(pg_engine* e, float* x_seq, const int32_t* kv_star
     const int M = (int)std::min(cap, rows - r0);
     int S = 1;
     TRY(head_gemms(e, (const char*)e->hbuf + r0 * d.D * e->esz, e->qbuf, M, &S, st));
-    TRY(k_sample(e, e->part, S, (size_t)M * d.img_vocab, b1, M / 2, 0.f, 1.f, 0, 0, 0, 0, 1.0, nullptr, image_tokens,
-                 (int)(r0 / 2), nullptr, n, nullptr, nullptr, nullptr, nullptr, st, &pi, logprobs_out, n));
+    TRY(k_sample(e, e->part, S, (size_t)M * d.img_vocab, b1, M / 2, 0, 0, nullptr, image_tokens, (int)(r0 / 2), nullptr, n,
+                 nullptr, nullptr, nullptr, nullptr, st, pi, logprobs_out, n));
   }
   return 0;
-}
-
-extern "C" int pg_score_image_tokens(pg_engine* e, float* x_seq, const int32_t* kv_start, int R, int P, int n,
-                                     const int32_t* image_tokens, const pg_image_sampling* per_image, float* logprobs_out,
-                                     void* stream) {
-  return score_image_tokens(e, x_seq, kv_start, R, P, n, image_tokens, per_image, nullptr, logprobs_out, stream);
-}
-
-extern "C" int pg_score_image_tokens_scheduled(pg_engine* e, float* x_seq, const int32_t* kv_start, int R, int P, int n,
-                                               const int32_t* image_tokens, const pg_image_sampling* per_image,
-                                               const float* cfg_schedule_host, float* logprobs_out, void* stream) {
-  if (!cfg_schedule_host) return fail("null argument");
-  return score_image_tokens(e, x_seq, kv_start, R, P, n, image_tokens, per_image, cfg_schedule_host, logprobs_out, stream);
 }
 
 // ------------------------------------------------------------------------------ f1: stage-1 text decode (x2t)

@@ -72,11 +72,12 @@ __device__ unsigned long long* g_sample_dbg = nullptr;   // debug timeline (tool
 // while mass_below + j * p <= thr.  The removed e_v are zeroed and the sum recomputed over the kept set.  Greedy
 // sampling skips it (the arg-max is always kept).
 //
-// per_image != nullptr (the per-image entry points): cluster b takes cfg_weight, temperature, top_k, top_p_thr, seed
-// and a start offset (added to offset_base) from per_image[b] instead of the scalar arguments, so one batch can mix
-// requests.  rng_per_image != 0 draws image b's variates at element v of a (1, V) tensor (stride and per-step offset of
-// numel = V, chosen by the host) instead of b * V + v: the image's tokens then depend only on its own seed and offset,
-// as torch.multinomial(probs[b:b+1], 1, generator=g_b) would draw them, not on its position or the batch size.
+// per_image[img] holds the image's settings: cfg_weight, temperature, top_k, top_p_thr, seed and a start offset (added
+// to offset_base), so one batch can mix requests; a batch-wide setting is the same entry repeated.  rng_per_image == 0
+// draws image b's variates at element b * V + v of one (B, V) tensor (every entry then holds the same seed and offset);
+// rng_per_image != 0 at element v of a (1, V) tensor (stride and per-step offset of numel = V, chosen by the host): the
+// image's tokens then depend only on its own seed and offset, as torch.multinomial(probs[b:b+1], 1, generator=g_b)
+// would draw them, not on its position or the batch size.
 //
 // logprobs != nullptr: log p(tok) of the distribution the draw uses (after top-k and top-p) goes to
 // logprobs[image * n_steps + step], written by the thread that visited tok in the filter loops: (t_tok - mx) - log(sum)
@@ -85,7 +86,7 @@ __device__ unsigned long long* g_sample_dbg = nullptr;   // debug timeline (tool
 // score_n > 0 (teacher-forced scoring): cluster b scores the pair g = step_base + b, image g / score_n, position
 // g % score_n (n_steps == score_n); the token is always gt_labels[g], no variates are drawn and there is no arg-max.
 // cfg_sched != nullptr (guidance schedules): the guidance weight is cfg_sched[image * n_steps + step] instead of the
-// scalar or per-image one, read wherever the weight is read; in score mode that index is g.
+// per-image one, read wherever the weight is read; in score mode that index is g.
 constexpr int SAMPLE_CLUSTER = 8;
 
 // device copy of one pg_image_sampling entry (engine.cu converts top_p to the threshold the kernel compares with)
@@ -203,9 +204,8 @@ PG_DEVINL float cfg_scaled_logit(float c, float u, float cfg_weight, float tempe
 template <typename T>
 __global__ void __cluster_dims__(SAMPLE_CLUSTER, 1, 1) __launch_bounds__(SAMPLE_CL_THREADS)
 cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t split_stride, const float* __restrict__ bias,
-                                int B, int V, float cfg_weight, float temperature, uint64_t seed, uint64_t offset_base,
-                                uint64_t offset_per_step, uint64_t philox_stride, int greedy, int top_k,
-                                float top_p_thr, const int32_t* __restrict__ edit_region, const int32_t* __restrict__ gt_labels,
+                                int B, int V, uint64_t offset_base, uint64_t offset_per_step, uint64_t philox_stride,
+                                int greedy, const int32_t* __restrict__ edit_region, const int32_t* __restrict__ gt_labels,
                                 int step_base, const int* __restrict__ step_ptr, int n_steps,
                                 int32_t* __restrict__ tokens_out, const T* __restrict__ embed_table, int D,
                                 float* __restrict__ x_next, const float* __restrict__ next_norm_w, T* __restrict__ xn_next,
@@ -233,16 +233,15 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
   // launches the host passes the step explicitly (step_ptr == nullptr), so reading it before the PDL wait is safe.
   const int step = score_n ? (step_base + b) % score_n : step_base + (step_ptr ? *step_ptr : 0);
   const int img = score_n ? (step_base + b) / score_n : b;
-  // The per-image settings and the guidance schedule are staged by a copy before the decode loop, never written by a
-  // kernel of the loop, so they are read before the PDL wait too: the Philox prefetch below needs the image's seed and
+  // The per-image settings and the guidance schedule are staged by a copy before the launch (or the decode loop), never
+  // written by a kernel, so they are read before the PDL wait too: the Philox prefetch below needs the image's seed and
   // offset.
-  if (per_image != nullptr) {
-    const ImageSampling s = per_image[img];
-    cfg_weight = s.cfg_weight; temperature = s.temperature; top_k = s.top_k; top_p_thr = s.top_p_thr;
-    seed = s.seed; offset_base += s.offset;
-  }
-  if (cfg_sched != nullptr) cfg_weight = cfg_sched[(size_t)img * n_steps + step];
-  const uint64_t offset = offset_base + offset_per_step * (uint64_t)(step - step_base);
+  const ImageSampling s = per_image[img];
+  const float cfg_weight = cfg_sched != nullptr ? cfg_sched[(size_t)img * n_steps + step] : s.cfg_weight;
+  const float temperature = s.temperature, top_p_thr = s.top_p_thr;
+  const int top_k = s.top_k;
+  const uint64_t seed = s.seed;
+  const uint64_t offset = offset_base + s.offset + offset_per_step * (uint64_t)(step - step_base);
   // The exponential variates of torch.multinomial depend on (seed, offset, element index) only - not on the logits: they
   // are drawn while the head contraction is still streaming its weights (this kernel is launched ahead of its dependency).
   constexpr int QPRE = 8;
@@ -462,9 +461,8 @@ cfg_sample_embed_cluster_kernel(const float* __restrict__ part, int S, size_t sp
   }
   if (logprobs != nullptr && tok >= v_lo && tok < v_hi && tid == (tok - v_lo) % SAMPLE_CL_THREADS) {
     // the settings are read again rather than kept in registers across the filters (the kernel is at its register limit)
-    const float w = cfg_sched ? __ldcg(cfg_sched + (size_t)img * n_steps + step)
-                              : per_image ? __ldcg(&per_image[img].cfg_weight) : cfg_weight;
-    const float temp = per_image ? __ldcg(&per_image[img].temperature) : temperature;
+    const float w = cfg_sched ? __ldcg(cfg_sched + (size_t)img * n_steps + step) : __ldcg(&per_image[img].cfg_weight);
+    const float temp = __ldcg(&per_image[img].temperature);
     const size_t c_at = (size_t)(2 * b) * V + tok, u_at = c_at + V;
     float c, u;
     if (S == 1) { c = __ldcg(part + c_at); u = __ldcg(part + u_at); }

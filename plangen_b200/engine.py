@@ -55,7 +55,6 @@ def _is_seq(v) -> bool:
 @dataclass
 class SamplingPlan:
     """Sampling arguments of one image batch, one entry per generated image (see sampling_plan)."""
-    per_image: bool                 # some setting or the generator differs per image: the *_per_image ops
     rng_per_image: bool             # one generator per image
     cfg_weight: List[float]
     temperature: List[float]
@@ -82,8 +81,8 @@ def sampling_plan(num_gen: int, cfg_weight, temperature, top_k, top_p, generator
             raise ValueError(f"`{name}` has {len(vals)} values for {num_gen} generated images")
         return [cast(x) for x in vals], True
 
-    cfg, s_cfg = values("cfg_weight", cfg_weight, float)
-    temp, s_temp = values("temperature", temperature, float)
+    cfg, _ = values("cfg_weight", cfg_weight, float)
+    temp, _ = values("temperature", temperature, float)
     ks, s_k = values("top_k", top_k, int)
     ps, s_p = values("top_p", top_p, float)
     if s_k:
@@ -120,15 +119,14 @@ def sampling_plan(num_gen: int, cfg_weight, temperature, top_k, top_p, generator
         if off != 0:
             raise ValueError("generator must be freshly seeded (the reference reseeds per t2i call, :526)")
         seeds, offs = [seed] * num_gen, [off] * num_gen
-    return SamplingPlan(rng_per_image or s_cfg or s_temp or s_k or s_p, rng_per_image, cfg, temp, ks, ps,
-                        [_i64(x) for x in seeds], offs, gens)
+    return SamplingPlan(rng_per_image, cfg, temp, ks, ps, [_i64(x) for x in seeds], offs, gens)
 
 
 def guidance_schedule(cfg_weight, num_gen: int, n: int) -> Optional[torch.Tensor]:
     """A guidance schedule: cfg_weight as a 2-D tensor or nested sequence of shape (num_gen, n), entry [j, i] the weight
     of image j at step i (image j = copy * B + b under t2i's parallel_size), returned as the CPU fp32 table the
-    *_scheduled ops take.  None for a scalar or 1-D cfg_weight, which sampling_plan handles as before.  A wrong shape,
-    more than two dimensions or a non-finite entry raises ValueError naming the entry."""
+    sample_image and score_image_tokens ops take.  None for a scalar or 1-D cfg_weight, which sampling_plan handles.  A
+    wrong shape, more than two dimensions or a non-finite entry raises ValueError naming the entry."""
     if isinstance(cfg_weight, torch.Tensor):
         if cfg_weight.dim() < 2:
             return None
@@ -354,7 +352,8 @@ class FastJanus:
         self.use_teacher_forcing = bool(use_teacher_forcing)      # args.use_teacher_forcing (plangen_base.py:528,556,593)
         self.top_k = int(top_k)                                   # 0 = off (the reference has no top-k)
         self.top_p = float(top_p)                                 # 1 = off (nor top-p)
-        _ops._top_p(self.top_p)
+        if not 0.0 <= self.top_p <= 1.0:                          # NaN fails too
+            raise ValueError(f"`top_p` has to be a float in [0, 1], but is {top_p}")
         self.device = torch.device(device)
         self.out_dtype = torch.bfloat16 if mode == "bf16" else torch.float32
         self.max_rows = 2 * max_batch
@@ -509,21 +508,12 @@ class FastJanus:
         lg = logits.to(device=self.device, dtype=torch.float32).contiguous()
         x_next = torch.empty(2 * B, self.dims.D, device=self.device, dtype=torch.float32)
         plan = sampling_plan(B, cfg_weight, temperature, top_k, top_p, list(seed) if _is_seq(seed) else int(seed), 0)
-        if not plan.per_image and logprobs_out is None:
-            OPS.cfg_sample_embed(self.handle, lg, float(cfg_weight), float(temperature), _i64(seed), int(offset), bool(greedy),
-                                 int(top_k), edit_region, gt_labels, int(step), int(n_steps), tokens_out, x_next, float(top_p))
-            return x_next
         offs = [int(o) for o in offset] if _is_seq(offset) else [int(offset)] * B
         if len(offs) != B:
             raise ValueError(f"`offset` has {len(offs)} values for {B} images")
-        if logprobs_out is not None:     # all-scalar settings too: uniform lists sample exactly as the scalar op
-            OPS.cfg_sample_embed_logprobs(self.handle, lg, plan.cfg_weight, plan.temperature, plan.top_k, plan.top_p, plan.seed,
-                                          offs, plan.rng_per_image, bool(greedy), edit_region, gt_labels, int(step),
-                                          int(n_steps), tokens_out, x_next, logprobs_out)
-            return x_next
-        OPS.cfg_sample_embed_per_image(self.handle, lg, plan.cfg_weight, plan.temperature, plan.top_k, plan.top_p, plan.seed,
-                                       offs, plan.rng_per_image, bool(greedy), edit_region, gt_labels, int(step), int(n_steps),
-                                       tokens_out, x_next)
+        OPS.cfg_sample_embed(self.handle, lg, plan.cfg_weight, plan.temperature, plan.top_k, plan.top_p, plan.seed, offs,
+                             plan.rng_per_image, bool(greedy), edit_region, gt_labels, int(step), int(n_steps), tokens_out,
+                             x_next, logprobs_out)
         return x_next
 
     def philox_offset_per_step(self, B: int) -> int:
@@ -600,18 +590,8 @@ class FastJanus:
         logprobs = None
         if return_logprobs:
             logprobs = torch.empty(num_gen, n, dtype=torch.float32, device=self.device)
-        if sched is not None:            # the schedule replaces the per-image cfg_weight
-            OPS.sample_image_scheduled(self.handle, x, kv_start, n, sched, plan.temperature, plan.top_k, plan.top_p, plan.seed,
-                                       plan.offset, plan.rng_per_image, bool(greedy), er, gl, tokens, logprobs)
-        elif return_logprobs:            # all-scalar settings too: uniform lists sample exactly as the scalar op
-            OPS.sample_image_logprobs(self.handle, x, kv_start, n, plan.cfg_weight, plan.temperature, plan.top_k, plan.top_p,
-                                      plan.seed, plan.offset, plan.rng_per_image, bool(greedy), er, gl, tokens, logprobs)
-        elif not plan.per_image:
-            OPS.sample_image(self.handle, x, kv_start, n, float(cfg_weight), float(temperature), plan.seed[0], bool(greedy), int(k),
-                             er, gl, tokens, float(p))
-        else:
-            OPS.sample_image_per_image(self.handle, x, kv_start, n, plan.cfg_weight, plan.temperature, plan.top_k, plan.top_p,
-                                       plan.seed, plan.offset, plan.rng_per_image, bool(greedy), er, gl, tokens)
+        OPS.sample_image(self.handle, x, kv_start, n, plan.cfg_weight, plan.temperature, plan.top_k, plan.top_p, plan.seed,
+                         plan.offset, plan.rng_per_image, bool(greedy), er, gl, tokens, sched, logprobs)
         self._serial += 1
         per_draw = self.philox_offset_per_step(1 if plan.rng_per_image else num_gen)
         for g in plan.generators:
@@ -699,12 +679,8 @@ class FastJanus:
         ids = image_tokens.to(device=self.device, dtype=torch.int32).contiguous()
         out = torch.empty(B, n, dtype=torch.float32, device=self.device)
         self._keep = (kv_start, x, ids)
-        if sched is not None:
-            OPS.score_image_tokens_scheduled(self.handle, x, kv_start, P, ids, sched, plan.temperature, plan.top_k,
-                                             plan.top_p, out)
-        else:
-            OPS.score_image_tokens(self.handle, x, kv_start, P, ids, plan.cfg_weight, plan.temperature, plan.top_k,
-                                   plan.top_p, out)
+        OPS.score_image_tokens(self.handle, x, kv_start, P, ids, plan.cfg_weight, plan.temperature, plan.top_k, plan.top_p,
+                               out, sched)
         self._serial += 1                # the KV cache now holds the scored sequence
         return out
 

@@ -5,11 +5,13 @@ Every hot-path entry point of include/plangen_b200.h is registered with `torch.l
 with their mutated arguments, run on torch's CURRENT CUDA stream and can be traced / profiled like any other operator.
 The ops take the engine as an integer handle (`FastJanus.handle`); all tensors are CUDA tensors owned by the caller.
 There is no CPU implementation: a CPU tensor fails in the dispatcher, a missing shared library fails at import of
-`_lib` - nothing falls back.  The *_per_image ops take one value per image as list arguments (seeds as two's-complement
-int64) and pass them to the C-ABI as a host array of pg_image_sampling.  The *_scheduled ops take the guidance schedule
-as a CPU fp32 (B, n) tensor, passed as the C-ABI's host array; it replaces the per-image cfg_weight, so they take none.
-A weight of 1 there is u + 1 * (c - u) rounded per op (not the conditional logits alone), and the unconditional rows are
-computed on every step whatever the schedule.
+`_lib` - nothing falls back.  The sampling ops take one value per image as list arguments (seeds as two's-complement
+int64; a batch-wide setting is the same value repeated) and pass them to the C-ABI as a host array of pg_image_sampling.
+sample_image and score_image_tokens take an optional guidance schedule as a CPU fp32 (B, n) tensor, passed as the
+C-ABI's host array; it replaces the per-image cfg_weight, which is then ignored.  A weight of 1 there is u + 1 * (c - u)
+rounded per op (not the conditional logits alone), and the unconditional rows are computed on every step whatever the
+schedule.  logprobs_out (None: none, for the step and the loop) receives log p(token) per image and step.  These
+optional arguments have no default: torch.library's version bookkeeping indexes every mutated argument positionally.
 
     op                          C-ABI                         reference call (plangen_base.py)
     embed_tokens                pg_embed_tokens               language_model.get_input_embeddings()(ids)      :548
@@ -18,15 +20,8 @@ computed on every step whatever the schedule.
     gen_head                    pg_gen_head                   gen_head(h)                                     :579
     prepare_gen_img_embeds      pg_prepare_gen_img_embeds     prepare_gen_img_embeds(ids)                     :603
     cfg_sample_embed            pg_cfg_sample_embed           CFG + softmax + multinomial + embed             :580-604
-    cfg_sample_embed_per_image  pg_cfg_sample_embed_per_image the same with per-image settings and seeds
     sample_image                pg_sample_image               System.sample_image                             :567-607
-    sample_image_per_image      pg_sample_image_per_image     the same with per-image settings and seeds
-    cfg_sample_embed_logprobs   pg_cfg_sample_embed_logprobs  cfg_sample_embed_per_image + log p(token) per image
-    sample_image_logprobs       pg_sample_image_logprobs      sample_image_per_image + log p(token) per image and step
     score_image_tokens          pg_score_image_tokens         log p(given tokens): one teacher-forced prefill + gen_head
-    sample_image_scheduled      pg_sample_image_scheduled     sample_image_per_image with a guidance weight per image and
-                                                              step (+ log-probs when logprobs_out is given)
-    score_image_tokens_scheduled  pg_score_image_tokens_scheduled  score_image_tokens with a weight per image and position
     vq_decode_code              pg_vq_decode_code             gen_vision_model.decode_code                    :555
     vq_encode                   pg_vq_encode                  gen_vision_model.encode(img)[-1][-1]            :532
     prepare_inputs_embeds       pg_prepare_inputs_embeds      prepare_inputs_embeds                           :289,366,855
@@ -35,7 +30,6 @@ computed on every step whatever the schedule.
 from __future__ import annotations
 
 import ctypes as C
-import math
 import weakref
 from typing import List, Optional
 
@@ -72,11 +66,6 @@ def _cuda(*ts):
     for t in ts:
         if t is not None and not t.is_cuda:
             raise RuntimeError("plangen_b200 ops take CUDA tensors only (there is no CPU path)")
-
-
-def _top_p(top_p: float):
-    if not 0.0 <= float(top_p) <= 1.0:          # NaN fails too
-        raise ValueError(f"`top_p` has to be a float in [0, 1], but is {top_p}")
 
 
 def _per_image(B: int, cfg_weight, temperature, top_k, top_p, seed, offset):
@@ -125,92 +114,10 @@ def prepare_gen_img_embeds(handle: int, ids: torch.Tensor, out: torch.Tensor) ->
     _lib.check(e._lib.pg_prepare_gen_img_embeds(e._h, _p(ids), ids.numel(), _p(out), _st(out)))
 
 
-@torch.library.custom_op(f"{NS}::cfg_sample_embed", mutates_args=("tokens_out", "x_next"), device_types="cuda")
-def cfg_sample_embed(handle: int, logits: torch.Tensor, cfg_weight: float, temperature: float, seed: int, philox_offset: int,
-                     greedy: bool, top_k: int, edit_region: Optional[torch.Tensor], gt_labels: Optional[torch.Tensor], step: int,
-                     n_steps: int, tokens_out: torch.Tensor, x_next: torch.Tensor, top_p: float = 1.0) -> None:
-    e = _eng(handle); _cuda(logits, edit_region, gt_labels, tokens_out, x_next); _top_p(top_p)
-    _lib.check(e._lib.pg_cfg_sample_embed(e._h, _p(logits), logits.shape[0] // 2, float(cfg_weight), float(temperature), int(seed) & 0xFFFFFFFFFFFFFFFF,
-                                          int(philox_offset), int(greedy), int(top_k), float(top_p), _p(edit_region), _p(gt_labels), int(step),
-                                          int(n_steps), _p(tokens_out), _p(x_next), _st(logits)))
-
-
-@torch.library.custom_op(f"{NS}::cfg_sample_embed_per_image", mutates_args=("tokens_out", "x_next"), device_types="cuda")
-def cfg_sample_embed_per_image(handle: int, logits: torch.Tensor, cfg_weight: List[float], temperature: List[float], top_k: List[int],
-                               top_p: List[float], seed: List[int], philox_offset: List[int], rng_per_image: bool, greedy: bool,
-                               edit_region: Optional[torch.Tensor], gt_labels: Optional[torch.Tensor], step: int, n_steps: int,
-                               tokens_out: torch.Tensor, x_next: torch.Tensor) -> None:
-    e = _eng(handle); _cuda(logits, edit_region, gt_labels, tokens_out, x_next)
-    B = logits.shape[0] // 2
-    pi = _per_image(B, cfg_weight, temperature, top_k, top_p, seed, philox_offset)
-    _lib.check(e._lib.pg_cfg_sample_embed_per_image(e._h, _p(logits), B, pi, int(rng_per_image), int(greedy), _p(edit_region),
-                                                    _p(gt_labels), int(step), int(n_steps), _p(tokens_out), _p(x_next), _st(logits)))
-
-
-@torch.library.custom_op(f"{NS}::sample_image", mutates_args=("x_prompt", "tokens_out"), device_types="cuda")
-def sample_image(handle: int, x_prompt: torch.Tensor, kv_start: torch.Tensor, n_steps: int, cfg_weight: float, temperature: float,
-                 seed: int, greedy: bool, top_k: int, edit_region: Optional[torch.Tensor], gt_labels: Optional[torch.Tensor],
-                 tokens_out: torch.Tensor, top_p: float = 1.0) -> None:
-    e = _eng(handle); _cuda(x_prompt, kv_start, edit_region, gt_labels, tokens_out); _top_p(top_p)
-    R, P = x_prompt.shape[0], x_prompt.shape[1]
-    _lib.check(e._lib.pg_sample_image(e._h, _p(x_prompt), _p(kv_start), R, P, int(n_steps), float(cfg_weight), float(temperature),
-                                      int(seed) & 0xFFFFFFFFFFFFFFFF, int(greedy), int(top_k), float(top_p), _p(edit_region), _p(gt_labels), _p(tokens_out), _st(x_prompt)))
-
-
-@torch.library.custom_op(f"{NS}::sample_image_per_image", mutates_args=("x_prompt", "tokens_out"), device_types="cuda")
-def sample_image_per_image(handle: int, x_prompt: torch.Tensor, kv_start: torch.Tensor, n_steps: int, cfg_weight: List[float],
-                           temperature: List[float], top_k: List[int], top_p: List[float], seed: List[int], philox_offset: List[int],
-                           rng_per_image: bool, greedy: bool, edit_region: Optional[torch.Tensor], gt_labels: Optional[torch.Tensor],
-                           tokens_out: torch.Tensor) -> None:
-    e = _eng(handle); _cuda(x_prompt, kv_start, edit_region, gt_labels, tokens_out)
-    R, P = x_prompt.shape[0], x_prompt.shape[1]
-    pi = _per_image(R // 2, cfg_weight, temperature, top_k, top_p, seed, philox_offset)
-    _lib.check(e._lib.pg_sample_image_per_image(e._h, _p(x_prompt), _p(kv_start), R, P, int(n_steps), pi, int(rng_per_image),
-                                                int(greedy), _p(edit_region), _p(gt_labels), _p(tokens_out), _st(x_prompt)))
-
-
-@torch.library.custom_op(f"{NS}::cfg_sample_embed_logprobs", mutates_args=("tokens_out", "x_next", "logprobs_out"),
-                         device_types="cuda")
-def cfg_sample_embed_logprobs(handle: int, logits: torch.Tensor, cfg_weight: List[float], temperature: List[float], top_k: List[int],
-                              top_p: List[float], seed: List[int], philox_offset: List[int], rng_per_image: bool, greedy: bool,
-                              edit_region: Optional[torch.Tensor], gt_labels: Optional[torch.Tensor], step: int, n_steps: int,
-                              tokens_out: torch.Tensor, x_next: torch.Tensor, logprobs_out: torch.Tensor) -> None:
-    e = _eng(handle); _cuda(logits, edit_region, gt_labels, tokens_out, x_next, logprobs_out)
-    B = logits.shape[0] // 2
-    pi = _per_image(B, cfg_weight, temperature, top_k, top_p, seed, philox_offset)
-    _lib.check(e._lib.pg_cfg_sample_embed_logprobs(e._h, _p(logits), B, pi, int(rng_per_image), int(greedy), _p(edit_region),
-                                                   _p(gt_labels), int(step), int(n_steps), _p(tokens_out), _p(x_next),
-                                                   _p(logprobs_out), _st(logits)))
-
-
-@torch.library.custom_op(f"{NS}::sample_image_logprobs", mutates_args=("x_prompt", "tokens_out", "logprobs_out"),
-                         device_types="cuda")
-def sample_image_logprobs(handle: int, x_prompt: torch.Tensor, kv_start: torch.Tensor, n_steps: int, cfg_weight: List[float],
-                          temperature: List[float], top_k: List[int], top_p: List[float], seed: List[int], philox_offset: List[int],
-                          rng_per_image: bool, greedy: bool, edit_region: Optional[torch.Tensor], gt_labels: Optional[torch.Tensor],
-                          tokens_out: torch.Tensor, logprobs_out: torch.Tensor) -> None:
-    e = _eng(handle); _cuda(x_prompt, kv_start, edit_region, gt_labels, tokens_out, logprobs_out)
-    R, P = x_prompt.shape[0], x_prompt.shape[1]
-    pi = _per_image(R // 2, cfg_weight, temperature, top_k, top_p, seed, philox_offset)
-    _lib.check(e._lib.pg_sample_image_logprobs(e._h, _p(x_prompt), _p(kv_start), R, P, int(n_steps), pi, int(rng_per_image),
-                                               int(greedy), _p(edit_region), _p(gt_labels), _p(tokens_out), _p(logprobs_out),
-                                               _st(x_prompt)))
-
-
-@torch.library.custom_op(f"{NS}::score_image_tokens", mutates_args=("x_seq", "logprobs_out"), device_types="cuda")
-def score_image_tokens(handle: int, x_seq: torch.Tensor, kv_start: torch.Tensor, P: int, image_tokens: torch.Tensor,
-                       cfg_weight: List[float], temperature: List[float], top_k: List[int], top_p: List[float],
-                       logprobs_out: torch.Tensor) -> None:
-    e = _eng(handle); _cuda(x_seq, kv_start, image_tokens, logprobs_out)
-    R, n = x_seq.shape[0], image_tokens.shape[1]
-    B = R // 2
-    pi = _per_image(B, cfg_weight, temperature, top_k, top_p, [0] * B, [0] * B)
-    _lib.check(e._lib.pg_score_image_tokens(e._h, _p(x_seq), _p(kv_start), R, int(P), n, _p(image_tokens), pi,
-                                            _p(logprobs_out), _st(x_seq)))
-
-
-def _schedule(cfg_schedule: torch.Tensor, B: int, n: int):
+def _schedule(cfg_schedule: Optional[torch.Tensor], B: int, n: int):
     """The host pointer of a guidance schedule: a CPU fp32 contiguous (B, n) tensor (the C-ABI checks the values)."""
+    if cfg_schedule is None:
+        return None
     if cfg_schedule.device.type != "cpu" or cfg_schedule.dtype != torch.float32 or not cfg_schedule.is_contiguous():
         raise ValueError("`cfg_schedule` must be a contiguous CPU float32 tensor (it is read on the host)")
     if tuple(cfg_schedule.shape) != (B, n):
@@ -218,34 +125,43 @@ def _schedule(cfg_schedule: torch.Tensor, B: int, n: int):
     return C.c_void_p(cfg_schedule.data_ptr())
 
 
-@torch.library.custom_op(f"{NS}::sample_image_scheduled", mutates_args=("x_prompt", "tokens_out", "logprobs_out"),
-                         device_types="cuda")
-def sample_image_scheduled(handle: int, x_prompt: torch.Tensor, kv_start: torch.Tensor, n_steps: int, cfg_schedule: torch.Tensor,
-                           temperature: List[float], top_k: List[int], top_p: List[float], seed: List[int],
-                           philox_offset: List[int], rng_per_image: bool, greedy: bool, edit_region: Optional[torch.Tensor],
-                           gt_labels: Optional[torch.Tensor], tokens_out: torch.Tensor,
-                           logprobs_out: Optional[torch.Tensor]) -> None:
+@torch.library.custom_op(f"{NS}::cfg_sample_embed", mutates_args=("tokens_out", "x_next", "logprobs_out"), device_types="cuda")
+def cfg_sample_embed(handle: int, logits: torch.Tensor, cfg_weight: List[float], temperature: List[float], top_k: List[int],
+                     top_p: List[float], seed: List[int], philox_offset: List[int], rng_per_image: bool, greedy: bool,
+                     edit_region: Optional[torch.Tensor], gt_labels: Optional[torch.Tensor], step: int, n_steps: int,
+                     tokens_out: torch.Tensor, x_next: torch.Tensor, logprobs_out: Optional[torch.Tensor]) -> None:
+    e = _eng(handle); _cuda(logits, edit_region, gt_labels, tokens_out, x_next, logprobs_out)
+    B = logits.shape[0] // 2
+    pi = _per_image(B, cfg_weight, temperature, top_k, top_p, seed, philox_offset)
+    _lib.check(e._lib.pg_cfg_sample_embed(e._h, _p(logits), B, pi, int(rng_per_image), int(greedy), _p(edit_region),
+                                          _p(gt_labels), int(step), int(n_steps), _p(tokens_out), _p(x_next),
+                                          _p(logprobs_out), _st(logits)))
+
+
+@torch.library.custom_op(f"{NS}::sample_image", mutates_args=("x_prompt", "tokens_out", "logprobs_out"), device_types="cuda")
+def sample_image(handle: int, x_prompt: torch.Tensor, kv_start: torch.Tensor, n_steps: int, cfg_weight: List[float],
+                 temperature: List[float], top_k: List[int], top_p: List[float], seed: List[int], philox_offset: List[int],
+                 rng_per_image: bool, greedy: bool, edit_region: Optional[torch.Tensor], gt_labels: Optional[torch.Tensor],
+                 tokens_out: torch.Tensor, cfg_schedule: Optional[torch.Tensor], logprobs_out: Optional[torch.Tensor]) -> None:
     e = _eng(handle); _cuda(x_prompt, kv_start, edit_region, gt_labels, tokens_out, logprobs_out)
     R, P = x_prompt.shape[0], x_prompt.shape[1]
-    B = R // 2
-    sched = _schedule(cfg_schedule, B, int(n_steps))
-    pi = _per_image(B, [math.nan] * B, temperature, top_k, top_p, seed, philox_offset)     # cfg_weight: the schedule's
-    _lib.check(e._lib.pg_sample_image_scheduled(e._h, _p(x_prompt), _p(kv_start), R, P, int(n_steps), pi, int(rng_per_image),
-                                                int(greedy), _p(edit_region), _p(gt_labels), sched, _p(tokens_out),
-                                                _p(logprobs_out), _st(x_prompt)))
+    sched = _schedule(cfg_schedule, R // 2, int(n_steps))
+    pi = _per_image(R // 2, cfg_weight, temperature, top_k, top_p, seed, philox_offset)
+    _lib.check(e._lib.pg_sample_image(e._h, _p(x_prompt), _p(kv_start), R, P, int(n_steps), pi, int(rng_per_image), int(greedy),
+                                      _p(edit_region), _p(gt_labels), sched, _p(tokens_out), _p(logprobs_out), _st(x_prompt)))
 
 
-@torch.library.custom_op(f"{NS}::score_image_tokens_scheduled", mutates_args=("x_seq", "logprobs_out"), device_types="cuda")
-def score_image_tokens_scheduled(handle: int, x_seq: torch.Tensor, kv_start: torch.Tensor, P: int, image_tokens: torch.Tensor,
-                                 cfg_schedule: torch.Tensor, temperature: List[float], top_k: List[int], top_p: List[float],
-                                 logprobs_out: torch.Tensor) -> None:
+@torch.library.custom_op(f"{NS}::score_image_tokens", mutates_args=("x_seq", "logprobs_out"), device_types="cuda")
+def score_image_tokens(handle: int, x_seq: torch.Tensor, kv_start: torch.Tensor, P: int, image_tokens: torch.Tensor,
+                       cfg_weight: List[float], temperature: List[float], top_k: List[int], top_p: List[float],
+                       logprobs_out: torch.Tensor, cfg_schedule: Optional[torch.Tensor]) -> None:
     e = _eng(handle); _cuda(x_seq, kv_start, image_tokens, logprobs_out)
     R, n = x_seq.shape[0], image_tokens.shape[1]
     B = R // 2
     sched = _schedule(cfg_schedule, B, n)
-    pi = _per_image(B, [math.nan] * B, temperature, top_k, top_p, [0] * B, [0] * B)
-    _lib.check(e._lib.pg_score_image_tokens_scheduled(e._h, _p(x_seq), _p(kv_start), R, int(P), n, _p(image_tokens), pi, sched,
-                                                      _p(logprobs_out), _st(x_seq)))
+    pi = _per_image(B, cfg_weight, temperature, top_k, top_p, [0] * B, [0] * B)
+    _lib.check(e._lib.pg_score_image_tokens(e._h, _p(x_seq), _p(kv_start), R, int(P), n, _p(image_tokens), pi, sched,
+                                            _p(logprobs_out), _st(x_seq)))
 
 
 @torch.library.custom_op(f"{NS}::vq_decode_code", mutates_args=("image_out",), device_types="cuda")
@@ -277,6 +193,4 @@ def images_to_u8(handle: int, image: torch.Tensor, out: torch.Tensor) -> None:
 
 
 OP_NAMES = ("embed_tokens", "prefill", "decode_step", "gen_head", "prepare_gen_img_embeds", "cfg_sample_embed", "sample_image",
-            "vq_decode_code", "vq_encode", "prepare_inputs_embeds", "images_to_u8", "cfg_sample_embed_per_image",
-            "sample_image_per_image", "cfg_sample_embed_logprobs", "sample_image_logprobs", "score_image_tokens",
-            "sample_image_scheduled", "score_image_tokens_scheduled")
+            "score_image_tokens", "vq_decode_code", "vq_encode", "prepare_inputs_embeds", "images_to_u8")

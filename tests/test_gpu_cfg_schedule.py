@@ -112,7 +112,7 @@ def test_fp32_loop_schedule_with_teacher_forcing_and_greedy_matches_the_oracle()
 
 # ------------------------------------------------------------------------- 2. a constant schedule is the per-image path
 def _c_abi_scheduled(eng, ids, mask, steps, sched, arr, rng_per_image=1):
-    """pg_sample_image_scheduled called directly (tokens, log-probs and the return code)."""
+    """pg_sample_image with a schedule, called directly (tokens, log-probs and the return code)."""
     emb = eng.language_model.get_input_embeddings()(ids)
     R, P, _ = emb.shape
     x = emb.contiguous().clone()
@@ -121,8 +121,8 @@ def _c_abi_scheduled(eng, ids, mask, steps, sched, arr, rng_per_image=1):
     lp = torch.zeros(R // 2, steps, device="cuda")
     sched = sched.float().contiguous()
     p = lambda t: C.c_void_p(t.data_ptr())
-    rc = eng._lib.pg_sample_image_scheduled(eng._h, p(x), p(kv), R, P, steps, arr, rng_per_image, 0, None, None, p(sched),
-                                            p(toks), p(lp), C.c_void_p(torch.cuda.current_stream().cuda_stream))
+    rc = eng._lib.pg_sample_image(eng._h, p(x), p(kv), R, P, steps, arr, rng_per_image, 0, None, None, p(sched), p(toks),
+                                  p(lp), C.c_void_p(torch.cuda.current_stream().cuda_stream))
     torch.cuda.synchronize()
     return rc, toks, lp
 
@@ -135,7 +135,7 @@ def _arr(s, seeds, cfg_weight):
 
 
 @pytest.mark.parametrize("mode", ["fp32", "bf16"])
-def test_constant_schedule_is_the_per_image_path_bit_for_bit(mode):
+def test_constant_schedule_samples_as_per_image_weights_bit_for_bit(mode):
     d, steps, B = O.SMALL, 6, 3
     eng = get_engine(d, mode, with_vq=False)
     ids, mask = _small_batch(d, B, d.n_img_tokens)
@@ -285,7 +285,7 @@ def test_fullsize_bf16_schedule_columns_land_on_their_steps_and_tokens_match_tor
 
 
 # ---------------------------------------------------------------------------------------------------------- 6. failures
-def test_bad_schedules_fail_naming_the_image_and_step():
+def test_bad_schedules_fail_naming_the_image_and_step_at_the_single_entry_points():
     d, B, steps = O.SMALL, 3, 4
     eng = get_engine(d, "fp32", with_vq=False)
     ids, mask = _small_batch(d, B, d.n_img_tokens)
@@ -302,8 +302,7 @@ def test_bad_schedules_fail_naming_the_image_and_step():
         rc, _, _ = _c_abi_scheduled(eng, ids, mask, steps, sched, arr)
         err = eng._lib.pg_last_error()
         assert rc != 0 and b"image 1, step 2" in err, err
-        rc = eng._lib.pg_score_image_tokens_scheduled(eng._h, p(x_seq), p(kv0), 2 * B, P, steps, p(img), arr, p(sched), p(lp),
-                                                      None)
+        rc = eng._lib.pg_score_image_tokens(eng._h, p(x_seq), p(kv0), 2 * B, P, steps, p(img), arr, p(sched), p(lp), None)
         err = eng._lib.pg_last_error()
         assert rc != 0 and b"image 1, step 2" in err, err
         with pytest.raises(ValueError, match=r"cfg_weight\[1, 2\]"):
@@ -325,5 +324,5 @@ def test_bad_schedules_fail_naming_the_image_and_step():
     toks = torch.zeros(B, steps, dtype=torch.int32, device="cuda")
     for bad in (torch.ones(B, steps + 1), torch.ones(B, steps, device="cuda"), torch.ones(B, steps, dtype=torch.float64)):
         with pytest.raises(ValueError, match="cfg_schedule"):
-            OPS.sample_image_scheduled(eng.handle, emb.clone(), kv, steps, bad, S3["temperature"], S3["top_k"], S3["top_p"],
-                                       SEEDS, [0] * B, True, False, None, None, toks, None)
+            OPS.sample_image(eng.handle, emb.clone(), kv, steps, [5.0] * B, S3["temperature"], S3["top_k"], S3["top_p"], SEEDS,
+                             [0] * B, True, False, None, None, toks, bad, None)

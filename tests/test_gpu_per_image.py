@@ -267,7 +267,7 @@ def test_fullsize_mixed_settings_per_image_generators_match_torch_and_are_determ
     assert torch.equal(got, run())
 
 
-def test_bad_per_image_values_fail_naming_the_image():
+def test_bad_sampling_entries_fail_naming_the_image():
     V = 2048
     eng = get_engine(_tiny(V), "fp32", max_batch=20, with_vq=False)
     B = 4
@@ -279,8 +279,8 @@ def test_bad_per_image_values_fail_naming_the_image():
         for b in range(B):
             arr[b] = _lib.PgImageSampling(b, 0, 5.0, 1.0, 0, 1.0)
         setattr(arr[3], field, bad)
-        rc = eng._lib.pg_cfg_sample_embed_per_image(eng._h, C.c_void_p(logits.data_ptr()), B, arr, 1, 0, None, None, 0, 1,
-                                                    C.c_void_p(t.data_ptr()), C.c_void_p(x.data_ptr()), None)
+        rc = eng._lib.pg_cfg_sample_embed(eng._h, C.c_void_p(logits.data_ptr()), B, arr, 1, 0, None, None, 0, 1,
+                                          C.c_void_p(t.data_ptr()), C.c_void_p(x.data_ptr()), None, None)
         err = eng._lib.pg_last_error()
         assert rc != 0 and b"image 3" in err and field.encode() in err, err
         vals = {"top_k": [0] * B, "top_p": [1.0] * B}

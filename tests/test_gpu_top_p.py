@@ -12,6 +12,7 @@ import pytest
 import torch
 
 from oracle import janus_oracle as O
+from plangen_b200 import _lib
 from tests import top_p_ref as R
 from tests.gpu_util import get_engine, product_dims
 
@@ -99,7 +100,7 @@ def test_sampler_top_p_matches_torch_idiom_multinomial(mode, B, V):
     tally.done(f"{mode} B={B} V={V}")
 
 
-def test_sampler_top_p_one_is_the_plain_path_and_bad_values_fail():
+def test_sampler_top_p_one_is_the_unfiltered_path_and_bad_values_fail():
     d = O.JanusDims(**{**O.TINY.__dict__, "name": "tiny-v16384", "img_vocab": 16384})
     eng = get_engine(d, "fp32", max_batch=4, with_vq=False)
     logits = torch.randn(8, 16384, device="cuda")
@@ -121,8 +122,9 @@ def test_sampler_top_p_one_is_the_plain_path_and_bad_values_fail():
         with pytest.raises(ValueError):
             eng.cfg_sample_embed(logits, CFG_W, 1.0, 5, 0, 0, 1, t, top_p=bad)
         x = torch.empty(8, d.D, device="cuda")
-        rc = eng._lib.pg_cfg_sample_embed(eng._h, C.c_void_p(logits.data_ptr()), 4, CFG_W, 1.0, 5, 0, 0, 0, bad, None,
-                                          None, 0, 1, C.c_void_p(t.data_ptr()), C.c_void_p(x.data_ptr()), None)
+        arr = (_lib.PgImageSampling * 4)(*[_lib.PgImageSampling(5, 0, CFG_W, 1.0, 0, bad)] * 4)
+        rc = eng._lib.pg_cfg_sample_embed(eng._h, C.c_void_p(logits.data_ptr()), 4, arr, 0, 0, None, None, 0, 1,
+                                          C.c_void_p(t.data_ptr()), C.c_void_p(x.data_ptr()), None, None)
         assert rc != 0 and b"top_p" in eng._lib.pg_last_error()
 
 

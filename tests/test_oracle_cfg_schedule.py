@@ -2,6 +2,7 @@
 (plangen_b200.engine.guidance_schedule)."""
 import ctypes
 import math
+import re
 
 import pytest
 import torch
@@ -52,7 +53,7 @@ def test_varying_schedule_changes_the_tokens_from_the_step_it_differs():
     assert torch.equal(a[:, :k], c[:, :k])
 
 
-def test_guidance_schedule_accepts_tensors_and_nested_sequences():
+def test_guidance_schedule_takes_tensors_and_nested_sequences():
     want = torch.tensor([[1.0, 2.0, 3.0], [4.0, 5.0, 6.0]])
     for arg in (want, want.double(), want.tolist(), tuple(tuple(r) for r in want.tolist()), [want[0], want[1]],
                 [[1, 2, 3], torch.tensor([4.0, 5.0, 6.0])]):
@@ -63,7 +64,7 @@ def test_guidance_schedule_accepts_tensors_and_nested_sequences():
     for arg in (5.0, torch.tensor(5.0), [3.0, 5.0], (3.0, 5.0), torch.tensor([3.0, 5.0])):
         assert guidance_schedule(arg, 2, 3) is None
     p = sampling_plan(2, [3.0, 5.0], 1.0, 0, 1.0, None, 0)
-    assert p.per_image and p.cfg_weight == [3.0, 5.0]
+    assert p.cfg_weight == [3.0, 5.0]
 
 
 def test_guidance_schedule_rejects_wrong_shapes_and_non_finite_entries_naming_them():
@@ -91,12 +92,25 @@ def test_guidance_schedule_rejects_wrong_shapes_and_non_finite_entries_naming_th
         sampling_plan(2, torch.ones(2, 3), 1.0, 0, 1.0, None, 0)
 
 
-def test_library_exports_the_scheduled_entry_points():
+def test_library_has_one_sampling_entry_point_per_job():
     from plangen_b200 import _lib, build, ops
-    for name in ("pg_sample_image_scheduled", "pg_score_image_tokens_scheduled"):
-        assert name in _lib.EXPORTS
-        getattr(ctypes.CDLL(build.build()), name)
-    assert {"sample_image_scheduled", "score_image_tokens_scheduled"} <= set(ops.OP_NAMES)
+    cdll = ctypes.CDLL(build.build())
     with open(build.os.path.join(build.HERE, "..", "include", "plangen_b200.h")) as f:
         header = f.read()
-    assert "pg_sample_image_scheduled(" in header and "pg_score_image_tokens_scheduled(" in header
+    # the loop and the scorer take the schedule as an optional argument of their one entry point each
+    for name in ("pg_sample_image", "pg_score_image_tokens"):
+        assert name in _lib.EXPORTS
+        getattr(cdll, name)
+        decl = re.search(rf"\b{name}\(([^;]*)\);", header)
+        assert decl and "cfg_schedule_host" in decl.group(1), name
+    for name in ("sample_image", "score_image_tokens"):
+        assert name in ops.OP_NAMES
+        assert "cfg_schedule" in str(getattr(torch.ops.plangen_b200, name).default._schema), name
+    # one entry point per job: no variants with a suffix for per-image settings, log-probs or schedules
+    jobs = ("pg_cfg_sample_embed", "pg_sample_image", "pg_score_image_tokens")
+    sampling = re.compile(r"\b(?:%s)\w*(?=\s*\()" % "|".join(jobs))
+    assert set(sampling.findall(header)) == set(jobs)
+    assert {n for n in _lib.EXPORTS if sampling.match(n + "(")} == set(jobs)
+    for job in jobs:
+        for suffix in ("_per_image", "_logprobs", "_scheduled"):
+            assert not hasattr(cdll, job + suffix), job + suffix

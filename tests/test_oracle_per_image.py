@@ -37,17 +37,17 @@ def test_per_row_reference_treats_each_row_as_its_own_batch():
         assert int(tok[b]) == int(alone)
 
 
-def test_sampling_plan_normalises_scalars_sequences_and_tensors():
+def test_sampling_plan_gives_one_entry_per_image_for_scalars_sequences_and_tensors():
     from plangen_b200.engine import sampling_plan
     p = sampling_plan(3, 5.0, 1.0, 0, 1.0, None, 42)
-    assert not p.per_image and not p.rng_per_image
+    assert not p.rng_per_image
     assert p.cfg_weight == [5.0] * 3 and p.seed == [42] * 3 and p.offset == [0] * 3 and p.generators == []
     p = sampling_plan(3, [1, 3, 5], torch.tensor([1.0, 0.5, 2.0]), torch.tensor(7), (1.0, 0.9, 0.5), 11, 0)
-    assert p.per_image and not p.rng_per_image
+    assert not p.rng_per_image
     assert p.cfg_weight == [1.0, 3.0, 5.0] and p.temperature == [1.0, 0.5, 2.0] and p.top_k == [7] * 3
     assert p.top_p == [1.0, 0.9, 0.5] and p.seed == [11] * 3
     p = sampling_plan(2, 5.0, 1.0, 0, 1.0, [5, 2 ** 64 - 1], 0)
-    assert p.per_image and p.rng_per_image and p.seed == [5, -1] and p.offset == [0, 0]
+    assert p.rng_per_image and p.seed == [5, -1] and p.offset == [0, 0]
 
 
 def test_sampling_plan_rejects_bad_arguments():

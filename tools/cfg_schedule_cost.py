@@ -2,8 +2,8 @@
 
 Times, alternated three times in this one process (ms per decode step = (n-token loop - 1-token loop) / (n - 1), CUDA
 events):
-  scalar      the scalar path (pg_sample_image), CFG 5, T 1, decode graph
-  uniform     the per-image path with every image at CFG 5, T 1 and one batch-wide seed, decode graph
+  scalar      scalar Python arguments, CFG 5, T 1 (passed on as a uniform settings array), decode graph
+  uniform     one-value-per-image lists with every image at CFG 5, T 1 and one batch-wide seed, the same decode graph
   ramp        a linear-ramp schedule, 1 -> w over the steps (w = 1 / 3 / 5 / 7.5 by image), decode graph
   const       the schedule with every entry 5 (its tokens are compared with `uniform`'s: they must be identical)
   stepwise    what a caller has to do without schedules: the loop in Python, one language_model.model(...) decode
@@ -98,5 +98,5 @@ for k in names:
 d = mean["ramp"] - mean["uniform"]
 print(f"ramp vs uniform {d:+.4f} ms ({100 * d / mean['uniform']:+.2f} %)")
 same = torch.equal(run(N, "const"), run(N, "uniform"))
-print(f"const schedule tokens == uniform per-image tokens ({B} x {N}): {same}")
+print(f"const schedule tokens == uniform tokens ({B} x {N}): {same}")
 print(f"graph captures: {eng.counter('graph_captures')}")

@@ -2,7 +2,7 @@
 
 Alternated three times in this one process, CUDA events:
   1. ms per decode step = (n-token loop - 1-token loop) / (n - 1), decode graph:
-       uniform / uniform_lp   per-image path, every image at CFG 5, T 1, one batch-wide seed; log-probs off / on
+       uniform / uniform_lp   one value per image, every image at CFG 5, T 1, one batch-wide seed; log-probs off / on
        mixed / mixed_lp       mixed CFG / T / top-k, top-p 0.9 on half the images, one generator per image; off / on
   2. ms per batch of scoring 576 given tokens per image: the teacher-forced scorer (one prefill over prompt + image
      tokens, one wide gen_head) against the teacher-forced decode loop (edit_region all 0) with log-probs, on the same

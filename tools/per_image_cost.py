@@ -2,11 +2,12 @@
 
 Times, alternated three times in this one process (ms per decode step = (n-token loop - 1-token loop) / (n - 1), CUDA
 events, decode graph):
-  scalar          the scalar path (pg_sample_image), CFG 5, T 1
-  uniform         the per-image path with every image at CFG 5, T 1 and one batch-wide seed
-  mixed           the per-image path with mixed CFG / T / top-k, top-p 0.9 on half the images, one generator per image
-  scalar_top_p    the scalar path with top-p 0.9 on every image
-  scalar_filters  the scalar path with top-k 50 and top-p 0.9 on every image (the filter work `mixed` asks for)
+  scalar          scalar Python arguments, CFG 5, T 1 (the op layer passes them as a uniform settings array)
+  uniform         one-value-per-image lists with every image at CFG 5, T 1 and one batch-wide seed (same graph as
+                  `scalar`)
+  mixed           mixed CFG / T / top-k, top-p 0.9 on half the images, one generator per image
+  scalar_top_p    scalar arguments with top-p 0.9 on every image
+  scalar_filters  scalar arguments with top-k 50 and top-p 0.9 on every image (the filter work `mixed` asks for)
 """
 import os
 import subprocess
