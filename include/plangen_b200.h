@@ -20,7 +20,7 @@
 extern "C" {
 #endif
 
-#define PG_ABI_VERSION 9
+#define PG_ABI_VERSION 10
 
 /* arithmetic regimes */
 #define PG_MODE_BF16 0 /* the reference's regime: fp32 master weights under autocast(bf16), plangen_base.py:360 */
@@ -247,6 +247,26 @@ int pg_debug_zero_part(pg_engine* e, size_t nbytes, void* stream);
 int pg_test_attn_decode_io(pg_engine* e, int impl, int splits, const float* part, int S, int R, int H, void* kcache,
                            void* vcache, int Tmax, const int32_t* kv_start, const int32_t* src_row, int alias_P, int pos,
                            const int32_t* step_ptr, int rope_flags, int ctas, void* out, uint64_t* ws, void* stream);
+
+/* One prefill-attention launch exactly as the prefill issues it (same kernel, grid, shared memory and TMA maps; PDL off)
+ * on caller-owned operands, for unit tests of the kernel's own operation.  Synchronises `stream` once (bounds checks).
+ *   impl 1: attn_prefill_tc_kernel (bf16 engine with use_tc); impl 0: attn_prefill_kernel in the engine's dtype.
+ *   kcache / vcache: [R][H][Tmax][128], P <= Tmax; kv_start[R] in [0, P] (left padding of each row).
+ *   row_off: NULL - q and out are the padded block [R*P][H*128] (pad queries get zeros); otherwise (impl 1 only) the
+ *           packed stream of the real tokens, row_off[R+1] monotone with row_off[r+1] - row_off[r] either 0 (a duplicate
+ *           row: no tokens, nothing written) or P - kv_start[r]; q and out then hold row_off[R] rows.
+ *   Masked cache columns inside the 128-key blocks a tile walks must be finite (they enter P.V with weight 0). */
+int pg_test_attn_prefill_io(pg_engine* e, int impl, const void* q, const void* kcache, const void* vcache,
+                            const int32_t* kv_start, const int32_t* row_off, int R, int P, int H, int Tmax, void* out,
+                            void* stream);
+
+/* One SigLIP attention launch exactly as the vision tower issues it (PDL off) on a caller qkv buffer [qkv_rows][3W] in the
+ * engine's dtype: image i is rows [i*NP, (i+1)*NP), n*NP <= qkv_rows; the tcgen05 kernel's TMA maps cover all qkv_rows,
+ * so rows after image n-1 hold data the kernel must not use.  out: [n*NP][W].
+ *   impl 1: vit_attn_tc_kernel (bf16 engine with use_tc, W / heads == 64); impl 0: vit_attn_kernel in the engine's dtype
+ *   (NP <= 1024, W / heads <= 128). */
+int pg_test_vit_attn_io(pg_engine* e, int impl, const void* qkv, int qkv_rows, int n, int NP, int W, int heads, void* out,
+                        void* stream);
 
 /* Host-only helper of the prefill (no device work, callable without a GPU): proposes, for every prompt row, the FIRST
  * row of the batch with the same left padding `start[r]` and the same 64-bit content hash (itself when there is none).

@@ -85,7 +85,11 @@ EXPORTS = {
     "pg_test_attn_decode_io": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                          C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int,
                                          C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
-    "pg_host_group_rows": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    "pg_test_attn_prefill_io": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                          C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "pg_test_vit_attn_io": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                      C.c_void_p, C.c_void_p]),
+    "pg_host_group_rows":(C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "pg_test_gemm": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                C.c_int, C.c_void_p, C.c_void_p]),
     "pg_test_contraction_run": (C.c_int, [C.c_void_p, C.POINTER(PgTestContraction), C.c_void_p]),
@@ -113,7 +117,7 @@ def load(build_if_missing: bool = True):
         fn = getattr(lib, name)      # AttributeError if the symbol is not exported
         fn.restype = res
         fn.argtypes = args
-    if lib.pg_abi_version() != 9:
+    if lib.pg_abi_version() != 10:
         raise PgError("ABI version mismatch")
     _LIB = lib
     return lib

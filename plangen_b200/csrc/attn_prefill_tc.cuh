@@ -2,7 +2,12 @@
 // Causal attention with LEFT padding: key j is visible to the query at column p iff kv_start[r] <= j <= p
 // (the reference's (R, P+576) 0/1 mask + HF create_causal_mask; eager_attention_forward, HF modeling_llama.py:199-221).
 //
-// One CTA = one (row, head, 128-query tile); it walks the 128-key blocks the tile can see (at most 4 for P <= 512):
+// Masked cache columns inside the key blocks a tile walks must hold finite values: they enter P V with weight 0, and
+// 0 * NaN or 0 * Inf would poison the tile.  The engine zero-fills the cache at bind and writes only bf16 results; packed
+// prefill leaves pad columns holding stale (finite) K / V.
+//
+// One CTA = one (row, head, 128-query tile); it walks the 128-key blocks from kv_start / 128 to the tile's last query
+// (up to ceil(P / 128); a scorer or x2t prompt with 576 image tokens has P of about 600-1100, so 5-9 blocks):
 //   S   = Q K_blk^T      tcgen05.mma 128x128x128, fp32 in TMEM columns 0..127      (operands by TMA, SWIZZLE_128B)
 //   P   = online softmax of S, one thread per query row (= TMEM lane): two passes over the row with tcgen05.ld
 //         (masked max, then exp2 + running sum), written as bf16 into shared memory in the K-major swizzled

@@ -878,6 +878,48 @@ extern "C" int pg_host_group_rows(const int32_t* start, const uint64_t* hash, in
   return proposals;
 }
 
+// One prefill-attention launch (prefill_impl and pg_test_attn_prefill_io).  q / out: [tok][H*128] in the engine's dtype,
+// tok = R*P (padded) or row_off[R] (packed stream, tcgen05 only); kcache / vcache: [R][H][Tmax][128].
+static int launch_prefill_attn(pg_engine* e, bool tc, const void* q, int tok, const void* kcache, const void* vcache,
+                               const int32_t* kv_start, const int32_t* row_off, void* out, int R, int P, int H, int Tmax,
+                               cudaStream_t st) {
+  const float scale = 1.0f / sqrtf((float)HEAD_DIM);
+  if (tc) {
+    // tensor-core path: one CTA per (row, head, 128-query tile); V is read from the cache rows as an MN-major operand
+    CUtensorMap mq, mk, mv;
+    TRY(make_map_2d(e, &mq, q, (uint64_t)tok, (uint64_t)H * HEAD_DIM, PA_BQ));
+    TRY(make_map_2d(e, &mk, kcache, (uint64_t)R * H * Tmax, (uint64_t)HEAD_DIM, PA_BK));
+    TRY(make_map_2d(e, &mv, vcache, (uint64_t)R * H * Tmax, (uint64_t)HEAD_DIM, PA_BK));
+    return launch(e, attn_prefill_tc_kernel, dim3((P + PA_BQ - 1) / PA_BQ, H, R), dim3(128), PA_SMEM, st, mq, mk, mv, kv_start,
+                  (bf16*)out, P, H, Tmax, scale, row_off);
+  }
+  DISPATCH_T(e,
+             launch(e, attn_prefill_kernel<bf16>, dim3((P + 63) / 64, H, R), dim3(256), ATTN_PREFILL_SMEM, st, (const bf16*)q,
+                    (const bf16*)kcache, (const bf16*)vcache, kv_start, (bf16*)out, P, H, Tmax, scale),
+             launch(e, attn_prefill_kernel<float>, dim3((P + 63) / 64, H, R), dim3(256), ATTN_PREFILL_SMEM, st, (const float*)q,
+                    (const float*)kcache, (const float*)vcache, kv_start, (float*)out, P, H, Tmax, scale));
+  return 0;
+}
+
+// One SigLIP attention launch (the vision tower and pg_test_vit_attn_io).  qkv: [qkv_rows][3W] in the engine's dtype,
+// image i in rows [i*NP, (i+1)*NP); out: [n*NP][W].  The tcgen05 kernel's maps cover all qkv_rows.
+static int launch_vit_attn(pg_engine* e, bool tc, const void* qkv, int qkv_rows, void* out, int n, int NP, int W, int heads,
+                           cudaStream_t st) {
+  const int hd = W / heads;
+  const float scale = 1.0f / sqrtf((float)hd);
+  if (tc) {
+    CUtensorMap mq, mk;      // K and V rows both through mk (V read in place as an MN-major operand)
+    TRY(make_map_2d(e, &mq, qkv, (uint64_t)qkv_rows, (uint64_t)3 * W, VT_BQ));
+    TRY(make_map_2d(e, &mk, qkv, (uint64_t)qkv_rows, (uint64_t)3 * W, VT_BK));
+    return launch(e, vit_attn_tc_kernel, dim3((NP + VT_BQ - 1) / VT_BQ, heads, n), dim3(128), VT_SMEM, st, mq, mk, (bf16*)out,
+                  NP, W, scale);
+  }
+  DISPATCH_T(e,
+             launch(e, vit_attn_kernel<bf16>, dim3((NP + 3) / 4, heads, n), dim3(128), 0, st, (const bf16*)qkv, (bf16*)out, NP, W, heads, hd, scale),
+             launch(e, vit_attn_kernel<float>, dim3((NP + 3) / 4, heads, n), dim3(128), 0, st, (const float*)qkv, (float*)out, NP, W, heads, hd, scale));
+  return 0;
+}
+
 // a3: prompt prefill.  x fp32 [R*P, D] in place.
 static int prefill_impl(pg_engine* e, float* x, const int32_t* kv_start, int R, int P, float* hidden_out, int all_positions,
                         bool rope_rel, void* stream, int tail = 0);
@@ -900,7 +942,6 @@ static int prefill_impl(pg_engine* e, float* x, const int32_t* kv_start, int R, 
   NEED(normw, float, "norm");
   const int D = d.D, HD = e->HD, F = d.F;
   int tok = R * P;
-  const float scale = 1.0f / sqrtf((float)HEAD_DIM);
   int S = 1;
   // ---- packed prefill (fused loops only: the drop-in call returns every position, pads included)
   const int32_t* row_off = nullptr;
@@ -995,22 +1036,8 @@ static int prefill_impl(pg_engine* e, float* x, const int32_t* kv_start, int R, 
                       (float*)e->qbuf, (float*)kv_ptr(e, l, 0, R), (float*)kv_ptr(e, l, 1, R), P, d.H, e->Tmax,
                       rope_rel ? kv_start : (const int32_t*)nullptr));
     }
-    if (e->bf16 && e->use_tc && e->prefill_attn_tc) {
-      // tensor-core path: one CTA per (row, head, 128-query tile); V is read from the cache rows as an MN-major operand
-      CUtensorMap mq, mk, mv;
-      TRY(make_map_2d(e, &mq, e->qbuf, (uint64_t)tok, (uint64_t)HD, PA_BQ));
-      TRY(make_map_2d(e, &mk, kv_ptr(e, l, 0, R), (uint64_t)R * d.H * e->Tmax, (uint64_t)HEAD_DIM, PA_BK));
-      TRY(make_map_2d(e, &mv, kv_ptr(e, l, 1, R), (uint64_t)R * d.H * e->Tmax, (uint64_t)HEAD_DIM, PA_BK));
-      TRY(launch(e, attn_prefill_tc_kernel, dim3((P + PA_BQ - 1) / PA_BQ, d.H, R), dim3(128), PA_SMEM, st, mq, mk, mv, kv_start,
-                 (bf16*)e->attn_out, P, d.H, e->Tmax, scale, row_off));
-    } else
-    DISPATCH_T(e,
-               launch(e, attn_prefill_kernel<bf16>, dim3((P + 63) / 64, d.H, R), dim3(256), ATTN_PREFILL_SMEM, st,
-                      (const bf16*)e->qbuf, (const bf16*)kv_ptr(e, l, 0, R), (const bf16*)kv_ptr(e, l, 1, R), kv_start,
-                      (bf16*)e->attn_out, P, d.H, e->Tmax, scale),
-               launch(e, attn_prefill_kernel<float>, dim3((P + 63) / 64, d.H, R), dim3(256), ATTN_PREFILL_SMEM, st,
-                      (const float*)e->qbuf, (const float*)kv_ptr(e, l, 0, R), (const float*)kv_ptr(e, l, 1, R), kv_start,
-                      (float*)e->attn_out, P, d.H, e->Tmax, scale));
+    TRY(launch_prefill_attn(e, e->bf16 && e->use_tc && e->prefill_attn_tc, e->qbuf, tok, kv_ptr(e, l, 0, R), kv_ptr(e, l, 1, R),
+                            kv_start, row_off, e->attn_out, R, P, d.H, e->Tmax, st));
     if (fuse) {
       EpiFuse er = {nullptr, nullptr, x, 0};
       TRY(run_gemm(e, e->attn_out, w.wo, tok, D, HD, e->part, e->part_bytes, &S, st, -1, 0, true, nullptr, nullptr, &er));
@@ -1651,17 +1678,7 @@ static int sig_tower(pg_engine* e, const float* pixel, int n, void* feat, cudaSt
     SIGT(wfc1, void, p + "fc1.w"); SIGT(bfc1, float, p + "fc1.b"); SIGT(wfc2, void, p + "fc2.w"); SIGT(bfc2, float, p + "fc2.b");
     if (l == 0) TRY(resid_ln(nullptr, nullptr, ln1w, ln1b));
     TRY(linear_out(e->sig_xn, wqkv, bqkv, e->sig_qkv, 3 * W, W, 0));
-    if (tc_attn) {
-      CUtensorMap mq, mk;      // K and V rows both through mk (V read in place as an MN-major operand)
-      TRY(make_map_2d(e, &mq, e->sig_qkv, (uint64_t)M, (uint64_t)3 * W, VT_BQ));
-      TRY(make_map_2d(e, &mk, e->sig_qkv, (uint64_t)M, (uint64_t)3 * W, VT_BK));
-      TRY(launch(e, vit_attn_tc_kernel, dim3((NP + VT_BQ - 1) / VT_BQ, heads, n), dim3(128), VT_SMEM, st, mq, mk, (bf16*)e->sig_attn, NP, W,
-                 1.0f / sqrtf((float)hd)));
-    } else {
-      DISPATCH_T(e,
-                 launch(e, vit_attn_kernel<bf16>, dim3((NP + 3) / 4, heads, n), dim3(128), 0, st, (const bf16*)e->sig_qkv, (bf16*)e->sig_attn, NP, W, heads, hd, 1.0f / sqrtf((float)hd)),
-                 launch(e, vit_attn_kernel<float>, dim3((NP + 3) / 4, heads, n), dim3(128), 0, st, (const float*)e->sig_qkv, (float*)e->sig_attn, NP, W, heads, hd, 1.0f / sqrtf((float)hd)));
-    }
+    TRY(launch_vit_attn(e, tc_attn, e->sig_qkv, M, e->sig_attn, n, NP, W, heads, st));
     TRY(linear_resid_ln(e->sig_attn, wproj, bproj, W, ln2w, ln2b));
     TRY(linear_out(e->sig_xn, wfc1, bfc1, e->sig_h, d.sig_mlp, W, 1));
     if (l + 1 < d.sig_layers) {
@@ -2180,6 +2197,67 @@ extern "C" int pg_test_attn_decode_io(pg_engine* e, int impl, int splits, const 
                   (float*)kcache, (float*)vcache, kv_start, (float*)out, e->attn_ws, e->attn_cnt, H, Tmax, pos,
                   (const int*)step_ptr, scale, rope_flags);
   }
+  e->use_pdl = saved;
+  return rc;
+}
+
+// One prefill-attention launch as prefill_impl issues it (launch_prefill_attn, PDL off) on caller-owned operands.
+extern "C" int pg_test_attn_prefill_io(pg_engine* e, int impl, const void* q, const void* kcache, const void* vcache,
+                                       const int32_t* kv_start, const int32_t* row_off, int R, int P, int H, int Tmax,
+                                       void* out, void* stream) {
+  TRY(check_ready(e));
+  cudaStream_t st = (cudaStream_t)stream;
+  if (impl != 0 && impl != 1) return fail("pg_test_attn_prefill_io: impl=%d must be 0 (CUDA-core kernel) or 1 (tcgen05)", impl);
+  if (impl == 1 && !(e->bf16 && e->use_tc)) return fail("pg_test_attn_prefill_io: impl 1 (tcgen05) needs a bf16 engine with use_tc");
+  if (row_off && impl != 1) return fail("pg_test_attn_prefill_io: row_off (packed stream) needs impl 1 (tcgen05)");
+  if (!q || !kcache || !vcache || !kv_start || !out) return fail("pg_test_attn_prefill_io: null operand");
+  if (R < 1 || H < 1 || P < 1) return fail("pg_test_attn_prefill_io: R=%d H=%d P=%d must be >= 1", R, H, P);
+  if (P > Tmax) return fail("pg_test_attn_prefill_io: P=%d must be <= Tmax=%d", P, Tmax);
+  std::vector<int32_t> ks(R), ro(R + 1);
+  CK(cudaMemcpyAsync(ks.data(), kv_start, (size_t)R * 4, cudaMemcpyDeviceToHost, st));
+  if (row_off) CK(cudaMemcpyAsync(ro.data(), row_off, (size_t)(R + 1) * 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  for (int r = 0; r < R; ++r)
+    if (ks[r] < 0 || ks[r] > P) return fail("pg_test_attn_prefill_io: kv_start[%d]=%d must be in [0, P=%d]", r, ks[r], P);
+  int tok = R * P;
+  if (row_off) {
+    if (ro[0] < 0) return fail("pg_test_attn_prefill_io: row_off[0]=%d must be >= 0", ro[0]);
+    for (int r = 0; r < R; ++r) {
+      const int n = ro[r + 1] - ro[r];
+      if (n != 0 && n != P - ks[r])
+        return fail("pg_test_attn_prefill_io: row_off[%d]-row_off[%d]=%d must be 0 or P-kv_start=%d (row_off monotone)", r + 1, r, n,
+                    P - ks[r]);
+    }
+    tok = ro[R];
+    if (tok < 1) return fail("pg_test_attn_prefill_io: row_off[R]=%d: the packed stream has no token", tok);
+  }
+  const int saved = e->use_pdl;
+  e->use_pdl = 0;
+  const int rc = launch_prefill_attn(e, impl == 1, q, tok, kcache, vcache, kv_start, row_off, out, R, P, H, Tmax, st);
+  e->use_pdl = saved;
+  return rc;
+}
+
+// One SigLIP attention launch as the vision tower issues it (launch_vit_attn, PDL off) on a caller-owned qkv buffer.
+extern "C" int pg_test_vit_attn_io(pg_engine* e, int impl, const void* qkv, int qkv_rows, int n, int NP, int W, int heads,
+                                   void* out, void* stream) {
+  TRY(check_ready(e));
+  if (impl != 0 && impl != 1) return fail("pg_test_vit_attn_io: impl=%d must be 0 (CUDA-core kernel) or 1 (tcgen05)", impl);
+  if (!qkv || !out) return fail("pg_test_vit_attn_io: null operand");
+  if (n < 1 || NP < 1 || heads < 1 || W < heads || W % heads != 0)
+    return fail("pg_test_vit_attn_io: n=%d NP=%d W=%d heads=%d: need n, NP >= 1 and W a multiple of heads", n, NP, W, heads);
+  if ((int64_t)n * NP > qkv_rows) return fail("pg_test_vit_attn_io: n*NP=%lld must be <= qkv_rows=%d", (long long)n * NP, qkv_rows);
+  const int hd = W / heads;
+  if (impl == 1) {
+    if (!(e->bf16 && e->use_tc)) return fail("pg_test_vit_attn_io: impl 1 (tcgen05) needs a bf16 engine with use_tc");
+    if (hd != VT_HD) return fail("pg_test_vit_attn_io: impl 1 (tcgen05) needs hd == %d (hd=%d)", VT_HD, hd);
+  } else {
+    if (NP > 32 * VA_MAXI) return fail("pg_test_vit_attn_io: NP=%d must be <= 32 * VA_MAXI = %d for impl 0", NP, 32 * VA_MAXI);
+    if (hd > 128) return fail("pg_test_vit_attn_io: hd=%d must be <= 128 for impl 0", hd);
+  }
+  const int saved = e->use_pdl;
+  e->use_pdl = 0;
+  const int rc = launch_vit_attn(e, impl == 1, qkv, qkv_rows, out, n, NP, W, heads, (cudaStream_t)stream);
   e->use_pdl = saved;
   return rc;
 }

@@ -659,6 +659,7 @@ bias_act_kernel(const float* __restrict__ part, int S, size_t split_stride, cons
 // kv_start[r] <= j <= p (the reference's (R, P+576) 0/1 mask + HF create_causal_mask).
 // CUDA-core flash-style kernel: CTA = 64 queries x one head x one row, 256 threads;
 // S = Q K^T in 4x4 register tiles, online softmax in fp32, O += P V in 4x8 register tiles.
+// Masked cache columns in [(kv_start / 64) * 64, P) must hold finite values: they enter O += P V with weight 0.
 template <typename T>
 __global__ void __launch_bounds__(256)
 attn_prefill_kernel(const T* __restrict__ q, const T* __restrict__ kcache, const T* __restrict__ vcache,
